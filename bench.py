@@ -12,6 +12,7 @@ kernel (3 launches), plus the DoA histogram (and its NCCL all-reduce when N > 1)
     python bench.py --gpus 1 --steps 5 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N
     python bench.py --impl reference ...        # the CPU path on the host cores
+    python bench.py ... --dump-outputs DIR      # + what the last timed step returned, as DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).
 """
@@ -36,6 +37,34 @@ SNR_GRID = np.linspace(-10, 20, 11)          # target_snn_localization.py:435
 METRIC = "clips_per_sec"
 UNIT = "clips/s"
 RHO_NOMINAL = 0.076                          # spikes per channel-sample (SURVEY.md 8d); measured value is reported
+DUMP_BYTES_MAX = 64 << 20
+DUMP_SPIKE_CLIPS = 4                         # spike rasters are [B, T, 14] int8 per band (4.8 GB at the default B)
+
+
+def dump_outputs(out_dir, outs, hist=None):
+    """Write what one step returned to its caller as <out_dir>/<name>.npy: per band `b`, `<key>_band<b>` for every array
+    of the band's result (DoA index and RZCC flags of every clip as float32), the spike rasters of a fixed, seeded
+    sample of clips as float32 (`spikes_band<b>_clips` holds their indices), and the step's DoA histogram as float64.
+    The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    arrays = {}
+    for b, out in enumerate(outs):
+        for key, v in out.items():
+            if not hasattr(v, "shape"):
+                continue
+            if key == "spikes":
+                rows = np.sort(np.random.default_rng(0).choice(len(v), min(DUMP_SPIKE_CLIPS, len(v)), replace=False))
+                arrays[f"spikes_band{b}_clips"] = rows.astype(np.float64)
+                v = v[rows.tolist()]
+            v = v.cpu().numpy() if hasattr(v, "cpu") else np.asarray(v)
+            arrays[f"{key}_band{b}"] = v.astype(np.float64 if v.dtype == np.float64 else np.float32)
+    if hist is not None:
+        arrays["doa_histogram"] = hist.cpu().numpy().astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES_MAX:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs, more than {DUMP_BYTES_MAX}; use fewer clips per band")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_workload():
@@ -193,8 +222,10 @@ def run_reference(args):
         cpu_pass(cfgs, [c[:1] for c in clips], cores)
     tot_n, tot_s = 0, 0.0
     for _ in range(args.steps):
-        n, s, _ = cpu_pass(cfgs, clips, cores)
+        n, s, outs = cpu_pass(cfgs, clips, cores)
         tot_n += n; tot_s += s
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs)
     v = tot_n / tot_s
     sample = f"{n_per_band} clips x {len(bands)} bands per step (1 s, 7 mics, G=449), {args.steps} steps"
     line = {
@@ -318,6 +349,8 @@ def run_gpu(args):
         m_, n_ = e.last_kernel_ms()
         kern_ms += m_; kern_n += n_
         e.enable_timing(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs, hist)
     # cross-check of the launch time with one launch at a time (no overlap between the bands): the library's CUDA events
     # around every k_fused_tc launch on its stream, two passes over the three bands, outside the timed region
     solo_ms, solo_n = 0.0, 0
@@ -769,7 +802,11 @@ def main():
     ap.add_argument("--extra-xylo-clips", type=int, default=3552,
                     help="clips of the config-3 extra (3552 = 148 SMs x 24: one full wave of the exact front end's one-warp-per-clip kernel)")
     ap.add_argument("--extra-c5-clips", type=int, default=4, help="10 s 64-microphone clips of the config-5 extra")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
