@@ -69,17 +69,20 @@ struct micloc_snn {
     int last_kernels = 0;
     int sm_count = 148;
     double pole_radius = 1.0;      // largest pole modulus of the band-pass: how fast it forgets (time-segmented kernels)
-    long long seg_reruns = 0;      // clips a segmented run handed back to the sequential kernel so far
 };
 
-// Few long clips (BASELINE config 5): cut the sequential stages into time segments (k_chain_seg / k_neuron_seg).
-struct SegPlan { int seg_len, warm, tail, nseg, nwarm, nseg_neuron, seg_len_neuron; };
-static bool plan_segments(const micloc_snn *c, long long B, long long T, int nb, SegPlan &sp) {
+// Time segments of the sequential stages (k_chain_blk / k_neuron_seg): the chain's, and neuron segments of
+// seg_len_neuron samples that start nwarm samples early.
+struct SegPlan { ChainSegs chain; int seg_len_neuron, nwarm, nseg_neuron; };
+static SegPlan sequential_plan(long long T) { return {sequential_chain(T), (int)T, 0, 1}; }
+
+// Few long clips (BASELINE config 5) are cut into time segments; everything else runs sequentially.
+static SegPlan plan_segments(const micloc_snn *c, long long B, long long T, int nb) {
     const ChainParams &p = c->p;
-    if (getenv("MICLOC_NO_SEGMENTS")) return false;
+    if (getenv("MICLOC_NO_SEGMENTS")) return sequential_plan(T);
     const long long chains = B * p.C2 * nb;
-    if (chains >= 16384 || T < 32768) return false;             // enough sequential chains to fill the GPU already
-    if (!(c->pole_radius > 0.0 && c->pole_radius < 0.9995)) return false;
+    if (chains >= 16384 || T < 32768) return sequential_plan(T);  // enough sequential chains to fill the GPU already
+    if (!(c->pole_radius > 0.0 && c->pole_radius < 0.9995)) return sequential_plan(T);
     // band-pass transient below 1e-9 of full scale, the decision latency of the RZCC encoder on top
     int warm = (int)std::ceil(std::log(1e-9) / std::log(c->pole_radius)) + 2 * rzcc_lag(p.w);
     warm = (warm + 31) & ~31;
@@ -92,14 +95,14 @@ static bool plan_segments(const micloc_snn *c, long long B, long long T, int nb,
     long long seg = (T + want - 1) / want;
     if (seg < warm) seg = warm;
     seg = (seg + 31) & ~31ll;
-    if (seg * 2 > T) return false;
-    sp.seg_len = (int)seg; sp.warm = warm; sp.tail = rzcc_lag(p.w) + kSeg;
-    sp.nseg = (int)((T + seg - 1) / seg);
+    if (seg * 2 > T) return sequential_plan(T);
+    SegPlan sp;
+    sp.chain = {(int)seg, warm, rzcc_lag(p.w) + kSeg, (int)((T + seg - 1) / seg)};
     // alpha kernel h[n] = c n a^n: below 1e-12 of its peak
     sp.nwarm = (int)std::ceil(std::log(1e-12) / std::log((double)p.na)) + p.nL + 64;
     sp.seg_len_neuron = 1024 > 4 * sp.nwarm ? 1024 : 4 * sp.nwarm;
     sp.nseg_neuron = (int)((T + sp.seg_len_neuron - 1) / sp.seg_len_neuron);
-    return true;
+    return sp;
 }
 
 static int upload_bf(micloc_snn *c, const double *bf, int G) {
@@ -343,32 +346,22 @@ int micloc::launch_stht_any(const ChainParams &p, const float *d_taps, const voi
                                : launch_stht<float>(p, d_taps, (const float *)audio, q, B, T, st);
 }
 
-int micloc::launch_chain_any(const ChainParams &p, const void *audio, int dtype, const float *q,
+int micloc::launch_chain_any(const ChainParams &p, const ChainSegs &segs, const void *audio, int dtype, const float *q,
                              const float *band_sos, int nb, float *z, int8_t *spikes, int32_t *flags,
                              long long B, long long T, cudaStream_t st) {
-    const long long n = B * p.C2 * nb;
-    const unsigned grid = (unsigned)((n + 127) / 128);
-    if (p.M > 8 && T < (1ll << 30) && !getenv("MICLOC_CHAIN_SEG_V1")) {
-        // wide arrays: the block-wise kernel with one segment per chain (32 channels of a warp make the per-sample
-        // kernel run its divergent candidate path on every step); it stores spikes only, into a zeroed raster.
-        // (Arrays of up to 8 microphones keep k_chain: the FFMA fused kernel is tested bit for bit against it.)
-        MICLOC_CUDA(cudaMemsetAsync(spikes, 0, (size_t)n * T, st));
-        const int seg_len = (int)((T + kSeg - 1) & ~(long long)(kSeg - 1));
-        const unsigned gb = (unsigned)((n + kChainBlkThreads - 1) / kChainBlkThreads);
-#define MICLOC_CHAIN_BLK1(IN_T, NSEC)                                                                                 \
-        k_chain_blk<IN_T, NSEC><<<gb, kChainBlkThreads, 0, st>>>((const IN_T *)audio, q, band_sos, z, spikes, flags, p, B, T, nb, \
-                                                                 seg_len, 0, 0, 1)
-        if (dtype == MICLOC_I16) { if (p.nsec == 2) MICLOC_CHAIN_BLK1(int16_t, 2); else MICLOC_CHAIN_BLK1(int16_t, 0); }
-        else { if (p.nsec == 2) MICLOC_CHAIN_BLK1(float, 2); else MICLOC_CHAIN_BLK1(float, 0); }
-#undef MICLOC_CHAIN_BLK1
-        count_launch(1);
-        MICLOC_CUDA(cudaGetLastError());
-        return MICLOC_OK;
-    }
+    // k_chain_blk counts time in int, up to one block of kSeg samples past the end
+    if (T >= (1ll << 31) - kSeg) return set_error(MICLOC_ERR_SHAPE, "T = %lld too long for the chain kernel", T);
+    MICLOC_CUDA(cudaMemsetAsync(spikes, 0, (size_t)B * T * p.C2 * nb, st));     // the kernel stores spikes only
+    const long long n = B * segs.nseg * p.C2 * nb;
+    const unsigned grid = (unsigned)((n + kChainBlkThreads - 1) / kChainBlkThreads);
+    auto launch = [&](auto kernel, auto *x) {
+        kernel<<<grid, kChainBlkThreads, 0, st>>>(x, q, band_sos, z, spikes, flags, p, B, T, nb, segs.seg_len, segs.warm,
+                                                  segs.tail, segs.nseg);
+    };
     if (dtype == MICLOC_I16)
-        k_chain<int16_t><<<grid, 128, 0, st>>>((const int16_t *)audio, q, band_sos, z, spikes, flags, p, B, T, nb);
+        launch(p.nsec == 2 ? k_chain_blk<int16_t, 2> : k_chain_blk<int16_t, 0>, (const int16_t *)audio);
     else
-        k_chain<float><<<grid, 128, 0, st>>>((const float *)audio, q, band_sos, z, spikes, flags, p, B, T, nb);
+        launch(p.nsec == 2 ? k_chain_blk<float, 2> : k_chain_blk<float, 0>, (const float *)audio);
     count_launch(1);
     MICLOC_CUDA(cudaGetLastError());
     return MICLOC_OK;
@@ -472,6 +465,17 @@ static int run_power(micloc_snn *c, const float *vmem, long long B, long long T,
     return MICLOC_OK;
 }
 
+// reads the clip flags back (synchronises `st`) and calls fn(i) for every clip i with bit 0 set, up to the first error
+template <typename Fn>
+static int for_flagged(const int32_t *flg, long long B, cudaStream_t st, Fn &&fn) {
+    std::vector<int32_t> hf((size_t)B);
+    MICLOC_CUDA(cudaMemcpyAsync(hf.data(), flg, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    MICLOC_CUDA(cudaStreamSynchronize(st));
+    for (long long i = 0; i < B; ++i)
+        if (hf[(size_t)i] & 1) MICLOC_TRY(fn(i));
+    return MICLOC_OK;
+}
+
 // ---------------------------------------------------------------------------
 // RZCC overflow (flags bit 0): the streaming encoder of the staged / fused kernels buffers kClusterMax candidates per
 // cluster and follows flat tops of kPlateauMax exact zeros (digital silence: the float32 band-pass output underflows
@@ -481,20 +485,17 @@ static int run_power(micloc_snn *c, const float *vmem, long long B, long long T,
 static int heal_overflow(micloc_snn *c, const void *audio, int dtype, const float *q, float *z_dev, int8_t *spk,
                          int32_t *flg, long long B, long long T, cudaStream_t st) {
     const ChainParams &p = c->p;
-    std::vector<int32_t> hf((size_t)B);
-    MICLOC_CUDA(cudaMemcpyAsync(hf.data(), flg, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MICLOC_CUDA(cudaStreamSynchronize(st));
     const size_t n_c = (size_t)T * p.C2, esz = dtype == MICLOC_I16 ? 2 : 4;
-    for (long long i = 0; i < B; ++i) {
-        if (!(hf[(size_t)i] & 1)) continue;
+    return for_flagged(flg, B, st, [&](long long i) -> int {
         MICLOC_TRY(c->rzd.reserve(n_c * sizeof(double)));
         const float *z = z_dev ? z_dev + (size_t)i * n_c : nullptr;
         if (!z) {      // the band-pass output was not kept: once more for this clip
             MICLOC_TRY(c->rz.reserve(n_c * sizeof(float)));
             MICLOC_TRY(c->rspk.reserve(n_c));
             MICLOC_TRY(c->rflag.reserve(sizeof(int32_t)));
-            MICLOC_TRY(launch_chain_any(p, (const char *)audio + (size_t)i * T * p.M * esz, dtype, q + (size_t)i * T * p.M,
-                                        c->d_sos, 1, (float *)c->rz.ptr, (int8_t *)c->rspk.ptr, (int32_t *)c->rflag.ptr, 1, T, st));
+            MICLOC_TRY(launch_chain_any(p, sequential_chain(T), (const char *)audio + (size_t)i * T * p.M * esz, dtype,
+                                        q + (size_t)i * T * p.M, c->d_sos, 1, (float *)c->rz.ptr, (int8_t *)c->rspk.ptr,
+                                        (int32_t *)c->rflag.ptr, 1, T, st));
             z = (const float *)c->rz.ptr;
         }
         k_f32_to_f64<<<(unsigned)((n_c + 255) / 256), 256, 0, st>>>(z, (double *)c->rzd.ptr, (long long)n_c);
@@ -504,7 +505,34 @@ static int heal_overflow(micloc_snn *c, const void *audio, int dtype, const floa
                                           c->device, st));
         MICLOC_CUDA(cudaMemsetAsync(flg + i, 0, sizeof(int32_t), st));
         c->refined++;
+        return MICLOC_OK;
+    });
+}
+
+// The staged front end: flags reset -> STHT (q) -> band-pass (z, optional) + RZCC (spk) -> overflow heal -> neuron filter
+// (vm; skipped when null).  Clips that a segmented chain could not vouch for (or whose cluster overflowed) are first
+// redone sequentially: the sequential kernel's own overflow flag is then the clip's.
+static int run_front(micloc_snn *c, const SegPlan &sp, const void *audio, int dtype, long long B, long long T, float *q,
+                     float *z, int8_t *spk, int32_t *flg, float *vm, cudaStream_t st) {
+    const ChainParams &p = c->p;
+    MICLOC_CUDA(cudaMemsetAsync(flg, 0, (size_t)B * sizeof(int32_t), st));
+    MICLOC_TRY(launch_stht_any(p, c->d_taps, audio, dtype, q, B, T, st));
+    MICLOC_TRY(launch_chain_any(p, sp.chain, audio, dtype, q, c->d_sos, 1, z, spk, flg, B, T, st));
+    if (sp.chain.nseg > 1) {
+        const size_t esz = dtype == MICLOC_I16 ? 2 : 4;
+        MICLOC_TRY(for_flagged(flg, B, st, [&](long long i) {
+            MICLOC_CUDA(cudaMemsetAsync(flg + i, 0, sizeof(int32_t), st));
+            return launch_chain_any(p, sequential_chain(T), (const char *)audio + (size_t)i * T * p.M * esz, dtype,
+                                    q + (size_t)i * T * p.M, c->d_sos, 1, z ? z + (size_t)i * T * p.C2 : nullptr,
+                                    spk + (size_t)i * T * p.C2, flg + i, 1, T, st);
+        }));
     }
+    MICLOC_TRY(heal_overflow(c, audio, dtype, q, z, spk, flg, B, T, st));
+    if (!vm) return MICLOC_OK;
+    const long long n = B * sp.nseg_neuron * p.C2;
+    k_neuron_seg<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(spk, vm, p, B, T, sp.seg_len_neuron, sp.nwarm, sp.nseg_neuron);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
     return MICLOC_OK;
 }
 
@@ -524,61 +552,8 @@ extern "C" int micloc_snn_run_taps(micloc_snn *c, const void *audio, int dtype, 
     if (!flg) { MICLOC_TRY(c->flags.reserve((size_t)B * sizeof(int32_t))); flg = (int32_t *)c->flags.ptr; }
     MICLOC_TRY(timing_mark(c, st));
     const long long l0 = g_launches.load();
-    MICLOC_CUDA(cudaMemsetAsync(flg, 0, (size_t)B * sizeof(int32_t), st));
-    MICLOC_TRY(launch_stht_any(p, c->d_taps, audio, dtype, q, B, T, st));
-    SegPlan sp{};
-    const bool segmented = plan_segments(c, B, T, 1, sp);
-    if (segmented) {
-        const long long n = B * sp.nseg * p.C2;
-        const unsigned grid = (unsigned)((n + 127) / 128);
-        if (getenv("MICLOC_CHAIN_SEG_V1")) {            // one sample at a time (the block-wise kernel's cross-check)
-            if (dtype == MICLOC_I16)
-                k_chain_seg<int16_t><<<grid, 128, 0, st>>>((const int16_t *)audio, q, c->d_sos, z_dev, spk, flg, p, B, T, 1,
-                                                           sp.seg_len, sp.warm, sp.tail, sp.nseg);
-            else
-                k_chain_seg<float><<<grid, 128, 0, st>>>((const float *)audio, q, c->d_sos, z_dev, spk, flg, p, B, T, 1,
-                                                         sp.seg_len, sp.warm, sp.tail, sp.nseg);
-        } else {
-            // 32 samples at a time: stores spikes only, into a zeroed raster
-            MICLOC_CUDA(cudaMemsetAsync(spk, 0, n_c, st));
-#define MICLOC_CHAIN_BLK(IN_T, NSEC)                                                                                     \
-            k_chain_blk<IN_T, NSEC><<<grid, kChainBlkThreads, 0, st>>>((const IN_T *)audio, q, c->d_sos, z_dev, spk, flg, p, B, T, 1, \
-                                                                       sp.seg_len, sp.warm, sp.tail, sp.nseg)
-            if (dtype == MICLOC_I16) { if (p.nsec == 2) MICLOC_CHAIN_BLK(int16_t, 2); else MICLOC_CHAIN_BLK(int16_t, 0); }
-            else { if (p.nsec == 2) MICLOC_CHAIN_BLK(float, 2); else MICLOC_CHAIN_BLK(float, 0); }
-#undef MICLOC_CHAIN_BLK
-        }
-        count_launch(1);
-        MICLOC_CUDA(cudaGetLastError());
-        // what the segments could not vouch for (or an overflowed cluster) is redone by the sequential kernel: its own
-        // overflow flag is then the clip's
-        std::vector<int32_t> hf((size_t)B);
-        MICLOC_CUDA(cudaMemcpyAsync(hf.data(), flg, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        MICLOC_CUDA(cudaStreamSynchronize(st));
-        const size_t esz = dtype == MICLOC_I16 ? 2 : 4;
-        for (long long i = 0; i < B; ++i)
-            if (hf[(size_t)i] & 1) {
-                MICLOC_CUDA(cudaMemsetAsync(flg + i, 0, sizeof(int32_t), st));
-                MICLOC_TRY(launch_chain_any(p, (const char *)audio + (size_t)i * T * p.M * esz, dtype, q + (size_t)i * T * p.M, c->d_sos, 1,
-                                            z_dev ? z_dev + (size_t)i * T * p.C2 : nullptr, spk + (size_t)i * T * p.C2, flg + i, 1, T, st));
-                c->seg_reruns++;
-            }
-    } else {
-        MICLOC_TRY(launch_chain_any(p, audio, dtype, q, c->d_sos, 1, z_dev, spk, flg, B, T, st));
-    }
-    MICLOC_TRY(heal_overflow(c, audio, dtype, q, z_dev, spk, flg, B, T, st));
     const bool need_vmem = vmem_dev || y_dev || power_dev || doa_dev;
-    if (need_vmem) {
-        if (segmented) {
-            const long long n = B * sp.nseg_neuron * p.C2;
-            k_neuron_seg<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(spk, vm, p, B, T, sp.seg_len_neuron, sp.nwarm, sp.nseg_neuron);
-        } else {
-            const long long n = B * p.C2;
-            k_neuron_seg<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(spk, vm, p, B, T, (int)T, 0, 1);   // one segment: the sequential recurrence, spike bytes requested ahead
-        }
-        count_launch(1);
-        MICLOC_CUDA(cudaGetLastError());
-    }
+    MICLOC_TRY(run_front(c, plan_segments(c, B, T, 1), audio, dtype, B, T, q, z_dev, spk, flg, need_vmem ? vm : nullptr, st));
     if (power_dev || doa_dev) MICLOC_TRY(run_power(c, vm, B, T, power_dev, doa_dev, st));
     if (y_dev) {
         const int slab = 256;
@@ -607,17 +582,11 @@ extern "C" int micloc_snn_gram(micloc_snn *c, const void *audio, int dtype, int6
     MICLOC_TRY(c->spikes.reserve(n_c));
     MICLOC_TRY(c->vmem.reserve(n_c * sizeof(float)));
     MICLOC_TRY(c->flags.reserve((size_t)B * sizeof(int32_t)));
-    MICLOC_CUDA(cudaMemsetAsync(c->flags.ptr, 0, (size_t)B * sizeof(int32_t), st));
-    MICLOC_TRY(launch_stht_any(p, c->d_taps, audio, dtype, (float *)c->q.ptr, B, T, st));
-    MICLOC_TRY(launch_chain_any(p, audio, dtype, (float *)c->q.ptr, c->d_sos, 1, nullptr, (int8_t *)c->spikes.ptr,
-                                (int32_t *)c->flags.ptr, B, T, st));
-    MICLOC_TRY(heal_overflow(c, audio, dtype, (const float *)c->q.ptr, nullptr, (int8_t *)c->spikes.ptr, (int32_t *)c->flags.ptr,
-                             B, T, st));
-    const long long n = B * p.C2;
-    k_neuron_seg<<<(unsigned)((n + 127) / 128), 128, 0, st>>>((const int8_t *)c->spikes.ptr, (float *)c->vmem.ptr, p, B, T, (int)T, 0, 1);
+    MICLOC_TRY(run_front(c, sequential_plan(T), audio, dtype, B, T, (float *)c->q.ptr, nullptr, (int8_t *)c->spikes.ptr,
+                         (int32_t *)c->flags.ptr, (float *)c->vmem.ptr, st));
     dim3 gg((unsigned)B, (unsigned)((p.C2 * p.C2 + 255) / 256));
     k_gram<<<gg, 256, 0, st>>>((const float *)c->vmem.ptr, gram_dev, p.C2, T, t_start);
-    count_launch(2);
+    count_launch(1);
     MICLOC_CUDA(cudaGetLastError());
     MICLOC_CUDA(cudaEventRecord(c->ev_last, st));
     return MICLOC_OK;
@@ -664,24 +633,18 @@ extern "C" int micloc_snn_refine(micloc_snn *c, const void *audio, int dtype, in
     if (n_refined) *n_refined = 0;
     if (!flags_dev) return set_error(MICLOC_ERR_SHAPE, "refine needs the flags of the run");
     MICLOC_CUDA(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    std::vector<int32_t> hf((size_t)B);
-    MICLOC_CUDA(cudaMemcpyAsync(hf.data(), flags_dev, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MICLOC_CUDA(cudaStreamSynchronize(st));
     const ChainParams &p = c->p;
     const size_t esz = dtype == MICLOC_I16 ? 2 : 4;
     const bool timing = c->timing;
     c->timing = false;                                   // the rerun is not a timed run of its own
     long long n = 0;
-    int rc = MICLOC_OK;
-    for (long long i = 0; i < B && rc == MICLOC_OK; ++i) {
-        if (!(hf[(size_t)i] & 1)) continue;
-        rc = micloc_snn_run_taps(c, (const char *)audio + (size_t)i * T * p.M * esz, dtype, 1, T, nullptr, nullptr,
-                                 spikes_dev ? spikes_dev + (size_t)i * T * p.C2 : nullptr, nullptr, nullptr,
-                                 power_dev ? power_dev + (size_t)i * p.G : nullptr, doa_dev ? doa_dev + i : nullptr,
-                                 flags_dev + i, stream);
+    const int rc = for_flagged(flags_dev, B, (cudaStream_t)stream, [&](long long i) {
         ++n;
-    }
+        return micloc_snn_run_taps(c, (const char *)audio + (size_t)i * T * p.M * esz, dtype, 1, T, nullptr, nullptr,
+                                   spikes_dev ? spikes_dev + (size_t)i * T * p.C2 : nullptr, nullptr, nullptr,
+                                   power_dev ? power_dev + (size_t)i * p.G : nullptr, doa_dev ? doa_dev + i : nullptr,
+                                   flags_dev + i, stream);
+    });
     c->timing = timing;
     if (n_refined) *n_refined = n;
     return rc;
@@ -800,8 +763,8 @@ extern "C" int micloc_hilbert_beamform(micloc_snn *c, const void *audio, int dty
     MICLOC_CUDA(cudaStreamSynchronize(st));  // w is a stack-owned vector
     float *z = (float *)c->vmem.ptr;
     MICLOC_TRY(launch_stht_any(p, c->d_taps, audio, dtype, (float *)c->q.ptr, B, T, st));
-    MICLOC_TRY(launch_chain_any(p, audio, dtype, (float *)c->q.ptr, c->d_sos, 1, z, (int8_t *)c->spikes.ptr,
-                                (int32_t *)c->flags.ptr, B, T, st));
+    MICLOC_TRY(launch_chain_any(p, sequential_chain(T), audio, dtype, (float *)c->q.ptr, c->d_sos, 1, z,
+                                (int8_t *)c->spikes.ptr, (int32_t *)c->flags.ptr, B, T, st));
     const int slab = 256;
     dim3 grid((unsigned)((G + 127) / 128), (unsigned)((T + slab - 1) / slab), (unsigned)B);
     const float *bfr = (const float *)c->part.ptr, *bfi = bfr + (size_t)p.M * G;

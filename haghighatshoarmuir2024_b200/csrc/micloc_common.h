@@ -72,8 +72,14 @@ namespace micloc {
 int sos_to_f32(const double *sos, int nsec, float *out);
 int launch_stht_any(const ChainParams &p, const float *d_taps, const void *audio, int dtype, float *q,
                     long long B, long long T, cudaStream_t st);
-int launch_chain_any(const ChainParams &p, const void *audio, int dtype, const float *q, const float *band_sos,
-                     int nb, float *z, int8_t *spikes, int32_t *flags, long long B, long long T, cudaStream_t st);
+// time segments of the band-pass + RZCC kernel (k_chain_blk): segment s keeps samples [s*seg_len, (s+1)*seg_len) and
+// runs from `warm` samples before them to `tail` samples after them; seg_len and warm are multiples of kSeg
+struct ChainSegs { int seg_len, warm, tail, nseg; };
+// one segment per chain: the sequential recurrence
+inline ChainSegs sequential_chain(long long T) { return {(int)((T + kSeg - 1) & ~(long long)(kSeg - 1)), 0, 0, 1}; }
+int launch_chain_any(const ChainParams &p, const ChainSegs &segs, const void *audio, int dtype, const float *q,
+                     const float *band_sos, int nb, float *z, int8_t *spikes, int32_t *flags, long long B, long long T,
+                     cudaStream_t st);
 int launch_fused(const ChainParams &p, const float *d_taps, const double *d_Wd, const void *audio, int dtype,
                  long long B, long long T, int8_t *spikes, float *power, int32_t *doa, int32_t *flags,
                  unsigned int *sm_slots, int sm_count, cudaStream_t st);

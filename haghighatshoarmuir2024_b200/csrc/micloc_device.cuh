@@ -158,9 +158,9 @@ __device__ __forceinline__ float biquad_step(const float (&sos)[kMaxSections][5]
 // flagged; micloc_rzcc_encode_f64 is the unbounded encoder).
 //
 // Two front ends feed the same cluster logic and give identical spikes:
-//   rzcc_detect         one sample at a time (staged kernel)
+//   rzcc_detect         one sample at a time (stream kernel)
 //   rzcc_segment_masks  kSeg samples at once from sign / zero bit masks and the
-//                       per-sample running sums (fused kernel)
+//                       per-sample running sums (k_chain_blk, fused kernels)
 // ---------------------------------------------------------------------------
 constexpr int kSeg = 32;          // samples between two cluster close checks
 constexpr int kPlateauMax = 16;   // longest run of exact zeros inside a flat top the streaming encoder follows

@@ -47,64 +47,6 @@ k_stht(const IN_T *__restrict__ audio, float *__restrict__ q, const float *__res
     }
 }
 
-// ---------------------------------------------------------------------------
-// S2: band-pass + RZCC, one thread per (clip, band, channel), sequential in time.
-//   channel c < M : in-phase  = x[(t - K/2) mod T]   (np.roll, snn_beamformer.py:325)
-//   channel c >= M: quadrature = q[t]
-//   z = SOS cascade (snn_beamformer.py:330-335 / filterbank.py:40-44)
-//   spikes = RZCC(z)          (spike_encoder.py:115-137)
-// Output channel index is band*C2 + c (Demo.spike_encoding's hstack over bands,
-// xylo_snn_localization.py:341-342); nb == 1 for the float SNN chain.
-// `band_sos` [nb][kMaxSections][5]; sos of band 0 also sits in p.sos.
-// ---------------------------------------------------------------------------
-template <typename IN_T>
-__global__ void __launch_bounds__(128)
-k_chain(const IN_T *__restrict__ audio, const float *__restrict__ q, const float *__restrict__ band_sos,
-        float *__restrict__ z_out, int8_t *__restrict__ spikes, int32_t *__restrict__ flags,
-        const __grid_constant__ ChainParams p, long long B, long long T, int nb) {
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const int CT = p.C2 * nb;
-    if (idx >= B * CT) return;
-    const long long b = idx / CT;
-    const int cc = (int)(idx % CT);
-    const int band = cc / p.C2, c = cc % p.C2;
-
-    float sos[kMaxSections][5];
-#pragma unroll
-    for (int k = 0; k < kMaxSections; ++k)
-#pragma unroll
-        for (int e = 0; e < 5; ++e) sos[k][e] = band_sos[(band * kMaxSections + k) * 5 + e];
-
-    BiquadState bq; biquad_reset(bq);
-    RzccState rz; rzcc_reset(rz);
-    int cl_pos[2 * kClusterMax]; float cl_h[2 * kClusterMax];
-    const RzccStore store{cl_pos, cl_h, 1};
-    int8_t *sp = spikes + b * T * CT + cc;
-    auto emit = [&](int pos, int sign) { sp[(long long)pos * CT] = (int8_t)sign; };
-
-    const bool inphase = c < p.M;
-    const IN_T *xa = audio + b * T * p.M + (inphase ? c : 0);
-    const float *xq = q + b * T * p.M + (inphase ? 0 : c - p.M);
-    long long src = ((-(long long)p.half) % T + T) % T;  // (t - K/2) mod T at t = 0
-    for (long long t = 0; t < T; ++t) {
-        float x;
-        if (inphase) { x = to_f32<IN_T>(xa[src * p.M]); if (++src == T) src = 0; }
-        else x = xq[t * p.M];
-        const float z = biquad_step(sos, p.nsec, bq, x);
-        if (z_out) z_out[(b * T + t) * CT + cc] = z;
-        sp[t * CT] = 0;
-        rzcc_detect(rz, store, p.bipolar, p.w, (int)t, z, emit);
-        const bool last = t == T - 1;
-        if (last || (t & (kSeg - 1)) == kSeg - 1) rzcc_close(rz, store, p.w, (int)t, last, emit);
-    }
-    if (rz.overflow && flags) atomicOr(flags + b, 1);
-}
-
-// ---------------------------------------------------------------------------
-// S3: neuron filter   vmem[b][t][c] = sum_{n<L} h[n] * spikes[b][t-n][c]   (snn_beamformer.py:364)
-//     is k_neuron_seg below (one segment per chain = the sequential recurrence).
-// ---------------------------------------------------------------------------
-
 // band-pass output of one clip -> input of the unbounded float64 encoder (heal_overflow).  Denormals become zeros:
 // in digital silence the float32 filter never decays to 0 but cycles through denormals, whose sign changes are noise.
 static __global__ void __launch_bounds__(256)
@@ -114,108 +56,36 @@ k_f32_to_f64(const float *__restrict__ x, double *__restrict__ y, long long n) {
 }
 
 // ---------------------------------------------------------------------------
-// S2' / S3': the same two stages cut into TIME SEGMENTS, for few long clips (BASELINE config 5: one 10 s clip of 64
-// microphones is 128 sequential chains of 480 000 steps -- 128 threads).  Band-pass and alpha kernel forget their
-// past geometrically and the RZCC decisions are local (a cluster ends at the first gap >= w), so segment s starts
-// from zero state `warm` samples early, runs `tail` samples past its end and keeps only the spikes / membrane values
-// of its own range: (clip, channel, segment) chains run in parallel.  What a segment cannot vouch for sets the
-// clip's flag bit 0 and the clip is redone sequentially by the host code: a cluster still open at the segment start
-// that began inside the settling half of the warm-up, or one that holds a spike of the segment and is still open at
-// the end of the tail.  The running sum restarts at every warm-up: heights are only compared inside a cluster, where
-// a common offset cancels (up to float32 rounding of the sum, i.e. within the path's tolerance, not bit for bit).
-// RZCC is scale-free: in digital silence the band-pass's decaying tail IS the signal and keeps spiking for tens of
-// milliseconds, so "forgetting" only holds relative to a live input -- a run of kSilenceRun exactly-zero input samples
-// anywhere in a segment's span flags the clip as well.
-constexpr int kSilenceRun = 64;
+// S2: band-pass + RZCC, one thread per (clip, time segment, band, channel).
+//   channel c < M : in-phase  = x[(t - K/2) mod T]   (np.roll, snn_beamformer.py:325)
+//   channel c >= M: quadrature = q[t]
+//   z = SOS cascade (snn_beamformer.py:330-335 / filterbank.py:40-44)
+//   spikes = RZCC(z)          (spike_encoder.py:115-137)
+// Output channel index is band*C2 + c (Demo.spike_encoding's hstack over bands,
+// xylo_snn_localization.py:341-342); nb == 1 for the float SNN chain.
+// `band_sos` [nb][kMaxSections][5]; sos of band 0 also sits in p.sos.
+//
+// TIME SEGMENTS, for few long clips (BASELINE config 5: one 10 s clip of 64 microphones is 128 sequential chains of
+// 480 000 steps -- 128 threads).  Band-pass and alpha kernel forget their past geometrically and the RZCC decisions are
+// local (a cluster ends at the first gap >= w), so segment s starts from zero state `warm` samples early, runs `tail`
+// samples past its end and keeps only the spikes / membrane values of its own range: (clip, channel, segment) chains
+// run in parallel.  What a segment cannot vouch for sets the clip's flag bit 0 and the clip is redone sequentially by
+// the host code: a cluster still open at the segment start that began inside the settling half of the warm-up, or one
+// that holds a spike of the segment and is still open at the end of the tail.  The running sum restarts at every
+// warm-up: heights are only compared inside a cluster, where a common offset cancels (up to float32 rounding of the
+// sum, i.e. within the path's tolerance, not bit for bit).  RZCC is scale-free: in digital silence the band-pass's
+// decaying tail IS the signal and keeps spiking for tens of milliseconds, so "forgetting" only holds relative to a live
+// input -- a block of kSeg exactly-zero input samples anywhere in a segment's span flags the clip as well.  One segment
+// per chain (seg_len >= T, warm = tail = 0) is the sequential recurrence: only an overflowed cluster flags the clip.
+//
+// 32 samples at a time: a per-sample candidate test (rzcc_detect) runs its divergent cluster path on almost every step,
+// because with 32 channels in a warp SOME lane has a zero crossing (ncu: 144 warp instructions per sample).  Here a
+// thread first runs the band-pass and the running sum over a block of kSeg samples without a branch (sign / flat-top
+// bit masks, the running sums of the block in shared memory), then hands the block to rzcc_segment_masks -- the front
+// end of the fused kernels, which visits only the sign changes -- and the next block's 32 inputs travel from HBM to
+// registers meanwhile.  The spike raster must be ZEROED before the launch (launch_chain_any does): only spikes are
+// stored.
 // ---------------------------------------------------------------------------
-template <typename IN_T>
-__global__ void __launch_bounds__(128)
-k_chain_seg(const IN_T *__restrict__ audio, const float *__restrict__ q, const float *__restrict__ band_sos,
-            float *__restrict__ z_out, int8_t *__restrict__ spikes, int32_t *__restrict__ flags,
-            const __grid_constant__ ChainParams p, long long B, long long T, int nb, int seg_len, int warm, int tail,
-            int nseg) {
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const int CT = p.C2 * nb;
-    if (idx >= B * nseg * CT) return;
-    const int cc = (int)(idx % CT);
-    const int seg = (int)((idx / CT) % nseg);
-    const long long b = idx / ((long long)CT * nseg);
-    const int band = cc / p.C2, c = cc % p.C2;
-
-    float sos[kMaxSections][5];
-#pragma unroll
-    for (int k = 0; k < kMaxSections; ++k)
-#pragma unroll
-        for (int e = 0; e < 5; ++e) sos[k][e] = band_sos[(band * kMaxSections + k) * 5 + e];
-
-    const long long start = (long long)seg * seg_len;
-    const long long end = min(T, start + seg_len);
-    const long long t_begin = max(0ll, start - warm);
-    const long long t_stop = min(T, end + tail);
-    BiquadState bq; biquad_reset(bq);
-    RzccState rz; rzcc_reset(rz);
-    int cl_pos[2 * kClusterMax]; float cl_h[2 * kClusterMax];
-    const RzccStore store{cl_pos, cl_h, 1};
-    int8_t *sp = spikes + b * T * CT + cc;
-    auto emit = [&](int pos, int sign) { if (pos >= start && pos < end) sp[(long long)pos * CT] = (int8_t)sign; };
-
-    const bool inphase = c < p.M;
-    const IN_T *xa = audio + b * T * p.M + (inphase ? c : 0);
-    const float *xq = q + b * T * p.M + (inphase ? 0 : c - p.M);
-    long long src = ((t_begin - (long long)p.half) % T + T) % T;      // (t - K/2) mod T at t = t_begin
-    auto fetch = [&](long long t) -> float {
-        if (t >= t_stop) return 0.f;
-        if (!inphase) return xq[t * p.M];
-        long long s2 = src + (t - t_begin);
-        if (s2 >= T) s2 -= T;
-        return to_f32<IN_T>(xa[s2 * p.M]);
-    };
-    bool unsynced = false;
-    int zrun = 0;
-    // (few chains per SM -- a handful of warps: nothing but this thread's own loads in flight hides the HBM latency)
-    constexpr int kPf = 4;
-    float xc[kPf], xn[kPf];
-#pragma unroll
-    for (int u = 0; u < kPf; ++u) xc[u] = fetch(t_begin + u);
-    for (long long t4 = t_begin; t4 < t_stop; t4 += kPf) {
-#pragma unroll
-        for (int u = 0; u < kPf; ++u) xn[u] = fetch(t4 + kPf + u);   // next inputs on their way while these steps run
-#pragma unroll
-        for (int u = 0; u < kPf; ++u) {
-            const long long t = t4 + u;
-            if (t < t_stop) {
-                if (t == start && seg > 0) {
-                    // decisions from here on are this segment's: every open cluster must have begun after the filters settled
-                    const long long settled = t_begin + (warm >> 1);
-                    if ((rz.n1 > 0 && cl_pos[kClusterMax] < settled) || (rz.n0 > 0 && cl_pos[0] < settled)) unsynced = true;
-                }
-                zrun = xc[u] == 0.f ? zrun + 1 : 0;
-                if (zrun >= kSilenceRun) unsynced = true;
-                const float z = biquad_step(sos, p.nsec, bq, xc[u]);
-                if (t >= start && t < end) {
-                    if (z_out) z_out[(b * T + t) * CT + cc] = z;
-                    sp[t * CT] = 0;
-                }
-                rzcc_detect(rz, store, p.bipolar, p.w, (int)t, z, emit);
-                const bool last = t == T - 1;
-                if (last || (t & (kSeg - 1)) == kSeg - 1) rzcc_close(rz, store, p.w, (int)t, last, emit);
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < kPf; ++u) xc[u] = xn[u];
-    }
-    // a cluster that is still open behind the tail and holds a candidate of this segment was not decided
-    if (t_stop < T && ((rz.n1 > 0 && cl_pos[kClusterMax] < end) || (rz.n0 > 0 && cl_pos[0] < end))) unsynced = true;
-    if ((rz.overflow || unsynced) && flags) atomicOr(flags + b, 1);
-}
-
-// The same segments, 32 samples at a time (ncu on k_chain_seg: 144 warp instructions per sample -- the per-sample
-// candidate test runs its divergent cluster path on almost every step, because with 32 channels in a warp SOME lane has a
-// zero crossing).  Here a thread first runs the band-pass and the running sum over a block of kSeg samples without a
-// branch (sign / flat-top bit masks, the running sums of the block in shared memory), then hands the block to
-// rzcc_segment_masks -- the front end of the fused kernels, which visits only the sign changes -- and the next block's
-// 32 inputs travel from HBM to registers meanwhile.  Same decisions as k_chain_seg (both front ends feed one cluster
-// logic).  The spike raster must be ZEROED by the caller: only spikes are stored.
 constexpr int kChainBlkThreads = 128;
 template <typename IN_T, int NSEC>          // NSEC: biquads of the band-pass (0 = p.nsec at run time)
 __global__ void __launch_bounds__(kChainBlkThreads, 3)
@@ -321,7 +191,7 @@ k_chain_blk(const IN_T *__restrict__ audio, const float *__restrict__ q, const f
             cs[i * kChainBlkThreads] = csum;
             if (keep_z && ts + i < end) zo[(long long)i * CT] = v;
         }
-        // digital silence: a run of kSilenceRun exactly-zero inputs (k_chain_seg's test) contains a whole block of zeros
+        // digital silence: a whole block of exactly-zero inputs (either sign)
         if ((any << 1) == 0u && nvalid == kSeg && nseg > 1) unsynced = true;
         // ---- the next block's inputs on their way while the candidates of this one are handled ----
         if (ts + kSeg < t_stop) load_block(ts + kSeg);

@@ -11,7 +11,7 @@
 //                         paper_plots/target_xylo_localization.py:594-605
 //
 // Two front ends produce the signed spike raster int8 [B][T][2M*F]:
-//   fast  (exact = 0): float32 STHT FIR (k_stht) + float32 SOS band filters + streaming RZCC (k_chain)
+//   fast  (exact = 0): float32 STHT FIR (k_stht) + float32 SOS band filters + streaming RZCC (k_chain_blk)
 //   exact (exact = 1): float64 throughout with the reference's own operation order -- lfilter's
 //                      direct-form-II-transposed FIR / IIR (product rounded, then added, oldest tap
 //                      first) and find_peaks on a float64 np.cumsum -- so that the spikes, and with
@@ -1220,7 +1220,8 @@ extern "C" int micloc_xylo_run(micloc_xylo *c, const void *audio, int dtype, int
             if (!done) {
                 MICLOC_TRY(c->q.reserve((size_t)chunk * T * p.M * sizeof(float)));
                 MICLOC_TRY(launch_stht_any(p, c->d_taps, a, dtype, (float *)c->q.ptr, nb, T, st));
-                MICLOC_TRY(launch_chain_any(p, a, dtype, (const float *)c->q.ptr, c->d_band_sos, c->F, nullptr, sgn, flg + b0, nb, T, st));
+                MICLOC_TRY(launch_chain_any(p, sequential_chain(T), a, dtype, (const float *)c->q.ptr, c->d_band_sos, c->F,
+                                            nullptr, sgn, flg + b0, nb, T, st));
             }
         }
         if (spikes_in_dev) {

@@ -2,7 +2,7 @@
 
 `evolve` keeps the reference's return layout (F x T x M) and runs on the host with
 scipy (it is only used to prepare live-demo frames); inside the Xylo chain the
-band filters run on the device as SOS cascades (csrc/micloc_staged.cuh:k_chain).
+band filters run on the device as SOS cascades (csrc/micloc_staged.cuh:k_chain_blk).
 """
 from __future__ import annotations
 

@@ -271,7 +271,7 @@ def test_full_size_config4_multi_source_360_grid():
 @pytest.mark.parametrize("name", ["snn_c5_random64", "snn_c5_linear64"])
 def test_full_size_config5_64_mics_10s_512_grid(name):
     """Config 5 size: one 10 s clip (T = 480 000) on the 64-microphone arrays, G = 512, against the oracle.  Few long
-    clips take the time-segmented kernels (k_chain_seg / k_neuron_seg / k_gram_slab)."""
+    clips take the time-segmented kernels (k_chain_blk / k_neuron_seg / k_gram_slab)."""
     import time
     g = H.load(name)
     T = 480_000
