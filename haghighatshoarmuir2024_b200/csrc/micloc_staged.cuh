@@ -256,17 +256,32 @@ k_neuron_seg(const int8_t *__restrict__ spikes, float *__restrict__ vmem, const 
 // S4a: Gram matrix of the membrane signals   C[b][i][j] = sum_t v[t][i] v[t][j]
 //      mean_t (v[t] . w_g)^2 == w_g^T (C/T) w_g, so the per-DoA power of
 //      snn_beamformer.py:368 + target_snn_localization.py:462 needs no T x G pass.
+//      rows_b (nullable, stream batches): clip b sums its first rows_b[b] rows only (T stays the row stride), and a
+//      clip with no rows is not written.
 // ---------------------------------------------------------------------------
 static __global__ void __launch_bounds__(256)
-k_gram(const float *__restrict__ vmem, double *__restrict__ gram, int C2, long long T, long long t_start) {
+k_gram(const float *__restrict__ vmem, double *__restrict__ gram, int C2, long long T, long long t_start,
+       const int32_t *__restrict__ rows_b = nullptr) {
     const long long b = blockIdx.x;
     const int pair = blockIdx.y * blockDim.x + threadIdx.x;
     if (pair >= C2 * C2) return;
     const int i = pair / C2, j = pair % C2;
     if (j < i) return;  // symmetric: upper triangle only
+    const long long t_end = rows_b ? rows_b[b] : T;
+    if (t_end == 0) return;
     const float *v = vmem + b * T * C2;
     double acc = 0.0;
-    for (long long t = t_start; t < T; ++t) acc = fma((double)v[t * C2 + i], (double)v[t * C2 + j], acc);
+    // the loads of 16 rows are issued before their FMAs (the sum is latency-bound otherwise; same order of FMAs)
+    constexpr int kU = 16;
+    long long t = t_start;
+    for (; t + kU <= t_end; t += kU) {
+        float a[kU], c[kU];
+#pragma unroll
+        for (int u = 0; u < kU; ++u) { a[u] = v[(t + u) * C2 + i]; c[u] = v[(t + u) * C2 + j]; }
+#pragma unroll
+        for (int u = 0; u < kU; ++u) acc = fma((double)a[u], (double)c[u], acc);
+    }
+    for (; t < t_end; ++t) acc = fma((double)v[t * C2 + i], (double)v[t * C2 + j], acc);
     gram[(b * C2 + i) * C2 + j] = acc;
     gram[(b * C2 + j) * C2 + i] = acc;
 }
@@ -761,16 +776,22 @@ k_gram_reduce(const double *__restrict__ part, double *__restrict__ gram, int C2
 // ---------------------------------------------------------------------------
 // S4b: power[b][g] = w_g^T C_b w_g / T (float64), doa[b] = first argmax.
 // One block per clip; dynamic smem: C2*C2 doubles + reduction scratch.
+// rows_b (nullable, stream batches): clip b averages over rows_b[b] samples instead of 1/inv_T, and a clip with no
+// rows is not written.
 // ---------------------------------------------------------------------------
 static __global__ void __launch_bounds__(256)
 k_power_argmax(const double *__restrict__ gram, const double *__restrict__ Wd, float *__restrict__ power,
                int32_t *__restrict__ doa, int C2, int G, double inv_T, int nchunk, double *__restrict__ chunk_v,
-               int *__restrict__ chunk_i) {
+               int *__restrict__ chunk_i, const int32_t *__restrict__ rows_b = nullptr) {
     extern __shared__ __align__(16) double sm_d[];
     double *Cs = sm_d;
     __shared__ double red_v[256];
     __shared__ int red_i[256];
     const long long b = blockIdx.x;
+    if (rows_b) {                            // (uniform across the block: before any barrier)
+        if (rows_b[b] == 0) return;
+        inv_T = 1.0 / (double)rows_b[b];
+    }
     // few clips and a wide array (BASELINE config 5): blockIdx.y takes a slice of the DoA grid, k_argmax_chunks finishes
     const int gper = (G + nchunk - 1) / nchunk;
     const int g_lo = blockIdx.y * gper, g_hi = min(G, g_lo + gper);

@@ -12,11 +12,17 @@
 // encoder, the neuron recurrences and the envelope state all carry over.  Differences to a one-shot clip, by nature of
 // a stream: the in-phase branch is the CAUSAL delay x[t - K/2] (zeros before the stream starts; np.roll's wrap-around
 // needs the clip's end), and results lag the input by D = rzcc_lag(robust_width) samples -- a spike at p is only final
-// once the distance rule has seen D more samples.  micloc_snn_stream_push returns the n_out samples that became final;
-// micloc_snn_stream_flush closes the stream like a clip end and returns the rest.
+// once the distance rule has seen D more samples.  A push returns the n_out samples that became final; a flush closes
+// the stream like a clip end and returns the rest.
 //
-// The kernels are the staged ones (micloc_staged.cuh) with their state in global memory: a stream is one clip wide
-// (7 microphones = 14 sequential channels), i.e. latency matters here, not throughput.
+// A STREAM BATCH carries S such recordings ("slots") at once; the single stream (micloc_snn_stream_*) is a batch of
+// one.  Slots are independent (own position, reset and flush), but a push hands every slot one frame of the same
+// length n, so that one launch per stage serves all of them.  Per push, whatever S:
+//   k_stream_assemble        [K-1 history rows | frame] of every slot (from the previous push's buffer: ping-pong)
+//   STHT                     launch_stht_any over S clips of K-1+n rows
+//   k_stream_blk             band-pass + RZCC of the new samples, then the neuron filter of the final ones
+//   k_gram, k_power_argmax   power / DoA over each slot's final rows            (when power or doa is requested)
+//   k_dense, k_envelope, k_argmax_rows                                      (when env or doa_t is requested)
 #include <cuda_runtime.h>
 
 #include <vector>
@@ -26,7 +32,7 @@
 
 namespace micloc {
 
-struct ChanState {            // one per real channel (in-phase | quadrature)
+struct ChanState {            // one per (slot, real channel): in-phase | quadrature
     BiquadState bq;
     RzccState rz;
     int cl_pos[2 * kClusterMax];
@@ -34,107 +40,251 @@ struct ChanState {            // one per real channel (in-phase | quadrature)
     NeuronState nr;
 };
 
-// frame (any integer / float PCM, `in_ch` >= M interleaved channels, extra channels dropped) -> float rows behind
-// the K-1 history rows of xbuf
+// where a slot stands: samples pushed (N), samples returned as final (F), 0 once flushed.  Positions stay below
+// 2^31 - 4096 (the host refuses a push beyond), so the kernels count time in int.
+struct SlotPos { int N, F, active, pad; };
+
+// [K-1 history rows | frame rows] of every slot: cur [S][hist + n][M].  History = the last hist rows of the previous
+// push's buffer prev [S][hist + n_prev][M], zeros for a slot that starts (N == 0); frame rows converted to float,
+// channels >= M dropped.
 template <typename IN_T>
 __global__ void __launch_bounds__(256)
-k_stream_ingest(const IN_T *__restrict__ frame, float *__restrict__ xbuf, long long n, int in_ch, int M, int hist) {
+k_stream_assemble(const IN_T *__restrict__ frames, const float *__restrict__ prev, float *__restrict__ cur,
+                  const SlotPos *__restrict__ pos, long long S, int n, int n_prev, int in_ch, int M, int hist) {
+    const long long rows = (long long)hist + n;
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n * M) return;
-    const long long t = i / M;
+    if (i >= S * rows * M) return;
     const int m = (int)(i % M);
-    xbuf[(hist + t) * M + m] = (float)frame[t * in_ch + m];
+    const long long r = (i / M) % rows, s = i / (rows * M);
+    float v;
+    if (r < hist) v = pos[s].N > 0 ? prev[(s * (hist + n_prev) + n_prev + r) * M + m] : 0.f;
+    else v = (float)frames[(s * n + (r - hist)) * in_ch + m];
+    cur[i] = v;
 }
 
-// the K-1 newest rows move to the front (history of the next frame)
+// Band-pass + RZCC of the new samples [N, N + n) of every slot, then the neuron filter of the samples that became
+// final, one thread per (slot, channel) with its state in global memory.  The chain is k_chain_blk's (32-sample blocks:
+// branch-free band-pass and running sum, sign / flat-top masks, rzcc_segment_masks, the next block's inputs loaded
+// meanwhile) with the blocks aligned to ABSOLUTE time: the head and tail of a frame that are no whole aligned block go
+// through the same masks with nvalid < 32, and the clusters are closed exactly where the one-clip chain closes them
+// (after every sample t with t % 32 == 31, and at the end), so the spikes are the one-shot clip's bits.  Spikes go to
+// the thread's ring row (int8 [S][C2][R], R a power of two >= n + D + L + 64) at their absolute position; the neuron
+// then reads the row at t and t - L.  Outputs: spikes / membrane rows [S][rows][C2], row i = sample F + i.
+// close_sel != nullptr: flush -- no new samples, the selected slots close their clusters like a clip end, return the
+// rest and stop.  pos_out / m_out: each slot's new position and its number of final rows (read by the later stages).
+// Register budget and CTA size: the chains are latency-bound (one dependent recurrence per thread), so what counts is
+// threads in flight.  152 registers (no spills) leave 13 warps per SM; one-warp CTAs use all 13 (larger CTAs round
+// down), i.e. 61 568 threads on 148 SMs: 4096 slots of 7 microphones (57 344 chains) run in ONE wave.
+constexpr int kStreamBlkThreads = 32;
+template <int NSEC>          // biquads of the band-pass (0 = p.nsec at run time)
+__global__ void __maxnreg__(152)
+k_stream_blk(const float *__restrict__ xbuf, const float *__restrict__ q, ChanState *__restrict__ state,
+             const SlotPos *__restrict__ pos_in, SlotPos *__restrict__ pos_out, int32_t *__restrict__ m_out,
+             const int32_t *__restrict__ close_sel, int8_t *__restrict__ ring, int ring_len, int32_t *__restrict__ flags,
+             int8_t *__restrict__ spikes_out, float *__restrict__ vmem, const __grid_constant__ ChainParams p,
+             long long S, int n, int hist, int rows, int D) {
+    __shared__ float cs_s[kSeg * kStreamBlkThreads];
+    const int C2 = p.C2, M = p.M;
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool in = idx < S * C2;                    // (no early return: keep the warp whole)
+    const long long idc = in ? idx : 0;
+    const int c = (int)(idc % C2);
+    const long long s = idc / C2;
+    const SlotPos ps = pos_in[s];
+    const bool flush = close_sel != nullptr;
+    const bool run = in && ps.active && (!flush || close_sel[s] != 0);
+    const int N0 = ps.N, F0 = ps.F;
+    const int t_end = run ? N0 + n : N0;
+    const int F1 = !run ? F0 : (flush ? N0 : max(t_end - D, F0));
+    if (in && c == 0) {
+        pos_out[s] = SlotPos{t_end, F1, (run && flush) ? 0 : ps.active, 0};
+        m_out[s] = F1 - F0;
+    }
+    constexpr int NS = NSEC ? NSEC : kMaxSections;
+    const int nsec = NSEC ? NSEC : p.nsec;
+    float sos[kMaxSections][5];
+#pragma unroll
+    for (int k = 0; k < kMaxSections; ++k)
+#pragma unroll
+        for (int e = 0; e < 5; ++e) sos[k][e] = p.sos[k][e];
+
+    ChanState &st = state[idc];
+    BiquadState bq = st.bq;
+    RzccState rz = st.rz;
+    NeuronState nr = st.nr;
+    int cl_pos[2 * kClusterMax]; float cl_h[2 * kClusterMax];
+#pragma unroll
+    for (int i = 0; i < 2 * kClusterMax; ++i) { cl_pos[i] = st.cl_pos[i]; cl_h[i] = st.cl_h[i]; }
+    const RzccStore store{cl_pos, cl_h, 1};
+    int8_t *rr = ring + idc * (long long)ring_len;
+    const int rmask = ring_len - 1;
+    auto emit = [&](int pos, int sign) { rr[pos & rmask] = (int8_t)sign; };
+
+    // in-phase: x[t - K/2] = row hist + i - K/2 of the slot's buffer; quadrature: q of row hist + i  (i = t - N0)
+    const bool inphase = c < M;
+    const long long base = s * ((long long)hist + n) * M;
+    const float *src = inphase ? xbuf + base + (long long)(hist - p.half) * M + c : q + base + (long long)hist * M + (c - M);
+    float x[kSeg];
+    auto load_block = [&](int t0, int nv) {
+        const float *pp = src + (long long)(t0 - N0) * M;
+        if (nv == kSeg) {
+#pragma unroll
+            for (int i = 0; i < kSeg; ++i) { x[i] = *pp; pp += M; }
+        } else {
+#pragma unroll
+            for (int i = 0; i < kSeg; ++i) x[i] = i < nv ? pp[(long long)i * M] : 0.f;
+        }
+    };
+    float *cs = cs_s + threadIdx.x;
+    int t = N0;
+    if (t < t_end) load_block(t, min(kSeg - (t & (kSeg - 1)), t_end - t));
+    while (t < t_end) {
+        const int nvalid = min(kSeg - (t & (kSeg - 1)), t_end - t);
+        // the ring bytes of this block: only spikes are stored
+        if (nvalid == kSeg) {
+            uint4 *r4 = reinterpret_cast<uint4 *>(rr + (t & rmask));
+            r4[0] = make_uint4(0u, 0u, 0u, 0u);
+            r4[1] = make_uint4(0u, 0u, 0u, 0u);
+        } else {
+            for (int i = 0; i < nvalid; ++i) rr[(t + i) & rmask] = 0;
+        }
+        // ---- band-pass + running sum of the block, branch-free ----
+        const float carry = rz.csum;
+        float csum = carry;
+        unsigned neg = 0u, zero = 0u;
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i) {
+            if (i < nvalid) {
+                float v = x[i];
+#pragma unroll
+                for (int k = 0; k < NS; ++k) {
+                    if (k < nsec) {
+                        const float y = fmaf(sos[k][0], v, bq.s1[k]);
+                        bq.s1[k] = fmaf(sos[k][1], v, fmaf(-sos[k][3], y, bq.s2[k]));
+                        bq.s2[k] = fmaf(sos[k][2], v, -sos[k][4] * y);
+                        v = y;
+                    }
+                }
+                const float cprev = csum;
+                csum = cprev + v;
+                neg |= (__float_as_uint(v) & 0x80000000u) >> i;
+                zero |= rzcc_flat(v, cprev) ? (0x80000000u >> i) : 0u;
+                cs[i * kStreamBlkThreads] = csum;
+            }
+        }
+        const int tn = t + nvalid;
+        // ---- the next block's inputs on their way while the candidates of this one are handled ----
+        if (tn < t_end) load_block(tn, min(kSeg, t_end - tn));
+        rzcc_segment_masks(rz, store, p.bipolar, p.w, t, nvalid, neg, zero, cs, kStreamBlkThreads, carry, emit);
+        rz.csum = csum;
+        if ((tn & (kSeg - 1)) == 0) rzcc_close(rz, store, p.w, tn - 1, false, emit);
+        t = tn;
+    }
+    if (run && flush && N0 > 0) rzcc_close(rz, store, p.w, N0 - 1, true, emit);
+
+    // ---- neuron filter of the final samples [F0, F1); the spike bytes of the next kNeuBlk steps are requested
+    //      before the current ones are computed (k_neuron_seg) ----
+    constexpr int kNeuBlk = 16;
+    const int nL = p.nL;
+    int nx_s[kNeuBlk], nx_d[kNeuBlk];
+    auto request = [&](int t0) {
+#pragma unroll
+        for (int u = 0; u < kNeuBlk; ++u) {
+            nx_s[u] = rr[(t0 + u) & rmask];
+            nx_d[u] = rr[(t0 + u - nL) & rmask];
+        }
+    };
+    int8_t *so = spikes_out ? spikes_out + s * (long long)rows * C2 + c : nullptr;
+    float *vo = vmem + s * (long long)rows * C2 + c;
+    if (F0 < F1) request(F0);
+    for (int t0 = F0; t0 < F1; t0 += kNeuBlk) {
+        int cur_s[kNeuBlk]; float cur_d[kNeuBlk];
+#pragma unroll
+        for (int u = 0; u < kNeuBlk; ++u) { cur_s[u] = nx_s[u]; cur_d[u] = t0 + u >= nL ? (float)nx_d[u] : 0.f; }
+        if (t0 + kNeuBlk < F1) request(t0 + kNeuBlk);
+#pragma unroll
+        for (int u = 0; u < kNeuBlk; ++u) {
+            if (t0 + u < F1) {
+                const long long i = t0 + u - F0;
+                if (so) so[i * C2] = (int8_t)cur_s[u];
+                vo[i * C2] = neuron_step(p, nr, (float)cur_s[u], cur_d[u]);
+            }
+        }
+    }
+    if (run) {
+        st.bq = bq;
+        st.rz = rz;
+        st.nr = nr;
+#pragma unroll
+        for (int i = 0; i < 2 * kClusterMax; ++i) { st.cl_pos[i] = cl_pos[i]; st.cl_h[i] = cl_h[i]; }
+        if (rz.overflow) atomicOr(flags + s, 1);
+    }
+}
+
+// fresh state for the selected slots (sel == nullptr: all): one thread per (slot, j < max(C2, G))
 __global__ void __launch_bounds__(256)
-k_stream_shift(float *__restrict__ xbuf, float *__restrict__ tmp, long long n, int M, int hist, int phase) {
+k_stream_reset(ChanState *__restrict__ state, SlotPos *__restrict__ pos, int32_t *__restrict__ flags,
+               float *__restrict__ env_state, int32_t *__restrict__ env_started, const int32_t *__restrict__ sel,
+               long long S, int C2, int G) {
+    const int W = C2 > G ? C2 : G;
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (long long)hist * M) return;
-    if (phase == 0) tmp[i] = xbuf[n * M + i]; else xbuf[i] = tmp[i];
-}
-
-// band-pass + RZCC of the new samples [N0, N0 + n), one thread per channel, state carried; spikes go to the ring
-// (int8 [R][C2], R a power of two) at their absolute position.  `final` closes the open clusters (stream end).
-__global__ void __launch_bounds__(32)
-k_stream_chain(const float *__restrict__ xbuf, const float *__restrict__ q, ChanState *__restrict__ state,
-               int8_t *__restrict__ ring, int ring_mask, int32_t *__restrict__ flags,
-               const __grid_constant__ ChainParams p, long long N0, long long n, int hist, int final) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= p.C2) return;
-    ChanState &cs = state[c];
-    BiquadState bq = cs.bq;
-    RzccState rz = cs.rz;
-    const RzccStore store{cs.cl_pos, cs.cl_h, 1};
-    auto emit = [&](int pos, int sign) { ring[(long long)(pos & ring_mask) * p.C2 + c] = (int8_t)sign; };
-    const bool inphase = c < p.M;
-    for (long long i = 0; i < n; ++i) {
-        const long long t = N0 + i;
-        // in-phase: x[t - K/2] (row hist + i - K/2 of xbuf); quadrature: q of the extended clip at row hist + i
-        const float x = inphase ? xbuf[(hist + i - p.half) * p.M + c] : q[(hist + i) * p.M + (c - p.M)];
-        const float z = biquad_step(p.sos, p.nsec, bq, x);
-        ring[(t & ring_mask) * p.C2 + c] = 0;
-        rzcc_detect(rz, store, p.bipolar, p.w, (int)t, z, emit);
-        if ((t & (kSeg - 1)) == kSeg - 1) rzcc_close(rz, store, p.w, (int)t, false, emit);
+    if (i >= S * W) return;
+    const long long s = i / W;
+    const int j = (int)(i % W);
+    if (sel && !sel[s]) return;
+    if (j < C2) {
+        ChanState &c = state[s * C2 + j];
+        biquad_reset(c.bq);
+        rzcc_reset(c.rz);
+        neuron_reset(c.nr);
+        for (int k = 0; k < 2 * kClusterMax; ++k) { c.cl_pos[k] = 0; c.cl_h[k] = 0.f; }
     }
-    if (final && N0 + n > 0) rzcc_close(rz, store, p.w, (int)(N0 + n - 1), true, emit);
-    cs.bq = bq;
-    cs.rz = rz;
-    if (rz.overflow && flags) atomicOr(flags, 1);
-}
-
-// neuron filter of the final samples [F0, F0 + m): spikes from the ring -> int8 spikes out + membrane rows
-__global__ void __launch_bounds__(32)
-k_stream_neuron(const int8_t *__restrict__ ring, int ring_mask, ChanState *__restrict__ state,
-                int8_t *__restrict__ spikes_out, float *__restrict__ vmem, const __grid_constant__ ChainParams p,
-                long long F0, long long m) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= p.C2) return;
-    NeuronState nr = state[c].nr;
-    for (long long i = 0; i < m; ++i) {
-        const long long t = F0 + i;
-        const int8_t s8 = ring[(t & ring_mask) * p.C2 + c];
-        const float sd = t >= p.nL ? (float)ring[((t - p.nL) & ring_mask) * p.C2 + c] : 0.f;
-        if (spikes_out) spikes_out[i * p.C2 + c] = s8;
-        vmem[i * p.C2 + c] = neuron_step(p, nr, (float)s8, sd);
-    }
-    state[c].nr = nr;
+    if (j < G) { env_state[s * G + j] = 0.f; env_started[s * G + j] = 0; }
+    if (j == 0) { pos[s] = SlotPos{0, 0, 1, 0}; flags[s] = 0; }
 }
 
 }  // namespace micloc
 
-// Envelope.evolve (micloc/utils.py:49-81) over rows of |x|, one thread per channel, state carried between calls:
-//   first row ever: state = |x[0]|, out[0] = state;  afterwards  rise = |x| >= state,  win = rise ? int(fs rise_time)
-//   : int(fs fall_time),  state = (1 - 1/win) state + (1/win) |x| rise,  out = state
+// Envelope.evolve (micloc/utils.py:49-81) over rows of |x|, one thread per (clip, channel), state carried between
+// calls:  first row ever: state = |x[0]|, out[0] = state;  afterwards  rise = |x| >= state,  win = rise ?
+// int(fs rise_time) : int(fs fall_time),  state = (1 - 1/win) state + (1/win) |x| rise,  out = state.
+// x, env [B][T][C]; state, started [B][C]; rows_b (nullable): clip b takes its first rows_b[b] rows (T = row stride).
 namespace micloc {
 __global__ void __launch_bounds__(128)
 k_envelope(const float *__restrict__ x, float *__restrict__ env, float *__restrict__ state, int32_t *__restrict__ started,
-           long long T, int C, float inv_fall, float inv_rise) {
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= C) return;
-    float s = state[c];
+           const int32_t *__restrict__ rows_b, long long B, long long T, int C, float inv_fall, float inv_rise) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= B * C) return;
+    const long long b = i / C;
+    const int c = (int)(i % C);
+    const long long Tn = rows_b ? rows_b[b] : T;
+    const float *xb = x + b * T * C;
+    float *eb = env + b * T * C;
+    float s = state[i];
     long long t = 0;
-    if (!*started && T > 0) { s = fabsf(x[c]); env[c] = s; t = 1; }
-    for (; t < T; ++t) {
-        const float a = fabsf(x[t * C + c]);
+    if (!started[i] && Tn > 0) { s = fabsf(xb[c]); eb[c] = s; t = 1; started[i] = 1; }
+    for (; t < Tn; ++t) {
+        const float a = fabsf(xb[t * C + c]);
         const bool rise = a >= s;
         const float iw = rise ? inv_rise : inv_fall;
         s = (1.f - iw) * s + (rise ? iw * a : 0.f);
-        env[t * C + c] = s;
+        eb[t * C + c] = s;
     }
-    state[c] = s;
+    state[i] = s;
 }
-__global__ void k_envelope_mark(int32_t *started, long long T) { if (T > 0) *started = 1; }
 
-// first argmax over the C channels of every row (np.argmax(env, axis=1)); one warp per row
+// first argmax over the C channels of every row (np.argmax(env, axis=1)); one warp per row of env [B][T][C]
+// (rows_b as in k_envelope: rows past a clip's count are not written)
 __global__ void __launch_bounds__(256)
-k_argmax_rows(const float *__restrict__ env, int32_t *__restrict__ idx, long long T, int C) {
-    const long long t = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+k_argmax_rows(const float *__restrict__ env, int32_t *__restrict__ idx, const int32_t *__restrict__ rows_b, long long B,
+              long long T, int C) {
+    const long long r = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
-    if (t >= T) return;
+    if (r >= B * T) return;
+    if (rows_b && r % T >= rows_b[r / T]) return;
     float best = -1.f; int bi = 0x7fffffff;
     for (int c = lane; c < C; c += 32) {
-        const float v = env[t * C + c];
+        const float v = env[r * C + c];
         if (v > best) { best = v; bi = c; }
     }
     for (int o = 16; o > 0; o >>= 1) {
@@ -142,64 +292,87 @@ k_argmax_rows(const float *__restrict__ env, int32_t *__restrict__ idx, long lon
         const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
         if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }
     }
-    if (lane == 0) idx[t] = bi;
+    if (lane == 0) idx[r] = bi;
 }
 }  // namespace micloc
 
 using namespace micloc;
 
-struct micloc_stream {
+struct micloc_stream_batch {
     micloc_snn_params prm{};        // copy of what the kernels need from the parent context
     int device = 0;
+    long long S = 0;
     long long max_frame = 0;
     int hist = 0;                   // K - 1
     int D = 0;                      // output latency in samples
     int ring_len = 0;
-    long long N = 0;                // samples pushed
-    long long F = 0;                // samples returned (final)
-    bool flushed = false;
-    float *xbuf = nullptr, *tmp = nullptr, *q = nullptr, *vmem = nullptr, *y = nullptr, *env = nullptr, *env_state = nullptr;
+    int xcur = 0;                   // xbuf[xcur] holds the newest [history | frame] rows (n_prev frame rows)
+    int pcur = 0;                   // pos[pcur] holds the slots' positions
+    long long n_prev = 0;
+    std::vector<long long> N, F;    // host mirror of the positions (n_out without a device synchronisation)
+    std::vector<char> active;
+    std::vector<int32_t> sel_h;     // staging of the slot lists
+    float *xbuf[2] = {nullptr, nullptr}, *q = nullptr, *vmem = nullptr, *env_state = nullptr;
     int8_t *ring = nullptr;
     ChanState *state = nullptr;
-    int32_t *flags = nullptr, *env_started = nullptr;
+    SlotPos *pos[2] = {nullptr, nullptr};
+    int32_t *m = nullptr, *flags = nullptr, *sel = nullptr, *env_started = nullptr;
     double *gram = nullptr;
+    DevBuf y, env;                  // envelope scratch: allocated on the first request, grow-only
     float rise_time = 10e-3f, fall_time = 100e-3f, fs = 48000.f;
 };
 
-extern "C" int micloc_snn_stream_destroy(micloc_stream *s) {
-    if (!s) return MICLOC_OK;
-    cudaSetDevice(s->device);
-    cudaFree(s->xbuf); cudaFree(s->tmp); cudaFree(s->q); cudaFree(s->vmem); cudaFree(s->y); cudaFree(s->env);
-    cudaFree(s->env_state); cudaFree(s->ring); cudaFree(s->state); cudaFree(s->flags); cudaFree(s->env_started);
-    cudaFree(s->gram);
-    delete s;
+// the single stream: a batch of one slot
+struct micloc_stream {
+    micloc_stream_batch *sb = nullptr;
+};
+
+extern "C" int micloc_snn_streams_destroy(micloc_stream_batch *sb) {
+    if (!sb) return MICLOC_OK;
+    cudaSetDevice(sb->device);
+    cudaFree(sb->xbuf[0]); cudaFree(sb->xbuf[1]); cudaFree(sb->q); cudaFree(sb->vmem); cudaFree(sb->env_state);
+    cudaFree(sb->ring); cudaFree(sb->state); cudaFree(sb->pos[0]); cudaFree(sb->pos[1]); cudaFree(sb->m);
+    cudaFree(sb->flags); cudaFree(sb->sel); cudaFree(sb->env_started); cudaFree(sb->gram);
+    sb->y.release(); sb->env.release();
+    delete sb;
     return MICLOC_OK;
 }
 
-static int stream_reset_state(micloc_stream *s, cudaStream_t st) {
-    const ChainParams &p = s->prm.chain;
-    MICLOC_CUDA(cudaMemsetAsync(s->xbuf, 0, (size_t)(s->hist + s->max_frame) * p.M * sizeof(float), st));
-    MICLOC_CUDA(cudaMemsetAsync(s->ring, 0, (size_t)s->ring_len * p.C2, st));
-    MICLOC_CUDA(cudaMemsetAsync(s->env_state, 0, (size_t)p.G * sizeof(float), st));
-    MICLOC_CUDA(cudaMemsetAsync(s->env_started, 0, sizeof(int32_t), st));
-    MICLOC_CUDA(cudaMemsetAsync(s->flags, 0, sizeof(int32_t), st));
-    std::vector<ChanState> init((size_t)p.C2);
-    for (auto &c : init) {
-        for (int k = 0; k < kMaxSections; ++k) { c.bq.s1[k] = 0.f; c.bq.s2[k] = 0.f; }
-        c.rz.csum = 0.f; c.rz.r = -1; c.rz.sgn = 0; c.rz.n0 = c.rz.n1 = 0; c.rz.last0 = c.rz.last1 = 0; c.rz.overflow = 0;
-        c.nr.p1 = c.nr.p2 = c.nr.q1 = c.nr.q2 = 0.f;
-        for (int i = 0; i < 2 * kClusterMax; ++i) { c.cl_pos[i] = 0; c.cl_h[i] = 0.f; }
-    }
-    MICLOC_CUDA(cudaMemcpyAsync(s->state, init.data(), init.size() * sizeof(ChanState), cudaMemcpyHostToDevice, st));
-    MICLOC_CUDA(cudaStreamSynchronize(st));      // `init` is a local vector
-    s->N = 0; s->F = 0; s->flushed = false;
+// slots_host [n_slots] (NULL = every slot) -> sb->sel on the device (1 = listed); synchronises `st`: the staging
+// vector is reused by the next call
+static int upload_slots(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots, cudaStream_t st) {
+    if (slots_host && n_slots < 0) return set_error(MICLOC_ERR_SHAPE, "n_slots %d < 0", n_slots);
+    for (int32_t i = 0; slots_host && i < n_slots; ++i)
+        if (slots_host[i] < 0 || slots_host[i] >= sb->S)
+            return set_error(MICLOC_ERR_SHAPE, "slot %d out of range [0, %lld)", slots_host[i], sb->S);
+    sb->sel_h.assign((size_t)sb->S, slots_host ? 0 : 1);
+    for (int32_t i = 0; slots_host && i < n_slots; ++i) sb->sel_h[(size_t)slots_host[i]] = 1;
+    MICLOC_CUDA(cudaMemcpyAsync(sb->sel, sb->sel_h.data(), (size_t)sb->S * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    MICLOC_CUDA(cudaStreamSynchronize(st));
     return MICLOC_OK;
 }
 
-extern "C" int micloc_snn_stream_create(micloc_snn *ctx, int64_t max_frame_len, double fs, double rise_time,
-                                        double fall_time, micloc_stream **out) {
+extern "C" int micloc_snn_streams_reset(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots, void *stream) {
+    if (!sb) return set_error(MICLOC_ERR_CONFIG, "null stream");
+    MICLOC_CUDA(cudaSetDevice(sb->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (slots_host) MICLOC_TRY(upload_slots(sb, slots_host, n_slots, st));
+    const ChainParams &p = sb->prm.chain;
+    const long long W = p.C2 > p.G ? p.C2 : p.G;
+    k_stream_reset<<<(unsigned)((sb->S * W + 255) / 256), 256, 0, st>>>(sb->state, sb->pos[sb->pcur], sb->flags, sb->env_state,
+                                                                       sb->env_started, slots_host ? sb->sel : nullptr, sb->S, p.C2, p.G);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    for (long long s = 0; s < sb->S; ++s)
+        if (!slots_host || sb->sel_h[(size_t)s]) { sb->N[(size_t)s] = 0; sb->F[(size_t)s] = 0; sb->active[(size_t)s] = 1; }
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_streams_create(micloc_snn *ctx, int32_t num_streams, int64_t max_frame_len, double fs,
+                                         double rise_time, double fall_time, micloc_stream_batch **out) {
     if (!ctx || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
     *out = nullptr;
+    if (num_streams < 1 || num_streams > 65535) return set_error(MICLOC_ERR_SHAPE, "num_streams %d out of range [1, 65535]", num_streams);
     if (max_frame_len < 1 || max_frame_len > (1ll << 24)) return set_error(MICLOC_ERR_SHAPE, "max_frame_len out of range");
     if (rise_time > fall_time)
         return set_error(MICLOC_ERR_CONFIG, "for proper functioning, an envelope estimator should have a larger fall time!");
@@ -208,128 +381,213 @@ extern "C" int micloc_snn_stream_create(micloc_snn *ctx, int64_t max_frame_len, 
     MICLOC_TRY(micloc_snn_get_params(ctx, &prm));
     const ChainParams &p = prm.chain;
     MICLOC_CUDA(cudaSetDevice(prm.device));
-    micloc_stream *s = new micloc_stream();
-    s->prm = prm; s->device = prm.device; s->max_frame = max_frame_len;
-    s->hist = p.K - 1;
-    s->D = rzcc_lag(p.w);
-    int need = (int)max_frame_len + s->D + p.nL + 2 * kSeg;
-    s->ring_len = 1;
-    while (s->ring_len < need) s->ring_len <<= 1;
-    s->fs = (float)fs; s->rise_time = (float)rise_time; s->fall_time = (float)fall_time;
-    const size_t rows = (size_t)s->hist + max_frame_len;
-    const size_t fin = (size_t)max_frame_len + s->D;                // most samples one call can finalise
-    bool ok = cudaMalloc(&s->xbuf, rows * p.M * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&s->tmp, (size_t)s->hist * p.M * sizeof(float) + 16) == cudaSuccess &&
-              cudaMalloc(&s->q, rows * p.M * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&s->vmem, fin * p.C2 * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&s->y, fin * p.G * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&s->env, fin * p.G * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&s->env_state, (size_t)p.G * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&s->ring, (size_t)s->ring_len * p.C2) == cudaSuccess &&
-              cudaMalloc(&s->state, (size_t)p.C2 * sizeof(ChanState)) == cudaSuccess &&
-              cudaMalloc(&s->flags, sizeof(int32_t)) == cudaSuccess &&
-              cudaMalloc(&s->env_started, sizeof(int32_t)) == cudaSuccess &&
-              cudaMalloc(&s->gram, (size_t)p.C2 * p.C2 * sizeof(double)) == cudaSuccess;
-    if (!ok) { micloc_snn_stream_destroy(s); return set_error(MICLOC_ERR_CUDA, "cudaMalloc(stream) failed"); }
-    const int rc = stream_reset_state(s, nullptr);
-    if (rc) { micloc_snn_stream_destroy(s); return rc; }
-    *out = s;
+    micloc_stream_batch *sb = new micloc_stream_batch();
+    sb->prm = prm; sb->device = prm.device; sb->S = num_streams; sb->max_frame = max_frame_len;
+    sb->hist = p.K - 1;
+    sb->D = rzcc_lag(p.w);
+    const long long need = max_frame_len + sb->D + p.nL + 2 * kSeg;
+    sb->ring_len = 32;
+    while (sb->ring_len < need) sb->ring_len <<= 1;
+    sb->fs = (float)fs; sb->rise_time = (float)rise_time; sb->fall_time = (float)fall_time;
+    sb->N.assign((size_t)num_streams, 0); sb->F.assign((size_t)num_streams, 0); sb->active.assign((size_t)num_streams, 1);
+    const size_t S = (size_t)num_streams;
+    const size_t rows = (size_t)sb->hist + max_frame_len;
+    const size_t fin = (size_t)max_frame_len + sb->D;                // most samples one call can finalise
+    bool ok = cudaMalloc(&sb->xbuf[0], S * rows * p.M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&sb->xbuf[1], S * rows * p.M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&sb->q, S * rows * p.M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&sb->vmem, S * fin * p.C2 * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&sb->env_state, S * p.G * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&sb->env_started, S * p.G * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&sb->ring, S * p.C2 * (size_t)sb->ring_len) == cudaSuccess &&
+              cudaMalloc(&sb->state, S * p.C2 * sizeof(ChanState)) == cudaSuccess &&
+              cudaMalloc(&sb->pos[0], S * sizeof(SlotPos)) == cudaSuccess &&
+              cudaMalloc(&sb->pos[1], S * sizeof(SlotPos)) == cudaSuccess &&
+              cudaMalloc(&sb->m, S * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&sb->flags, S * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&sb->sel, S * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&sb->gram, S * p.C2 * p.C2 * sizeof(double)) == cudaSuccess;
+    if (!ok) { micloc_snn_streams_destroy(sb); return set_error(MICLOC_ERR_CUDA, "cudaMalloc(stream batch) failed"); }
+    int rc = micloc_snn_streams_reset(sb, nullptr, 0, nullptr);
+    if (!rc && cudaStreamSynchronize(nullptr) != cudaSuccess) rc = set_error(MICLOC_ERR_CUDA, "stream batch reset failed");
+    if (rc) { micloc_snn_streams_destroy(sb); return rc; }
+    *out = sb;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_streams_latency(micloc_stream_batch *sb) { return sb ? sb->D : 0; }
+
+// shared tail of push / flush: power / DoA and envelope over each slot's final rows (sb->m, written by k_stream_blk);
+// outputs [S][rows][...]
+static int streams_finalise(micloc_stream_batch *sb, long long rows, float *power_dev, int32_t *doa_dev, float *env_dev,
+                            int32_t *doa_t_dev, cudaStream_t st) {
+    const ChainParams &p = sb->prm.chain;
+    const long long S = sb->S;
+    if (power_dev || doa_dev) {
+        dim3 gg((unsigned)S, (unsigned)((p.C2 * p.C2 + 255) / 256));
+        k_gram<<<gg, 256, 0, st>>>(sb->vmem, sb->gram, p.C2, rows, 0, sb->m);
+        const size_t smem = (size_t)p.C2 * p.C2 * sizeof(double);
+        MICLOC_CUDA(cudaFuncSetAttribute(k_power_argmax, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_power_argmax<<<(unsigned)S, 256, smem, st>>>(sb->gram, (const double *)sb->prm.bf_f64_dev, power_dev, doa_dev, p.C2,
+                                                       p.G, 1.0, 1, nullptr, nullptr, sb->m);
+        count_launch(2);
+    }
+    if (env_dev || doa_t_dev) {
+        const size_t bytes = (size_t)S * rows * p.G * sizeof(float);
+        MICLOC_TRY(sb->y.reserve(bytes));
+        if (!env_dev) MICLOC_TRY(sb->env.reserve(bytes));
+        float *y = (float *)sb->y.ptr;
+        float *env = env_dev ? env_dev : (float *)sb->env.ptr;
+        const int slab = 256;
+        dim3 grid((unsigned)((p.G + 127) / 128), (unsigned)((rows + slab - 1) / slab), (unsigned)S);
+        if (p.C2 <= 16) k_dense<16><<<grid, 128, 0, st>>>(sb->vmem, (const float *)sb->prm.bf_f32_dev, y, p.C2, p.G, rows, slab);
+        else k_dense<0><<<grid, 128, 0, st>>>(sb->vmem, (const float *)sb->prm.bf_f32_dev, y, p.C2, p.G, rows, slab);
+        k_envelope<<<(unsigned)((S * p.G + 127) / 128), 128, 0, st>>>(y, env, sb->env_state, sb->env_started, sb->m, S, rows, p.G,
+                                                                      1.f / (float)(int)(sb->fs * sb->fall_time),
+                                                                      1.f / (float)(int)(sb->fs * sb->rise_time));
+        count_launch(2);
+        if (doa_t_dev) {
+            k_argmax_rows<<<(unsigned)((S * rows * 32 + 255) / 256), 256, 0, st>>>(env, doa_t_dev, sb->m, S, rows, p.G);
+            count_launch(1);
+        }
+    }
+    MICLOC_CUDA(cudaGetLastError());
+    return MICLOC_OK;
+}
+
+static int launch_stream_blk(micloc_stream_batch *sb, const int32_t *close_sel, int n, int rows, int8_t *spikes_dev,
+                             cudaStream_t st) {
+    const ChainParams &p = sb->prm.chain;
+    const long long lanes = sb->S * p.C2;
+    const unsigned grid = (unsigned)((lanes + kStreamBlkThreads - 1) / kStreamBlkThreads);
+    auto kernel = p.nsec == 2 ? k_stream_blk<2> : k_stream_blk<0>;
+    kernel<<<grid, kStreamBlkThreads, 0, st>>>(sb->xbuf[sb->xcur], sb->q, sb->state, sb->pos[sb->pcur], sb->pos[sb->pcur ^ 1],
+                                              sb->m, close_sel, sb->ring, sb->ring_len, sb->flags, spikes_dev, sb->vmem, p,
+                                              sb->S, n, sb->hist, rows, sb->D);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    sb->pcur ^= 1;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_streams_push(micloc_stream_batch *sb, const void *frames_dev, int dtype, int64_t n,
+                                       int32_t in_channels, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev,
+                                       float *env_dev, int32_t *doa_t_dev, int64_t *n_out_host, void *stream) {
+    if (!sb || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
+    const ChainParams &p = sb->prm.chain;
+    if (n < 1 || n > sb->max_frame) return set_error(MICLOC_ERR_SHAPE, "frame of %lld samples (stream takes 1..%lld)", (long long)n, sb->max_frame);
+    if (in_channels < p.M)
+        return set_error(MICLOC_ERR_SHAPE, "number of channels in the input siganl %d should be the same as the number of microphones %d!", in_channels, p.M);
+    if (dtype != MICLOC_F32 && dtype != MICLOC_I16 && dtype != MICLOC_I32)
+        return set_error(MICLOC_ERR_SHAPE, "dtype must be MICLOC_F32, MICLOC_I16 or MICLOC_I32");
+    for (long long s = 0; s < sb->S; ++s)
+        if (sb->active[(size_t)s] && sb->N[(size_t)s] + n >= (1ll << 31) - 4096)
+            return set_error(MICLOC_ERR_SHAPE, "stream position exceeds 2^31 samples: reset the stream");
+    MICLOC_CUDA(cudaSetDevice(sb->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nxt = sb->xcur ^ 1;
+    const long long total = sb->S * (sb->hist + n) * p.M;
+    const unsigned ga = (unsigned)((total + 255) / 256);
+    const float *prev = sb->xbuf[sb->xcur];
+    const SlotPos *pos = sb->pos[sb->pcur];
+    if (dtype == MICLOC_F32)
+        k_stream_assemble<float><<<ga, 256, 0, st>>>((const float *)frames_dev, prev, sb->xbuf[nxt], pos, sb->S, (int)n, (int)sb->n_prev, in_channels, p.M, sb->hist);
+    else if (dtype == MICLOC_I16)
+        k_stream_assemble<int16_t><<<ga, 256, 0, st>>>((const int16_t *)frames_dev, prev, sb->xbuf[nxt], pos, sb->S, (int)n, (int)sb->n_prev, in_channels, p.M, sb->hist);
+    else
+        k_stream_assemble<int32_t><<<ga, 256, 0, st>>>((const int32_t *)frames_dev, prev, sb->xbuf[nxt], pos, sb->S, (int)n, (int)sb->n_prev, in_channels, p.M, sb->hist);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    sb->xcur = nxt;
+    sb->n_prev = n;
+    // STHT of the extended clips [history | frame]: rows >= hist see their whole window
+    MICLOC_TRY(launch_stht_any(p, (const float *)sb->prm.taps_dev, sb->xbuf[nxt], MICLOC_F32, sb->q, sb->S, sb->hist + n, st));
+    const long long rows = n + sb->D;
+    MICLOC_TRY(launch_stream_blk(sb, nullptr, (int)n, (int)rows, spikes_dev, st));
+    for (long long s = 0; s < sb->S; ++s) {
+        const size_t i = (size_t)s;
+        n_out_host[s] = 0;
+        if (!sb->active[i]) continue;
+        sb->N[i] += n;
+        const long long f = sb->N[i] - sb->D > sb->F[i] ? sb->N[i] - sb->D : sb->F[i];
+        n_out_host[s] = f - sb->F[i];
+        sb->F[i] = f;
+    }
+    return streams_finalise(sb, rows, power_dev, doa_dev, env_dev, doa_t_dev, st);
+}
+
+extern "C" int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots,
+                                        int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev,
+                                        int32_t *doa_t_dev, int64_t *n_out_host, int32_t *flags_host, void *stream) {
+    if (!sb || !n_out_host) return set_error(MICLOC_ERR_CONFIG, "null stream");
+    MICLOC_CUDA(cudaSetDevice(sb->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    MICLOC_TRY(upload_slots(sb, slots_host, n_slots, st));
+    const long long rows = sb->max_frame + sb->D;
+    MICLOC_TRY(launch_stream_blk(sb, sb->sel, 0, (int)rows, spikes_dev, st));
+    for (long long s = 0; s < sb->S; ++s) {
+        const size_t i = (size_t)s;
+        n_out_host[s] = 0;
+        if (!sb->active[i] || !sb->sel_h[i]) continue;
+        n_out_host[s] = sb->N[i] - sb->F[i];
+        sb->F[i] = sb->N[i];
+        sb->active[i] = 0;
+    }
+    MICLOC_TRY(streams_finalise(sb, rows, power_dev, doa_dev, env_dev, doa_t_dev, st));
+    if (flags_host) {
+        MICLOC_CUDA(cudaMemcpyAsync(flags_host, sb->flags, (size_t)sb->S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        MICLOC_CUDA(cudaStreamSynchronize(st));
+    }
+    return MICLOC_OK;
+}
+
+// ---- the single stream: slot 0 of a one-slot batch ----
+extern "C" int micloc_snn_stream_create(micloc_snn *ctx, int64_t max_frame_len, double fs, double rise_time,
+                                        double fall_time, micloc_stream **out) {
+    if (!ctx || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
+    *out = nullptr;
+    micloc_stream_batch *sb = nullptr;
+    MICLOC_TRY(micloc_snn_streams_create(ctx, 1, max_frame_len, fs, rise_time, fall_time, &sb));
+    *out = new micloc_stream{sb};
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_stream_destroy(micloc_stream *s) {
+    if (!s) return MICLOC_OK;
+    micloc_snn_streams_destroy(s->sb);
+    delete s;
     return MICLOC_OK;
 }
 
 extern "C" int micloc_snn_stream_reset(micloc_stream *s, void *stream) {
     if (!s) return set_error(MICLOC_ERR_CONFIG, "null stream");
-    MICLOC_CUDA(cudaSetDevice(s->device));
-    return stream_reset_state(s, (cudaStream_t)stream);
-}
-
-extern "C" int micloc_snn_stream_latency(micloc_stream *s) { return s ? s->D : 0; }
-
-// shared tail of push / flush: the samples [F, F_new) are final -> neuron, spikes, Gram power, envelope, argmax
-static int stream_finalise(micloc_stream *s, long long F_new, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev,
-                           float *env_dev, int32_t *doa_t_dev, int64_t *n_out, cudaStream_t st) {
-    const ChainParams &p = s->prm.chain;
-    const long long m = F_new - s->F;
-    if (n_out) *n_out = m;
-    if (m <= 0) return MICLOC_OK;
-    k_stream_neuron<<<(p.C2 + 31) / 32, 32, 0, st>>>(s->ring, s->ring_len - 1, s->state, spikes_dev, s->vmem, p, s->F, m);
-    count_launch(1);
-    if (power_dev || doa_dev) {
-        dim3 gg(1, (unsigned)((p.C2 * p.C2 + 255) / 256));
-        k_gram<<<gg, 256, 0, st>>>(s->vmem, s->gram, p.C2, m, 0);
-        const size_t smem = (size_t)p.C2 * p.C2 * sizeof(double);
-        MICLOC_CUDA(cudaFuncSetAttribute(k_power_argmax, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_power_argmax<<<1, 256, smem, st>>>(s->gram, (const double *)s->prm.bf_f64_dev, power_dev, doa_dev, p.C2, p.G, 1.0 / (double)m, 1, nullptr, nullptr);
-        count_launch(2);
-    }
-    if (env_dev || doa_t_dev) {
-        const int slab = 256;
-        dim3 grid((unsigned)((p.G + 127) / 128), (unsigned)((m + slab - 1) / slab), 1);
-        if (p.C2 <= 16) k_dense<16><<<grid, 128, 0, st>>>(s->vmem, (const float *)s->prm.bf_f32_dev, s->y, p.C2, p.G, m, slab);
-        else k_dense<0><<<grid, 128, 0, st>>>(s->vmem, (const float *)s->prm.bf_f32_dev, s->y, p.C2, p.G, m, slab);
-        float *env = env_dev ? env_dev : s->env;
-        k_envelope<<<(p.G + 127) / 128, 128, 0, st>>>(s->y, env, s->env_state, s->env_started, m, p.G,
-                                                      1.f / (float)(int)(s->fs * s->fall_time), 1.f / (float)(int)(s->fs * s->rise_time));
-        k_envelope_mark<<<1, 1, 0, st>>>(s->env_started, m);
-        count_launch(3);
-        if (doa_t_dev) {
-            k_argmax_rows<<<(unsigned)((m * 32 + 255) / 256), 256, 0, st>>>(env, doa_t_dev, m, p.G);
-            count_launch(1);
-        }
-    }
-    MICLOC_CUDA(cudaGetLastError());
-    s->F = F_new;
+    MICLOC_TRY(micloc_snn_streams_reset(s->sb, nullptr, 0, stream));
+    MICLOC_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
     return MICLOC_OK;
 }
+
+extern "C" int micloc_snn_stream_latency(micloc_stream *s) { return s ? s->sb->D : 0; }
 
 extern "C" int micloc_snn_stream_push(micloc_stream *s, const void *frame_dev, int dtype, int64_t n, int32_t in_channels,
                                       int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev,
                                       int32_t *doa_t_dev, int64_t *n_out, void *stream) {
     if (!s || !frame_dev) return set_error(MICLOC_ERR_SHAPE, "null argument");
-    const ChainParams &p = s->prm.chain;
-    if (s->flushed) return set_error(MICLOC_ERR_CONFIG, "stream was flushed: reset it before pushing again");
-    if (n < 1 || n > s->max_frame) return set_error(MICLOC_ERR_SHAPE, "frame of %lld samples (stream takes 1..%lld)", (long long)n, s->max_frame);
-    if (in_channels < p.M)
-        return set_error(MICLOC_ERR_SHAPE, "number of channels in the input siganl %d should be the same as the number of microphones %d!", in_channels, p.M);
-    if (s->N + n >= (1ll << 31) - 4096) return set_error(MICLOC_ERR_SHAPE, "stream position exceeds 2^31 samples: reset the stream");
-    MICLOC_CUDA(cudaSetDevice(s->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const unsigned gi = (unsigned)((n * p.M + 255) / 256);
-    if (dtype == MICLOC_F32) k_stream_ingest<float><<<gi, 256, 0, st>>>((const float *)frame_dev, s->xbuf, n, in_channels, p.M, s->hist);
-    else if (dtype == MICLOC_I16) k_stream_ingest<int16_t><<<gi, 256, 0, st>>>((const int16_t *)frame_dev, s->xbuf, n, in_channels, p.M, s->hist);
-    else if (dtype == MICLOC_I32) k_stream_ingest<int32_t><<<gi, 256, 0, st>>>((const int32_t *)frame_dev, s->xbuf, n, in_channels, p.M, s->hist);
-    else return set_error(MICLOC_ERR_SHAPE, "dtype must be MICLOC_F32, MICLOC_I16 or MICLOC_I32");
-    count_launch(1);
-    // STHT of the extended clip [history | frame]: rows >= hist see their whole window
-    MICLOC_TRY(launch_stht_any(p, (const float *)s->prm.taps_dev, s->xbuf, MICLOC_F32, s->q, 1, s->hist + n, st));
-    k_stream_chain<<<(p.C2 + 31) / 32, 32, 0, st>>>(s->xbuf, s->q, s->state, s->ring, s->ring_len - 1, s->flags, p, s->N, n, s->hist, 0);
-    const unsigned gs = (unsigned)(((long long)s->hist * p.M + 255) / 256);
-    k_stream_shift<<<gs, 256, 0, st>>>(s->xbuf, s->tmp, n, p.M, s->hist, 0);
-    k_stream_shift<<<gs, 256, 0, st>>>(s->xbuf, s->tmp, n, p.M, s->hist, 1);
-    count_launch(3);
-    MICLOC_CUDA(cudaGetLastError());
-    s->N += n;
-    const long long F_new = s->N - s->D > s->F ? s->N - s->D : s->F;
-    return stream_finalise(s, F_new, spikes_dev, power_dev, doa_dev, env_dev, doa_t_dev, n_out, st);
+    if (!s->sb->active[0]) return set_error(MICLOC_ERR_CONFIG, "stream was flushed: reset it before pushing again");
+    int64_t m = 0;
+    MICLOC_TRY(micloc_snn_streams_push(s->sb, frame_dev, dtype, n, in_channels, spikes_dev, power_dev, doa_dev, env_dev,
+                                       doa_t_dev, &m, stream));
+    if (n_out) *n_out = m;
+    return MICLOC_OK;
 }
 
 extern "C" int micloc_snn_stream_flush(micloc_stream *s, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev,
                                        float *env_dev, int32_t *doa_t_dev, int64_t *n_out, int32_t *flags_host,
                                        void *stream) {
     if (!s) return set_error(MICLOC_ERR_CONFIG, "null stream");
-    const ChainParams &p = s->prm.chain;
-    MICLOC_CUDA(cudaSetDevice(s->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!s->flushed) {
-        k_stream_chain<<<(p.C2 + 31) / 32, 32, 0, st>>>(s->xbuf, s->q, s->state, s->ring, s->ring_len - 1, s->flags, p, s->N, 0, s->hist, 1);
-        count_launch(1);
-        s->flushed = true;
-    }
-    MICLOC_TRY(stream_finalise(s, s->N, spikes_dev, power_dev, doa_dev, env_dev, doa_t_dev, n_out, st));
-    if (flags_host) {
-        MICLOC_CUDA(cudaMemcpyAsync(flags_host, s->flags, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        MICLOC_CUDA(cudaStreamSynchronize(st));
-    }
+    int64_t m = 0;
+    MICLOC_TRY(micloc_snn_streams_flush(s->sb, nullptr, 0, spikes_dev, power_dev, doa_dev, env_dev, doa_t_dev, &m,
+                                        flags_host, stream));
+    if (n_out) *n_out = m;
     return MICLOC_OK;
 }
 
@@ -345,13 +603,13 @@ extern "C" int micloc_envelope(const float *x_dev, int64_t T, int32_t C, double 
     cudaStream_t st = (cudaStream_t)stream;
     float *state = nullptr; int32_t *started = nullptr;
     MICLOC_CUDA(cudaMallocAsync(&state, (size_t)C * sizeof(float), st));
-    MICLOC_CUDA(cudaMallocAsync(&started, sizeof(int32_t), st));
+    MICLOC_CUDA(cudaMallocAsync(&started, (size_t)C * sizeof(int32_t), st));
     MICLOC_CUDA(cudaMemsetAsync(state, 0, (size_t)C * sizeof(float), st));
-    MICLOC_CUDA(cudaMemsetAsync(started, 0, sizeof(int32_t), st));
-    k_envelope<<<(C + 127) / 128, 128, 0, st>>>(x_dev, env_dev, state, started, T, C, 1.f / (float)wf, 1.f / (float)wr);
+    MICLOC_CUDA(cudaMemsetAsync(started, 0, (size_t)C * sizeof(int32_t), st));
+    k_envelope<<<(C + 127) / 128, 128, 0, st>>>(x_dev, env_dev, state, started, nullptr, 1, T, C, 1.f / (float)wf, 1.f / (float)wr);
     count_launch(1);
     if (argmax_dev) {
-        k_argmax_rows<<<(unsigned)((T * 32 + 255) / 256), 256, 0, st>>>(env_dev, argmax_dev, T, C);
+        k_argmax_rows<<<(unsigned)((T * 32 + 255) / 256), 256, 0, st>>>(env_dev, argmax_dev, nullptr, 1, T, C);
         count_launch(1);
     }
     MICLOC_CUDA(cudaGetLastError());

@@ -297,6 +297,98 @@ class SnnStream:
         return res
 
 
+class SnnStreamBatch:
+    """`num_streams` independent recordings ("slots") advanced together (micloc_snn_streams_*): one push hands every
+    slot one frame of the same length and runs a fixed number of kernels whatever the number of slots.  Each slot
+    behaves as an `SnnStream`; `reset` and `flush` act on a list of slots only, and a flushed slot ignores its rows of
+    later pushes (n_out = 0) until it is reset.  Frames are [num_streams, n, channels] device tensors, float32 / int16 /
+    int32 (channels beyond the microphones are dropped)."""
+
+    def __init__(self, engine: SnnEngine, num_streams: int, max_frame_len: int, fs: float = 48_000.0,
+                 rise_time: float = 10e-3, fall_time: float = 100e-3):
+        self.engine = engine
+        self._lib = engine._lib
+        self.num_streams = int(num_streams)
+        self.max_frame_len = int(max_frame_len)
+        h = C.c_void_p()
+        N.check(self._lib.micloc_snn_streams_create(engine._h, self.num_streams, self.max_frame_len, float(fs),
+                                                    float(rise_time), float(fall_time), C.byref(h)))
+        self._h = h
+        self.latency = int(self._lib.micloc_snn_streams_latency(h))
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.micloc_snn_streams_destroy(self._h)
+            self._h = None
+
+    __del__ = close
+
+    @staticmethod
+    def _slots(slots):
+        if slots is None:
+            return None, None, 0
+        arr = np.ascontiguousarray(np.atleast_1d(np.asarray(slots)), dtype=np.int32)
+        return arr, arr.ctypes.data_as(C.c_void_p), len(arr)
+
+    def reset(self, slots=None):
+        """Fresh state for the listed slots (None: all); they restart at sample 0."""
+        arr, p, n = self._slots(slots)
+        N.check(self._lib.micloc_snn_streams_reset(self._h, p, n, _stream_ptr(self.engine.device)))
+
+    def _outputs(self, rows, want_env):
+        e, S = self.engine, self.num_streams
+        dev = e.device
+        return {"spikes": torch.empty((S, rows, e.C2), dtype=torch.int8, device=dev),
+                "power": torch.empty((S, e.G), dtype=torch.float32, device=dev),
+                "doa": torch.empty(S, dtype=torch.int32, device=dev),
+                "env": torch.empty((S, rows, e.G), dtype=torch.float32, device=dev) if want_env else None,
+                "doa_t": torch.empty((S, rows), dtype=torch.int32, device=dev) if want_env else None}
+
+    def push(self, frames: torch.Tensor, want_env: bool = False) -> Dict[str, object]:
+        """One frame per slot in, the samples that became final out: dict(n_out numpy int64 [S], spikes [S, n + D, 2M],
+        power [S, G], doa [S], + env [S, n + D, G] and doa_t [S, n + D] when `want_env`).  Slot s fills its first
+        n_out[s] rows; the other rows, and power / doa of a slot with n_out[s] == 0, are left as allocated."""
+        e = self.engine
+        if frames.dim() != 3 or frames.shape[2] < e.M:
+            raise ValueError(
+                f"number of channels in the input siganl {frames.shape[-1]} should be the same as the number of microphones {e.M}!")
+        if frames.shape[0] != self.num_streams:
+            raise ValueError(f"frames hold {frames.shape[0]} slots, the batch has {self.num_streams}")
+        if frames.device != e.device:
+            raise ValueError(f"frame lives on {frames.device}, engine on {e.device}")
+        dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frames.dtype)
+        if dt is None:
+            raise ValueError(f"frame must be float32, int16 or int32, got {frames.dtype}")
+        frames = frames.contiguous()
+        n = frames.shape[1]
+        out = self._outputs(n + self.latency, want_env)
+        n_out = np.zeros(self.num_streams, dtype=np.int64)
+        N.check(self._lib.micloc_snn_streams_push(self._h, _ptr(frames), dt, n, frames.shape[2], _ptr(out["spikes"]),
+                                                  _ptr(out["power"]), _ptr(out["doa"]), _ptr(out["env"]),
+                                                  _ptr(out["doa_t"]), n_out.ctypes.data_as(C.c_void_p),
+                                                  _stream_ptr(e.device)))
+        out["n_out"] = n_out
+        if not want_env:
+            del out["env"], out["doa_t"]
+        return out
+
+    def flush(self, slots=None, want_env: bool = False) -> Dict[str, object]:
+        """End of the listed recordings (None: all): their remaining samples as in `push` (rows: max_frame_len +
+        latency) + 'flags' numpy int32 [S], bit 0 = RZCC overflow anywhere in that slot's recording."""
+        arr, p, ns = self._slots(slots)
+        out = self._outputs(self.max_frame_len + self.latency, want_env)
+        n_out = np.zeros(self.num_streams, dtype=np.int64)
+        flags = np.zeros(self.num_streams, dtype=np.int32)
+        N.check(self._lib.micloc_snn_streams_flush(self._h, p, ns, _ptr(out["spikes"]), _ptr(out["power"]),
+                                                   _ptr(out["doa"]), _ptr(out["env"]), _ptr(out["doa_t"]),
+                                                   n_out.ctypes.data_as(C.c_void_p), flags.ctypes.data_as(C.c_void_p),
+                                                   _stream_ptr(self.engine.device)))
+        out["n_out"], out["flags"] = n_out, flags
+        if not want_env:
+            del out["env"], out["doa_t"]
+        return out
+
+
 def envelope(x: torch.Tensor, fs: float, rise_time: float, fall_time: float, want_argmax: bool = False):
     """Envelope(rise_time, fall_time, fs).evolve on a device array [T, C] float32 (micloc/utils.py:15-81);
     with `want_argmax` also the per-row argmax (tests/test_snn_hilbert_localization.py:284-293)."""

@@ -150,6 +150,43 @@ int micloc_snn_stream_push(micloc_stream *s, const void *frame_dev, int dtype, i
                            int64_t *n_out, void *stream);
 int micloc_snn_stream_flush(micloc_stream *s, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev,
                             int32_t *doa_t_dev, int64_t *n_out, int32_t *flags_host, void *stream);
+
+/* ---- stream batches: many live recordings, one push per frame tick ---------------------------------------------- */
+/* A stream batch holds S independent slots on one context; each slot is one continuous recording with the semantics
+ * of a micloc_stream above (N pushed frames = one clip of their concatenation, causal in-phase delay, results lag the
+ * input by micloc_snn_streams_latency() = D samples).  A single micloc_stream is a batch of one slot.
+ *   - Slots are independent: reset and flush act on the listed slots only (slots_host [n_slots], NULL = every slot).
+ *     A flushed slot ignores its rows of later pushes (n_out = 0, state untouched) until it is reset, so one slot can be
+ *     recycled while the others keep running; a push after every slot was flushed is no error (all n_out = 0).
+ *   - Positions are per slot: a slot reset mid-run restarts at sample 0 while the others go on.  n_out_host[s] is the
+ *     number of samples of slot s that became final with this call (N_s - D - F_s for a push, the rest at a flush); the
+ *     library computes it on the host, without a device synchronisation.
+ *   - push: frames_dev [S][n][in_channels] float32 / int16 / int32 (one frame of n samples per slot, the same n for all
+ *     slots, 1 <= n <= max_frame_len; channels >= num_mic are dropped).  Outputs, all nullable device pointers:
+ *       spikes_dev [S][n + D][2M] int8, power_dev [S][G] (mean over the slot's final samples of y^2), doa_dev [S] (its
+ *       first argmax), env_dev [S][n + D][G] (Envelope continued across calls), doa_t_dev [S][n + D] (per-sample argmax
+ *       of the envelope).  Slot s fills its first n_out_host[s] rows; the other rows, and power / doa of a slot with
+ *       n_out = 0, are NOT written.
+ *   - flush closes the listed slots like a clip end; outputs as in push with [S][max_frame_len + D] rows;
+ *     flags_host [S] (nullable, host): bit 0 = RZCC overflow anywhere in that slot's recording (synchronises).
+ *   - reset / flush copy the slot list to the device and synchronise `stream`; a push does not synchronise.
+ * Kernel launches per push, whatever S: 5 (frame assembly, STHT, band-pass + RZCC + neuron, Gram, power), of which Gram
+ * and power only when power_dev or doa_dev is given; +2 (dense y, envelope) when env_dev or doa_t_dev is given, +1
+ * (argmax) when doa_t_dev is given.  The envelope scratch (S (n + D) G floats, twice when env_dev is NULL) is allocated
+ * on the first call that asks for it.  1 <= num_streams <= 65535.  Same lifetime rules as micloc_stream. */
+typedef struct micloc_stream_batch micloc_stream_batch;
+int micloc_snn_streams_create(micloc_snn *ctx, int32_t num_streams, int64_t max_frame_len, double fs,
+                              double rise_time, double fall_time, micloc_stream_batch **out);
+int micloc_snn_streams_destroy(micloc_stream_batch *sb);
+int micloc_snn_streams_latency(micloc_stream_batch *sb);
+int micloc_snn_streams_reset(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots, void *stream);
+int micloc_snn_streams_push(micloc_stream_batch *sb, const void *frames_dev, int dtype, int64_t n, int32_t in_channels,
+                            int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev, int32_t *doa_t_dev,
+                            int64_t *n_out_host, void *stream);
+int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots,
+                             int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev, int32_t *doa_t_dev,
+                             int64_t *n_out_host, int32_t *flags_host, void *stream);
+
 /* Envelope.evolve on a whole device array x_dev [T][C] float32 (fresh state) -> env_dev [T][C]; argmax_dev [T]
  * (nullable) = first argmax over the C channels of every row. */
 int micloc_envelope(const float *x_dev, int64_t T, int32_t C, double fs, double rise_time, double fall_time,
