@@ -78,7 +78,14 @@ SYMBOLS = {
     "micloc_snn_streams_reset": (C.c_int, [_vp, _vp, _i32, _vp]),
     "micloc_snn_streams_push": (C.c_int, [_vp, _vp, C.c_int, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "micloc_snn_streams_flush": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "micloc_envelope": (C.c_int, [_vp, _i64, _i32, C.c_double, C.c_double, C.c_double, _vp, _vp, C.c_int, _vp]),
+    "micloc_snn_mb_streams_create": (C.c_int, [C.POINTER(_vp), _i32, _i32, _dp, _dp, _i32, _i64, C.POINTER(_vp)]),
+    "micloc_snn_mb_streams_destroy": (C.c_int, [_vp]),
+    "micloc_snn_mb_streams_latency": (C.c_int, [_vp]),
+    "micloc_snn_mb_streams_reset": (C.c_int, [_vp, _vp, _i32, _vp]),
+    "micloc_snn_mb_streams_push": (C.c_int, [_vp, _vp, C.c_int, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                             _vp]),
+    "micloc_snn_mb_streams_flush": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "micloc_envelope":(C.c_int, [_vp, _i64, _i32, C.c_double, C.c_double, C.c_double, _vp, _vp, C.c_int, _vp]),
     "micloc_filterbank": (C.c_int, [_vp, C.c_int, _i64, _i64, _i32, _i32, _i32, _i32, _dp, _vp, _vp, C.c_int, _vp]),
     "micloc_power_fuse": (C.c_int, [_vp, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, _vp]),
     "micloc_synth_clips": (C.c_int, [C.POINTER(SynthConfig), _i64, _vp, _vp, _vp, _vp, _vp, C.c_uint64, _vp, _vp,

@@ -70,6 +70,18 @@ int micloc_snn_get_params(micloc_snn *ctx, micloc_snn_params *out);
 
 namespace micloc {
 int sos_to_f32(const double *sos, int nsec, float *out);
+// the float32 band-pass sections of a filterbank of F <= 8 bands (micloc_multiband.cu)
+struct FilterbankParams {
+    int F, nsec;
+    float sos[8][kMaxSections][5];
+};
+// checks F (1..8) and n_sections (1..kMaxSections), converts sos [F][n_sections][6] (host, float64)
+int filterbank_params(int32_t F, int32_t n_sections, const double *sos, FilterbankParams *out);
+// k_power_fuse over power [F][B][G]; rows_b (nullable): clip b with rows_b[b] == 0 is not written;
+// band_flags (nullable, F device pointers [B]): flags[b] = OR of their bit 0 before the estimator bit is added
+int launch_power_fuse(const float *power, int F, long long B, int G, const double *doa_list, float *power_sum,
+                      int32_t *doa, double *ml, double *trimmed, int32_t *flags, const int32_t *rows_b,
+                      const int32_t *const *band_flags, cudaStream_t st);
 int launch_stht_any(const ChainParams &p, const float *d_taps, const void *audio, int dtype, float *q,
                     long long B, long long T, cudaStream_t st);
 // time segments of the band-pass + RZCC kernel (k_chain_blk): segment s keeps samples [s*seg_len, (s+1)*seg_len) and

@@ -18,11 +18,6 @@
 
 namespace micloc {
 
-struct FilterbankParams {
-    int F, nsec;
-    float sos[8][kMaxSections][5];
-};
-
 template <typename T> __device__ __forceinline__ float fb_to_f32(T v) { return (float)v; }
 
 // one thread per (clip, microphone): reads its sample once, steps the F band-pass cascades, writes F rows.
@@ -53,22 +48,26 @@ k_filterbank(const IN_T *__restrict__ audio, float *__restrict__ out, double *__
 }
 
 struct FuseParams {
-    int F, G, want_ml;
+    int F, G;
+    const int32_t *band_flags[8];              // multi-band stream batches: each band's per-slot flags, or all null
 };
 
 // one CTA per clip: power_sum[g] = sum_f power[f][b][g] (bands added in order, float64 like the reference's
 // power_grid), first argmax, periodic ML = angle(mean(p e^{j doa})), trimmed periodic ML = the same over
 // arange(-G/2 // 2, G/2 // 2 + 1) - argmax with numpy's negative-index wrap (an index below -G is the reference's
-// IndexError: flags bit 1, estimate NaN)
+// IndexError: flags bit 1, estimate NaN).  rows_b (nullable, multi-band stream batches): a clip with rows_b[b] == 0
+// has no power rows and is not written.  With band_flags, flags[b] is first set to the OR of the bands' bit 0;
+// without, the caller zeroes flags.
 __global__ void __launch_bounds__(256)
 k_power_fuse(const float *__restrict__ power, const double *__restrict__ doa_list, float *__restrict__ power_sum,
              int32_t *__restrict__ doa, double *__restrict__ ml, double *__restrict__ trimmed, int32_t *__restrict__ flags,
-             const __grid_constant__ FuseParams fp, long long B) {
+             const int32_t *__restrict__ rows_b, const __grid_constant__ FuseParams fp, long long B) {
     extern __shared__ double s_p[];            // [G] summed pattern
     __shared__ double s_red[3][8];
     __shared__ int s_idx[8];
     __shared__ int s_arg;
     const long long b = blockIdx.x;
+    if (rows_b && rows_b[b] == 0) return;      // (uniform across the block: before any barrier)
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int G = fp.G;
     double best = -1.0; int bi = 0x7fffffff;
@@ -98,6 +97,11 @@ k_power_fuse(const float *__restrict__ power, const double *__restrict__ doa_lis
         }
         s_arg = bi;
         if (doa) doa[b] = bi;
+        if (flags && fp.band_flags[0]) {
+            int v = 0;
+            for (int f = 0; f < fp.F; ++f) v |= fp.band_flags[f][b] & 1;
+            flags[b] = v;
+        }
         if (ml && doa_list) ml[b] = atan2(im / G, re / G);
     }
     __syncthreads();
@@ -130,6 +134,30 @@ k_power_fuse(const float *__restrict__ power, const double *__restrict__ doa_lis
 
 }  // namespace micloc
 
+int micloc::filterbank_params(int32_t F, int32_t n_sections, const double *sos, FilterbankParams *out) {
+    if (F < 1 || F > 8) return set_error(MICLOC_ERR_CONFIG, "filterbank of %d bands (1..8 supported)", F);
+    if (n_sections < 1 || n_sections > kMaxSections) return set_error(MICLOC_ERR_CONFIG, "n_sections must be 1..%d", kMaxSections);
+    FilterbankParams fp{};
+    fp.F = F; fp.nsec = n_sections;
+    for (int f = 0; f < F; ++f) MICLOC_TRY(sos_to_f32(sos + (size_t)f * n_sections * 6, n_sections, &fp.sos[f][0][0]));
+    *out = fp;
+    return MICLOC_OK;
+}
+
+int micloc::launch_power_fuse(const float *power, int F, long long B, int G, const double *doa_list, float *power_sum,
+                              int32_t *doa, double *ml, double *trimmed, int32_t *flags, const int32_t *rows_b,
+                              const int32_t *const *band_flags, cudaStream_t st) {
+    FuseParams fp{};
+    fp.F = F; fp.G = G;
+    for (int f = 0; band_flags && f < F; ++f) fp.band_flags[f] = band_flags[f];
+    const size_t smem = (size_t)G * sizeof(double);
+    if (smem > 48 * 1024) MICLOC_CUDA(cudaFuncSetAttribute(k_power_fuse, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_power_fuse<<<(unsigned)B, 256, smem, st>>>(power, doa_list, power_sum, doa, ml, trimmed, flags, rows_b, fp, B);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    return MICLOC_OK;
+}
+
 using namespace micloc;
 
 extern "C" int micloc_filterbank(const void *audio_dev, int dtype, int64_t B, int64_t T, int32_t in_channels, int32_t M,
@@ -139,11 +167,8 @@ extern "C" int micloc_filterbank(const void *audio_dev, int dtype, int64_t B, in
     if (B < 1 || T < 1 || M < 1) return set_error(MICLOC_ERR_SHAPE, "empty batch");
     if (in_channels < M)
         return set_error(MICLOC_ERR_SHAPE, "number of channels in the input siganl %d should be the same as the number of microphones %d!", in_channels, M);
-    if (F < 1 || F > 8) return set_error(MICLOC_ERR_CONFIG, "filterbank of %d bands (1..8 supported)", F);
-    if (n_sections < 1 || n_sections > kMaxSections) return set_error(MICLOC_ERR_CONFIG, "n_sections must be 1..%d", kMaxSections);
-    FilterbankParams fp{};
-    fp.F = F; fp.nsec = n_sections;
-    for (int f = 0; f < F; ++f) MICLOC_TRY(sos_to_f32(sos + (size_t)f * n_sections * 6, n_sections, &fp.sos[f][0][0]));
+    FilterbankParams fp;
+    MICLOC_TRY(filterbank_params(F, n_sections, sos, &fp));
     MICLOC_CUDA(cudaSetDevice(device));
     cudaStream_t st = (cudaStream_t)stream;
     if (sumsq_dev) MICLOC_CUDA(cudaMemsetAsync(sumsq_dev, 0, (size_t)B * sizeof(double), st));
@@ -165,13 +190,7 @@ extern "C" int micloc_power_fuse(const float *power_dev, int32_t F, int64_t B, i
     if ((periodic_ml_dev || trimmed_ml_dev) && !doa_list_dev) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
     MICLOC_CUDA(cudaSetDevice(device));
     cudaStream_t st = (cudaStream_t)stream;
-    FuseParams fp{F, G, 0};
-    const size_t smem = (size_t)G * sizeof(double);
-    if (smem > 48 * 1024) MICLOC_CUDA(cudaFuncSetAttribute(k_power_fuse, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (flags_dev) MICLOC_CUDA(cudaMemsetAsync(flags_dev, 0, (size_t)B * sizeof(int32_t), st));
-    k_power_fuse<<<(unsigned)B, 256, smem, st>>>(power_dev, doa_list_dev, power_sum_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev,
-                                               flags_dev, fp, B);
-    count_launch(1);
-    MICLOC_CUDA(cudaGetLastError());
-    return MICLOC_OK;
+    return launch_power_fuse(power_dev, F, B, G, doa_list_dev, power_sum_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev,
+                             flags_dev, nullptr, nullptr, st);
 }

@@ -23,8 +23,18 @@
 //   k_stream_blk             band-pass + RZCC of the new samples, then the neuron filter of the final ones
 //   k_gram, k_power_argmax   power / DoA over each slot's final rows            (when power or doa is requested)
 //   k_dense, k_envelope, k_argmax_rows                                      (when env or doa_t is requested)
+//
+// A MULTI-BAND STREAM BATCH (micloc_snn_mb_streams_*) is the live localiser of micloc/localization_demo_snn.py:125-193
+// made continuous: a Butterworth filterbank on the raw frame, one chain per band, power summed over the bands.  It owns
+// one stream batch per band, created with a common latency D = max_f rzcc_lag(w_f) so that every band finalises the
+// same samples in a push, and replaces their frame assembly by one kernel that runs the filterbank with its state
+// carried across pushes and writes every band's [history | frame] rows (k_mb_stream_assemble).  Per push, whatever S:
+//   k_mb_stream_assemble                                                    1
+//   per band: STHT, k_stream_blk, k_gram, k_power_argmax (into band f's slice of [F][S][G])   4 F
+//   k_power_fuse       sum over bands, argmax, periodic-ML estimators over each slot's final rows   1
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "micloc_common.h"
@@ -60,6 +70,88 @@ k_stream_assemble(const IN_T *__restrict__ frames, const float *__restrict__ pre
     if (r < hist) v = pos[s].N > 0 ? prev[(s * (hist + n_prev) + n_prev + r) * M + m] : 0.f;
     else v = (float)frames[(s * n + (r - hist)) * in_ch + m];
     cur[i] = v;
+}
+
+// Multi-band frame assembly: one thread per (slot, microphone) steps the F band-pass cascades of the filterbank
+// (biquad_step with the float32 sections of k_filterbank, so band f's rows are micloc_filterbank's bits for the whole
+// recording) from its state in fb_state [F][S][M], and writes band f's [hist_f history rows | frame] buffer cur[f]
+// [S][hist_f + n][M] directly; history from the band's previous buffer prev[f] [S][hist_f + n_prev][M].  A slot at
+// N == 0 (new or reset) starts from zero filter state and zero history.  sumsq [S] (nullable, zeroed by the caller)
+// += sum of x^2 over the frame's kept channels, float32 partials of 256 samples added in float64 as in k_filterbank.
+struct MbAssembleParams {
+    FilterbankParams fb;
+    const float *prev[8];
+    float *cur[8];
+    int hist[8];
+};
+
+// NF = F is a template argument: the bands stay in registers, and the unrolled loop body stays small enough for the
+// instruction cache.  A predicated loop over 8 bands inside a 16-sample unroll did not (20 k instructions): 3.5 ms per
+// push at 1024 slots against 2.0 ms at 4096 slots in this form (F = 3, one B200).
+template <typename IN_T, int NF>
+__global__ void __launch_bounds__(128)
+k_mb_stream_assemble(const IN_T *__restrict__ frames, BiquadState *__restrict__ fb_state, double *__restrict__ sumsq,
+                     const SlotPos *__restrict__ pos, const __grid_constant__ MbAssembleParams ap, long long S, int n,
+                     int n_prev, int in_ch, int M) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= S * M) return;
+    const long long s = i / M;
+    const int m = (int)(i % M);
+    const bool fresh = pos[s].N == 0;
+    BiquadState st[NF];
+    float *row[NF];                       // band f's first frame row of this (slot, microphone)
+#pragma unroll
+    for (int f = 0; f < NF; ++f) {
+        if (fresh) biquad_reset(st[f]);
+        else st[f] = fb_state[f * S * M + i];
+        const int hist = ap.hist[f];
+        float *cur = ap.cur[f] + s * ((long long)hist + n) * M + m;
+        const float *prev = ap.prev[f] + (s * ((long long)hist + n_prev) + n_prev) * M + m;
+#pragma unroll 4
+        for (int r = 0; r < hist; ++r) cur[(long long)r * M] = fresh ? 0.f : prev[(long long)r * M];
+        row[f] = cur + (long long)hist * M;
+    }
+    // the frame in blocks of 8 samples, the next block's loads issued before the current one is filtered
+    constexpr int kBlk = 8;
+    const IN_T *src = frames + s * (long long)n * in_ch + m;
+    float nx[kBlk];
+    auto load = [&](int t0) {
+#pragma unroll
+        for (int u = 0; u < kBlk; ++u) nx[u] = t0 + u < n ? (float)src[(long long)(t0 + u) * in_ch] : 0.f;
+    };
+    double ss = 0.0;
+    float part = 0.f;
+    load(0);
+    for (int t0 = 0; t0 < n; t0 += kBlk) {
+        float x[kBlk];
+#pragma unroll
+        for (int u = 0; u < kBlk; ++u) x[u] = nx[u];
+        if (t0 + kBlk < n) load(t0 + kBlk);
+#pragma unroll
+        for (int u = 0; u < kBlk; ++u) {
+            const int t = t0 + u;
+            if (t < n) {
+                part = fmaf(x[u], x[u], part);
+                if ((t & 255) == 255) { ss += (double)part; part = 0.f; }
+#pragma unroll
+                for (int f = 0; f < NF; ++f) row[f][(long long)t * M] = biquad_step(ap.fb.sos[f], ap.fb.nsec, st[f], x[u]);
+            }
+        }
+    }
+    if (sumsq) atomicAdd(sumsq + s, ss + (double)part);
+#pragma unroll
+    for (int f = 0; f < NF; ++f) fb_state[f * S * M + i] = st[f];
+}
+
+template <typename IN_T>
+static void launch_mb_assemble(int F, unsigned grid, cudaStream_t st, const void *frames, BiquadState *fb_state,
+                               double *sumsq, const SlotPos *pos, const MbAssembleParams &ap, long long S, int n,
+                               int n_prev, int in_ch, int M) {
+    static decltype(&k_mb_stream_assemble<IN_T, 1>) const ks[8] = {
+        k_mb_stream_assemble<IN_T, 1>, k_mb_stream_assemble<IN_T, 2>, k_mb_stream_assemble<IN_T, 3>,
+        k_mb_stream_assemble<IN_T, 4>, k_mb_stream_assemble<IN_T, 5>, k_mb_stream_assemble<IN_T, 6>,
+        k_mb_stream_assemble<IN_T, 7>, k_mb_stream_assemble<IN_T, 8>};
+    ks[F - 1]<<<grid, 128, 0, st>>>((const IN_T *)frames, fb_state, sumsq, pos, ap, S, n, n_prev, in_ch, M);
 }
 
 // Band-pass + RZCC of the new samples [N, N + n) of every slot, then the neuron filter of the samples that became
@@ -368,8 +460,9 @@ extern "C" int micloc_snn_streams_reset(micloc_stream_batch *sb, const int32_t *
     return MICLOC_OK;
 }
 
-extern "C" int micloc_snn_streams_create(micloc_snn *ctx, int32_t num_streams, int64_t max_frame_len, double fs,
-                                         double rise_time, double fall_time, micloc_stream_batch **out) {
+// D_floor: the multi-band batch aligns its bands on one latency, D = max(rzcc_lag(w), D_floor) (ring and vmem follow)
+static int streams_create(micloc_snn *ctx, int32_t num_streams, int64_t max_frame_len, double fs, double rise_time,
+                          double fall_time, int D_floor, micloc_stream_batch **out) {
     if (!ctx || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
     *out = nullptr;
     if (num_streams < 1 || num_streams > 65535) return set_error(MICLOC_ERR_SHAPE, "num_streams %d out of range [1, 65535]", num_streams);
@@ -384,7 +477,7 @@ extern "C" int micloc_snn_streams_create(micloc_snn *ctx, int32_t num_streams, i
     micloc_stream_batch *sb = new micloc_stream_batch();
     sb->prm = prm; sb->device = prm.device; sb->S = num_streams; sb->max_frame = max_frame_len;
     sb->hist = p.K - 1;
-    sb->D = rzcc_lag(p.w);
+    sb->D = std::max(rzcc_lag(p.w), D_floor);
     const long long need = max_frame_len + sb->D + p.nL + 2 * kSeg;
     sb->ring_len = 32;
     while (sb->ring_len < need) sb->ring_len <<= 1;
@@ -413,6 +506,11 @@ extern "C" int micloc_snn_streams_create(micloc_snn *ctx, int32_t num_streams, i
     if (rc) { micloc_snn_streams_destroy(sb); return rc; }
     *out = sb;
     return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_streams_create(micloc_snn *ctx, int32_t num_streams, int64_t max_frame_len, double fs,
+                                         double rise_time, double fall_time, micloc_stream_batch **out) {
+    return streams_create(ctx, num_streams, max_frame_len, fs, rise_time, fall_time, 0, out);
 }
 
 extern "C" int micloc_snn_streams_latency(micloc_stream_batch *sb) { return sb ? sb->D : 0; }
@@ -470,10 +568,8 @@ static int launch_stream_blk(micloc_stream_batch *sb, const int32_t *close_sel, 
     return MICLOC_OK;
 }
 
-extern "C" int micloc_snn_streams_push(micloc_stream_batch *sb, const void *frames_dev, int dtype, int64_t n,
-                                       int32_t in_channels, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev,
-                                       float *env_dev, int32_t *doa_t_dev, int64_t *n_out_host, void *stream) {
-    if (!sb || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
+// the frame arguments of a push against the batch
+static int check_frames(const micloc_stream_batch *sb, int dtype, int64_t n, int32_t in_channels) {
     const ChainParams &p = sb->prm.chain;
     if (n < 1 || n > sb->max_frame) return set_error(MICLOC_ERR_SHAPE, "frame of %lld samples (stream takes 1..%lld)", (long long)n, sb->max_frame);
     if (in_channels < p.M)
@@ -483,6 +579,36 @@ extern "C" int micloc_snn_streams_push(micloc_stream_batch *sb, const void *fram
     for (long long s = 0; s < sb->S; ++s)
         if (sb->active[(size_t)s] && sb->N[(size_t)s] + n >= (1ll << 31) - 4096)
             return set_error(MICLOC_ERR_SHAPE, "stream position exceeds 2^31 samples: reset the stream");
+    return MICLOC_OK;
+}
+
+// everything of a push after the frame assembly, which left [history | frame] rows in sb->xbuf[sb->xcur]: STHT,
+// band-pass + RZCC + neuron, the slots' new positions (n_out_host, on the host), power / DoA / envelope
+static int streams_advance(micloc_stream_batch *sb, int64_t n, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev,
+                           float *env_dev, int32_t *doa_t_dev, int64_t *n_out_host, cudaStream_t st) {
+    const ChainParams &p = sb->prm.chain;
+    // STHT of the extended clips [history | frame]: rows >= hist see their whole window
+    MICLOC_TRY(launch_stht_any(p, (const float *)sb->prm.taps_dev, sb->xbuf[sb->xcur], MICLOC_F32, sb->q, sb->S, sb->hist + n, st));
+    const long long rows = n + sb->D;
+    MICLOC_TRY(launch_stream_blk(sb, nullptr, (int)n, (int)rows, spikes_dev, st));
+    for (long long s = 0; s < sb->S; ++s) {
+        const size_t i = (size_t)s;
+        n_out_host[s] = 0;
+        if (!sb->active[i]) continue;
+        sb->N[i] += n;
+        const long long f = sb->N[i] - sb->D > sb->F[i] ? sb->N[i] - sb->D : sb->F[i];
+        n_out_host[s] = f - sb->F[i];
+        sb->F[i] = f;
+    }
+    return streams_finalise(sb, rows, power_dev, doa_dev, env_dev, doa_t_dev, st);
+}
+
+extern "C" int micloc_snn_streams_push(micloc_stream_batch *sb, const void *frames_dev, int dtype, int64_t n,
+                                       int32_t in_channels, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev,
+                                       float *env_dev, int32_t *doa_t_dev, int64_t *n_out_host, void *stream) {
+    if (!sb || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
+    MICLOC_TRY(check_frames(sb, dtype, n, in_channels));
+    const ChainParams &p = sb->prm.chain;
     MICLOC_CUDA(cudaSetDevice(sb->device));
     cudaStream_t st = (cudaStream_t)stream;
     const int nxt = sb->xcur ^ 1;
@@ -500,20 +626,7 @@ extern "C" int micloc_snn_streams_push(micloc_stream_batch *sb, const void *fram
     MICLOC_CUDA(cudaGetLastError());
     sb->xcur = nxt;
     sb->n_prev = n;
-    // STHT of the extended clips [history | frame]: rows >= hist see their whole window
-    MICLOC_TRY(launch_stht_any(p, (const float *)sb->prm.taps_dev, sb->xbuf[nxt], MICLOC_F32, sb->q, sb->S, sb->hist + n, st));
-    const long long rows = n + sb->D;
-    MICLOC_TRY(launch_stream_blk(sb, nullptr, (int)n, (int)rows, spikes_dev, st));
-    for (long long s = 0; s < sb->S; ++s) {
-        const size_t i = (size_t)s;
-        n_out_host[s] = 0;
-        if (!sb->active[i]) continue;
-        sb->N[i] += n;
-        const long long f = sb->N[i] - sb->D > sb->F[i] ? sb->N[i] - sb->D : sb->F[i];
-        n_out_host[s] = f - sb->F[i];
-        sb->F[i] = f;
-    }
-    return streams_finalise(sb, rows, power_dev, doa_dev, env_dev, doa_t_dev, st);
+    return streams_advance(sb, n, spikes_dev, power_dev, doa_dev, env_dev, doa_t_dev, n_out_host, st);
 }
 
 extern "C" int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots,
@@ -539,6 +652,151 @@ extern "C" int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *
         MICLOC_CUDA(cudaStreamSynchronize(st));
     }
     return MICLOC_OK;
+}
+
+// ---- multi-band stream batches: F stream batches with one latency behind one filterbank ----
+struct micloc_mb_streams {
+    int F = 0, device = 0, M = 0, C2 = 0, G = 0, D = 0;
+    long long S = 0, max_frame = 0;
+    micloc_stream_batch *band[8] = {};
+    FilterbankParams fb{};
+    BiquadState *fb_state = nullptr;    // [F][S][M] filterbank state
+    double *doa_list = nullptr;         // [G] on the device, null: no ML estimators
+    float *power = nullptr;             // [F][S][G] per-band power when the caller passes no power_dev
+    std::vector<int32_t> flags_h;       // staging of a band's flags at a flush
+};
+
+extern "C" int micloc_snn_mb_streams_destroy(micloc_mb_streams *mb) {
+    if (!mb) return MICLOC_OK;
+    cudaSetDevice(mb->device);
+    for (int f = 0; f < mb->F; ++f) micloc_snn_streams_destroy(mb->band[f]);
+    cudaFree(mb->fb_state); cudaFree(mb->doa_list); cudaFree(mb->power);
+    delete mb;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_mb_streams_create(micloc_snn *const *ctxs, int32_t F, int32_t n_sections, const double *sos,
+                                            const double *doa_list, int32_t num_streams, int64_t max_frame_len,
+                                            micloc_mb_streams **out) {
+    if (!ctxs || !sos || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
+    *out = nullptr;
+    if (F < 1 || F > 8) return set_error(MICLOC_ERR_CONFIG, "multi-band stream batch of %d bands (1..8 supported)", F);
+    FilterbankParams fb;
+    MICLOC_TRY(filterbank_params(F, n_sections, sos, &fb));
+    micloc_snn_params prm[8];
+    int D = 0;
+    for (int f = 0; f < F; ++f) {
+        if (!ctxs[f]) return set_error(MICLOC_ERR_CONFIG, "null context of band %d", f);
+        MICLOC_TRY(micloc_snn_get_params(ctxs[f], &prm[f]));
+        if (prm[f].device != prm[0].device)
+            return set_error(MICLOC_ERR_CONFIG, "band %d's context is on device %d, band 0's on device %d", f, prm[f].device, prm[0].device);
+        if (prm[f].chain.M != prm[0].chain.M || prm[f].chain.G != prm[0].chain.G)
+            return set_error(MICLOC_ERR_SHAPE, "band %d's context has %d microphones and %d DoAs, band 0's %d and %d", f,
+                             prm[f].chain.M, prm[f].chain.G, prm[0].chain.M, prm[0].chain.G);
+        D = std::max(D, rzcc_lag(prm[f].chain.w));
+    }
+    MICLOC_CUDA(cudaSetDevice(prm[0].device));
+    micloc_mb_streams *mb = new micloc_mb_streams();
+    mb->device = prm[0].device; mb->M = prm[0].chain.M; mb->C2 = prm[0].chain.C2; mb->G = prm[0].chain.G; mb->D = D;
+    mb->S = num_streams; mb->max_frame = max_frame_len; mb->fb = fb;
+    for (int f = 0; f < F; ++f) {
+        const int rc = streams_create(ctxs[f], num_streams, max_frame_len, 48000.0, 10e-3, 100e-3, D, &mb->band[f]);
+        if (rc) { micloc_snn_mb_streams_destroy(mb); return rc; }
+        mb->F = f + 1;
+    }
+    const size_t S = (size_t)num_streams;
+    bool ok = cudaMalloc(&mb->fb_state, (size_t)F * S * mb->M * sizeof(BiquadState)) == cudaSuccess &&
+              cudaMalloc(&mb->power, (size_t)F * S * mb->G * sizeof(float)) == cudaSuccess &&
+              (!doa_list || cudaMalloc(&mb->doa_list, (size_t)mb->G * sizeof(double)) == cudaSuccess);
+    if (!ok) { micloc_snn_mb_streams_destroy(mb); return set_error(MICLOC_ERR_CUDA, "cudaMalloc(multi-band stream batch) failed"); }
+    if ((doa_list && cudaMemcpy(mb->doa_list, doa_list, (size_t)mb->G * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) ||
+        cudaMemset(mb->fb_state, 0, (size_t)F * S * mb->M * sizeof(BiquadState)) != cudaSuccess) {
+        micloc_snn_mb_streams_destroy(mb);
+        return set_error(MICLOC_ERR_CUDA, "multi-band stream batch set-up failed");
+    }
+    *out = mb;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_mb_streams_latency(micloc_mb_streams *mb) { return mb ? mb->D : 0; }
+
+// the filterbank state of a reset slot is dropped by k_mb_stream_assemble (it restarts at N == 0)
+extern "C" int micloc_snn_mb_streams_reset(micloc_mb_streams *mb, const int32_t *slots_host, int32_t n_slots, void *stream) {
+    if (!mb) return set_error(MICLOC_ERR_CONFIG, "null stream");
+    for (int f = 0; f < mb->F; ++f) MICLOC_TRY(micloc_snn_streams_reset(mb->band[f], slots_host, n_slots, stream));
+    return MICLOC_OK;
+}
+
+// sum over the bands + estimators over each slot's final rows (band 0's row counts: the same in every band)
+static int mb_fuse(micloc_mb_streams *mb, const float *power, float *power_grid_dev, int32_t *doa_dev, double *periodic_ml_dev,
+                   double *trimmed_ml_dev, int32_t *flags_dev, cudaStream_t st) {
+    const int32_t *band_flags[8];
+    for (int f = 0; f < mb->F; ++f) band_flags[f] = mb->band[f]->flags;
+    return launch_power_fuse(power, mb->F, mb->S, mb->G, mb->doa_list, power_grid_dev, doa_dev, periodic_ml_dev,
+                             trimmed_ml_dev, flags_dev, mb->band[0]->m, band_flags, st);
+}
+
+extern "C" int micloc_snn_mb_streams_push(micloc_mb_streams *mb, const void *frames_dev, int dtype, int64_t n,
+                                          int32_t in_channels, int8_t *spikes_dev, float *power_dev, float *power_grid_dev,
+                                          int32_t *doa_dev, double *periodic_ml_dev, double *trimmed_ml_dev,
+                                          double *sumsq_dev, int32_t *flags_dev, int64_t *n_out_host, void *stream) {
+    if (!mb || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
+    micloc_stream_batch *b0 = mb->band[0];
+    MICLOC_TRY(check_frames(b0, dtype, n, in_channels));        // (positions and shapes are the same in every band)
+    if ((periodic_ml_dev || trimmed_ml_dev) && !mb->doa_list) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
+    MICLOC_CUDA(cudaSetDevice(mb->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    MbAssembleParams ap{};
+    ap.fb = mb->fb;
+    for (int f = 0; f < mb->F; ++f) {
+        micloc_stream_batch *sb = mb->band[f];
+        ap.prev[f] = sb->xbuf[sb->xcur];
+        ap.cur[f] = sb->xbuf[sb->xcur ^ 1];
+        ap.hist[f] = sb->hist;
+    }
+    if (sumsq_dev) MICLOC_CUDA(cudaMemsetAsync(sumsq_dev, 0, (size_t)mb->S * sizeof(double), st));
+    const unsigned grid = (unsigned)((mb->S * mb->M + 127) / 128);
+    const SlotPos *pos = b0->pos[b0->pcur];
+    auto launch = dtype == MICLOC_F32 ? launch_mb_assemble<float> : dtype == MICLOC_I16 ? launch_mb_assemble<int16_t>
+                                                                                    : launch_mb_assemble<int32_t>;
+    launch(mb->F, grid, st, frames_dev, mb->fb_state, sumsq_dev, pos, ap, mb->S, (int)n, (int)b0->n_prev, in_channels, mb->M);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    const bool fuse = power_dev || power_grid_dev || doa_dev || periodic_ml_dev || trimmed_ml_dev || flags_dev;
+    float *power = power_dev ? power_dev : mb->power;
+    const long long rows = n + mb->D;
+    for (int f = 0; f < mb->F; ++f) {
+        micloc_stream_batch *sb = mb->band[f];
+        sb->xcur ^= 1;
+        sb->n_prev = n;
+        MICLOC_TRY(streams_advance(sb, n, spikes_dev ? spikes_dev + f * mb->S * rows * mb->C2 : nullptr,
+                                   fuse ? power + f * mb->S * mb->G : nullptr, nullptr, nullptr, nullptr, n_out_host, st));
+    }
+    if (!fuse) return MICLOC_OK;
+    return mb_fuse(mb, power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, st);
+}
+
+extern "C" int micloc_snn_mb_streams_flush(micloc_mb_streams *mb, const int32_t *slots_host, int32_t n_slots,
+                                           int8_t *spikes_dev, float *power_dev, float *power_grid_dev, int32_t *doa_dev,
+                                           double *periodic_ml_dev, double *trimmed_ml_dev, int32_t *flags_dev,
+                                           int64_t *n_out_host, int32_t *flags_host, void *stream) {
+    if (!mb || !n_out_host) return set_error(MICLOC_ERR_CONFIG, "null stream");
+    if ((periodic_ml_dev || trimmed_ml_dev) && !mb->doa_list) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
+    const bool fuse = power_dev || power_grid_dev || doa_dev || periodic_ml_dev || trimmed_ml_dev || flags_dev;
+    float *power = power_dev ? power_dev : mb->power;
+    const long long rows = mb->max_frame + mb->D;
+    if (flags_host) for (long long s = 0; s < mb->S; ++s) flags_host[s] = 0;
+    mb->flags_h.assign((size_t)mb->S, 0);
+    for (int f = 0; f < mb->F; ++f) {
+        MICLOC_TRY(micloc_snn_streams_flush(mb->band[f], slots_host, n_slots,
+                                            spikes_dev ? spikes_dev + f * mb->S * rows * mb->C2 : nullptr,
+                                            fuse ? power + f * mb->S * mb->G : nullptr, nullptr, nullptr, nullptr,
+                                            n_out_host, flags_host ? mb->flags_h.data() : nullptr, stream));
+        for (long long s = 0; flags_host && s < mb->S; ++s) flags_host[s] |= mb->flags_h[(size_t)s] & 1;
+    }
+    if (!fuse) return MICLOC_OK;
+    MICLOC_CUDA(cudaSetDevice(mb->device));
+    return mb_fuse(mb, power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, (cudaStream_t)stream);
 }
 
 // ---- the single stream: slot 0 of a one-slot batch ----

@@ -187,6 +187,54 @@ int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *slots_host,
                              int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev, int32_t *doa_t_dev,
                              int64_t *n_out_host, int32_t *flags_host, void *stream);
 
+/* ---- multi-band stream batches: the live localiser, continuous, over many arrays -------------------------------- */
+/* The multi-band localiser of micloc/localization_demo_snn.py:125-193 (filterbank, one chain per band, power summed
+ * over the bands, estimators) with the state carried across pushes.  A batch holds S independent slots over F contexts
+ * ctxs[F] (one per band, 1 <= F <= 8, same device, M and G) and the F band-pass filters of the filterbank
+ * (sos [F][n_sections][6], host; the sections of micloc_filterbank).
+ *   - Concatenation rule: N pushed frames give, for every band f, what micloc_filterbank of the concatenation followed
+ *     by band f's stream batch gives.  The filterbank state carries over, so band f's chain input is bit for bit the
+ *     filterbank output of the whole recording; the chain has the semantics of a stream batch slot.
+ *   - One latency for all bands: D = micloc_snn_mb_streams_latency() = max_f rzcc_lag(w_f).  Every band finalises
+ *     the same samples [F_s, N_s - D) of slot s in a push, and the rest at a flush, so n_out_host[s] is one number per
+ *     slot (computed on the host, no synchronisation).  A band with a smaller lag finalises later than it could; its
+ *     spikes are unchanged by that.
+ *   - push: frames_dev [S][n][in_channels] float32 / int16 / int32, as for micloc_snn_streams_push.  Outputs, all
+ *     nullable device pointers, over the n_out_host[s] final samples of slot s:
+ *       spikes_dev [F][S][n + D][2M] int8;  power_dev [F][S][G] float32 (per band, mean of y^2);  power_grid_dev [S][G]
+ *       float32 (sum over the bands in band order, float64, as micloc_power_fuse);  doa_dev [S] (first argmax);
+ *       periodic_ml_dev / trimmed_ml_dev [S] float64 (the estimators of micloc_power_fuse; they need doa_list);
+ *       flags_dev [S]: bit 0 = RZCC overflow so far in any band of the slot, bit 1 = the trimmed estimator's
+ *       IndexError case (estimate NaN).  A slot with n_out = 0 (a first push shorter than D, a flushed slot) gets none
+ *       of these written.
+ *       sumsq_dev [S] float64 = sum of x^2 over the kept channels of the frame just pushed, every slot (activity
+ *       detection, localization_demo_snn.py:151-163): float32 partials of 256 samples added in float64, so it equals
+ *       micloc_filterbank's sumsq of that frame up to the order in which the microphones are added.  The gate looks
+ *       at the newest frame, D samples ahead of the samples the power describes.
+ *   - flush closes the listed slots (slots_host [n_slots], NULL = every slot) like a clip end; outputs as in push with
+ *     [max_frame_len + D] rows; flags_host [S] (nullable, host): bit 0 = RZCC overflow anywhere in that slot's
+ *     recording, any band.  reset / flush / flushed slots behave as in micloc_snn_streams_*; reset also restarts the
+ *     filterbank of the listed slots from zero state.  reset and flush synchronise `stream`, a push does not.
+ * Kernel launches per push, whatever S: 4 F + 2 (filterbank + frame assembly; per band STHT, band-pass + RZCC +
+ * neuron, Gram, power; the sum over bands with its estimators), 2 F + 1 when no power, fused output or flags are
+ * requested.  1 <= num_streams <= 65535; doa_list [G] (host, nullable: no ML estimators).  The contexts' constants
+ * are used: destroy the batch before any of its contexts, re-create it after micloc_snn_set_bf. */
+typedef struct micloc_mb_streams micloc_mb_streams;
+int micloc_snn_mb_streams_create(micloc_snn *const *ctxs, int32_t F, int32_t n_sections, const double *sos,
+                                 const double *doa_list, int32_t num_streams, int64_t max_frame_len,
+                                 micloc_mb_streams **out);
+int micloc_snn_mb_streams_destroy(micloc_mb_streams *mb);
+int micloc_snn_mb_streams_latency(micloc_mb_streams *mb);
+int micloc_snn_mb_streams_reset(micloc_mb_streams *mb, const int32_t *slots_host, int32_t n_slots, void *stream);
+int micloc_snn_mb_streams_push(micloc_mb_streams *mb, const void *frames_dev, int dtype, int64_t n, int32_t in_channels,
+                               int8_t *spikes_dev, float *power_dev, float *power_grid_dev, int32_t *doa_dev,
+                               double *periodic_ml_dev, double *trimmed_ml_dev, double *sumsq_dev, int32_t *flags_dev,
+                               int64_t *n_out_host, void *stream);
+int micloc_snn_mb_streams_flush(micloc_mb_streams *mb, const int32_t *slots_host, int32_t n_slots, int8_t *spikes_dev,
+                                float *power_dev, float *power_grid_dev, int32_t *doa_dev, double *periodic_ml_dev,
+                                double *trimmed_ml_dev, int32_t *flags_dev, int64_t *n_out_host, int32_t *flags_host,
+                                void *stream);
+
 /* Envelope.evolve on a whole device array x_dev [T][C] float32 (fresh state) -> env_dev [T][C]; argmax_dev [T]
  * (nullable) = first argmax over the C channels of every row. */
 int micloc_envelope(const float *x_dev, int64_t T, int32_t C, double fs, double rise_time, double fall_time,
