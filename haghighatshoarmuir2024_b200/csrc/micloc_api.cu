@@ -430,8 +430,6 @@ static int run_power(micloc_snn *c, const float *vmem, long long B, long long T,
         k_gram<<<gg, 256, 0, st>>>(vmem, (double *)c->gram.ptr, p.C2, T, 0);
         count_launch(1);
     }
-    const size_t smem = (size_t)p.C2 * p.C2 * sizeof(double);
-    MICLOC_CUDA(cudaFuncSetAttribute(k_power_argmax, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // few clips: slices of the DoA grid on separate CTAs (one CTA per clip would run G x C2^2 float64 FMAs on one SM)
     int nchunk = 1;
     if (B < c->sm_count && (long long)p.G * p.C2 * p.C2 >= (1ll << 20)) {
@@ -446,15 +444,32 @@ static int run_power(micloc_snn *c, const float *vmem, long long B, long long T,
         cv = (double *)c->chunkbuf.ptr;
         ci = (int *)(cv + (size_t)B * nchunk);
     }
-    const size_t smem_w = smem + ((size_t)p.C2 * 32 + (size_t)kPwSlices * 32) * sizeof(double);
-    if (p.C2 >= 32 && smem_w <= 200 * 1024 && !getenv("MICLOC_POWER_NARROW")) {
+    return launch_power((const double *)c->gram.ptr, c->d_Wd, power, doa, p.C2, p.G, B, 1.0 / (double)T, nullptr, nchunk,
+                        cv, ci, st);
+}
+
+int micloc::launch_power(const double *gram, const double *Wd, float *power, int32_t *doa, int C2, int G, long long B,
+                         double inv_T, const int32_t *rows_b, int nchunk, double *cv, int *ci, cudaStream_t st) {
+    const size_t smem = (size_t)C2 * C2 * sizeof(double);
+    const size_t smem_w = smem + ((size_t)C2 * 32 + (size_t)kPwSlices * 32) * sizeof(double);
+    const dim3 grid((unsigned)B, (unsigned)nchunk);
+    if (!rows_b && C2 >= 32 && smem_w <= 200 * 1024 && !getenv("MICLOC_POWER_NARROW")) {
         // wide arrays: a warp per slice of Gram rows x 32 DoAs (one thread per DoA leaves most of the CTA idle)
         MICLOC_CUDA(cudaFuncSetAttribute(k_power_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));
-        k_power_wide<<<dim3((unsigned)B, (unsigned)nchunk), 32 * kPwSlices, smem_w, st>>>((const double *)c->gram.ptr, c->d_Wd, power, doa,
-                                                                                          p.C2, p.G, 1.0 / (double)T, nchunk, cv, ci);
+        k_power_wide<<<grid, 32 * kPwSlices, smem_w, st>>>(gram, Wd, power, doa, C2, G, inv_T, nchunk, cv, ci);
     } else {
-        k_power_argmax<<<dim3((unsigned)B, (unsigned)nchunk), 256, smem, st>>>((const double *)c->gram.ptr, c->d_Wd, power, doa, p.C2, p.G,
-                                                                              1.0 / (double)T, nchunk, cv, ci);
+        // the Gram matrix in shared memory while it fits next to the kernel's static reduction scratch
+        int dev = 0, optin = 0;
+        cudaFuncAttributes fa{};
+        MICLOC_CUDA(cudaGetDevice(&dev));
+        MICLOC_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+        MICLOC_CUDA(cudaFuncGetAttributes(&fa, k_power_argmax<true>));
+        if (smem + fa.sharedSizeBytes <= (size_t)optin) {
+            MICLOC_CUDA(cudaFuncSetAttribute(k_power_argmax<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            k_power_argmax<true><<<grid, 256, smem, st>>>(gram, Wd, power, doa, C2, G, inv_T, nchunk, cv, ci, rows_b);
+        } else {
+            k_power_argmax<false><<<grid, 256, 0, st>>>(gram, Wd, power, doa, C2, G, inv_T, nchunk, cv, ci, rows_b);
+        }
     }
     count_launch(1);
     if (nchunk > 1 && doa) {

@@ -82,6 +82,16 @@ int filterbank_params(int32_t F, int32_t n_sections, const double *sos, Filterba
 int launch_power_fuse(const float *power, int F, long long B, int G, const double *doa_list, float *power_sum,
                       int32_t *doa, double *ml, double *trimmed, int32_t *flags, const int32_t *rows_b,
                       const int32_t *const *band_flags, cudaStream_t st);
+// power[b][g] = w_g^T gram_b w_g * inv_T (float64, stored as float32) and doa[b] = first argmax over g, for gram
+// [B][C2][C2] float64.  The one place that picks the power kernel (micloc_snn_run_taps and the stream batches):
+//   k_power_wide               C2 >= 32 and Gram + steering tile in <= 200 KB of shared memory (M <= 72), unless
+//                              MICLOC_POWER_NARROW or rows_b
+//   k_power_argmax<true>       otherwise while the Gram matrix fits the block's shared memory (M <= 84 on sm_100)
+//   k_power_argmax<false>      beyond: Gram rows read from global memory
+// rows_b (nullable): clip b averages over rows_b[b] rows (inv_T unused), a clip with no rows is not written.
+// nchunk > 1: DoA slices on separate CTAs into cv / ci [B][nchunk], k_argmax_chunks then writes doa.
+int launch_power(const double *gram, const double *Wd, float *power, int32_t *doa, int C2, int G, long long B,
+                 double inv_T, const int32_t *rows_b, int nchunk, double *cv, int *ci, cudaStream_t st);
 int launch_stht_any(const ChainParams &p, const float *d_taps, const void *audio, int dtype, float *q,
                     long long B, long long T, cudaStream_t st);
 // time segments of the band-pass + RZCC kernel (k_chain_blk): segment s keeps samples [s*seg_len, (s+1)*seg_len) and

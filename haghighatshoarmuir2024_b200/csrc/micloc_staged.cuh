@@ -775,16 +775,19 @@ k_gram_reduce(const double *__restrict__ part, double *__restrict__ gram, int C2
 
 // ---------------------------------------------------------------------------
 // S4b: power[b][g] = w_g^T C_b w_g / T (float64), doa[b] = first argmax.
-// One block per clip; dynamic smem: C2*C2 doubles + reduction scratch.
+// One block per clip; dynamic smem: C2*C2 doubles (kSmemGram) + reduction scratch.  Without kSmemGram the Gram rows are
+// read from global memory (C2 > 168: C2^2 doubles exceed the shared memory of a block; all threads read the same
+// element, so each load is one broadcast from L1 / L2).
 // rows_b (nullable, stream batches): clip b averages over rows_b[b] samples instead of 1/inv_T, and a clip with no
 // rows is not written.
 // ---------------------------------------------------------------------------
+template <bool kSmemGram>
 static __global__ void __launch_bounds__(256)
 k_power_argmax(const double *__restrict__ gram, const double *__restrict__ Wd, float *__restrict__ power,
                int32_t *__restrict__ doa, int C2, int G, double inv_T, int nchunk, double *__restrict__ chunk_v,
                int *__restrict__ chunk_i, const int32_t *__restrict__ rows_b = nullptr) {
     extern __shared__ __align__(16) double sm_d[];
-    double *Cs = sm_d;
+    const double *Cs = kSmemGram ? sm_d : gram + blockIdx.x * (long long)C2 * C2;
     __shared__ double red_v[256];
     __shared__ int red_i[256];
     const long long b = blockIdx.x;
@@ -795,8 +798,10 @@ k_power_argmax(const double *__restrict__ gram, const double *__restrict__ Wd, f
     // few clips and a wide array (BASELINE config 5): blockIdx.y takes a slice of the DoA grid, k_argmax_chunks finishes
     const int gper = (G + nchunk - 1) / nchunk;
     const int g_lo = blockIdx.y * gper, g_hi = min(G, g_lo + gper);
-    for (int e = threadIdx.x; e < C2 * C2; e += blockDim.x) Cs[e] = gram[b * C2 * C2 + e];
-    __syncthreads();
+    if (kSmemGram) {
+        for (int e = threadIdx.x; e < C2 * C2; e += blockDim.x) sm_d[e] = gram[b * C2 * C2 + e];
+        __syncthreads();
+    }
     double best = -1.0; int besti = 0x7fffffff;
     for (int g = g_lo + threadIdx.x; g < g_hi; g += blockDim.x) {
         double acc = 0.0;

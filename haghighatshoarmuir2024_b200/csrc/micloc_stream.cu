@@ -524,11 +524,9 @@ static int streams_finalise(micloc_stream_batch *sb, long long rows, float *powe
     if (power_dev || doa_dev) {
         dim3 gg((unsigned)S, (unsigned)((p.C2 * p.C2 + 255) / 256));
         k_gram<<<gg, 256, 0, st>>>(sb->vmem, sb->gram, p.C2, rows, 0, sb->m);
-        const size_t smem = (size_t)p.C2 * p.C2 * sizeof(double);
-        MICLOC_CUDA(cudaFuncSetAttribute(k_power_argmax, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_power_argmax<<<(unsigned)S, 256, smem, st>>>(sb->gram, (const double *)sb->prm.bf_f64_dev, power_dev, doa_dev, p.C2,
-                                                       p.G, 1.0, 1, nullptr, nullptr, sb->m);
-        count_launch(2);
+        count_launch(1);
+        MICLOC_TRY(launch_power(sb->gram, (const double *)sb->prm.bf_f64_dev, power_dev, doa_dev, p.C2, p.G, S, 1.0, sb->m,
+                                1, nullptr, nullptr, st));
     }
     if (env_dev || doa_t_dev) {
         const size_t bytes = (size_t)S * rows * p.G * sizeof(float);
