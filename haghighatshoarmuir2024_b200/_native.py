@@ -104,7 +104,6 @@ SYMBOLS = {
     "micloc_snn_debug_counters": (C.c_int, [_vp, C.POINTER(C.c_uint64)]),
     "micloc_snn_debug_cta_times": (C.c_int, [_vp, C.POINTER(C.c_uint64), _i32]),
     "micloc_fp32_peak": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double)]),
-    "micloc_sched_probe": (C.c_int, [C.c_int, C.POINTER(_i32), C.c_int, C.POINTER(C.c_uint64)]),
 }
 
 _lib = None

@@ -34,7 +34,7 @@
 // One CTA of sixteen warps per SM holds two such groups (own barrier, own shared memory, own clip pairs): one
 // FIR warp of each group per SM sub-partition.  What bounds the kernel is the issue port of the sub-partitions:
 // an FFMA2 with three register operands issues every ~2.6 cycles, and every instruction of a serial role displaces
-// FIR work (tools/sched_probe.py, DESIGN.md 4.1).  micloc_fused_tc.cu (the default) runs the FIR on the tensor cores instead.
+// FIR work (a scheduler micro-benchmark, DESIGN.md 4.1).  micloc_fused_tc.cu (the default) runs the FIR on the tensor cores instead.
 #include <cstdlib>
 
 #include "micloc_fused_common.cuh"
@@ -52,9 +52,7 @@ struct FusedGeom {
     int nblk;        // FIR tap blocks of 8 (multiple of 6: two halves walked in groups of three)
     int dtile;       // the neuron warp runs dtile tiles behind the pipeline step (RZCC decision latency)
     int tiles_is;    // tiles whose in-phase input comes from the clip tail (t < K/2)
-    int fir_blocks;  // debug (MICLOC_FUSED_FIRBLOCKS): tap blocks each FIR warp really computes (0 = all; results are garbage)
     int perm;        // serial roles of group 1 on sub-partitions 0..3, two bits each (see k_fused)
-    int skip;        // debug (MICLOC_FUSED_SKIP): bit r set = role r only attends the tile barriers (results are garbage)
     int off_x, off_q, off_vm, off_is, off_cs, off_seg, off_clus, off_bits, off_stage, off_qa;   // byte offsets in dynamic smem
     int smem_bytes;
 };
@@ -79,8 +77,8 @@ __device__ __forceinline__ void load_taps(Taps8 &t, const float *__restrict__ ta
 // Written window-major (the window pair is shared by consecutive multiply-adds).  ptxas schedules the 64 FFMA2 of a
 // block in its own order whatever the source says (`volatile` does not pin it); the sequence it emits for this
 // source measured fastest of five source forms (FIR warps alone 290 k clips/s; tap-major 278 k, accumulator-major
-// 283 k, older chunk first 285-291 k; whole kernel 171.8-174.1 k).  tools/sched_probe.py (roles 9, 12-14): between 2.4 and 5.2 cycles per FFMA2 and sub-partition
-// depending on the sequence.
+// 283 k, older chunk first 285-291 k; whole kernel 171.8-174.1 k).  A scheduler micro-benchmark of the FIR's operand
+// patterns measured between 2.4 and 5.2 cycles per FFMA2 and sub-partition depending on the sequence.
 __device__ __forceinline__ void ffma2_ordered(unsigned long long &acc, unsigned long long w, unsigned long long g2) {
     asm volatile("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc) : "l"(w), "l"(g2));
 }
@@ -175,13 +173,8 @@ __device__ __forceinline__ void fir_role(const FusedSmem &sm, const ChainParams 
                 const float *tp = sm.taps + 8 * half * nb2;
                 Taps8 t0, t1;
                 load_taps(t0, tp);
-#ifdef MICLOC_DEBUG_SWITCHES
-                const int nb_run = g.fir_blocks ? g.fir_blocks : nb2;
-#else
-                const int nb_run = nb2;
-#endif
 #pragma unroll 1
-                for (int jb = 0; jb < nb_run; jb += 3) {
+                for (int jb = 0; jb < nb2; jb += 3) {
                     load_chunk(Cq, row, cn); cn -= 16; if (cn < 0) cn += g.ring_x;
                     load_taps(t1, tp + 8);
                     fir_block(acc, A, Bq, t0);
@@ -415,7 +408,7 @@ k_fused(const IN_T *__restrict__ audio, const float *__restrict__ taps, const do
     } else {
         // warps 0..3: FIR of group 0, 4..7: FIR of group 1 (one per sub-partition each); warps 8..11 / 12..15:
         // band-pass, RZCC, neuron, Gram of group 0 / 1; group 1's order (g.perm) decides which roles share a
-        // sub-partition (default: band-pass + Gram, RZCC + neuron)
+        // sub-partition (band-pass + Gram, RZCC + neuron)
         if (warp < 2 * kFirWarps) {
             group = warp >> 2;
             role = warp & 3;
@@ -482,11 +475,6 @@ k_fused(const IN_T *__restrict__ audio, const float *__restrict__ taps, const do
         }
         group_sync();
 
-#ifdef MICLOC_DEBUG_SWITCHES
-        if ((g.skip >> role) & 1) {
-            for (int k = -1; k <= k_last; ++k) tile_barrier(bar_id);
-        } else
-#endif
         if (role < kFirWarps)
             fir_role<IN_T, MM>(sm, p, g, audio, clip0 + (role >> 1), clip0 + (role >> 1) < B, T, role >> 1, role & 1, lane,
                                NT, k_last);
@@ -608,18 +596,9 @@ int launch_fused(const ChainParams &p, const float *d_taps, const double *d_Wd, 
                          "fused kernel covers Hilbert-type STHT kernels (every other tap zero), a 2-section band-pass "
                          "and up to %d microphones; use the staged path", kRows);
     FusedGeom g{};
-#ifdef MICLOC_DEBUG_SWITCHES   // role ablation (tools/build_rt.sh builds only): these make the results garbage
-    if (const char *e = getenv("MICLOC_FUSED_SKIP")) g.skip = (int)strtol(e, nullptr, 0);
-    if (const char *e = getenv("MICLOC_FUSED_FIRBLOCKS")) g.fir_blocks = (int)strtol(e, nullptr, 0);
-#endif
-    {
-        // group 0 runs band-pass, RZCC, neuron, Gram on sub-partitions 0..3; group 1's order decides which roles share one
-        static const int perms[3][4] = {{3, 2, 1, 0}, {2, 3, 0, 1}, {1, 0, 3, 2}};
-        int layout = 0;
-        if (const char *e = getenv("MICLOC_FUSED_LAYOUT")) layout = atoi(e);
-        if (layout < 0 || layout > 2) layout = 0;
-        g.perm = perms[layout][0] | perms[layout][1] << 2 | perms[layout][2] << 4 | perms[layout][3] << 6;
-    }
+    // group 0 runs band-pass, RZCC, neuron, Gram on sub-partitions 0..3; group 1's order decides which roles share one.
+    // The reverse order (band-pass + Gram, RZCC + neuron) measured fastest of the three pairings.
+    g.perm = 3 | 2 << 2 | 1 << 4 | 0 << 6;
     // FIR tap blocks of 8, two halves walked in groups of three (zero taps appended up to a multiple of 48)
     g.nblk = (p.n_taps / 8 + 5) / 6 * 6;
     const int lookback = p.tap_first + 14 + 16 * (g.nblk - 1);      // oldest sample a tile's FIR windows load
@@ -653,9 +632,8 @@ int launch_fused(const ChainParams &p, const float *d_taps, const double *d_Wd, 
         return set_error(MICLOC_ERR_UNSUPPORTED, "fused kernel needs %d B of shared memory; use the staged path", g.smem_bytes);
     if (T + 16 * kTile >= (1ll << 31)) return set_error(MICLOC_ERR_SHAPE, "T too large for the fused kernel");
     // one CTA of two clip-pair groups per SM when both fit its shared memory (the usual case), else the
-    // single-group CTA twice per SM; MICLOC_FUSED_GROUPS=1 forces the latter (A/B measurements)
-    int groups = 2 * g.smem_bytes <= 227 * 1024 ? 2 : 1;
-    if (const char *e = getenv("MICLOC_FUSED_GROUPS")) { if (atoi(e) == 1) groups = 1; }
+    // single-group CTA twice per SM
+    const int groups = 2 * g.smem_bytes <= 227 * 1024 ? 2 : 1;
 #define MICLOC_FUSED_CASE(IN, MMV)                                                                                \
     do {                                                                                                          \
         if (groups == 2)                                                                                          \

@@ -36,7 +36,6 @@
 // next clip pair's largest magnitude, warp 3 issues the MMAs through one elected lane).  The same role of both groups
 // sits on the same SM sub-partition (warp id mod 4): a sub-partition then runs ~20 KB of code (one serial role + the
 // front end), which is what its instruction cache holds -- other pairings measured 3-7 % slower.
-#include <cstdlib>
 
 #include "micloc_fused_common.cuh"
 
@@ -880,7 +879,6 @@ int launch_fused(const ChainParams &p, const float *d_taps, const double *d_Wd, 
     if (!tc::fused_supported(p)) return set_error(MICLOC_ERR_UNSUPPORTED, "tensor-core fused kernel: unsupported chain geometry");
     TcGeom g;
     int groups = 2;
-    if (const char *e = getenv("MICLOC_FUSED_GROUPS")) { if (atoi(e) == 1) groups = 1; }
     make_geom(p, dtype, groups, g);
     if (groups == 2 && g.smem_bytes > 227 * 1024) { groups = 1; make_geom(p, dtype, groups, g); }
     if (g.smem_bytes > 227 * 1024)

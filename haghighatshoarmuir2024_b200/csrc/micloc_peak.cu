@@ -67,378 +67,12 @@ k_peak_dfma(float *out, int iters, double a, double b) {
     if (s == 123.456) out[0] = (float)s;
 }
 
-// variant 3: FFMA2 and DFMA streams side by side in every warp (do the two pipes overlap?)
-__global__ void __launch_bounds__(256)
-k_peak_mixed(float *out, int iters, float a, float b, double da, double db) {
-    unsigned long long acc[8], av, bv;
-    asm("mov.b64 %0, {%1, %1};" : "=l"(av) : "f"(a));
-    asm("mov.b64 %0, {%1, %1};" : "=l"(bv) : "f"(b));
-    double dacc[4];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const float lo = (float)(threadIdx.x + i), hi = lo + 0.5f;
-        asm("mov.b64 %0, {%1, %2};" : "=l"(acc[i]) : "f"(lo), "f"(hi));
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) dacc[i] = (double)(threadIdx.x + i);
-    for (int it = 0; it < iters; ++it) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            asm volatile("fma.rn.f32x2 %0, %0, %1, %2;" : "+l"(acc[i]) : "l"(av), "l"(bv));
-            if ((i & 1) == 0) dacc[i >> 1] = fma(dacc[i >> 1], da, db);
-        }
-    }
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        float lo, hi;
-        asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(acc[i]));
-        s += lo + hi;
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) s += (float)dacc[i];
-    if (s == 123.456f) out[0] = s;
-}
-
-
-// ---------------------------------------------------------------------------
-// Scheduler probe (diagnostics for the warp-specialised fused kernel): one CTA of up to 16 warps per SM,
-// every warp runs one instruction stream chosen by roles[warp] for iters x 1000 cycles (all warps run side
-// by side for the whole measurement) and reports its clock64 cycles and the instructions it got through.  Hardware warp slot w belongs to SM sub-partition w % 4.
-//   0 idle   1 FFMA2 stream (8 independent accumulators)   2 dependent scalar FFMA chain
-//   3 independent ALU stream (8 chains of LOP3/IADD3)       4 independent scalar FFMA stream (16 accumulators)
-//   5 dependent chain alternating FFMA and ALU               6 FFMA2 stream, 64 per round then 8 ALU ops
-//   7 dependent DFMA chain                                    8 independent DFMA stream (8 accumulators)
-//   9 / 11 FFMA2 with the FIR operand pattern (all operands in non-uniform registers; tap scalar / tap pair)
-//   10 scalar FFMA with the FIR operand pattern
-//   12 / 13 FIR pattern with the taps in kernel parameters (uniform registers), tap-major / window-major order
-//   14 FIR pattern, window-major order, taps in registers
-//   15 independent mma.sync m16n8k16 f16 stream (legacy tensor-core path)
-// out[warp] = cycles of CTA 0's warp, out[16 + warp] = instructions of the measured kind it issued.
-// ---------------------------------------------------------------------------
-struct ProbeTaps { float t[64]; };
-
-__global__ void __launch_bounds__(512, 1)
-k_sched_probe(const int *__restrict__ roles, int iters, float a, float b, unsigned long long *out, float *sink,
-              const __grid_constant__ ProbeTaps ptaps) {
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int role = roles[warp];
-    __syncthreads();
-    long long t0, t1;
-    unsigned long long n_inst = 0;
-    float res = 0.f;
-    int rounds_done = 0;
-    auto probe_running = [&](long long start, int kcyc, int it) {
-        long long now;
-        asm volatile("mov.u64 %0, %%clock64;" : "=l"(now));
-        rounds_done = it;
-        return now - start < 1000ll * kcyc;
-    };
-    asm volatile("mov.u64 %0, %%clock64;" : "=l"(t0));
-    if (role == 1 || role == 6) {
-        unsigned long long acc[8], av, bv;
-        asm("mov.b64 %0, {%1, %1};" : "=l"(av) : "f"(a));
-        asm("mov.b64 %0, {%1, %1};" : "=l"(bv) : "f"(b));
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const float lo = (float)(threadIdx.x + i), hi = lo + 0.5f;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(acc[i]) : "f"(lo), "f"(hi));
-        }
-        unsigned int x = threadIdx.x;
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int r = 0; r < 8; ++r)
-#pragma unroll
-                for (int i = 0; i < 8; ++i)
-                    asm volatile("fma.rn.f32x2 %0, %0, %1, %2;" : "+l"(acc[i]) : "l"(av), "l"(bv));
-            if (role == 6) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) asm volatile("lop3.b32 %0, %0, %1, %2, 0x96;" : "+r"(x) : "r"(it), "r"(i));
-            }
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            float lo, hi;
-            asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(acc[i]));
-            res += lo + hi;
-        }
-        res += (float)x;
-    } else if (role == 2) {
-        float x = (float)threadIdx.x;
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int i = 0; i < 64; ++i) asm volatile("fma.rn.f32 %0, %0, %1, %2;" : "+f"(x) : "f"(a), "f"(b));
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-        res = x;
-    } else if (role == 3) {
-        unsigned int x[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) x[i] = threadIdx.x + i;
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int r = 0; r < 8; ++r)
-#pragma unroll
-                for (int i = 0; i < 8; ++i) asm volatile("lop3.b32 %0, %0, %1, %2, 0x96;" : "+r"(x[i]) : "r"(it), "r"(r));
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) res += (float)x[i];
-    } else if (role == 4) {
-        float acc[16];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) acc[i] = (float)(threadIdx.x + i);
-        const float ar = a + (float)lane * 1e-9f, br = b + (float)lane * 1e-9f;   // register operands, not constants
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int r = 0; r < 4; ++r)
-#pragma unroll
-                for (int i = 0; i < 16; ++i) asm volatile("fma.rn.f32 %0, %0, %1, %2;" : "+f"(acc[i]) : "f"(ar), "f"(br));
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) res += acc[i];
-    } else if (role == 5) {
-        float x = (float)threadIdx.x;
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) {
-                asm volatile("fma.rn.f32 %0, %0, %1, %2;" : "+f"(x) : "f"(a), "f"(b));
-                unsigned int u = __float_as_uint(x);
-                asm volatile("lop3.b32 %0, %0, %1, %2, 0x96;" : "+r"(u) : "r"(it), "r"(i));
-                x = __uint_as_float(u);
-            }
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-        res = x;
-    }
-    else if (role == 7) {
-        double x = (double)threadIdx.x;
-        const double da = (double)a, db = (double)b;
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int i = 0; i < 64; ++i) asm volatile("fma.rn.f64 %0, %0, %1, %2;" : "+d"(x) : "d"(da), "d"(db));
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-        res = (float)x;
-    } else if (role == 8) {
-        double acc[8];
-        const double da = (double)a, db = (double)b;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) acc[i] = (double)(threadIdx.x + i);
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int r = 0; r < 8; ++r)
-#pragma unroll
-                for (int i = 0; i < 8; ++i) asm volatile("fma.rn.f64 %0, %0, %1, %2;" : "+d"(acc[i]) : "d"(da), "d"(db));
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) res += (float)acc[i];
-    }
-    else if (role == 9 || role == 11) {
-        // the FIR's operand pattern: accumulator pair += window pair * tap, all from (non-uniform) registers;
-        // role 9: the tap is one scalar register broadcast to both halves, role 11: the tap is a register pair
-        unsigned long long acc[8], win[16], tap2[8];
-        float tap[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const float lo = (float)(threadIdx.x + i), hi = lo + 0.5f;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(acc[i]) : "f"(lo), "f"(hi));
-            tap[i] = a + 1e-6f * (float)(lane + i);
-            const float tl = tap[i], th = tap[i] + 1e-7f;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(tap2[i]) : "f"(tl), "f"(th));
-        }
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const float lo = b + 1e-6f * (float)(lane + i), hi = lo + 1e-7f;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(win[i]) : "f"(lo), "f"(hi));
-        }
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    if (role == 9) {
-                        unsigned long long t2;
-                        asm("mov.b64 %0, {%1, %1};" : "=l"(t2) : "f"(tap[j]));
-                        asm volatile("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[i]) : "l"(win[i + 7 - j]), "l"(t2));
-                    } else {
-                        asm volatile("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[i]) : "l"(win[i + 7 - j]), "l"(tap2[j]));
-                    }
-                }
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            float lo, hi;
-            asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(acc[i]));
-            res += lo + hi;
-        }
-    } else if (role == 10) {
-        // scalar FFMA with the FIR's operand pattern: 16 accumulators, 23 window values, 8 taps, all registers
-        float acc[16], win[24], tap[8];
-#pragma unroll
-        for (int i = 0; i < 16; ++i) acc[i] = (float)(threadIdx.x + i);
-#pragma unroll
-        for (int i = 0; i < 24; ++i) win[i] = b + 1e-6f * (float)(lane + i);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) tap[i] = a + 1e-6f * (float)(lane + i);
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 8; ++sub) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-#pragma unroll
-                for (int i = 0; i < 16; ++i)
-                    asm volatile("fma.rn.f32 %0, %1, %2, %0;" : "+f"(acc[i]) : "f"(win[i + 7 - j]), "f"(tap[j]));
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) res += acc[i];
-    }
-    else if (role == 12 || role == 13) {
-        // the FIR's operand pattern with the taps in the kernel parameters (constant bank -> uniform registers):
-        // role 12 in tap-major order (the tap is reused by 8 consecutive FFMA2), role 13 window-major (the window
-        // pair is reused by up to 8 consecutive FFMA2)
-        unsigned long long acc[8], win[16];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const float lo = (float)(threadIdx.x + i), hi = lo + 0.5f;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(acc[i]) : "f"(lo), "f"(hi));
-        }
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const float lo = b + 1e-6f * (float)(lane + i), hi = lo + 1e-7f;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(win[i]) : "f"(lo), "f"(hi));
-        }
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-            const int tb = 8 * (sub & 7);
-            if (role == 12) {
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    unsigned long long t2;
-                    asm("mov.b64 %0, {%1, %1};" : "=l"(t2) : "f"(ptaps.t[tb + j]));
-#pragma unroll
-                    for (int i = 0; i < 8; ++i)
-                        asm volatile("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[i]) : "l"(win[i + 7 - j]), "l"(t2));
-                }
-            } else {
-#pragma unroll
-                for (int w = 0; w < 15; ++w)
-#pragma unroll
-                    for (int j = 0; j < 8; ++j) {
-                        const int i = w - 7 + j;
-                        if (i >= 0 && i < 8) {
-                            unsigned long long t2;
-                            asm("mov.b64 %0, {%1, %1};" : "=l"(t2) : "f"(ptaps.t[tb + j]));
-                            asm volatile("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[i]) : "l"(win[w]), "l"(t2));
-                        }
-                    }
-            }
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            float lo, hi;
-            asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(acc[i]));
-            res += lo + hi;
-        }
-    } else if (role == 14) {
-        // window-major order with the tap in a (non-uniform) register
-        unsigned long long acc[8], win[16];
-        float tap[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const float lo = (float)(threadIdx.x + i), hi = lo + 0.5f;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(acc[i]) : "f"(lo), "f"(hi));
-            tap[i] = a + 1e-6f * (float)(lane + i);
-        }
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const float lo = b + 1e-6f * (float)(lane + i), hi = lo + 1e-7f;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(win[i]) : "f"(lo), "f"(hi));
-        }
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int w = 0; w < 15; ++w)
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const int i = w - 7 + j;
-                    if (i >= 0 && i < 8) {
-                        unsigned long long t2;
-                        asm("mov.b64 %0, {%1, %1};" : "=l"(t2) : "f"(tap[j]));
-                        asm volatile("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[i]) : "l"(win[w]), "l"(t2));
-                    }
-                }
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            float lo, hi;
-            asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(acc[i]));
-            res += lo + hi;
-        }
-    }
-    else if (role == 15) {
-        // independent legacy tensor-core MMAs (mma.sync m16n8k16 f16, four accumulator sets): what do they cost the
-        // sub-partition's issue port / FMA pipe beside FFMA2 streams?
-        float d[4][4];
-        unsigned ar[4], br[2];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            ar[i] = 0x3c003c00u + (unsigned)lane;        // fp16 pairs near 1.0
-#pragma unroll
-            for (int j = 0; j < 4; ++j) d[i][j] = 0.f;
-        }
-        br[0] = 0x3c003c00u; br[1] = 0x38003800u;
-        for (int it = 0; probe_running(t0, iters, it); ++it)
-#pragma unroll 1
-        for (int sub = 0; sub < 16; ++sub) {
-#pragma unroll
-            for (int r = 0; r < 16; ++r)
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                                 : "+f"(d[i][0]), "+f"(d[i][1]), "+f"(d[i][2]), "+f"(d[i][3])
-                                 : "r"(ar[0]), "r"(ar[1]), "r"(ar[2]), "r"(ar[3]), "r"(br[0]), "r"(br[1]));
-        }
-        n_inst = 1024ull * (unsigned long long)rounds_done;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) res += d[i][0] + d[i][1] + d[i][2] + d[i][3];
-    }
-    asm volatile("mov.u64 %0, %%clock64;" : "=l"(t1));
-    if (res == 123.456f) sink[0] = res;
-    if (blockIdx.x == 0 && lane == 0) { out[warp] = (unsigned long long)(t1 - t0); out[16 + warp] = n_inst; }
-}
-
 }  // namespace micloc
 
 using namespace micloc;
 
 extern "C" int micloc_fp32_peak(int device, int variant, double *tflops) {
-    if (!tflops || variant < 0 || variant > 3) return set_error(MICLOC_ERR_CONFIG, "bad arguments");
+    if (!tflops || variant < 0 || variant > 2) return set_error(MICLOC_ERR_CONFIG, "bad arguments");
     MICLOC_CUDA(cudaSetDevice(device));
     int sms = 0;
     MICLOC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
@@ -453,14 +87,13 @@ extern "C" int micloc_fp32_peak(int device, int variant, double *tflops) {
         MICLOC_CUDA(cudaEventRecord(e0, 0));
         if (variant == 0) k_peak_ffma<<<grid, 256>>>(out, iters, 0.999f, 0.001f);
         else if (variant == 1) k_peak_ffma2<<<grid, 256>>>(out, iters, 0.999f, 0.001f);
-        else if (variant == 2) k_peak_dfma<<<grid, 256>>>(out, iters / 4, 0.999, 0.001);
-        else k_peak_mixed<<<grid, 256>>>(out, iters, 0.999f, 0.001f, 0.999, 0.001);
+        else k_peak_dfma<<<grid, 256>>>(out, iters / 4, 0.999, 0.001);
         MICLOC_CUDA(cudaEventRecord(e1, 0));
         MICLOC_CUDA(cudaEventSynchronize(e1));
         float ms = 0.f;
         MICLOC_CUDA(cudaEventElapsedTime(&ms, e0, e1));
         count_launch(1);
-        // flop counted: 16 FP32 FMA per iteration (variants 0, 1, 3: the FP32 part), 8 FP64 FMA (variant 2)
+        // flop counted: 16 FP32 FMA per iteration (variants 0, 1), 8 FP64 FMA (variant 2)
         const double fl = variant == 2 ? 2.0 * 8.0 * (double)(iters / 4) * 256.0 * (double)grid
                                        : 2.0 * 16.0 * (double)iters * 256.0 * (double)grid;
         const double tf = fl / (ms * 1e-3) / 1e12;
@@ -469,32 +102,5 @@ extern "C" int micloc_fp32_peak(int device, int variant, double *tflops) {
     cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(out);
     MICLOC_CUDA(cudaGetLastError());
     *tflops = best;
-    return MICLOC_OK;
-}
-
-extern "C" int micloc_sched_probe(int device, const int32_t roles[16], int iters, uint64_t out[32]) {
-    if (!roles || !out || iters <= 0) return set_error(MICLOC_ERR_CONFIG, "bad arguments");
-    MICLOC_CUDA(cudaSetDevice(device));
-    int sms = 0;
-    MICLOC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-    int nw = 0;
-    for (int w = 0; w < 16; ++w) if (roles[w]) nw = w + 1;
-    if (nw == 0) return set_error(MICLOC_ERR_CONFIG, "no active warp");
-    int *d_roles = nullptr; unsigned long long *d_out = nullptr; float *d_sink = nullptr;
-    MICLOC_CUDA(cudaMalloc(&d_roles, 16 * sizeof(int)));
-    MICLOC_CUDA(cudaMalloc(&d_out, 32 * sizeof(unsigned long long)));
-    MICLOC_CUDA(cudaMalloc(&d_sink, sizeof(float)));
-    MICLOC_CUDA(cudaMemcpy(d_roles, roles, 16 * sizeof(int), cudaMemcpyHostToDevice));
-    MICLOC_CUDA(cudaMemset(d_out, 0, 32 * sizeof(unsigned long long)));
-    for (int rep = 0; rep < 2; ++rep) {     // the second run is the one reported (warm instruction cache)
-        ProbeTaps pt;
-        for (int i = 0; i < 64; ++i) pt.t[i] = 0.999f + 1e-6f * (float)i;
-        k_sched_probe<<<sms, 32 * nw>>>(d_roles, iters, 0.999f, 0.001f, d_out, d_sink, pt);
-        count_launch(1);
-        MICLOC_CUDA(cudaDeviceSynchronize());
-    }
-    MICLOC_CUDA(cudaMemcpy(out, d_out, 32 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    cudaFree(d_roles); cudaFree(d_out); cudaFree(d_sink);
-    MICLOC_CUDA(cudaGetLastError());
     return MICLOC_OK;
 }

@@ -419,11 +419,9 @@ __device__ __forceinline__ void bar_arrive_named(int id, int count) { asm volati
 // handed over with named barriers).  Neuron threads: one (clip, hidden neuron) each, state in registers.
 // SAT_ISYN = false when the host proved that I_syn cannot leave the int16 range
 // (2^dash_syn * (sum_i |w_i| + 1) <= 32767 for every neuron).
-#ifndef MICLOC_LIF_MINB
-#define MICLOC_LIF_MINB 3      // CTAs of 512 threads per SM the register budget is cut for
-#endif
+constexpr int kLifMinBlocks = 3;     // CTAs of 512 threads per SM the register budget is cut for
 template <bool SIGNED_IN, int W, bool SAT_ISYN, bool RASTER>
-__global__ void __launch_bounds__(512, MICLOC_LIF_MINB)
+__global__ void __launch_bounds__(512, kLifMinBlocks)
 k_xylo_lif(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, const int16_t *__restrict__ w,
            const int16_t *__restrict__ thr, const int8_t *__restrict__ dash_syn, const int8_t *__restrict__ dash_mem,
            const int16_t *__restrict__ bias, int max_spikes, int N, int npb, long long T,
@@ -574,9 +572,7 @@ k_xylo_lif(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, con
 // Needs N_in <= 32 and |sum| < 2^15 (checked by the host); otherwise the event-loop kernel runs.
 // ---------------------------------------------------------------------------
 constexpr int kMmaTile = 24;     // time steps per tile: 3 MMA column blocks
-#ifndef MICLOC_LIF_MMA_MINB
-#define MICLOC_LIF_MMA_MINB 2
-#endif
+constexpr int kLifMmaMinBlocks = 2;
 
 __device__ __forceinline__ void mma_s8_16x8x32(int (&d)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
     asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.s8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%10,%10,%10};"
@@ -591,7 +587,7 @@ __device__ __forceinline__ int imad_pipe(int a, int b, int c) {
 }
 constexpr int kTrPitch = 28;      // int32 words per neuron row of the hand-over buffer: 24 steps + 4 (conflict-free 128-bit reads)
 template <bool SIGNED_IN, bool SAT_ISYN, bool SAT_V, bool HAS_BIAS, bool RASTER>
-__global__ void __launch_bounds__(512, MICLOC_LIF_MMA_MINB)
+__global__ void __launch_bounds__(512, kLifMmaMinBlocks)
 k_xylo_lif_mma(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, const int8_t *__restrict__ w8, int w_shift,
                const int16_t *__restrict__ thr, const int8_t *__restrict__ dash_syn, const int8_t *__restrict__ dash_mem,
                const int16_t *__restrict__ bias, int max_spikes, int N, int npb, long long T,

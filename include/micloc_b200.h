@@ -377,15 +377,9 @@ int micloc_snn_debug_counters(micloc_snn *ctx, uint64_t out[32]);
  * cycles of the eight roles, unused) of CTA i of the last fused launch, i < n <= 512 (MICLOC_ROLE_TIMING builds only). */
 int micloc_snn_debug_cta_times(micloc_snn *ctx, uint64_t *out, int32_t n);
 /* FP32 FMA-pipe micro-benchmark on `device` (the measured denominator of the
- * roofline in bench.py): variant 0 = scalar FFMA, 1 = packed fma.rn.f32x2; diagnostics: 2 = FP64 DFMA
- * (FP64 TFLOP/s), 3 = FFMA2 with one DFMA per two FFMA2 in the same warps (FP32 TFLOP/s of the FFMA2 part). */
+ * roofline in bench.py): variant 0 = scalar FFMA, 1 = packed fma.rn.f32x2, 2 = FP64 DFMA (FP64 TFLOP/s).
+ * Any other variant returns MICLOC_ERR_CONFIG. */
 int micloc_fp32_peak(int device, int variant, double *tflops);
-/* Scheduler probe (diagnostics behind the fused kernel's warp-role layout, DESIGN.md): one CTA of up to 16 warps
- * per SM, warp w runs instruction stream roles[w] (0 idle, 1 FFMA2 stream, 2 dependent FFMA chain, 3 independent
- * ALU stream, 4 independent scalar FFMA stream, 5 dependent FFMA/ALU chain, 6 FFMA2 stream with ALU gaps) for
- * iters x 1000 cycles, all warps side by side; out[w] = clock64 cycles of CTA 0's warp w, out[16 + w] = the
- * instructions it got through. */
-int micloc_sched_probe(int device, const int32_t roles[16], int iters, uint64_t out[32]);
 
 #ifdef __cplusplus
 }
