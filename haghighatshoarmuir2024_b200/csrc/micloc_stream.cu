@@ -39,6 +39,7 @@
 
 #include "micloc_common.h"
 #include "micloc_staged.cuh"
+#include "micloc_stream.cuh"
 
 namespace micloc {
 
@@ -50,27 +51,7 @@ struct ChanState {            // one per (slot, real channel): in-phase | quadra
     NeuronState nr;
 };
 
-// where a slot stands: samples pushed (N), samples returned as final (F), 0 once flushed.  Positions stay below
-// 2^31 - 4096 (the host refuses a push beyond), so the kernels count time in int.
-struct SlotPos { int N, F, active, pad; };
-
-// [K-1 history rows | frame rows] of every slot: cur [S][hist + n][M].  History = the last hist rows of the previous
-// push's buffer prev [S][hist + n_prev][M], zeros for a slot that starts (N == 0); frame rows converted to float,
-// channels >= M dropped.
-template <typename IN_T>
-__global__ void __launch_bounds__(256)
-k_stream_assemble(const IN_T *__restrict__ frames, const float *__restrict__ prev, float *__restrict__ cur,
-                  const SlotPos *__restrict__ pos, long long S, int n, int n_prev, int in_ch, int M, int hist) {
-    const long long rows = (long long)hist + n;
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= S * rows * M) return;
-    const int m = (int)(i % M);
-    const long long r = (i / M) % rows, s = i / (rows * M);
-    float v;
-    if (r < hist) v = pos[s].N > 0 ? prev[(s * (hist + n_prev) + n_prev + r) * M + m] : 0.f;
-    else v = (float)frames[(s * n + (r - hist)) * in_ch + m];
-    cur[i] = v;
-}
+// SlotPos and k_stream_assemble (the [K-1 history rows | frame] buffer of every slot): micloc_stream.cuh
 
 // Multi-band frame assembly: one thread per (slot, microphone) steps the F band-pass cascades of the filterbank
 // (biquad_step with the float32 sections of k_filterbank, so band f's rows are micloc_filterbank's bits for the whole

@@ -19,12 +19,17 @@
 // The integer network then runs as ONE kernel, one thread per (clip, hidden neuron) looping over
 // time with I_syn / V_mem / spike count in registers; the input spikes of a clip are turned into
 // per-step event masks in shared memory and each event is one predicated add of an int16 weight.
+// Xylo stream batches (end of this file) run the same exact front end and network on many continuous recordings, with
+// the chain and neuron state carried across pushes (STREAM / STATE forms of the kernels).
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 #include <vector>
 
 #include "micloc_common.h"
+#include "micloc_stream.cuh"
 
 namespace micloc {
 
@@ -102,14 +107,14 @@ __device__ __forceinline__ void stht_f64_taps4(double (&acc)[kSR], const double 
 template <typename IN_T>
 __global__ void __launch_bounds__(256)
 k_stht_f64_sparse(const IN_T *__restrict__ audio, const double *__restrict__ g, double *__restrict__ q,
-                  int M, int K, int ntap, long long T, int ntiles) {
+                  int M, int K, int ntap, long long T, int ntiles, long long t_first = 0) {
     extern __shared__ __align__(16) double smd[];
     double *gs = smd;                                   // [ntap]
     const int npos = kSTile + K - 1;                    // positions per row: x[t0 - (K-1) + p]
     const int pitch = (f64_pad(npos) + 9) & ~1;
     double *xs = smd + ntap;                            // [mg][pitch], microphone-major
     const long long b = blockIdx.x / ntiles;
-    const long long t0 = (long long)(blockIdx.x % ntiles) * kSTile;
+    const long long t0 = t_first + (long long)(blockIdx.x % ntiles) * kSTile;   // (t_first: outputs before it are not wanted)
     const int m0 = blockIdx.y * kF64MG;
     const int mg = min(kF64MG, M - m0);
     const IN_T *clip = audio + b * T * M;
@@ -190,21 +195,74 @@ __device__ __forceinline__ void f64_push(RzccState &s, const F64Store &st, int p
     if (POL) { s.last1 = pos; s.n1 = n + 1; } else { s.last0 = pos; s.n0 = n + 1; }
 }
 
-template <typename IN_T, int NBA>
+// Stream form (STREAM = true, Xylo stream batches): warp b is slot b, its lanes' chain state is parked in global memory
+// between pushes, and time runs in the slot's ABSOLUTE positions [N, N + n): the 64-step tiles start at the same
+// samples as in a one-shot clip of the whole recording.  A push may end inside a tile; the clusters are then checked
+// for closing there too, which emits nothing a later check would not (a cluster closed that way can no longer grow).
+// Spikes go to the slot's ring at their absolute position; the rows [F, N + n - D) are final and copied out.
+constexpr int kF64FlatTop = 64;         // flat-top allowance of the stream latency (samples)
+
+struct XyloChanState {                  // one per (slot, band, channel)
+    double zs[5];                       // band-filter delays (NBA <= 5)
+    double cs;                          // running sum
+    int rise, fall;                     // start of the running sum's current flat top / bottom (-1: none)
+    RzccState rz;
+    int cl_pos[2 * kF64Cluster];
+    double cl_h[2 * kF64Cluster];
+};
+
+struct XyloChainStream {
+    XyloChanState *state;               // [S][CT]
+    const SlotPos *pos_in;
+    SlotPos *pos_out;
+    int32_t *m_out;                     // [S] final rows of this call
+    const int32_t *close_sel;           // flush: 1 = close this slot like a clip end; nullptr: push
+    int8_t *ring;                       // [S][ring_len][CT] spikes at (absolute position mod ring_len)
+    int ring_len;                       // power of two >= max_frame_len + D
+    int hist;                           // rows of the assembled buffer before the frame (K - 1)
+    int rows;                           // row stride of the output raster (n + D)
+    int D;                              // latency
+};
+
+template <typename IN_T, int NBA, bool STREAM = false>
 __global__ void __launch_bounds__(32 * kChainWarps, 3)
 k_xylo_chain_f64(const IN_T *__restrict__ audio, const double *__restrict__ q, const double *__restrict__ ba_b,
                  const double *__restrict__ ba_a, int8_t *__restrict__ spikes, int32_t *__restrict__ flags,
-                 int M, int half, int nba, int F, int w, int bipolar, long long B, long long T) {
+                 int M, int half, int nba, int F, int w, int bipolar, long long B, long long T,
+                 const XyloChainStream sa = XyloChainStream{}) {
+    // STREAM: audio = assembled rows [S][hist + T][M] (float64), q the same rows' STHT, T = frame rows (0: flush)
+    using XS_T = typename std::conditional<STREAM, double, float>::type;
     extern __shared__ __align__(16) double smd[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const long long b = (long long)blockIdx.x * kChainWarps + warp;
+    const int nw = STREAM ? (int)(blockDim.x >> 5) : kChainWarps;   // (the stream form stages float64 in-phase rows)
+    const long long b = (long long)blockIdx.x * nw + warp;
     if (b >= B) return;
     const int C2 = 2 * M, CT = C2 * F;
     const int passes = (CT + 31) >> 5;
     double *qs = smd + (size_t)warp * kChainTile * M;                                                       // [tile][M]
-    float *xs = reinterpret_cast<float *>(smd + (size_t)kChainWarps * kChainTile * M) + (size_t)warp * kChainTile * M;   // [tile][M]
-    const IN_T *clip = audio + b * T * M;
-    const double *qc = q + b * T * M;
+    XS_T *xs = reinterpret_cast<XS_T *>(smd + (size_t)nw * kChainTile * M) + (size_t)warp * kChainTile * M;   // [tile][M]
+    const long long rows_in = STREAM ? sa.hist + T : T;
+    const IN_T *clip = audio + b * rows_in * M;
+    const double *qc = q + b * rows_in * M;
+
+    long long tstart = 0, tstop = T;
+    bool flush = false;
+    int F0 = 0, F1 = 0;
+    if constexpr (STREAM) {
+        const SlotPos sp = sa.pos_in[b];
+        flush = sa.close_sel != nullptr;
+        const bool run = sp.active && (!flush || sa.close_sel[b] != 0);
+        const int N0 = sp.N;
+        const int t_end = (run && !flush) ? N0 + (int)T : N0;
+        F0 = sp.F;
+        F1 = !run ? F0 : (flush ? N0 : max(t_end - sa.D, F0));
+        if (lane == 0) {
+            sa.pos_out[b] = SlotPos{t_end, F1, (run && flush) ? 0 : sp.active, 0};
+            sa.m_out[b] = F1 - F0;
+        }
+        if (!run) return;
+        tstart = N0; tstop = t_end;
+    }
 
     // per-pass chain state (CT <= 64: at most two (band, channel) per lane)
     // (parked in local memory between tiles: only the pass at work lives in registers)
@@ -215,22 +273,45 @@ k_xylo_chain_f64(const IN_T *__restrict__ audio, const double *__restrict__ q, c
     double q_h[kChainTile + 1];
 #pragma unroll 1
     for (int ps = 0; ps < 2; ++ps) {
+        if constexpr (STREAM) {
+            const int cc = lane + 32 * ps;
+            if (cc < CT) {
+                const XyloChanState &g = sa.state[b * CT + cc];
 #pragma unroll
-        for (int k = 0; k < NBA; ++k) sv[ps].zs[k] = 0.0;
-        sv[ps].cs = 0.0; sv[ps].rise = sv[ps].fall = -1;
-        rzcc_reset(sv[ps].rz);
+                for (int k = 0; k < NBA; ++k) sv[ps].zs[k] = g.zs[k];
+                sv[ps].cs = g.cs; sv[ps].rise = g.rise; sv[ps].fall = g.fall;
+                sv[ps].rz = g.rz;
+                for (int i = 0; i < sv[ps].rz.n0; ++i) { cl_pos[ps][i] = g.cl_pos[i]; cl_h[ps][i] = g.cl_h[i]; }
+                for (int i = 0; i < sv[ps].rz.n1; ++i) {
+                    cl_pos[ps][kF64Cluster + i] = g.cl_pos[kF64Cluster + i];
+                    cl_h[ps][kF64Cluster + i] = g.cl_h[kF64Cluster + i];
+                }
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < NBA; ++k) sv[ps].zs[k] = 0.0;
+            sv[ps].cs = 0.0; sv[ps].rise = sv[ps].fall = -1;
+            rzcc_reset(sv[ps].rz);
+        }
     }
-    const int NT = (int)((T + kChainTile - 1) / kChainTile);
-    for (int tile = 0; tile < NT; ++tile) {
-        const long long t0 = (long long)tile * kChainTile;
-        const int len = (int)min((long long)kChainTile, T - t0);
+    int8_t *const sbase = STREAM ? sa.ring + b * (long long)sa.ring_len * CT : spikes + b * T * CT;
+    const int rmask = sa.ring_len - 1;
+    // tiles of kChainTile ABSOLUTE samples (the first and last of a stream push may be partial)
+    for (long long t0 = tstart; t0 < tstop;) {
+        const int len = (int)min((long long)(kChainTile - (int)(t0 & (kChainTile - 1))), tstop - t0);
         __syncwarp();
         for (int e = lane; e < len * M; e += 32) {
-            qs[e] = qc[t0 * M + e];
             const int i = e / M, m = e - i * M;
-            long long src = t0 + i - half;                       // np.roll: x[(t - K/2) mod T]
-            if (src < 0) { src %= T; if (src < 0) src += T; }
-            xs[e] = (float)clip[src * M + m];
+            if constexpr (STREAM) {
+                const long long r = sa.hist + (t0 - tstart) + i;              // row of sample t0 + i
+                qs[e] = qc[r * M + m];
+                xs[e] = clip[(r - half) * M + m];                             // causal x[t - K/2] (zeros before the slot starts)
+            } else {
+                qs[e] = qc[t0 * M + e];
+                long long src = t0 + i - half;                       // np.roll: x[(t - K/2) mod T]
+                if (src < 0) { src %= T; if (src < 0) src += T; }
+                xs[e] = (float)clip[src * M + m];
+            }
         }
         __syncwarp();
 #pragma unroll 1
@@ -241,8 +322,11 @@ k_xylo_chain_f64(const IN_T *__restrict__ audio, const double *__restrict__ q, c
                 const bool inphase = c < M;
                 const int col = inphase ? c : c - M;
                 const F64Store store{cl_pos[ps], cl_h[ps], 1};
-                int8_t *out = spikes + b * T * CT + cc;
-                auto emit = [&](int pos, int sign) { out[(long long)pos * CT] = (int8_t)sign; };
+                int8_t *out = sbase + cc;
+                auto emit = [&](int pos, int sign) {
+                    if constexpr (STREAM) out[(long long)(pos & rmask) * CT] = (int8_t)sign;
+                    else out[(long long)pos * CT] = (int8_t)sign;
+                };
                 double bb[NBA], aa[NBA], zs[NBA];
 #pragma unroll
                 for (int k = 0; k < NBA; ++k) {
@@ -295,13 +379,58 @@ k_xylo_chain_f64(const IN_T *__restrict__ audio, const double *__restrict__ q, c
                     if (s.n1 > 0 && e1 - s.last1 >= w) f64_resolve<1>(s, store, w, emit);
                     if (s.n0 > 0 && e0 - s.last0 >= w) f64_resolve<0>(s, store, w, emit);
                 }
-                if (tile == NT - 1) {
+                if (!STREAM && t0 + len == tstop) {
                     rzcc_close(s, store, w, (int)(T - 1), true, emit);
                     if (s.overflow) atomicOr(flags + b, 1);
                 }
 #pragma unroll
                 for (int k = 0; k < NBA; ++k) sv[ps].zs[k] = zs[k];
                 sv[ps].rz = s; sv[ps].cs = acc; sv[ps].rise = rs; sv[ps].fall = fl;
+            }
+        }
+        t0 += len;
+    }
+    if constexpr (STREAM) {
+        // flush: close like a clip end.  Push: every spike below F1 must have been emitted -- the earliest position a
+        // spike can still take is the first candidate of an open cluster or the midpoint of an open flat top / bottom
+        // and a sample after the push; if that lies below F1 (or a cluster overflowed) the slot is flagged (bit 0).
+        // Then the final rows [F0, F1) of the lane's channels leave the ring (which is cleared behind them).
+#pragma unroll 1
+        for (int ps = 0; ps < passes; ++ps) {
+            const int cc = lane + 32 * ps;
+            if (cc >= CT) continue;
+            const F64Store store{cl_pos[ps], cl_h[ps], 1};
+            int8_t *ring = sbase + cc;
+            auto emit = [&](int pos, int sign) { ring[(long long)(pos & rmask) * CT] = (int8_t)sign; };
+            RzccState s = sv[ps].rz;
+            const int t_end = (int)tstop;
+            if (flush) {
+                if (t_end > 0) rzcc_close(s, store, w, t_end - 1, true, emit);
+            } else {
+                int h = t_end;
+                if (s.n1 > 0) h = min(h, cl_pos[ps][kF64Cluster]);
+                if (s.n0 > 0) h = min(h, cl_pos[ps][0]);
+                if (sv[ps].rise >= 0) h = min(h, (sv[ps].rise + t_end - 1) >> 1);
+                if (bipolar && sv[ps].fall >= 0) h = min(h, (sv[ps].fall + t_end - 1) >> 1);
+                if (h < F1) s.overflow = 1;
+            }
+            if (s.overflow) atomicOr(flags + b, 1);
+            XyloChanState &g = sa.state[b * CT + cc];
+#pragma unroll
+            for (int k = 0; k < NBA; ++k) g.zs[k] = sv[ps].zs[k];
+            g.cs = sv[ps].cs; g.rise = sv[ps].rise; g.fall = sv[ps].fall;
+            g.rz = s;
+            for (int i = 0; i < s.n0; ++i) { g.cl_pos[i] = cl_pos[ps][i]; g.cl_h[i] = cl_h[ps][i]; }
+            for (int i = 0; i < s.n1; ++i) {
+                g.cl_pos[kF64Cluster + i] = cl_pos[ps][kF64Cluster + i];
+                g.cl_h[kF64Cluster + i] = cl_h[ps][kF64Cluster + i];
+            }
+            int8_t *o = spikes + b * (long long)sa.rows * CT + cc;
+#pragma unroll 4
+            for (int t = F0; t < F1; ++t) {
+                int8_t *r = ring + (long long)(t & rmask) * CT;
+                o[(long long)(t - F0) * CT] = *r;
+                *r = 0;
             }
         }
     }
@@ -420,12 +549,16 @@ __device__ __forceinline__ void bar_arrive_named(int id, int count) { asm volati
 // SAT_ISYN = false when the host proved that I_syn cannot leave the int16 range
 // (2^dash_syn * (sum_i |w_i| + 1) <= 32767 for every neuron).
 constexpr int kLifMinBlocks = 3;     // CTAs of 512 threads per SM the register budget is cut for
-template <bool SIGNED_IN, int W, bool SAT_ISYN, bool RASTER>
+// STATE (Xylo stream batches): clip b runs over its first rows_b[b] rows only (T is then the row stride), from the
+// I_syn / V_mem it left in nstate [B][N] at its previous call, and leaves them there; counts are those of this call
+// (not written for a clip with no rows).
+template <bool SIGNED_IN, int W, bool SAT_ISYN, bool RASTER, bool STATE = false>
 __global__ void __launch_bounds__(512, kLifMinBlocks)
 k_xylo_lif(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, const int16_t *__restrict__ w,
            const int16_t *__restrict__ thr, const int8_t *__restrict__ dash_syn, const int8_t *__restrict__ dash_mem,
            const int16_t *__restrict__ bias, int max_spikes, int N, int npb, long long T,
-           uint8_t *__restrict__ raster, int32_t *__restrict__ counts) {
+           uint8_t *__restrict__ raster, int32_t *__restrict__ counts, const int32_t *__restrict__ rows_b = nullptr,
+           int2 *__restrict__ nstate = nullptr) {
     extern __shared__ __align__(16) unsigned char sm_raw[];
     int16_t *w_s = reinterpret_cast<int16_t *>(sm_raw);                            // [N_in][npb_pad]
     const int npb_pad = (npb + 7) & ~7;
@@ -438,7 +571,8 @@ k_xylo_lif(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, con
     const int tid = threadIdx.x;
     const int nthreads = blockDim.x;
     const int n_cons = nthreads - 32;                     // neuron threads
-    const int ntiles = (int)((T + kLifTile - 1) / kLifTile);
+    const long long Tb = STATE ? (long long)rows_b[b] : T;                // steps of this clip
+    const int ntiles = (int)((Tb + kLifTile - 1) / kLifTile);
     for (int e = tid; e < N_in * npb; e += nthreads) {
         const int i = e / npb, j = e % npb;
         w_s[i * npb_pad + j] = (n0 + j < N) ? w[(long long)i * N + n0 + j] : (int16_t)0;
@@ -451,7 +585,7 @@ k_xylo_lif(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, con
         const int8_t *src = spikes + b * T * row;
         for (int k = 0; k < ntiles; ++k) {
             const long long t0 = (long long)k * kLifTile;
-            const int len = (int)min((long long)kLifTile, T - t0);
+            const int len = (int)min((long long)kLifTile, Tb - t0);
             {   // raw spike bytes of the tile (coalesced; 16-byte vectors when aligned)
                 const int8_t *g = src + t0 * row;
                 const int nbytes = len * row;
@@ -499,6 +633,7 @@ k_xylo_lif(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, con
     const int n = n0 + tid;
     const bool live = tid < npb && n < N;
     int isyn = 0, vmem = 0, count = 0;
+    if (STATE && live) { const int2 v = nstate[b * N + n]; isyn = v.x; vmem = v.y; }
     const int th = live ? thr[n] : 0x3fffffff;
     const int th2 = 2 * th;
     const int ds = live ? dash_syn[n] : 0, dm = live ? dash_mem[n] : 0;
@@ -508,7 +643,7 @@ k_xylo_lif(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, con
     uint8_t *rp = (RASTER && live) ? raster + b * T * N + n : nullptr;
 
     for (int k = 0; k < ntiles; ++k) {
-        const int len = (int)min((long long)kLifTile, T - (long long)k * kLifTile);
+        const int len = (int)min((long long)kLifTile, Tb - (long long)k * kLifTile);
         bar_sync_named(1 + (k & 1), nthreads);                       // wait for the masks of tile k
         if (live) {
             const unsigned int *mk = masks + (k & 1) * kLifTile * W;
@@ -555,7 +690,8 @@ k_xylo_lif(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, con
         }
         if (k + 2 < ntiles) bar_arrive_named(3 + (k & 1), nthreads); // buffer k&1 may be refilled (tile k+2)
     }
-    if (live && counts) counts[b * N + n] = count;
+    if (STATE && live) nstate[b * N + n] = make_int2(isyn, vmem);
+    if (live && counts && (!STATE || Tb > 0)) counts[b * N + n] = count;
 }
 
 
@@ -586,12 +722,15 @@ __device__ __forceinline__ int imad_pipe(int a, int b, int c) {
     return r;
 }
 constexpr int kTrPitch = 28;      // int32 words per neuron row of the hand-over buffer: 24 steps + 4 (conflict-free 128-bit reads)
-template <bool SIGNED_IN, bool SAT_ISYN, bool SAT_V, bool HAS_BIAS, bool RASTER>
+// STATE: as in k_xylo_lif (per-clip row counts rows_b, I_syn / V_mem carried in nstate, counts of this call).  A group of
+// 8 steps that straddles a clip's last row takes the tail path, so the multi-spike redo never sees a step beyond it.
+template <bool SIGNED_IN, bool SAT_ISYN, bool SAT_V, bool HAS_BIAS, bool RASTER, bool STATE = false>
 __global__ void __launch_bounds__(512, kLifMmaMinBlocks)
 k_xylo_lif_mma(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in, const int8_t *__restrict__ w8, int w_shift,
                const int16_t *__restrict__ thr, const int8_t *__restrict__ dash_syn, const int8_t *__restrict__ dash_mem,
                const int16_t *__restrict__ bias, int max_spikes, int N, int npb, long long T,
-               uint8_t *__restrict__ raster, int32_t *__restrict__ counts) {
+               uint8_t *__restrict__ raster, int32_t *__restrict__ counts, const int32_t *__restrict__ rows_b = nullptr,
+               int2 *__restrict__ nstate = nullptr) {
     extern __shared__ __align__(16) unsigned char sm_raw[];
     uint8_t *Sb = sm_raw;                                                                // [2][kMmaTile][32] binary spikes
     int *tr_all = reinterpret_cast<int *>(sm_raw + 2 * kMmaTile * 32);                   // [neuron warps][32][kTrPitch]
@@ -602,7 +741,8 @@ k_xylo_lif_mma(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in,
     const int tid = threadIdx.x;
     const int nthreads = blockDim.x;
     const int n_cons = nthreads - 32;
-    const int ntiles = (int)((T + kMmaTile - 1) / kMmaTile);
+    const long long Tb = STATE ? (long long)rows_b[b] : T;                // steps of this clip
+    const int ntiles = (int)((Tb + kMmaTile - 1) / kMmaTile);
     for (int e = tid; e < 2 * kMmaTile * 32; e += nthreads) Sb[e] = 0;       // columns beyond the inputs stay zero
     __syncthreads();
 
@@ -615,7 +755,7 @@ k_xylo_lif_mma(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in,
         unsigned short pre[kPreW];
         auto prefetch = [&](int k) {
             const long long t = (long long)k * kMmaTile + lane;
-            const bool valid = k < ntiles && lane < kMmaTile && t < T;
+            const bool valid = k < ntiles && lane < kMmaTile && t < Tb;
             const unsigned short *gp = reinterpret_cast<const unsigned short *>(src + t * row);
 #pragma unroll
             for (int j = 0; j < kPreW; ++j) pre[j] = (valid && 2 * j < row) ? __ldg(gp + j) : (unsigned short)0;
@@ -651,6 +791,7 @@ k_xylo_lif_mma(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in,
     const int n = n0 + tid;
     const bool live = tid < npb && n < N;
     int isyn = 0, vmem = 0, count = 0;
+    if (STATE && live) { const int2 v = nstate[b * N + n]; isyn = v.x; vmem = v.y; }
     const int th = live ? thr[n] : 0x3fffffff;
     const int ds = live ? dash_syn[n] : 0, dm = live ? dash_mem[n] : 0;
     const int bs = (live && bias) ? bias[n] : 0;
@@ -676,7 +817,7 @@ k_xylo_lif_mma(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in,
         }
 
     for (int k = 0; k < ntiles; ++k) {
-        const int len = (int)min((long long)kMmaTile, T - (long long)k * kMmaTile);
+        const int len = (int)min((long long)kMmaTile, Tb - (long long)k * kMmaTile);
         bar_sync_named(1 + (k & 1), nthreads);                       // wait for the binary rows of tile k
         const uint8_t *S = Sb + (k & 1) * kMmaTile * 32;
         unsigned bf[kMmaTile / 8][2];
@@ -748,18 +889,20 @@ k_xylo_lif_mma(const int8_t *__restrict__ spikes, int CI, int bipolar, int N_in,
         }
         __syncwarp();                                                // the next tile overwrites this warp's buffer
     }
-    if (live && counts) counts[b * N + n] = count;
+    if (STATE && live) nstate[b * N + n] = make_int2(isyn, vmem);
+    if (live && counts && (!STATE || Tb > 0)) counts[b * N + n] = count;
 }
 
 // One CTA per clip: S[g] = sum_f counts[f*G + g]; doa = first argmax S; doa_peak = first argmax of the
 // 'full' box-car sums of S, minus win/2, modulo G (micloc/utils.py:84-121 on integers).
 __global__ void __launch_bounds__(128)
 k_xylo_doa(const int32_t *__restrict__ counts, int G, int F, int win, int32_t *__restrict__ doa,
-           int32_t *__restrict__ doa_peak) {
+           int32_t *__restrict__ doa_peak, const int32_t *__restrict__ rows_b = nullptr) {
     extern __shared__ __align__(16) long long S[];      // [G]
     __shared__ long long red_v[128];
     __shared__ int red_i[128];
     const long long b = blockIdx.x;
+    if (rows_b && rows_b[b] == 0) return;               // (stream batches: a slot with no final rows; uniform per block)
     const int32_t *c = counts + b * (long long)G * F;
     for (int g = threadIdx.x; g < G; g += blockDim.x) {
         long long a = 0;
@@ -804,12 +947,15 @@ k_xylo_doa(const int32_t *__restrict__ counts, int G, int F, int win, int32_t *_
     }
 }
 
-// signed raster [n][CI] -> Demo.spike_encoding's layout [n][N_in] in {0,1}
+// signed raster [n][CI] -> Demo.spike_encoding's layout [n][N_in] in {0,1}; rows_b (nullable, stream batches): row r
+// of clip r / T is only converted below rows_b[r / T]
 __global__ void __launch_bounds__(256)
-k_xylo_split(const int8_t *__restrict__ s, int8_t *__restrict__ out, long long rows, int CI, int bipolar) {
+k_xylo_split(const int8_t *__restrict__ s, int8_t *__restrict__ out, long long rows, int CI, int bipolar,
+             const int32_t *__restrict__ rows_b = nullptr, long long T = 1) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= rows * CI) return;
     const long long r = i / CI;
+    if (rows_b && r % T >= rows_b[r / T]) return;
     const int c = (int)(i % CI);
     const int v = s[i];
     if (bipolar) {
@@ -1001,10 +1147,10 @@ static int check_xylo_args(micloc_xylo *c, const void *in, int64_t B, int64_t T)
     return MICLOC_OK;
 }
 
-// integer network on a spike raster already on the device
-template <bool SIGNED_IN>
+// integer network on a spike raster already on the device (STATE: stream batches, see k_xylo_lif)
+template <bool SIGNED_IN, bool STATE = false>
 static int launch_lif(micloc_xylo *c, const int8_t *spikes, long long B, long long T, uint8_t *raster,
-                      int32_t *counts, cudaStream_t st) {
+                      int32_t *counts, cudaStream_t st, const int32_t *rows_b = nullptr, int2 *nstate = nullptr) {
     const int N = c->N;
     const int nchunks = (N + 479) / 480;                       // <= 480 neurons (15 warps) per CTA
     const int npb = (N + nchunks - 1) / nchunks;
@@ -1014,17 +1160,17 @@ static int launch_lif(micloc_xylo *c, const int8_t *spikes, long long B, long lo
         const size_t smem_m = (size_t)2 * kMmaTile * 32 + (size_t)((threads - 32) / 32) * 32 * kTrPitch * 4 + 16;
         dim3 grid_m((unsigned)B, (unsigned)nchunks);
         void (*kern)(const int8_t *, int, int, int, const int8_t *, int, const int16_t *, const int8_t *, const int8_t *,
-                     const int16_t *, int, int, int, long long, uint8_t *, int32_t *) = nullptr;
+                     const int16_t *, int, int, int, long long, uint8_t *, int32_t *, const int32_t *, int2 *) = nullptr;
         const bool hb = c->d_bias != nullptr;
 #define MICLOC_MMA_PICK(SI, SV, HB)                                                                          \
-        kern = raster ? k_xylo_lif_mma<SIGNED_IN, SI, SV, HB, true> : k_xylo_lif_mma<SIGNED_IN, SI, SV, HB, false>
+        kern = raster ? k_xylo_lif_mma<SIGNED_IN, SI, SV, HB, true, STATE> : k_xylo_lif_mma<SIGNED_IN, SI, SV, HB, false, STATE>
         if (c->sat_isyn) { if (hb) MICLOC_MMA_PICK(true, true, true); else MICLOC_MMA_PICK(true, true, false); }
         else if (c->sat_v) { if (hb) MICLOC_MMA_PICK(false, true, true); else MICLOC_MMA_PICK(false, true, false); }
         else { if (hb) MICLOC_MMA_PICK(false, false, true); else MICLOC_MMA_PICK(false, false, false); }
 #undef MICLOC_MMA_PICK
         MICLOC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m));
         kern<<<grid_m, threads, smem_m, st>>>(spikes, c->CT, c->p.bipolar, c->N_in, c->d_w8, c->w_shift, c->d_thr, c->d_ds, c->d_dm,
-                                              c->d_bias, c->max_spikes, N, npb, T, raster, counts);
+                                              c->d_bias, c->max_spikes, N, npb, T, raster, counts, rows_b, nstate);
         count_launch(1);
         MICLOC_CUDA(cudaGetLastError());
         return MICLOC_OK;
@@ -1037,11 +1183,11 @@ static int launch_lif(micloc_xylo *c, const int8_t *spikes, long long B, long lo
     dim3 grid((unsigned)B, (unsigned)nchunks);
 #define MICLOC_LIF_CASE(WW)                                                                                       \
     case WW: {                                                                                                    \
-        auto kern = raster ? (c->sat_isyn ? k_xylo_lif<SIGNED_IN, WW, true, true> : k_xylo_lif<SIGNED_IN, WW, false, true>)   \
-                           : (c->sat_isyn ? k_xylo_lif<SIGNED_IN, WW, true, false> : k_xylo_lif<SIGNED_IN, WW, false, false>); \
+        auto kern = raster ? (c->sat_isyn ? k_xylo_lif<SIGNED_IN, WW, true, true, STATE> : k_xylo_lif<SIGNED_IN, WW, false, true, STATE>)   \
+                           : (c->sat_isyn ? k_xylo_lif<SIGNED_IN, WW, true, false, STATE> : k_xylo_lif<SIGNED_IN, WW, false, false, STATE>); \
         MICLOC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));          \
         kern<<<grid, threads, smem, st>>>(spikes, c->CT, c->p.bipolar, c->N_in, c->d_w, c->d_thr, c->d_ds, c->d_dm, \
-                                          c->d_bias, c->max_spikes, N, npb, T, raster, counts);                   \
+                                          c->d_bias, c->max_spikes, N, npb, T, raster, counts, rows_b, nstate);   \
     } break
     switch (W) {
         MICLOC_LIF_CASE(1);
@@ -1056,14 +1202,20 @@ static int launch_lif(micloc_xylo *c, const int8_t *spikes, long long B, long lo
     return MICLOC_OK;
 }
 
+static int check_peak_win(const micloc_xylo *c, const int32_t *doa_peak, int win) {
+    if (doa_peak && (win < 1 || (win & 1) == 0 || win > c->G / 2))
+        return set_error(MICLOC_ERR_CONFIG, "averaging window size should be odd and at most half the DoA grid");  // utils.py:103-111
+    return MICLOC_OK;
+}
+
 static int launch_doa(micloc_xylo *c, const int32_t *counts, long long B, int32_t *doa, int32_t *doa_peak, int win,
-                      cudaStream_t st) {
+                      cudaStream_t st, const int32_t *rows_b = nullptr) {
     if (!doa && !doa_peak) return MICLOC_OK;
     if (doa_peak && (win < 1 || (win & 1) == 0 || win > c->G / 2))
         return set_error(MICLOC_ERR_CONFIG, "averaging window size should be odd and at most half the DoA grid");  // utils.py:103-111
     const size_t smem = (size_t)c->G * sizeof(long long);
     MICLOC_CUDA(cudaFuncSetAttribute(k_xylo_doa, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_xylo_doa<<<(unsigned)B, 128, smem, st>>>(counts, c->G, c->F, doa_peak ? win : 0, doa, doa_peak);
+    k_xylo_doa<<<(unsigned)B, 128, smem, st>>>(counts, c->G, c->F, doa_peak ? win : 0, doa, doa_peak, rows_b);
     count_launch(1);
     MICLOC_CUDA(cudaGetLastError());
     return MICLOC_OK;
@@ -1112,10 +1264,10 @@ static int exact_front_staged(micloc_xylo *c, const void *a, int dtype, long lon
 
 // exact float64 front end, fast form: register-blocked STHT (q in HBM) + one warp per clip for everything behind it;
 // clips whose clusters overflow the streaming encoder are redone by the unbounded staged kernels
-static bool chain_f64_supported(const micloc_xylo *c) {
-    return c->n_g > 0 && c->n_g % 4 == 0 && c->nba >= 1 && c->nba <= 5 && c->CT <= 64 && c->p.M <= 32 &&
-           !getenv("MICLOC_XYLO_STAGED_F64");
+static bool chain_f64_geometry(const micloc_xylo *c) {
+    return c->n_g > 0 && c->n_g % 4 == 0 && c->nba >= 1 && c->nba <= 5 && c->CT <= 64 && c->p.M <= 32;
 }
+static bool chain_f64_supported(const micloc_xylo *c) { return chain_f64_geometry(c) && !getenv("MICLOC_XYLO_STAGED_F64"); }
 
 template <typename IN_T>
 static int launch_front_f64(micloc_xylo *c, const IN_T *a, long long nb, long long T, int8_t *sgn, int32_t *flg, cudaStream_t st) {
@@ -1242,5 +1394,279 @@ extern "C" int micloc_xylo_process(micloc_xylo *c, const int8_t *spikes_in_dev, 
     if (!counts) { MICLOC_TRY(c->counts.reserve((size_t)B * c->N * sizeof(int32_t))); counts = (int32_t *)c->counts.ptr; }
     MICLOC_TRY(launch_lif<false>(c, spikes_in_dev, B, T, raster_dev, counts, st));
     MICLOC_TRY(launch_doa(c, counts, B, doa_dev, doa_peak_dev, peak_win, st));
+    return MICLOC_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Xylo stream batches: S continuous recordings through the exact front end and the integer network, one push per
+// frame tick (see include/micloc_b200.h).  Per push: k_stream_assemble (float64 rows) -> k_stht_f64_sparse over the
+// frame rows only -> k_xylo_chain_f64<STREAM> -> k_xylo_lif(_mma)<STATE> -> [k_xylo_doa] -> [k_xylo_split].
+// ---------------------------------------------------------------------------
+namespace micloc {
+// fresh chain state, LIF state, ring, position and flags of the selected slots (sel == nullptr: all); one thread per
+// (slot, j < max(CT, N, ring bytes / 16))
+__global__ void __launch_bounds__(256)
+k_xylo_streams_reset(XyloChanState *__restrict__ state, int2 *__restrict__ nstate, int8_t *__restrict__ ring,
+                     SlotPos *__restrict__ pos, int32_t *__restrict__ flags, const int32_t *__restrict__ sel, long long S,
+                     int CT, int N, int ring16, int W) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= S * W) return;
+    const long long s = i / W;
+    const int j = (int)(i % W);
+    if (sel && !sel[s]) return;
+    if (j < CT) {
+        XyloChanState &g = state[s * CT + j];
+        for (int k = 0; k < 5; ++k) g.zs[k] = 0.0;
+        g.cs = 0.0; g.rise = g.fall = -1;
+        rzcc_reset(g.rz);
+    }
+    if (j < N) nstate[s * N + j] = make_int2(0, 0);
+    if (j < ring16) reinterpret_cast<uint4 *>(ring)[s * ring16 + j] = make_uint4(0u, 0u, 0u, 0u);
+    if (j == 0) { pos[s] = SlotPos{0, 0, 1, 0}; flags[s] = 0; }
+}
+}  // namespace micloc
+
+struct micloc_xylo_streams {
+    micloc_xylo *c = nullptr;
+    int device = 0;
+    long long S = 0, max_frame = 0;
+    int hist = 0;                   // K - 1
+    int D = 0;                      // latency
+    int ring_len = 0;
+    int chain_warps = kChainWarps;  // slots per CTA of the chain kernel (fewer when float64 tiles of many microphones)
+    int xcur = 0, pcur = 0;
+    long long n_prev = 0;
+    std::vector<long long> N, F;    // host mirror of the positions (n_out without a device synchronisation)
+    std::vector<char> active;
+    std::vector<int32_t> sel_h;
+    double *xbuf[2] = {nullptr, nullptr}, *q = nullptr;
+    XyloChanState *state = nullptr;
+    int2 *nstate = nullptr;
+    int8_t *ring = nullptr, *sgn = nullptr;
+    SlotPos *pos[2] = {nullptr, nullptr};
+    int32_t *m = nullptr, *flags = nullptr, *sel = nullptr, *counts = nullptr;
+};
+
+extern "C" int micloc_xylo_streams_destroy(micloc_xylo_streams *xs) {
+    if (!xs) return MICLOC_OK;
+    cudaSetDevice(xs->device);
+    cudaFree(xs->xbuf[0]); cudaFree(xs->xbuf[1]); cudaFree(xs->q); cudaFree(xs->state); cudaFree(xs->nstate);
+    cudaFree(xs->ring); cudaFree(xs->sgn); cudaFree(xs->pos[0]); cudaFree(xs->pos[1]); cudaFree(xs->m);
+    cudaFree(xs->flags); cudaFree(xs->sel); cudaFree(xs->counts);
+    delete xs;
+    return MICLOC_OK;
+}
+
+static size_t xylo_stht_smem(const micloc_xylo *c) {
+    const int mgmax = c->p.M < kF64MG ? c->p.M : kF64MG;
+    return ((size_t)c->n_g + (size_t)mgmax * ((f64_pad(kSTile + c->p.K - 1) + 9) & ~1)) * sizeof(double);
+}
+
+// slots_host [n_slots] (NULL = every slot) -> xs->sel on the device (1 = listed); synchronises `st`
+static int xylo_upload_slots(micloc_xylo_streams *xs, const int32_t *slots_host, int32_t n_slots, cudaStream_t st) {
+    if (slots_host && n_slots < 0) return set_error(MICLOC_ERR_SHAPE, "n_slots %d < 0", n_slots);
+    for (int32_t i = 0; slots_host && i < n_slots; ++i)
+        if (slots_host[i] < 0 || slots_host[i] >= xs->S)
+            return set_error(MICLOC_ERR_SHAPE, "slot %d out of range [0, %lld)", slots_host[i], xs->S);
+    xs->sel_h.assign((size_t)xs->S, slots_host ? 0 : 1);
+    for (int32_t i = 0; slots_host && i < n_slots; ++i) xs->sel_h[(size_t)slots_host[i]] = 1;
+    MICLOC_CUDA(cudaMemcpyAsync(xs->sel, xs->sel_h.data(), (size_t)xs->S * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    MICLOC_CUDA(cudaStreamSynchronize(st));
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_xylo_streams_reset(micloc_xylo_streams *xs, const int32_t *slots_host, int32_t n_slots, void *stream) {
+    if (!xs) return set_error(MICLOC_ERR_CONFIG, "null stream batch");
+    MICLOC_CUDA(cudaSetDevice(xs->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (slots_host) MICLOC_TRY(xylo_upload_slots(xs, slots_host, n_slots, st));
+    const micloc_xylo *c = xs->c;
+    const int ring16 = (int)((long long)xs->ring_len * c->CT / 16);
+    const int W = std::max(std::max(c->CT, c->N), ring16);
+    k_xylo_streams_reset<<<(unsigned)((xs->S * W + 255) / 256), 256, 0, st>>>(
+        xs->state, xs->nstate, xs->ring, xs->pos[xs->pcur], xs->flags, slots_host ? xs->sel : nullptr, xs->S, c->CT, c->N,
+        ring16, W);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    MICLOC_CUDA(cudaStreamSynchronize(st));
+    for (long long s = 0; s < xs->S; ++s)
+        if (!slots_host || xs->sel_h[(size_t)s]) { xs->N[(size_t)s] = 0; xs->F[(size_t)s] = 0; xs->active[(size_t)s] = 1; }
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_xylo_streams_create(micloc_xylo *c, int32_t num_streams, int64_t max_frame_len, micloc_xylo_streams **out) {
+    if (!c || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
+    *out = nullptr;
+    if (num_streams < 1 || num_streams > 65535) return set_error(MICLOC_ERR_SHAPE, "num_streams %d out of range [1, 65535]", num_streams);
+    if (max_frame_len < 1 || max_frame_len > (1ll << 24)) return set_error(MICLOC_ERR_SHAPE, "max_frame_len out of range");
+    if (c->nba < 1) return set_error(MICLOC_ERR_CONFIG, "the exact front end needs the band filters in b/a form (n_ba)");
+    if (!chain_f64_geometry(c))
+        return set_error(MICLOC_ERR_UNSUPPORTED,
+                         "Xylo stream batches need the fast exact front end: a Hilbert kernel with every other tap zero "
+                         "(K a multiple of 8), len(b) <= 5, 2 M F <= 64 and M <= 32 (got K %d, len(b) %d, M %d, F %d)",
+                         c->p.K, c->nba, c->p.M, c->F);
+    if (xylo_stht_smem(c) > 227 * 1024) return set_error(MICLOC_ERR_UNSUPPORTED, "exact STHT tile needs too much shared memory");
+    MICLOC_CUDA(cudaSetDevice(c->device));
+    micloc_xylo_streams *xs = new micloc_xylo_streams();
+    xs->c = c; xs->device = c->device; xs->S = num_streams; xs->max_frame = max_frame_len;
+    xs->hist = c->p.K - 1;
+    const int w = c->p.w;
+    xs->D = (kF64Cluster - 1) * (w - 1) + w + kChainTile + kF64FlatTop / 2;
+    xs->ring_len = 64;
+    while (xs->ring_len < max_frame_len + xs->D) xs->ring_len <<= 1;
+    const size_t per_warp = (size_t)kChainTile * c->p.M * 2 * sizeof(double);
+    xs->chain_warps = (int)std::min<size_t>(kChainWarps, (size_t)(227 * 1024) / per_warp);
+    xs->N.assign((size_t)num_streams, 0); xs->F.assign((size_t)num_streams, 0); xs->active.assign((size_t)num_streams, 1);
+    const size_t S = (size_t)num_streams, M = (size_t)c->p.M, CT = (size_t)c->CT;
+    const size_t rows = (size_t)xs->hist + max_frame_len;
+    const size_t fin = (size_t)max_frame_len + xs->D;
+    bool ok = cudaMalloc(&xs->xbuf[0], S * rows * M * sizeof(double)) == cudaSuccess &&
+              cudaMalloc(&xs->xbuf[1], S * rows * M * sizeof(double)) == cudaSuccess &&
+              cudaMalloc(&xs->q, S * rows * M * sizeof(double)) == cudaSuccess &&
+              cudaMalloc(&xs->state, S * CT * sizeof(XyloChanState)) == cudaSuccess &&
+              cudaMalloc(&xs->nstate, S * c->N * sizeof(int2)) == cudaSuccess &&
+              cudaMalloc(&xs->ring, S * CT * (size_t)xs->ring_len) == cudaSuccess &&
+              cudaMalloc(&xs->sgn, S * fin * CT) == cudaSuccess &&
+              cudaMalloc(&xs->pos[0], S * sizeof(SlotPos)) == cudaSuccess &&
+              cudaMalloc(&xs->pos[1], S * sizeof(SlotPos)) == cudaSuccess &&
+              cudaMalloc(&xs->m, S * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&xs->flags, S * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&xs->sel, S * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&xs->counts, S * c->N * sizeof(int32_t)) == cudaSuccess;
+    if (!ok) { micloc_xylo_streams_destroy(xs); return set_error(MICLOC_ERR_CUDA, "cudaMalloc(Xylo stream batch) failed"); }
+    const int rc = micloc_xylo_streams_reset(xs, nullptr, 0, nullptr);
+    if (rc) { micloc_xylo_streams_destroy(xs); return rc; }
+    *out = xs;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_xylo_streams_latency(micloc_xylo_streams *xs) { return xs ? xs->D : 0; }
+
+// shared by push and flush: chain of the new samples (n = 0: flush of the slots in close_sel), then the integer
+// network, DoA and the {0,1} input spikes over each slot's final rows (row stride `rows`)
+template <int NBA>
+static void launch_chain_stream(micloc_xylo_streams *xs, const int32_t *close_sel, long long n, long long rows, cudaStream_t st) {
+    const micloc_xylo *c = xs->c;
+    const ChainParams &p = c->p;
+    XyloChainStream sa;
+    sa.state = xs->state; sa.pos_in = xs->pos[xs->pcur]; sa.pos_out = xs->pos[xs->pcur ^ 1]; sa.m_out = xs->m;
+    sa.close_sel = close_sel; sa.ring = xs->ring; sa.ring_len = xs->ring_len; sa.hist = xs->hist; sa.rows = (int)rows;
+    sa.D = xs->D;
+    const int nw = xs->chain_warps;
+    const size_t smem = (size_t)nw * kChainTile * p.M * 2 * sizeof(double);
+    cudaFuncSetAttribute(k_xylo_chain_f64<double, NBA, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    k_xylo_chain_f64<double, NBA, true><<<(unsigned)((xs->S + nw - 1) / nw), 32 * nw, smem, st>>>(
+        xs->xbuf[xs->xcur], xs->q, c->d_ba_b, c->d_ba_a, xs->sgn, xs->flags, p.M, p.half, c->nba, c->F, p.w, p.bipolar, xs->S,
+        n, sa);
+}
+
+static int xylo_streams_advance(micloc_xylo_streams *xs, const int32_t *close_sel, long long n, long long rows,
+                                int8_t *spikes_in_dev, uint8_t *raster_dev, int32_t *counts_dev, int32_t *doa_dev,
+                                int32_t *doa_peak_dev, int32_t peak_win, int32_t *flags_dev, cudaStream_t st) {
+    micloc_xylo *c = xs->c;
+    if (c->nba <= 3) launch_chain_stream<3>(xs, close_sel, n, rows, st);
+    else launch_chain_stream<5>(xs, close_sel, n, rows, st);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    xs->pcur ^= 1;
+    int32_t *counts = counts_dev ? counts_dev : xs->counts;
+    MICLOC_TRY((launch_lif<true, true>(c, xs->sgn, xs->S, rows, raster_dev, counts, st, xs->m, xs->nstate)));
+    MICLOC_TRY(launch_doa(c, counts, xs->S, doa_dev, doa_peak_dev, peak_win, st, xs->m));
+    if (spikes_in_dev) {
+        const long long r = xs->S * rows;
+        k_xylo_split<<<(unsigned)((r * c->CT + 255) / 256), 256, 0, st>>>(xs->sgn, spikes_in_dev, r, c->CT, c->p.bipolar, xs->m, rows);
+        count_launch(1);
+        MICLOC_CUDA(cudaGetLastError());
+    }
+    if (flags_dev) MICLOC_CUDA(cudaMemcpyAsync(flags_dev, xs->flags, (size_t)xs->S * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_xylo_streams_push(micloc_xylo_streams *xs, const void *frames_dev, int dtype, int64_t n, int32_t in_channels,
+                                        int8_t *spikes_in_dev, uint8_t *raster_dev, int32_t *counts_dev, int32_t *doa_dev,
+                                        int32_t *doa_peak_dev, int32_t peak_win, int32_t *flags_dev, int64_t *n_out_host,
+                                        void *stream) {
+    if (!xs || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
+    micloc_xylo *c = xs->c;
+    const ChainParams &p = c->p;
+    if (n < 1 || n > xs->max_frame) return set_error(MICLOC_ERR_SHAPE, "frame of %lld samples (stream takes 1..%lld)", (long long)n, xs->max_frame);
+    if (!frames_dev) return set_error(MICLOC_ERR_SHAPE, "null frame pointer");
+    if (in_channels < p.M)
+        return set_error(MICLOC_ERR_SHAPE, "number of channels in the input siganl %d should be the same as the number of microphones %d!", in_channels, p.M);
+    if (dtype != MICLOC_F32 && dtype != MICLOC_I16 && dtype != MICLOC_I32)
+        return set_error(MICLOC_ERR_SHAPE, "dtype must be MICLOC_F32, MICLOC_I16 or MICLOC_I32");
+    for (long long s = 0; s < xs->S; ++s)
+        if (xs->active[(size_t)s] && xs->N[(size_t)s] + n >= (1ll << 31) - 4096)
+            return set_error(MICLOC_ERR_SHAPE, "stream position exceeds 2^31 samples: reset the stream");
+    MICLOC_TRY(check_peak_win(c, doa_peak_dev, peak_win));
+    MICLOC_CUDA(cudaSetDevice(xs->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    // [K-1 history rows | frame] in float64
+    const int nxt = xs->xcur ^ 1;
+    const long long total = xs->S * (xs->hist + n) * p.M;
+    const unsigned ga = (unsigned)((total + 255) / 256);
+    const double *prev = xs->xbuf[xs->xcur];
+    const SlotPos *pos = xs->pos[xs->pcur];
+    if (dtype == MICLOC_F32)
+        k_stream_assemble<float, double><<<ga, 256, 0, st>>>((const float *)frames_dev, prev, xs->xbuf[nxt], pos, xs->S, (int)n, (int)xs->n_prev, in_channels, p.M, xs->hist);
+    else if (dtype == MICLOC_I16)
+        k_stream_assemble<int16_t, double><<<ga, 256, 0, st>>>((const int16_t *)frames_dev, prev, xs->xbuf[nxt], pos, xs->S, (int)n, (int)xs->n_prev, in_channels, p.M, xs->hist);
+    else
+        k_stream_assemble<int32_t, double><<<ga, 256, 0, st>>>((const int32_t *)frames_dev, prev, xs->xbuf[nxt], pos, xs->S, (int)n, (int)xs->n_prev, in_channels, p.M, xs->hist);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    xs->xcur = nxt;
+    xs->n_prev = n;
+    // STHT of the frame rows only (the history rows were the previous push's frame rows)
+    {
+        const long long rows_in = xs->hist + n;
+        const int ntiles = (int)((n + kSTile - 1) / kSTile);
+        const size_t smem = xylo_stht_smem(c);
+        dim3 grid((unsigned)(xs->S * ntiles), (unsigned)((p.M + kF64MG - 1) / kF64MG));
+        MICLOC_CUDA(cudaFuncSetAttribute(k_stht_f64_sparse<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_stht_f64_sparse<double><<<grid, 256, smem, st>>>(xs->xbuf[xs->xcur], c->d_g, xs->q, p.M, p.K, c->n_g, rows_in, ntiles,
+                                                          (long long)xs->hist);
+        count_launch(1);
+        MICLOC_CUDA(cudaGetLastError());
+    }
+    const long long rows = n + xs->D;
+    MICLOC_TRY(xylo_streams_advance(xs, nullptr, n, rows, spikes_in_dev, raster_dev, counts_dev, doa_dev, doa_peak_dev,
+                                    peak_win, flags_dev, st));
+    for (long long s = 0; s < xs->S; ++s) {
+        const size_t i = (size_t)s;
+        n_out_host[s] = 0;
+        if (!xs->active[i]) continue;
+        xs->N[i] += n;
+        const long long f = xs->N[i] - xs->D > xs->F[i] ? xs->N[i] - xs->D : xs->F[i];
+        n_out_host[s] = f - xs->F[i];
+        xs->F[i] = f;
+    }
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_xylo_streams_flush(micloc_xylo_streams *xs, const int32_t *slots_host, int32_t n_slots,
+                                         int8_t *spikes_in_dev, uint8_t *raster_dev, int32_t *counts_dev, int32_t *doa_dev,
+                                         int32_t *doa_peak_dev, int32_t peak_win, int32_t *flags_dev, int64_t *n_out_host,
+                                         int32_t *flags_host, void *stream) {
+    if (!xs || !n_out_host) return set_error(MICLOC_ERR_CONFIG, "null stream batch");
+    MICLOC_TRY(check_peak_win(xs->c, doa_peak_dev, peak_win));
+    MICLOC_CUDA(cudaSetDevice(xs->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    MICLOC_TRY(xylo_upload_slots(xs, slots_host, n_slots, st));
+    const long long rows = xs->max_frame + xs->D;
+    MICLOC_TRY(xylo_streams_advance(xs, xs->sel, 0, rows, spikes_in_dev, raster_dev, counts_dev, doa_dev, doa_peak_dev,
+                                    peak_win, flags_dev, st));
+    for (long long s = 0; s < xs->S; ++s) {
+        const size_t i = (size_t)s;
+        n_out_host[s] = 0;
+        if (!xs->active[i] || !xs->sel_h[i]) continue;
+        n_out_host[s] = xs->N[i] - xs->F[i];
+        xs->F[i] = xs->N[i];
+        xs->active[i] = 0;
+    }
+    if (flags_host) {
+        MICLOC_CUDA(cudaMemcpyAsync(flags_host, xs->flags, (size_t)xs->S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        MICLOC_CUDA(cudaStreamSynchronize(st));
+    }
     return MICLOC_OK;
 }

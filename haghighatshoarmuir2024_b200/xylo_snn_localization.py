@@ -227,6 +227,138 @@ class XyloEngine:
         return {"counts": counts, "doa": doa, "doa_peak": doa_peak, "raster": raster}
 
 
+class XyloStreamBatch:
+    """`num_streams` independent recordings ("slots") through the exact (float64) front end and the integer network
+    with their state carried across pushes (micloc_xylo_streams_*).  N pushed frames plus a flush give, for every slot,
+    bit for bit what `XyloEngine.run(exact=True)` gives on one clip of their concatenation (in-phase branch: the causal
+    delay x[t - K/2]); results lag the input by `latency` samples.  Slot lists, positions, flushed slots and unwritten
+    rows as in `MultibandStreamBatch`.  Frames are [num_streams, n, channels] device tensors, int32 / int16 / float32
+    (channels beyond the microphones are dropped).
+
+    `fs` and `doa_list` (the DoA grid, radians) serve the per-call estimators: rate [S, G] as `Demo.extract_rate` over
+    each slot's final samples, periodic_ml / trimmed_periodic_ml [S] as `Demo.estimate_doa_from_rate` (through
+    micloc_power_fuse: the angle is scale-free, so the band-summed counts go in as they are)."""
+
+    def __init__(self, engine: XyloEngine, num_streams: int, max_frame_len: int, fs: float = 48_000.0,
+                 doa_list: Optional[np.ndarray] = None):
+        self.engine = engine
+        self.num_streams = int(num_streams)
+        self.max_frame_len = int(max_frame_len)
+        self.device = engine.device
+        self.fs = float(fs)
+        self.M, self.F, self.G, self.N, self.N_in = engine.M, engine.F, engine.G, engine.N, engine.N_in
+        self._lib = N.lib()
+        h = C.c_void_p()
+        rc = self._lib.micloc_xylo_streams_create(engine._h, self.num_streams, self.max_frame_len, C.byref(h))
+        if rc in (N.ERR_CONFIG, N.ERR_UNSUPPORTED):
+            raise N.MiclocError(rc, self._lib.micloc_last_error().decode("utf-8", "replace"))
+        N.check(rc)
+        self._h = h
+        self.latency = int(self._lib.micloc_xylo_streams_latency(h))
+        self._doa_dev = None
+        if doa_list is not None:
+            doa_list = np.ascontiguousarray(doa_list, dtype=np.float64)
+            if doa_list.shape != (self.G,):
+                raise ValueError(f"doa_list should hold {self.G} angles")
+            self._doa_dev = torch.from_numpy(doa_list).to(self.device)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.micloc_xylo_streams_destroy(self._h)
+            self._h = None
+
+    __del__ = close
+
+    @staticmethod
+    def _slots(slots):
+        if slots is None:
+            return None, None, 0
+        arr = np.ascontiguousarray(np.atleast_1d(np.asarray(slots)), dtype=np.int32)
+        return arr, arr.ctypes.data_as(C.c_void_p), len(arr)
+
+    def reset(self, slots=None):
+        """Fresh state for the listed slots (None: all); they restart at sample 0."""
+        arr, p, n = self._slots(slots)
+        N.check(self._lib.micloc_xylo_streams_reset(self._h, p, n, self.engine._stream()))
+
+    def _outputs(self, rows, want_spikes_in, want_raster, peak_win):
+        S, dev = self.num_streams, self.device
+        return {"spikes_in": torch.empty((S, rows, self.N_in), dtype=torch.int8, device=dev) if want_spikes_in else None,
+                "raster": torch.empty((S, rows, self.N), dtype=torch.uint8, device=dev) if want_raster else None,
+                "counts": torch.zeros((S, self.N), dtype=torch.int32, device=dev),
+                "doa": torch.full((S,), -1, dtype=torch.int32, device=dev),          # -1: not written (n_out == 0)
+                "doa_peak": torch.full((S,), -1, dtype=torch.int32, device=dev) if peak_win else None,
+                "flags": torch.empty(S, dtype=torch.int32, device=dev)}
+
+    def _estimators(self, out, n_out):
+        """rate [S, G] (Demo.extract_rate over the final samples) and the periodic-ML estimators; NaN where n_out == 0."""
+        S, F, G = self.num_streams, self.F, self.G
+        cnt = out["counts"].view(S, F, G)
+        n = torch.from_numpy(n_out).to(self.device)
+        live = n > 0
+        rate = cnt.sum(1, dtype=torch.int64).double() * self.fs / (F * n.clamp(min=1).double()).unsqueeze(1)
+        out["rate"] = torch.where(live.unsqueeze(1), rate, torch.full_like(rate, float("nan")))
+        fflags = torch.zeros(S, dtype=torch.int32, device=self.device)
+        if self._doa_dev is not None:
+            power = cnt.permute(1, 0, 2).float().contiguous()                       # [F][S][G]
+            ml = torch.empty(S, dtype=torch.float64, device=self.device)
+            trimmed = torch.empty(S, dtype=torch.float64, device=self.device)
+            N.check(self._lib.micloc_power_fuse(_ptr(power), F, S, G, _ptr(self._doa_dev), None, None, _ptr(ml),
+                                                _ptr(trimmed), _ptr(fflags), self.device.index or 0, self.engine._stream()))
+            nan = torch.full_like(ml, float("nan"))
+            out["periodic_ml"] = torch.where(live, ml, nan)
+            out["trimmed_periodic_ml"] = torch.where(live, trimmed, nan)
+            fflags = torch.where(live, fflags & 2, torch.zeros_like(fflags))
+        return fflags
+
+    def push(self, frames: torch.Tensor, want_spikes_in: bool = False, want_raster: bool = False,
+             peak_win: int = 0) -> Dict[str, object]:
+        """One frame per slot in, the samples that became final out: n_out (numpy int64 [S]), counts [S, N] (zero
+        where n_out == 0), doa / doa_peak [S] (-1 where n_out == 0), rate [S, G], periodic_ml / trimmed_periodic_ml
+        [S] (with a doa_list; NaN where n_out == 0), flags [S] (bit 0: the slot's results are not guaranteed to be the
+        clip's bits since its reset; bit 1: the trimmed estimator's IndexError, estimate NaN), spikes_in [S, n + D,
+        N_in] / raster [S, n + D, N] on request (slot s fills its first n_out[s] rows).  No host synchronisation
+        beyond the row counts."""
+        if frames.dim() != 3 or frames.shape[2] < self.M:
+            raise ValueError(
+                f"number of channels in the input siganl {frames.shape[-1]} should be the same as the number of microphones {self.M}!")
+        if frames.shape[0] != self.num_streams:
+            raise ValueError(f"frames hold {frames.shape[0]} slots, the batch has {self.num_streams}")
+        if frames.device != self.device:
+            raise ValueError(f"frames live on {frames.device}, the batch on {self.device}")
+        dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frames.dtype)
+        if dt is None:
+            raise ValueError(f"frames must be float32, int16 or int32, got {frames.dtype}")
+        frames = frames.contiguous()
+        S, n, ch = frames.shape
+        out = self._outputs(n + self.latency, want_spikes_in, want_raster, peak_win)
+        n_out = np.zeros(S, dtype=np.int64)
+        N.check(self._lib.micloc_xylo_streams_push(
+            self._h, _ptr(frames), dt, n, ch, _ptr(out["spikes_in"]), _ptr(out["raster"]), _ptr(out["counts"]),
+            _ptr(out["doa"]), _ptr(out["doa_peak"]), int(peak_win), _ptr(out["flags"]), n_out.ctypes.data_as(C.c_void_p),
+            self.engine._stream()))
+        out["flags"] = out["flags"] | self._estimators(out, n_out)
+        out["n_out"] = n_out
+        return out
+
+    def flush(self, slots=None, want_spikes_in: bool = False, want_raster: bool = False,
+              peak_win: int = 0) -> Dict[str, object]:
+        """End of the listed recordings (None: all): their remaining samples as in `push` (rows: max_frame_len +
+        latency).  'flags' is numpy int32 [S] on the host: bit 0 as in push, bit 1 the trimmed estimator's IndexError
+        on the flushed samples."""
+        arr, p, ns = self._slots(slots)
+        out = self._outputs(self.max_frame_len + self.latency, want_spikes_in, want_raster, peak_win)
+        n_out = np.zeros(self.num_streams, dtype=np.int64)
+        flags = np.zeros(self.num_streams, dtype=np.int32)
+        N.check(self._lib.micloc_xylo_streams_flush(
+            self._h, p, ns, _ptr(out["spikes_in"]), _ptr(out["raster"]), _ptr(out["counts"]), _ptr(out["doa"]),
+            _ptr(out["doa_peak"]), int(peak_win), _ptr(out["flags"]), n_out.ctypes.data_as(C.c_void_p),
+            flags.ctypes.data_as(C.c_void_p), self.engine._stream()))
+        fflags = self._estimators(out, n_out).cpu().numpy()
+        out.update({"n_out": n_out, "flags": flags | fflags})
+        return out
+
+
 class Demo:
     """Same constructor and processing methods as the reference's `Demo`
     (micloc/xylo_snn_localization.py:74-444); `localize` is the batched call."""
@@ -318,6 +450,10 @@ class Demo:
         num_DoA = len(self.doa_list) // 2
         DoA_range = np.arange(-num_DoA // 2, num_DoA // 2 + 1) - DoA_index
         return np.angle(np.mean(spike_rate[DoA_range] * np.exp(1j * self.doa_list[DoA_range])))
+
+    def stream_batch(self, num_streams: int, max_frame_len: int) -> XyloStreamBatch:
+        """`num_streams` continuous recordings through this network's exact chain, one push per frame tick."""
+        return XyloStreamBatch(self.engine, num_streams, max_frame_len, fs=self.fs, doa_list=self.doa_list)
 
     def localize(self, audio: torch.Tensor, peak_win: int = 0, exact: Optional[bool] = None):
         """Batched chain: audio [B,T,M] CUDA tensor -> dict(counts, doa, doa_peak, flags)."""

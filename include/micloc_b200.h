@@ -357,6 +357,59 @@ int micloc_xylo_process(micloc_xylo *ctx, const int8_t *spikes_in_dev, int64_t B
                         uint8_t *raster_dev, int32_t *counts_dev, int32_t *doa_dev,
                         int32_t *doa_peak_dev, int32_t peak_win, void *stream);
 
+/* ---- Xylo stream batches: many live recordings through the bit-exact integer chain ------------------------------ */
+/* A Xylo stream batch holds S independent slots (1 <= S <= 65535) on one micloc_xylo context; each slot is one
+ * continuous recording through the EXACT (float64) front end and the integer network.
+ *   - Concatenation rule: N pushed frames plus a flush give, for every slot, what micloc_xylo_run(exact = 1) gives on
+ *     one clip of their concatenation -- signed input spikes, hidden raster and (summed over the calls) hidden spike
+ *     counts, bit for bit -- with the usual stream differences: the in-phase branch is the causal delay x[t - K/2]
+ *     (zeros before the slot starts; identical to np.roll whenever the clip's last K/2 samples are zero), and results
+ *     lag the input by D = micloc_xylo_streams_latency() samples.  Band-filter delays, running sum, flat-top starts,
+ *     open candidate clusters (kF64Cluster = 32 per polarity) and I_syn / V_mem carry over.  The sample path is float64
+ *     from the frame on, so int32 wav samples beyond 2^24 are taken exactly.
+ *   - Latency: D = (kF64Cluster - 1)(w - 1) + w + 64 + 32 with w = robust_width: a cluster of up to 32 candidates
+ *     spaced by at most w - 1, the distance w that closes it, the 64-sample tile of the chain kernel and a flat-top
+ *     allowance of 64 samples (a candidate sits at the midpoint of its flat top).  At the end of a push, every spike at
+ *     a position below N_s - D has been emitted, or the slot's flags bit 0 is set: the kernel checks the earliest
+ *     position a spike can still take (the first candidate of an open cluster, the midpoint of an open flat top or
+ *     bottom) against N_s - D, and sets the bit as well when a cluster overflows its 32 candidates (where the one-shot
+ *     path redoes the clip with the unbounded kernels).  Bit 0 stays set until the slot is reset.
+ *     INVARIANT: bit 0 clear => the slot's results are the clip's bits.  A push never synchronises nor redoes anything.
+ *   - Slots, positions, flushed slots, n_out_host and unwritten rows as in micloc_snn_streams_*: slots_host [n_slots]
+ *     (NULL = every slot); a slot reset mid-run restarts at 0 while the others go on; a flushed slot ignores later pushes
+ *     (n_out = 0, state untouched) until it is reset; n_out_host[s] (host, computed without a synchronisation) is the
+ *     number of samples of slot s that became final with this call; reset and flush synchronise `stream`, a push does
+ *     not; a push that would take a slot's position to 2^31 - 4096 samples or beyond is refused.
+ *   - push: frames_dev [S][n][in_channels] float32 / int16 / int32, 1 <= n <= max_frame_len (channels >= num_mic are
+ *     dropped).  Outputs, all nullable device pointers, over the n_out_host[s] final samples of slot s:
+ *       spikes_in_dev [S][n + D][N_in] int8 {0,1} (Demo.spike_encoding's layout);  raster_dev [S][n + D][N] uint8;
+ *       counts_dev [S][N] int32 hidden spikes over those samples;  doa_dev / doa_peak_dev [S] int32: first argmax of the
+ *       band-summed counts / utils.find_peak_location of them (peak_win odd, at most G / 2);  flags_dev [S] int32 bit 0
+ *       as above.  Rows past n_out_host[s], and counts / doa / doa_peak of a slot with n_out = 0, are NOT written.
+ *   - flush closes the listed slots like a clip end; outputs as in push with [S][max_frame_len + D] rows; flags_host [S]
+ *     (nullable, host, synchronises) = the flags after the flush.
+ *   - create: MICLOC_ERR_CONFIG without the b/a band filters (n_ba == 0); MICLOC_ERR_UNSUPPORTED where the fast exact
+ *     front end does not apply (a Hilbert kernel with every other tap zero and K a multiple of 8, n_ba <= 5,
+ *     2 M F <= 64, M <= 32).
+ * Kernel launches per push, whatever S: 4 (frame assembly, STHT of the frame rows, band filters + cumsum + find_peaks,
+ * integer network), +1 (DoA) when doa_dev or doa_peak_dev is given, +1 (pos / neg split) when spikes_in_dev is given.
+ * Device memory: 3 S (K - 1 + max_frame_len) M float64 (two assembly buffers and the STHT), S 2 M F x 856 bytes of chain
+ * state, S N x 8 bytes of neuron state, S 2 M F (R + max_frame_len + D) bytes of spike ring and raster (R = the
+ * power of two >= max_frame_len + D, at least 64), S N x 4 bytes of counts.  The batch uses its context's constants:
+ * destroy it before the context. */
+typedef struct micloc_xylo_streams micloc_xylo_streams;
+int micloc_xylo_streams_create(micloc_xylo *ctx, int32_t num_streams, int64_t max_frame_len, micloc_xylo_streams **out);
+int micloc_xylo_streams_destroy(micloc_xylo_streams *xs);
+int micloc_xylo_streams_latency(micloc_xylo_streams *xs);
+int micloc_xylo_streams_reset(micloc_xylo_streams *xs, const int32_t *slots_host, int32_t n_slots, void *stream);
+int micloc_xylo_streams_push(micloc_xylo_streams *xs, const void *frames_dev, int dtype, int64_t n, int32_t in_channels,
+                             int8_t *spikes_in_dev, uint8_t *raster_dev, int32_t *counts_dev, int32_t *doa_dev,
+                             int32_t *doa_peak_dev, int32_t peak_win, int32_t *flags_dev, int64_t *n_out_host, void *stream);
+int micloc_xylo_streams_flush(micloc_xylo_streams *xs, const int32_t *slots_host, int32_t n_slots,
+                              int8_t *spikes_in_dev, uint8_t *raster_dev, int32_t *counts_dev, int32_t *doa_dev,
+                              int32_t *doa_peak_dev, int32_t peak_win, int32_t *flags_dev, int64_t *n_out_host,
+                              int32_t *flags_host, void *stream);
+
 /* ---- misc ------------------------------------------------------------------ */
 const char *micloc_last_error(void);
 int micloc_version(void);
