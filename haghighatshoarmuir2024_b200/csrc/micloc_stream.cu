@@ -17,7 +17,8 @@
 //
 // A STREAM BATCH carries S such recordings ("slots") at once; the single stream (micloc_snn_stream_*) is a batch of
 // one.  Slots are independent (own position, reset and flush), but a push hands every slot one frame of the same
-// length n, so that one launch per stage serves all of them.  Per push, whatever S:
+// length n, so that one launch per stage serves all of them.  A batch is a SlotBook (micloc_stream.cuh: positions,
+// slot lists, frame checks, host mirror) plus one StreamBand (the chain's device state).  Per push, whatever S:
 //   k_stream_assemble        [K-1 history rows | frame] of every slot (from the previous push's buffer: ping-pong)
 //   STHT                     launch_stht_any over S clips of K-1+n rows
 //   k_stream_blk             band-pass + RZCC of the new samples, then the neuron filter of the final ones
@@ -25,10 +26,11 @@
 //   k_dense, k_envelope, k_argmax_rows                                      (when env or doa_t is requested)
 //
 // A MULTI-BAND STREAM BATCH (micloc_snn_mb_streams_*) is the live localiser of micloc/localization_demo_snn.py:125-193
-// made continuous: a Butterworth filterbank on the raw frame, one chain per band, power summed over the bands.  It owns
-// one stream batch per band, created with a common latency D = max_f rzcc_lag(w_f) so that every band finalises the
-// same samples in a push, and replaces their frame assembly by one kernel that runs the filterbank with its state
-// carried across pushes and writes every band's [history | frame] rows (k_mb_stream_assemble).  Per push, whatever S:
+// made continuous: a Butterworth filterbank on the raw frame, one chain per band, power summed over the bands.  It is
+// one SlotBook plus F StreamBands; the book's latency D = max_f rzcc_lag(w_f) is common, so every band finalises the
+// same samples in a push and every band's k_stream_blk writes the same positions and row counts.  One kernel runs the
+// filterbank with its state carried across pushes and writes every band's [history | frame] rows
+// (k_mb_stream_assemble).  Per push, whatever S:
 //   k_mb_stream_assemble                                                    1
 //   per band: STHT, k_stream_blk, k_gram, k_power_argmax (into band f's slice of [F][S][G])   4 F
 //   k_power_fuse       sum over bands, argmax, periodic-ML estimators over each slot's final rows   1
@@ -294,7 +296,8 @@ k_stream_blk(const float *__restrict__ xbuf, const float *__restrict__ q, ChanSt
     }
 }
 
-// fresh state for the selected slots (sel == nullptr: all): one thread per (slot, j < max(C2, G))
+// fresh state for the selected slots (sel == nullptr: all): one thread per (slot, j < max(C2, G)); pos == nullptr:
+// the positions are left alone (the bands of a multi-band batch share them: one band's reset writes them)
 __global__ void __launch_bounds__(256)
 k_stream_reset(ChanState *__restrict__ state, SlotPos *__restrict__ pos, int32_t *__restrict__ flags,
                float *__restrict__ env_state, int32_t *__restrict__ env_started, const int32_t *__restrict__ sel,
@@ -313,7 +316,10 @@ k_stream_reset(ChanState *__restrict__ state, SlotPos *__restrict__ pos, int32_t
         for (int k = 0; k < 2 * kClusterMax; ++k) { c.cl_pos[k] = 0; c.cl_h[k] = 0.f; }
     }
     if (j < G) { env_state[s * G + j] = 0.f; env_started[s * G + j] = 0; }
-    if (j == 0) { pos[s] = SlotPos{0, 0, 1, 0}; flags[s] = 0; }
+    if (j == 0) {
+        if (pos) pos[s] = SlotPos{0, 0, 1, 0};
+        flags[s] = 0;
+    }
 }
 
 }  // namespace micloc
@@ -371,28 +377,25 @@ k_argmax_rows(const float *__restrict__ env, int32_t *__restrict__ idx, const in
 
 using namespace micloc;
 
-struct micloc_stream_batch {
-    micloc_snn_params prm{};        // copy of what the kernels need from the parent context
-    int device = 0;
-    long long S = 0;
-    long long max_frame = 0;
+// one band's chain over the slots of a SlotBook: its [history | frame] buffers, STHT output, chain state, spike ring,
+// membrane, flags, Gram and envelope
+struct StreamBand {
+    micloc_snn_params prm{};        // copy of what the kernels need from the band's context
     int hist = 0;                   // K - 1
-    int D = 0;                      // output latency in samples
     int ring_len = 0;
-    int xcur = 0;                   // xbuf[xcur] holds the newest [history | frame] rows (n_prev frame rows)
-    int pcur = 0;                   // pos[pcur] holds the slots' positions
-    long long n_prev = 0;
-    std::vector<long long> N, F;    // host mirror of the positions (n_out without a device synchronisation)
-    std::vector<char> active;
-    std::vector<int32_t> sel_h;     // staging of the slot lists
     float *xbuf[2] = {nullptr, nullptr}, *q = nullptr, *vmem = nullptr, *env_state = nullptr;
     int8_t *ring = nullptr;
     ChanState *state = nullptr;
-    SlotPos *pos[2] = {nullptr, nullptr};
-    int32_t *m = nullptr, *flags = nullptr, *sel = nullptr, *env_started = nullptr;
+    int32_t *flags = nullptr, *env_started = nullptr;
     double *gram = nullptr;
     DevBuf y, env;                  // envelope scratch: allocated on the first request, grow-only
     float rise_time = 10e-3f, fall_time = 100e-3f, fs = 48000.f;
+};
+
+struct micloc_stream_batch {
+    int device = 0;
+    SlotBook book;
+    StreamBand band;
 };
 
 // the single stream: a batch of one slot
@@ -400,131 +403,101 @@ struct micloc_stream {
     micloc_stream_batch *sb = nullptr;
 };
 
-extern "C" int micloc_snn_streams_destroy(micloc_stream_batch *sb) {
-    if (!sb) return MICLOC_OK;
-    cudaSetDevice(sb->device);
-    cudaFree(sb->xbuf[0]); cudaFree(sb->xbuf[1]); cudaFree(sb->q); cudaFree(sb->vmem); cudaFree(sb->env_state);
-    cudaFree(sb->ring); cudaFree(sb->state); cudaFree(sb->pos[0]); cudaFree(sb->pos[1]); cudaFree(sb->m);
-    cudaFree(sb->flags); cudaFree(sb->sel); cudaFree(sb->env_started); cudaFree(sb->gram);
-    sb->y.release(); sb->env.release();
-    delete sb;
-    return MICLOC_OK;
+static void band_free(StreamBand &b) {
+    cudaFree(b.xbuf[0]); cudaFree(b.xbuf[1]); cudaFree(b.q); cudaFree(b.vmem); cudaFree(b.env_state);
+    cudaFree(b.ring); cudaFree(b.state); cudaFree(b.flags); cudaFree(b.env_started); cudaFree(b.gram);
+    b.y.release(); b.env.release();
 }
 
-// slots_host [n_slots] (NULL = every slot) -> sb->sel on the device (1 = listed); synchronises `st`: the staging
-// vector is reused by the next call
-static int upload_slots(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots, cudaStream_t st) {
-    if (slots_host && n_slots < 0) return set_error(MICLOC_ERR_SHAPE, "n_slots %d < 0", n_slots);
-    for (int32_t i = 0; slots_host && i < n_slots; ++i)
-        if (slots_host[i] < 0 || slots_host[i] >= sb->S)
-            return set_error(MICLOC_ERR_SHAPE, "slot %d out of range [0, %lld)", slots_host[i], sb->S);
-    sb->sel_h.assign((size_t)sb->S, slots_host ? 0 : 1);
-    for (int32_t i = 0; slots_host && i < n_slots; ++i) sb->sel_h[(size_t)slots_host[i]] = 1;
-    MICLOC_CUDA(cudaMemcpyAsync(sb->sel, sb->sel_h.data(), (size_t)sb->S * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    MICLOC_CUDA(cudaStreamSynchronize(st));
-    return MICLOC_OK;
+// the band's buffers for the book's slots, frame length and latency
+static int band_alloc(StreamBand &b, const micloc_snn_params &prm, const SlotBook &bk) {
+    b.prm = prm;
+    const ChainParams &p = prm.chain;
+    b.hist = p.K - 1;
+    const long long need = bk.max_frame + bk.D + p.nL + 2 * kSeg;
+    b.ring_len = 32;
+    while (b.ring_len < need) b.ring_len <<= 1;
+    const size_t S = (size_t)bk.S;
+    const size_t rows = (size_t)b.hist + bk.max_frame;
+    const size_t fin = (size_t)bk.max_frame + bk.D;                // most samples one call can finalise
+    bool ok = cudaMalloc(&b.xbuf[0], S * rows * p.M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&b.xbuf[1], S * rows * p.M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&b.q, S * rows * p.M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&b.vmem, S * fin * p.C2 * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&b.env_state, S * p.G * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&b.env_started, S * p.G * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&b.ring, S * p.C2 * (size_t)b.ring_len) == cudaSuccess &&
+              cudaMalloc(&b.state, S * p.C2 * sizeof(ChanState)) == cudaSuccess &&
+              cudaMalloc(&b.flags, S * sizeof(int32_t)) == cudaSuccess &&
+              cudaMalloc(&b.gram, S * p.C2 * p.C2 * sizeof(double)) == cudaSuccess;
+    return ok ? MICLOC_OK : set_error(MICLOC_ERR_CUDA, "cudaMalloc(stream batch) failed");
 }
 
-extern "C" int micloc_snn_streams_reset(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots, void *stream) {
-    if (!sb) return set_error(MICLOC_ERR_CONFIG, "null stream");
-    MICLOC_CUDA(cudaSetDevice(sb->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    if (slots_host) MICLOC_TRY(upload_slots(sb, slots_host, n_slots, st));
-    const ChainParams &p = sb->prm.chain;
-    const long long W = p.C2 > p.G ? p.C2 : p.G;
-    k_stream_reset<<<(unsigned)((sb->S * W + 255) / 256), 256, 0, st>>>(sb->state, sb->pos[sb->pcur], sb->flags, sb->env_state,
-                                                                       sb->env_started, slots_host ? sb->sel : nullptr, sb->S, p.C2, p.G);
+// fresh state for the listed slots (slots_host NULL: every slot) of every band; band 0's launch writes the positions.
+// Synchronises `st`.
+static int reset_bands(SlotBook &bk, StreamBand *band, int F, const int32_t *slots_host, int32_t n_slots, cudaStream_t st) {
+    if (slots_host) MICLOC_TRY(bk.upload(slots_host, n_slots, st));
+    for (int f = 0; f < F; ++f) {
+        StreamBand &b = band[f];
+        const ChainParams &p = b.prm.chain;
+        const long long W = p.C2 > p.G ? p.C2 : p.G;
+        k_stream_reset<<<(unsigned)((bk.S * W + 255) / 256), 256, 0, st>>>(b.state, f == 0 ? bk.pos[bk.pcur] : nullptr, b.flags,
+                                                                          b.env_state, b.env_started,
+                                                                          slots_host ? bk.sel : nullptr, bk.S, p.C2, p.G);
+        count_launch(1);
+        MICLOC_CUDA(cudaGetLastError());
+    }
+    return bk.reset_done(slots_host != nullptr, st);
+}
+
+// envelope scratch for outputs of `rows` rows, taken before a push or flush launches anything: a failed allocation
+// leaves every slot where it stood
+static int reserve_env(StreamBand &b, long long S, long long rows, const float *env_dev, const int32_t *doa_t_dev) {
+    if (!env_dev && !doa_t_dev) return MICLOC_OK;
+    const size_t bytes = (size_t)S * rows * b.prm.chain.G * sizeof(float);
+    MICLOC_TRY(b.y.reserve(bytes));
+    return env_dev ? MICLOC_OK : b.env.reserve(bytes);
+}
+
+// One band's part of a push of n samples (close_sel == nullptr: STHT of the newest [history | frame] buffer first) or
+// of a flush of the slots in close_sel (n = 0): band-pass + RZCC + neuron (k_stream_blk reads the book's positions and
+// writes the next ones and the final row counts m), then power / DoA and envelope over each slot's final rows; outputs
+// [S][rows][...].  The owner flips the book once every band has run.
+static int band_step(StreamBand &b, const SlotBook &bk, const int32_t *close_sel, long long n, long long rows,
+                     int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev, int32_t *doa_t_dev,
+                     cudaStream_t st) {
+    const ChainParams &p = b.prm.chain;
+    const long long S = bk.S;
+    // STHT of the extended clips [history | frame]: rows >= hist see their whole window
+    if (!close_sel)
+        MICLOC_TRY(launch_stht_any(p, (const float *)b.prm.taps_dev, b.xbuf[bk.xcur], MICLOC_F32, b.q, S, b.hist + n, st));
+    const unsigned grid = (unsigned)((S * p.C2 + kStreamBlkThreads - 1) / kStreamBlkThreads);
+    auto kernel = p.nsec == 2 ? k_stream_blk<2> : k_stream_blk<0>;
+    kernel<<<grid, kStreamBlkThreads, 0, st>>>(b.xbuf[bk.xcur], b.q, b.state, bk.pos[bk.pcur], bk.pos[bk.pcur ^ 1], bk.m,
+                                              close_sel, b.ring, b.ring_len, b.flags, spikes_dev, b.vmem, p, S, (int)n,
+                                              b.hist, (int)rows, bk.D);
     count_launch(1);
     MICLOC_CUDA(cudaGetLastError());
-    for (long long s = 0; s < sb->S; ++s)
-        if (!slots_host || sb->sel_h[(size_t)s]) { sb->N[(size_t)s] = 0; sb->F[(size_t)s] = 0; sb->active[(size_t)s] = 1; }
-    return MICLOC_OK;
-}
-
-// D_floor: the multi-band batch aligns its bands on one latency, D = max(rzcc_lag(w), D_floor) (ring and vmem follow)
-static int streams_create(micloc_snn *ctx, int32_t num_streams, int64_t max_frame_len, double fs, double rise_time,
-                          double fall_time, int D_floor, micloc_stream_batch **out) {
-    if (!ctx || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
-    *out = nullptr;
-    if (num_streams < 1 || num_streams > 65535) return set_error(MICLOC_ERR_SHAPE, "num_streams %d out of range [1, 65535]", num_streams);
-    if (max_frame_len < 1 || max_frame_len > (1ll << 24)) return set_error(MICLOC_ERR_SHAPE, "max_frame_len out of range");
-    if (rise_time > fall_time)
-        return set_error(MICLOC_ERR_CONFIG, "for proper functioning, an envelope estimator should have a larger fall time!");
-    if ((int)(fs * rise_time) < 1 || (int)(fs * fall_time) < 1) return set_error(MICLOC_ERR_CONFIG, "envelope windows shorter than one sample");
-    micloc_snn_params prm;
-    MICLOC_TRY(micloc_snn_get_params(ctx, &prm));
-    const ChainParams &p = prm.chain;
-    MICLOC_CUDA(cudaSetDevice(prm.device));
-    micloc_stream_batch *sb = new micloc_stream_batch();
-    sb->prm = prm; sb->device = prm.device; sb->S = num_streams; sb->max_frame = max_frame_len;
-    sb->hist = p.K - 1;
-    sb->D = std::max(rzcc_lag(p.w), D_floor);
-    const long long need = max_frame_len + sb->D + p.nL + 2 * kSeg;
-    sb->ring_len = 32;
-    while (sb->ring_len < need) sb->ring_len <<= 1;
-    sb->fs = (float)fs; sb->rise_time = (float)rise_time; sb->fall_time = (float)fall_time;
-    sb->N.assign((size_t)num_streams, 0); sb->F.assign((size_t)num_streams, 0); sb->active.assign((size_t)num_streams, 1);
-    const size_t S = (size_t)num_streams;
-    const size_t rows = (size_t)sb->hist + max_frame_len;
-    const size_t fin = (size_t)max_frame_len + sb->D;                // most samples one call can finalise
-    bool ok = cudaMalloc(&sb->xbuf[0], S * rows * p.M * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&sb->xbuf[1], S * rows * p.M * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&sb->q, S * rows * p.M * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&sb->vmem, S * fin * p.C2 * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&sb->env_state, S * p.G * sizeof(float)) == cudaSuccess &&
-              cudaMalloc(&sb->env_started, S * p.G * sizeof(int32_t)) == cudaSuccess &&
-              cudaMalloc(&sb->ring, S * p.C2 * (size_t)sb->ring_len) == cudaSuccess &&
-              cudaMalloc(&sb->state, S * p.C2 * sizeof(ChanState)) == cudaSuccess &&
-              cudaMalloc(&sb->pos[0], S * sizeof(SlotPos)) == cudaSuccess &&
-              cudaMalloc(&sb->pos[1], S * sizeof(SlotPos)) == cudaSuccess &&
-              cudaMalloc(&sb->m, S * sizeof(int32_t)) == cudaSuccess &&
-              cudaMalloc(&sb->flags, S * sizeof(int32_t)) == cudaSuccess &&
-              cudaMalloc(&sb->sel, S * sizeof(int32_t)) == cudaSuccess &&
-              cudaMalloc(&sb->gram, S * p.C2 * p.C2 * sizeof(double)) == cudaSuccess;
-    if (!ok) { micloc_snn_streams_destroy(sb); return set_error(MICLOC_ERR_CUDA, "cudaMalloc(stream batch) failed"); }
-    int rc = micloc_snn_streams_reset(sb, nullptr, 0, nullptr);
-    if (!rc && cudaStreamSynchronize(nullptr) != cudaSuccess) rc = set_error(MICLOC_ERR_CUDA, "stream batch reset failed");
-    if (rc) { micloc_snn_streams_destroy(sb); return rc; }
-    *out = sb;
-    return MICLOC_OK;
-}
-
-extern "C" int micloc_snn_streams_create(micloc_snn *ctx, int32_t num_streams, int64_t max_frame_len, double fs,
-                                         double rise_time, double fall_time, micloc_stream_batch **out) {
-    return streams_create(ctx, num_streams, max_frame_len, fs, rise_time, fall_time, 0, out);
-}
-
-extern "C" int micloc_snn_streams_latency(micloc_stream_batch *sb) { return sb ? sb->D : 0; }
-
-// shared tail of push / flush: power / DoA and envelope over each slot's final rows (sb->m, written by k_stream_blk);
-// outputs [S][rows][...]
-static int streams_finalise(micloc_stream_batch *sb, long long rows, float *power_dev, int32_t *doa_dev, float *env_dev,
-                            int32_t *doa_t_dev, cudaStream_t st) {
-    const ChainParams &p = sb->prm.chain;
-    const long long S = sb->S;
     if (power_dev || doa_dev) {
         dim3 gg((unsigned)S, (unsigned)((p.C2 * p.C2 + 255) / 256));
-        k_gram<<<gg, 256, 0, st>>>(sb->vmem, sb->gram, p.C2, rows, 0, sb->m);
+        k_gram<<<gg, 256, 0, st>>>(b.vmem, b.gram, p.C2, rows, 0, bk.m);
         count_launch(1);
-        MICLOC_TRY(launch_power(sb->gram, (const double *)sb->prm.bf_f64_dev, power_dev, doa_dev, p.C2, p.G, S, 1.0, sb->m,
-                                1, nullptr, nullptr, st));
+        MICLOC_TRY(launch_power(b.gram, (const double *)b.prm.bf_f64_dev, power_dev, doa_dev, p.C2, p.G, S, 1.0, bk.m, 1,
+                                nullptr, nullptr, st));
     }
-    if (env_dev || doa_t_dev) {
-        const size_t bytes = (size_t)S * rows * p.G * sizeof(float);
-        MICLOC_TRY(sb->y.reserve(bytes));
-        if (!env_dev) MICLOC_TRY(sb->env.reserve(bytes));
-        float *y = (float *)sb->y.ptr;
-        float *env = env_dev ? env_dev : (float *)sb->env.ptr;
+    if (env_dev || doa_t_dev) {                         // scratch: reserve_env
+        float *y = (float *)b.y.ptr;
+        float *env = env_dev ? env_dev : (float *)b.env.ptr;
         const int slab = 256;
         dim3 grid((unsigned)((p.G + 127) / 128), (unsigned)((rows + slab - 1) / slab), (unsigned)S);
-        if (p.C2 <= 16) k_dense<16><<<grid, 128, 0, st>>>(sb->vmem, (const float *)sb->prm.bf_f32_dev, y, p.C2, p.G, rows, slab);
-        else k_dense<0><<<grid, 128, 0, st>>>(sb->vmem, (const float *)sb->prm.bf_f32_dev, y, p.C2, p.G, rows, slab);
-        k_envelope<<<(unsigned)((S * p.G + 127) / 128), 128, 0, st>>>(y, env, sb->env_state, sb->env_started, sb->m, S, rows, p.G,
-                                                                      1.f / (float)(int)(sb->fs * sb->fall_time),
-                                                                      1.f / (float)(int)(sb->fs * sb->rise_time));
+        if (p.C2 <= 16) k_dense<16><<<grid, 128, 0, st>>>(b.vmem, (const float *)b.prm.bf_f32_dev, y, p.C2, p.G, rows, slab);
+        else k_dense<0><<<grid, 128, 0, st>>>(b.vmem, (const float *)b.prm.bf_f32_dev, y, p.C2, p.G, rows, slab);
+        k_envelope<<<(unsigned)((S * p.G + 127) / 128), 128, 0, st>>>(y, env, b.env_state, b.env_started, bk.m, S, rows, p.G,
+                                                                      1.f / (float)(int)(b.fs * b.fall_time),
+                                                                      1.f / (float)(int)(b.fs * b.rise_time));
         count_launch(2);
         if (doa_t_dev) {
-            k_argmax_rows<<<(unsigned)((S * rows * 32 + 255) / 256), 256, 0, st>>>(env, doa_t_dev, sb->m, S, rows, p.G);
+            k_argmax_rows<<<(unsigned)((S * rows * 32 + 255) / 256), 256, 0, st>>>(env, doa_t_dev, bk.m, S, rows, p.G);
             count_launch(1);
         }
     }
@@ -532,80 +505,93 @@ static int streams_finalise(micloc_stream_batch *sb, long long rows, float *powe
     return MICLOC_OK;
 }
 
-static int launch_stream_blk(micloc_stream_batch *sb, const int32_t *close_sel, int n, int rows, int8_t *spikes_dev,
-                             cudaStream_t st) {
-    const ChainParams &p = sb->prm.chain;
-    const long long lanes = sb->S * p.C2;
-    const unsigned grid = (unsigned)((lanes + kStreamBlkThreads - 1) / kStreamBlkThreads);
-    auto kernel = p.nsec == 2 ? k_stream_blk<2> : k_stream_blk<0>;
-    kernel<<<grid, kStreamBlkThreads, 0, st>>>(sb->xbuf[sb->xcur], sb->q, sb->state, sb->pos[sb->pcur], sb->pos[sb->pcur ^ 1],
-                                              sb->m, close_sel, sb->ring, sb->ring_len, sb->flags, spikes_dev, sb->vmem, p,
-                                              sb->S, n, sb->hist, rows, sb->D);
-    count_launch(1);
-    MICLOC_CUDA(cudaGetLastError());
-    sb->pcur ^= 1;
-    return MICLOC_OK;
-}
-
-// the frame arguments of a push against the batch
-static int check_frames(const micloc_stream_batch *sb, int dtype, int64_t n, int32_t in_channels) {
-    const ChainParams &p = sb->prm.chain;
-    if (n < 1 || n > sb->max_frame) return set_error(MICLOC_ERR_SHAPE, "frame of %lld samples (stream takes 1..%lld)", (long long)n, sb->max_frame);
-    if (in_channels < p.M)
-        return set_error(MICLOC_ERR_SHAPE, "number of channels in the input siganl %d should be the same as the number of microphones %d!", in_channels, p.M);
-    if (dtype != MICLOC_F32 && dtype != MICLOC_I16 && dtype != MICLOC_I32)
-        return set_error(MICLOC_ERR_SHAPE, "dtype must be MICLOC_F32, MICLOC_I16 or MICLOC_I32");
-    for (long long s = 0; s < sb->S; ++s)
-        if (sb->active[(size_t)s] && sb->N[(size_t)s] + n >= (1ll << 31) - 4096)
-            return set_error(MICLOC_ERR_SHAPE, "stream position exceeds 2^31 samples: reset the stream");
-    return MICLOC_OK;
-}
-
-// everything of a push after the frame assembly, which left [history | frame] rows in sb->xbuf[sb->xcur]: STHT,
-// band-pass + RZCC + neuron, the slots' new positions (n_out_host, on the host), power / DoA / envelope
-static int streams_advance(micloc_stream_batch *sb, int64_t n, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev,
-                           float *env_dev, int32_t *doa_t_dev, int64_t *n_out_host, cudaStream_t st) {
-    const ChainParams &p = sb->prm.chain;
-    // STHT of the extended clips [history | frame]: rows >= hist see their whole window
-    MICLOC_TRY(launch_stht_any(p, (const float *)sb->prm.taps_dev, sb->xbuf[sb->xcur], MICLOC_F32, sb->q, sb->S, sb->hist + n, st));
-    const long long rows = n + sb->D;
-    MICLOC_TRY(launch_stream_blk(sb, nullptr, (int)n, (int)rows, spikes_dev, st));
-    for (long long s = 0; s < sb->S; ++s) {
-        const size_t i = (size_t)s;
-        n_out_host[s] = 0;
-        if (!sb->active[i]) continue;
-        sb->N[i] += n;
-        const long long f = sb->N[i] - sb->D > sb->F[i] ? sb->N[i] - sb->D : sb->F[i];
-        n_out_host[s] = f - sb->F[i];
-        sb->F[i] = f;
+// a push (close_sel == nullptr) or flush of every band, then the slots' new positions; band f's spikes and power go to
+// spikes_dev + f S rows 2M and power_dev + f S G
+static int step_bands(SlotBook &bk, StreamBand *band, int F, const int32_t *close_sel, long long n, long long rows,
+                      int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev, int32_t *doa_t_dev,
+                      int64_t *n_out_host, cudaStream_t st) {
+    for (int f = 0; f < F; ++f) {
+        const ChainParams &p = band[f].prm.chain;
+        MICLOC_TRY(band_step(band[f], bk, close_sel, n, rows, spikes_dev ? spikes_dev + f * bk.S * rows * p.C2 : nullptr,
+                             power_dev ? power_dev + f * bk.S * p.G : nullptr, doa_dev, env_dev, doa_t_dev, st));
     }
-    return streams_finalise(sb, rows, power_dev, doa_dev, env_dev, doa_t_dev, st);
+    if (close_sel) bk.flushed(n_out_host);
+    else bk.pushed(n, n_out_host);
+    return MICLOC_OK;
 }
+
+// the listed slots (slots_host NULL: every slot) of every band close like a clip end; flags_host [S] (nullable, host):
+// bit 0 = RZCC overflow in any band (the only bit k_stream_blk sets).  Synchronises `st`.
+static int flush_bands(SlotBook &bk, StreamBand *band, int F, const int32_t *slots_host, int32_t n_slots,
+                       int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev, int32_t *doa_t_dev,
+                       int64_t *n_out_host, int32_t *flags_host, cudaStream_t st) {
+    MICLOC_TRY(bk.upload(slots_host, n_slots, st));
+    MICLOC_TRY(step_bands(bk, band, F, bk.sel, 0, bk.max_frame + bk.D, spikes_dev, power_dev, doa_dev, env_dev, doa_t_dev,
+                          n_out_host, st));
+    if (!flags_host) return MICLOC_OK;
+    const size_t S = (size_t)bk.S;
+    std::vector<int32_t> h((size_t)F * S);
+    for (int f = 0; f < F; ++f)
+        MICLOC_CUDA(cudaMemcpyAsync(h.data() + f * S, band[f].flags, S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    MICLOC_CUDA(cudaStreamSynchronize(st));
+    for (size_t s = 0; s < S; ++s) {
+        flags_host[s] = 0;
+        for (int f = 0; f < F; ++f) flags_host[s] |= h[f * S + s] & 1;
+    }
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_streams_destroy(micloc_stream_batch *sb) {
+    if (!sb) return MICLOC_OK;
+    cudaSetDevice(sb->device);
+    sb->book.destroy();
+    band_free(sb->band);
+    delete sb;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_streams_reset(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots, void *stream) {
+    if (!sb) return set_error(MICLOC_ERR_CONFIG, "null stream");
+    MICLOC_CUDA(cudaSetDevice(sb->device));
+    return reset_bands(sb->book, &sb->band, 1, slots_host, n_slots, (cudaStream_t)stream);
+}
+
+extern "C" int micloc_snn_streams_create(micloc_snn *ctx, int32_t num_streams, int64_t max_frame_len, double fs,
+                                         double rise_time, double fall_time, micloc_stream_batch **out) {
+    if (!ctx || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
+    *out = nullptr;
+    if (rise_time > fall_time)
+        return set_error(MICLOC_ERR_CONFIG, "for proper functioning, an envelope estimator should have a larger fall time!");
+    if ((int)(fs * rise_time) < 1 || (int)(fs * fall_time) < 1) return set_error(MICLOC_ERR_CONFIG, "envelope windows shorter than one sample");
+    micloc_snn_params prm;
+    MICLOC_TRY(micloc_snn_get_params(ctx, &prm));
+    MICLOC_CUDA(cudaSetDevice(prm.device));
+    micloc_stream_batch *sb = new micloc_stream_batch();
+    sb->device = prm.device;
+    sb->band.fs = (float)fs; sb->band.rise_time = (float)rise_time; sb->band.fall_time = (float)fall_time;
+    sb->book.D = rzcc_lag(prm.chain.w);
+    int rc = sb->book.create(num_streams, max_frame_len);
+    if (!rc) rc = band_alloc(sb->band, prm, sb->book);
+    if (!rc) rc = reset_bands(sb->book, &sb->band, 1, nullptr, 0, nullptr);
+    if (rc) { micloc_snn_streams_destroy(sb); return rc; }
+    *out = sb;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_snn_streams_latency(micloc_stream_batch *sb) { return sb ? sb->book.D : 0; }
 
 extern "C" int micloc_snn_streams_push(micloc_stream_batch *sb, const void *frames_dev, int dtype, int64_t n,
                                        int32_t in_channels, int8_t *spikes_dev, float *power_dev, int32_t *doa_dev,
                                        float *env_dev, int32_t *doa_t_dev, int64_t *n_out_host, void *stream) {
     if (!sb || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
-    MICLOC_TRY(check_frames(sb, dtype, n, in_channels));
-    const ChainParams &p = sb->prm.chain;
+    SlotBook &bk = sb->book;
+    StreamBand &b = sb->band;
+    MICLOC_TRY(bk.check_push(dtype, n, in_channels, b.prm.chain.M));
     MICLOC_CUDA(cudaSetDevice(sb->device));
     cudaStream_t st = (cudaStream_t)stream;
-    const int nxt = sb->xcur ^ 1;
-    const long long total = sb->S * (sb->hist + n) * p.M;
-    const unsigned ga = (unsigned)((total + 255) / 256);
-    const float *prev = sb->xbuf[sb->xcur];
-    const SlotPos *pos = sb->pos[sb->pcur];
-    if (dtype == MICLOC_F32)
-        k_stream_assemble<float><<<ga, 256, 0, st>>>((const float *)frames_dev, prev, sb->xbuf[nxt], pos, sb->S, (int)n, (int)sb->n_prev, in_channels, p.M, sb->hist);
-    else if (dtype == MICLOC_I16)
-        k_stream_assemble<int16_t><<<ga, 256, 0, st>>>((const int16_t *)frames_dev, prev, sb->xbuf[nxt], pos, sb->S, (int)n, (int)sb->n_prev, in_channels, p.M, sb->hist);
-    else
-        k_stream_assemble<int32_t><<<ga, 256, 0, st>>>((const int32_t *)frames_dev, prev, sb->xbuf[nxt], pos, sb->S, (int)n, (int)sb->n_prev, in_channels, p.M, sb->hist);
-    count_launch(1);
-    MICLOC_CUDA(cudaGetLastError());
-    sb->xcur = nxt;
-    sb->n_prev = n;
-    return streams_advance(sb, n, spikes_dev, power_dev, doa_dev, env_dev, doa_t_dev, n_out_host, st);
+    MICLOC_TRY(reserve_env(b, bk.S, n + bk.D, env_dev, doa_t_dev));
+    MICLOC_TRY(bk.assemble(b.xbuf, frames_dev, dtype, n, in_channels, b.prm.chain.M, b.hist, st));
+    return step_bands(bk, &b, 1, nullptr, n, n + bk.D, spikes_dev, power_dev, doa_dev, env_dev, doa_t_dev, n_out_host, st);
 }
 
 extern "C" int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *slots_host, int32_t n_slots,
@@ -613,42 +599,27 @@ extern "C" int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *
                                         int32_t *doa_t_dev, int64_t *n_out_host, int32_t *flags_host, void *stream) {
     if (!sb || !n_out_host) return set_error(MICLOC_ERR_CONFIG, "null stream");
     MICLOC_CUDA(cudaSetDevice(sb->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    MICLOC_TRY(upload_slots(sb, slots_host, n_slots, st));
-    const long long rows = sb->max_frame + sb->D;
-    MICLOC_TRY(launch_stream_blk(sb, sb->sel, 0, (int)rows, spikes_dev, st));
-    for (long long s = 0; s < sb->S; ++s) {
-        const size_t i = (size_t)s;
-        n_out_host[s] = 0;
-        if (!sb->active[i] || !sb->sel_h[i]) continue;
-        n_out_host[s] = sb->N[i] - sb->F[i];
-        sb->F[i] = sb->N[i];
-        sb->active[i] = 0;
-    }
-    MICLOC_TRY(streams_finalise(sb, rows, power_dev, doa_dev, env_dev, doa_t_dev, st));
-    if (flags_host) {
-        MICLOC_CUDA(cudaMemcpyAsync(flags_host, sb->flags, (size_t)sb->S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        MICLOC_CUDA(cudaStreamSynchronize(st));
-    }
-    return MICLOC_OK;
+    MICLOC_TRY(reserve_env(sb->band, sb->book.S, sb->book.max_frame + sb->book.D, env_dev, doa_t_dev));
+    return flush_bands(sb->book, &sb->band, 1, slots_host, n_slots, spikes_dev, power_dev, doa_dev, env_dev, doa_t_dev,
+                       n_out_host, flags_host, (cudaStream_t)stream);
 }
 
-// ---- multi-band stream batches: F stream batches with one latency behind one filterbank ----
+// ---- multi-band stream batches: F bands on one slot book, behind one filterbank ----
 struct micloc_mb_streams {
-    int F = 0, device = 0, M = 0, C2 = 0, G = 0, D = 0;
-    long long S = 0, max_frame = 0;
-    micloc_stream_batch *band[8] = {};
+    int F = 0, device = 0, M = 0, G = 0;
+    SlotBook book;
+    StreamBand band[8];
     FilterbankParams fb{};
     BiquadState *fb_state = nullptr;    // [F][S][M] filterbank state
     double *doa_list = nullptr;         // [G] on the device, null: no ML estimators
     float *power = nullptr;             // [F][S][G] per-band power when the caller passes no power_dev
-    std::vector<int32_t> flags_h;       // staging of a band's flags at a flush
 };
 
 extern "C" int micloc_snn_mb_streams_destroy(micloc_mb_streams *mb) {
     if (!mb) return MICLOC_OK;
     cudaSetDevice(mb->device);
-    for (int f = 0; f < mb->F; ++f) micloc_snn_streams_destroy(mb->band[f]);
+    mb->book.destroy();
+    for (int f = 0; f < mb->F; ++f) band_free(mb->band[f]);
     cudaFree(mb->fb_state); cudaFree(mb->doa_list); cudaFree(mb->power);
     delete mb;
     return MICLOC_OK;
@@ -672,47 +643,44 @@ extern "C" int micloc_snn_mb_streams_create(micloc_snn *const *ctxs, int32_t F, 
         if (prm[f].chain.M != prm[0].chain.M || prm[f].chain.G != prm[0].chain.G)
             return set_error(MICLOC_ERR_SHAPE, "band %d's context has %d microphones and %d DoAs, band 0's %d and %d", f,
                              prm[f].chain.M, prm[f].chain.G, prm[0].chain.M, prm[0].chain.G);
-        D = std::max(D, rzcc_lag(prm[f].chain.w));
+        D = std::max(D, rzcc_lag(prm[f].chain.w));      // one latency: every band finalises the same samples
     }
     MICLOC_CUDA(cudaSetDevice(prm[0].device));
     micloc_mb_streams *mb = new micloc_mb_streams();
-    mb->device = prm[0].device; mb->M = prm[0].chain.M; mb->C2 = prm[0].chain.C2; mb->G = prm[0].chain.G; mb->D = D;
-    mb->S = num_streams; mb->max_frame = max_frame_len; mb->fb = fb;
-    for (int f = 0; f < F; ++f) {
-        const int rc = streams_create(ctxs[f], num_streams, max_frame_len, 48000.0, 10e-3, 100e-3, D, &mb->band[f]);
-        if (rc) { micloc_snn_mb_streams_destroy(mb); return rc; }
-        mb->F = f + 1;
-    }
+    mb->F = F; mb->device = prm[0].device; mb->M = prm[0].chain.M; mb->G = prm[0].chain.G; mb->fb = fb;
+    mb->book.D = D;
+    int rc = mb->book.create(num_streams, max_frame_len);
+    for (int f = 0; f < F && !rc; ++f) rc = band_alloc(mb->band[f], prm[f], mb->book);
     const size_t S = (size_t)num_streams;
-    bool ok = cudaMalloc(&mb->fb_state, (size_t)F * S * mb->M * sizeof(BiquadState)) == cudaSuccess &&
-              cudaMalloc(&mb->power, (size_t)F * S * mb->G * sizeof(float)) == cudaSuccess &&
-              (!doa_list || cudaMalloc(&mb->doa_list, (size_t)mb->G * sizeof(double)) == cudaSuccess);
-    if (!ok) { micloc_snn_mb_streams_destroy(mb); return set_error(MICLOC_ERR_CUDA, "cudaMalloc(multi-band stream batch) failed"); }
-    if ((doa_list && cudaMemcpy(mb->doa_list, doa_list, (size_t)mb->G * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) ||
-        cudaMemset(mb->fb_state, 0, (size_t)F * S * mb->M * sizeof(BiquadState)) != cudaSuccess) {
-        micloc_snn_mb_streams_destroy(mb);
-        return set_error(MICLOC_ERR_CUDA, "multi-band stream batch set-up failed");
-    }
+    if (!rc && !(cudaMalloc(&mb->fb_state, (size_t)F * S * mb->M * sizeof(BiquadState)) == cudaSuccess &&
+                 cudaMalloc(&mb->power, (size_t)F * S * mb->G * sizeof(float)) == cudaSuccess &&
+                 (!doa_list || cudaMalloc(&mb->doa_list, (size_t)mb->G * sizeof(double)) == cudaSuccess)))
+        rc = set_error(MICLOC_ERR_CUDA, "cudaMalloc(multi-band stream batch) failed");
+    if (!rc && ((doa_list && cudaMemcpy(mb->doa_list, doa_list, (size_t)mb->G * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) ||
+                cudaMemset(mb->fb_state, 0, (size_t)F * S * mb->M * sizeof(BiquadState)) != cudaSuccess))
+        rc = set_error(MICLOC_ERR_CUDA, "multi-band stream batch set-up failed");
+    if (!rc) rc = reset_bands(mb->book, mb->band, F, nullptr, 0, nullptr);
+    if (rc) { micloc_snn_mb_streams_destroy(mb); return rc; }
     *out = mb;
     return MICLOC_OK;
 }
 
-extern "C" int micloc_snn_mb_streams_latency(micloc_mb_streams *mb) { return mb ? mb->D : 0; }
+extern "C" int micloc_snn_mb_streams_latency(micloc_mb_streams *mb) { return mb ? mb->book.D : 0; }
 
 // the filterbank state of a reset slot is dropped by k_mb_stream_assemble (it restarts at N == 0)
 extern "C" int micloc_snn_mb_streams_reset(micloc_mb_streams *mb, const int32_t *slots_host, int32_t n_slots, void *stream) {
     if (!mb) return set_error(MICLOC_ERR_CONFIG, "null stream");
-    for (int f = 0; f < mb->F; ++f) MICLOC_TRY(micloc_snn_streams_reset(mb->band[f], slots_host, n_slots, stream));
-    return MICLOC_OK;
+    MICLOC_CUDA(cudaSetDevice(mb->device));
+    return reset_bands(mb->book, mb->band, mb->F, slots_host, n_slots, (cudaStream_t)stream);
 }
 
-// sum over the bands + estimators over each slot's final rows (band 0's row counts: the same in every band)
+// sum over the bands + estimators over each slot's final rows
 static int mb_fuse(micloc_mb_streams *mb, const float *power, float *power_grid_dev, int32_t *doa_dev, double *periodic_ml_dev,
                    double *trimmed_ml_dev, int32_t *flags_dev, cudaStream_t st) {
     const int32_t *band_flags[8];
-    for (int f = 0; f < mb->F; ++f) band_flags[f] = mb->band[f]->flags;
-    return launch_power_fuse(power, mb->F, mb->S, mb->G, mb->doa_list, power_grid_dev, doa_dev, periodic_ml_dev,
-                             trimmed_ml_dev, flags_dev, mb->band[0]->m, band_flags, st);
+    for (int f = 0; f < mb->F; ++f) band_flags[f] = mb->band[f].flags;
+    return launch_power_fuse(power, mb->F, mb->book.S, mb->G, mb->doa_list, power_grid_dev, doa_dev, periodic_ml_dev,
+                             trimmed_ml_dev, flags_dev, mb->book.m, band_flags, st);
 }
 
 extern "C" int micloc_snn_mb_streams_push(micloc_mb_streams *mb, const void *frames_dev, int dtype, int64_t n,
@@ -720,37 +688,32 @@ extern "C" int micloc_snn_mb_streams_push(micloc_mb_streams *mb, const void *fra
                                           int32_t *doa_dev, double *periodic_ml_dev, double *trimmed_ml_dev,
                                           double *sumsq_dev, int32_t *flags_dev, int64_t *n_out_host, void *stream) {
     if (!mb || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
-    micloc_stream_batch *b0 = mb->band[0];
-    MICLOC_TRY(check_frames(b0, dtype, n, in_channels));        // (positions and shapes are the same in every band)
+    SlotBook &bk = mb->book;
+    MICLOC_TRY(bk.check_push(dtype, n, in_channels, mb->M));
     if ((periodic_ml_dev || trimmed_ml_dev) && !mb->doa_list) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
     MICLOC_CUDA(cudaSetDevice(mb->device));
     cudaStream_t st = (cudaStream_t)stream;
     MbAssembleParams ap{};
     ap.fb = mb->fb;
     for (int f = 0; f < mb->F; ++f) {
-        micloc_stream_batch *sb = mb->band[f];
-        ap.prev[f] = sb->xbuf[sb->xcur];
-        ap.cur[f] = sb->xbuf[sb->xcur ^ 1];
-        ap.hist[f] = sb->hist;
+        ap.prev[f] = mb->band[f].xbuf[bk.xcur];
+        ap.cur[f] = mb->band[f].xbuf[bk.xcur ^ 1];
+        ap.hist[f] = mb->band[f].hist;
     }
-    if (sumsq_dev) MICLOC_CUDA(cudaMemsetAsync(sumsq_dev, 0, (size_t)mb->S * sizeof(double), st));
-    const unsigned grid = (unsigned)((mb->S * mb->M + 127) / 128);
-    const SlotPos *pos = b0->pos[b0->pcur];
+    if (sumsq_dev) MICLOC_CUDA(cudaMemsetAsync(sumsq_dev, 0, (size_t)bk.S * sizeof(double), st));
+    const unsigned grid = (unsigned)((bk.S * mb->M + 127) / 128);
     auto launch = dtype == MICLOC_F32 ? launch_mb_assemble<float> : dtype == MICLOC_I16 ? launch_mb_assemble<int16_t>
                                                                                     : launch_mb_assemble<int32_t>;
-    launch(mb->F, grid, st, frames_dev, mb->fb_state, sumsq_dev, pos, ap, mb->S, (int)n, (int)b0->n_prev, in_channels, mb->M);
+    launch(mb->F, grid, st, frames_dev, mb->fb_state, sumsq_dev, bk.pos[bk.pcur], ap, bk.S, (int)n, (int)bk.n_prev,
+           in_channels, mb->M);
     count_launch(1);
     MICLOC_CUDA(cudaGetLastError());
+    bk.xcur ^= 1;
+    bk.n_prev = n;
     const bool fuse = power_dev || power_grid_dev || doa_dev || periodic_ml_dev || trimmed_ml_dev || flags_dev;
     float *power = power_dev ? power_dev : mb->power;
-    const long long rows = n + mb->D;
-    for (int f = 0; f < mb->F; ++f) {
-        micloc_stream_batch *sb = mb->band[f];
-        sb->xcur ^= 1;
-        sb->n_prev = n;
-        MICLOC_TRY(streams_advance(sb, n, spikes_dev ? spikes_dev + f * mb->S * rows * mb->C2 : nullptr,
-                                   fuse ? power + f * mb->S * mb->G : nullptr, nullptr, nullptr, nullptr, n_out_host, st));
-    }
+    MICLOC_TRY(step_bands(bk, mb->band, mb->F, nullptr, n, n + bk.D, spikes_dev, fuse ? power : nullptr, nullptr, nullptr,
+                          nullptr, n_out_host, st));
     if (!fuse) return MICLOC_OK;
     return mb_fuse(mb, power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, st);
 }
@@ -761,21 +724,14 @@ extern "C" int micloc_snn_mb_streams_flush(micloc_mb_streams *mb, const int32_t 
                                            int64_t *n_out_host, int32_t *flags_host, void *stream) {
     if (!mb || !n_out_host) return set_error(MICLOC_ERR_CONFIG, "null stream");
     if ((periodic_ml_dev || trimmed_ml_dev) && !mb->doa_list) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
+    MICLOC_CUDA(cudaSetDevice(mb->device));
+    cudaStream_t st = (cudaStream_t)stream;
     const bool fuse = power_dev || power_grid_dev || doa_dev || periodic_ml_dev || trimmed_ml_dev || flags_dev;
     float *power = power_dev ? power_dev : mb->power;
-    const long long rows = mb->max_frame + mb->D;
-    if (flags_host) for (long long s = 0; s < mb->S; ++s) flags_host[s] = 0;
-    mb->flags_h.assign((size_t)mb->S, 0);
-    for (int f = 0; f < mb->F; ++f) {
-        MICLOC_TRY(micloc_snn_streams_flush(mb->band[f], slots_host, n_slots,
-                                            spikes_dev ? spikes_dev + f * mb->S * rows * mb->C2 : nullptr,
-                                            fuse ? power + f * mb->S * mb->G : nullptr, nullptr, nullptr, nullptr,
-                                            n_out_host, flags_host ? mb->flags_h.data() : nullptr, stream));
-        for (long long s = 0; flags_host && s < mb->S; ++s) flags_host[s] |= mb->flags_h[(size_t)s] & 1;
-    }
+    MICLOC_TRY(flush_bands(mb->book, mb->band, mb->F, slots_host, n_slots, spikes_dev, fuse ? power : nullptr, nullptr,
+                           nullptr, nullptr, n_out_host, flags_host, st));
     if (!fuse) return MICLOC_OK;
-    MICLOC_CUDA(cudaSetDevice(mb->device));
-    return mb_fuse(mb, power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, (cudaStream_t)stream);
+    return mb_fuse(mb, power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, st);
 }
 
 // ---- the single stream: slot 0 of a one-slot batch ----
@@ -798,18 +754,16 @@ extern "C" int micloc_snn_stream_destroy(micloc_stream *s) {
 
 extern "C" int micloc_snn_stream_reset(micloc_stream *s, void *stream) {
     if (!s) return set_error(MICLOC_ERR_CONFIG, "null stream");
-    MICLOC_TRY(micloc_snn_streams_reset(s->sb, nullptr, 0, stream));
-    MICLOC_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
-    return MICLOC_OK;
+    return micloc_snn_streams_reset(s->sb, nullptr, 0, stream);
 }
 
-extern "C" int micloc_snn_stream_latency(micloc_stream *s) { return s ? s->sb->D : 0; }
+extern "C" int micloc_snn_stream_latency(micloc_stream *s) { return s ? s->sb->book.D : 0; }
 
 extern "C" int micloc_snn_stream_push(micloc_stream *s, const void *frame_dev, int dtype, int64_t n, int32_t in_channels,
                                       int8_t *spikes_dev, float *power_dev, int32_t *doa_dev, float *env_dev,
                                       int32_t *doa_t_dev, int64_t *n_out, void *stream) {
     if (!s || !frame_dev) return set_error(MICLOC_ERR_SHAPE, "null argument");
-    if (!s->sb->active[0]) return set_error(MICLOC_ERR_CONFIG, "stream was flushed: reset it before pushing again");
+    if (!s->sb->book.active[0]) return set_error(MICLOC_ERR_CONFIG, "stream was flushed: reset it before pushing again");
     int64_t m = 0;
     MICLOC_TRY(micloc_snn_streams_push(s->sb, frame_dev, dtype, n, in_channels, spikes_dev, power_dev, doa_dev, env_dev,
                                        doa_t_dev, &m, stream));

@@ -1399,8 +1399,10 @@ extern "C" int micloc_xylo_process(micloc_xylo *c, const int8_t *spikes_in_dev, 
 
 // ---------------------------------------------------------------------------
 // Xylo stream batches: S continuous recordings through the exact front end and the integer network, one push per
-// frame tick (see include/micloc_b200.h).  Per push: k_stream_assemble (float64 rows) -> k_stht_f64_sparse over the
-// frame rows only -> k_xylo_chain_f64<STREAM> -> k_xylo_lif(_mma)<STATE> -> [k_xylo_doa] -> [k_xylo_split].
+// frame tick (see include/micloc_b200.h).  Positions, slot lists, frame checks, the host mirror and the frame assembly
+// are the SlotBook's (micloc_stream.cuh, as for the float batches); the chain, network state and flags are this
+// batch's.  Per push: k_stream_assemble (float64 rows) -> k_stht_f64_sparse over the frame rows only ->
+// k_xylo_chain_f64<STREAM> -> k_xylo_lif(_mma)<STATE> -> [k_xylo_doa] -> [k_xylo_split].
 // ---------------------------------------------------------------------------
 namespace micloc {
 // fresh chain state, LIF state, ring, position and flags of the selected slots (sel == nullptr: all); one thread per
@@ -1429,30 +1431,23 @@ k_xylo_streams_reset(XyloChanState *__restrict__ state, int2 *__restrict__ nstat
 struct micloc_xylo_streams {
     micloc_xylo *c = nullptr;
     int device = 0;
-    long long S = 0, max_frame = 0;
+    SlotBook book;
     int hist = 0;                   // K - 1
-    int D = 0;                      // latency
     int ring_len = 0;
     int chain_warps = kChainWarps;  // slots per CTA of the chain kernel (fewer when float64 tiles of many microphones)
-    int xcur = 0, pcur = 0;
-    long long n_prev = 0;
-    std::vector<long long> N, F;    // host mirror of the positions (n_out without a device synchronisation)
-    std::vector<char> active;
-    std::vector<int32_t> sel_h;
     double *xbuf[2] = {nullptr, nullptr}, *q = nullptr;
     XyloChanState *state = nullptr;
     int2 *nstate = nullptr;
     int8_t *ring = nullptr, *sgn = nullptr;
-    SlotPos *pos[2] = {nullptr, nullptr};
-    int32_t *m = nullptr, *flags = nullptr, *sel = nullptr, *counts = nullptr;
+    int32_t *flags = nullptr, *counts = nullptr;
 };
 
 extern "C" int micloc_xylo_streams_destroy(micloc_xylo_streams *xs) {
     if (!xs) return MICLOC_OK;
     cudaSetDevice(xs->device);
+    xs->book.destroy();
     cudaFree(xs->xbuf[0]); cudaFree(xs->xbuf[1]); cudaFree(xs->q); cudaFree(xs->state); cudaFree(xs->nstate);
-    cudaFree(xs->ring); cudaFree(xs->sgn); cudaFree(xs->pos[0]); cudaFree(xs->pos[1]); cudaFree(xs->m);
-    cudaFree(xs->flags); cudaFree(xs->sel); cudaFree(xs->counts);
+    cudaFree(xs->ring); cudaFree(xs->sgn); cudaFree(xs->flags); cudaFree(xs->counts);
     delete xs;
     return MICLOC_OK;
 }
@@ -1462,43 +1457,26 @@ static size_t xylo_stht_smem(const micloc_xylo *c) {
     return ((size_t)c->n_g + (size_t)mgmax * ((f64_pad(kSTile + c->p.K - 1) + 9) & ~1)) * sizeof(double);
 }
 
-// slots_host [n_slots] (NULL = every slot) -> xs->sel on the device (1 = listed); synchronises `st`
-static int xylo_upload_slots(micloc_xylo_streams *xs, const int32_t *slots_host, int32_t n_slots, cudaStream_t st) {
-    if (slots_host && n_slots < 0) return set_error(MICLOC_ERR_SHAPE, "n_slots %d < 0", n_slots);
-    for (int32_t i = 0; slots_host && i < n_slots; ++i)
-        if (slots_host[i] < 0 || slots_host[i] >= xs->S)
-            return set_error(MICLOC_ERR_SHAPE, "slot %d out of range [0, %lld)", slots_host[i], xs->S);
-    xs->sel_h.assign((size_t)xs->S, slots_host ? 0 : 1);
-    for (int32_t i = 0; slots_host && i < n_slots; ++i) xs->sel_h[(size_t)slots_host[i]] = 1;
-    MICLOC_CUDA(cudaMemcpyAsync(xs->sel, xs->sel_h.data(), (size_t)xs->S * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    MICLOC_CUDA(cudaStreamSynchronize(st));
-    return MICLOC_OK;
-}
-
 extern "C" int micloc_xylo_streams_reset(micloc_xylo_streams *xs, const int32_t *slots_host, int32_t n_slots, void *stream) {
     if (!xs) return set_error(MICLOC_ERR_CONFIG, "null stream batch");
     MICLOC_CUDA(cudaSetDevice(xs->device));
     cudaStream_t st = (cudaStream_t)stream;
-    if (slots_host) MICLOC_TRY(xylo_upload_slots(xs, slots_host, n_slots, st));
+    SlotBook &bk = xs->book;
+    if (slots_host) MICLOC_TRY(bk.upload(slots_host, n_slots, st));
     const micloc_xylo *c = xs->c;
     const int ring16 = (int)((long long)xs->ring_len * c->CT / 16);
     const int W = std::max(std::max(c->CT, c->N), ring16);
-    k_xylo_streams_reset<<<(unsigned)((xs->S * W + 255) / 256), 256, 0, st>>>(
-        xs->state, xs->nstate, xs->ring, xs->pos[xs->pcur], xs->flags, slots_host ? xs->sel : nullptr, xs->S, c->CT, c->N,
+    k_xylo_streams_reset<<<(unsigned)((bk.S * W + 255) / 256), 256, 0, st>>>(
+        xs->state, xs->nstate, xs->ring, bk.pos[bk.pcur], xs->flags, slots_host ? bk.sel : nullptr, bk.S, c->CT, c->N,
         ring16, W);
     count_launch(1);
     MICLOC_CUDA(cudaGetLastError());
-    MICLOC_CUDA(cudaStreamSynchronize(st));
-    for (long long s = 0; s < xs->S; ++s)
-        if (!slots_host || xs->sel_h[(size_t)s]) { xs->N[(size_t)s] = 0; xs->F[(size_t)s] = 0; xs->active[(size_t)s] = 1; }
-    return MICLOC_OK;
+    return bk.reset_done(slots_host != nullptr, st);
 }
 
 extern "C" int micloc_xylo_streams_create(micloc_xylo *c, int32_t num_streams, int64_t max_frame_len, micloc_xylo_streams **out) {
     if (!c || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
     *out = nullptr;
-    if (num_streams < 1 || num_streams > 65535) return set_error(MICLOC_ERR_SHAPE, "num_streams %d out of range [1, 65535]", num_streams);
-    if (max_frame_len < 1 || max_frame_len > (1ll << 24)) return set_error(MICLOC_ERR_SHAPE, "max_frame_len out of range");
     if (c->nba < 1) return set_error(MICLOC_ERR_CONFIG, "the exact front end needs the band filters in b/a form (n_ba)");
     if (!chain_f64_geometry(c))
         return set_error(MICLOC_ERR_UNSUPPORTED,
@@ -1508,18 +1486,20 @@ extern "C" int micloc_xylo_streams_create(micloc_xylo *c, int32_t num_streams, i
     if (xylo_stht_smem(c) > 227 * 1024) return set_error(MICLOC_ERR_UNSUPPORTED, "exact STHT tile needs too much shared memory");
     MICLOC_CUDA(cudaSetDevice(c->device));
     micloc_xylo_streams *xs = new micloc_xylo_streams();
-    xs->c = c; xs->device = c->device; xs->S = num_streams; xs->max_frame = max_frame_len;
+    xs->c = c; xs->device = c->device;
     xs->hist = c->p.K - 1;
     const int w = c->p.w;
-    xs->D = (kF64Cluster - 1) * (w - 1) + w + kChainTile + kF64FlatTop / 2;
+    SlotBook &bk = xs->book;
+    bk.D = (kF64Cluster - 1) * (w - 1) + w + kChainTile + kF64FlatTop / 2;
+    int rc = bk.create(num_streams, max_frame_len);
+    if (rc) { micloc_xylo_streams_destroy(xs); return rc; }
     xs->ring_len = 64;
-    while (xs->ring_len < max_frame_len + xs->D) xs->ring_len <<= 1;
+    while (xs->ring_len < max_frame_len + bk.D) xs->ring_len <<= 1;
     const size_t per_warp = (size_t)kChainTile * c->p.M * 2 * sizeof(double);
     xs->chain_warps = (int)std::min<size_t>(kChainWarps, (size_t)(227 * 1024) / per_warp);
-    xs->N.assign((size_t)num_streams, 0); xs->F.assign((size_t)num_streams, 0); xs->active.assign((size_t)num_streams, 1);
     const size_t S = (size_t)num_streams, M = (size_t)c->p.M, CT = (size_t)c->CT;
     const size_t rows = (size_t)xs->hist + max_frame_len;
-    const size_t fin = (size_t)max_frame_len + xs->D;
+    const size_t fin = (size_t)max_frame_len + bk.D;
     bool ok = cudaMalloc(&xs->xbuf[0], S * rows * M * sizeof(double)) == cudaSuccess &&
               cudaMalloc(&xs->xbuf[1], S * rows * M * sizeof(double)) == cudaSuccess &&
               cudaMalloc(&xs->q, S * rows * M * sizeof(double)) == cudaSuccess &&
@@ -1527,20 +1507,16 @@ extern "C" int micloc_xylo_streams_create(micloc_xylo *c, int32_t num_streams, i
               cudaMalloc(&xs->nstate, S * c->N * sizeof(int2)) == cudaSuccess &&
               cudaMalloc(&xs->ring, S * CT * (size_t)xs->ring_len) == cudaSuccess &&
               cudaMalloc(&xs->sgn, S * fin * CT) == cudaSuccess &&
-              cudaMalloc(&xs->pos[0], S * sizeof(SlotPos)) == cudaSuccess &&
-              cudaMalloc(&xs->pos[1], S * sizeof(SlotPos)) == cudaSuccess &&
-              cudaMalloc(&xs->m, S * sizeof(int32_t)) == cudaSuccess &&
               cudaMalloc(&xs->flags, S * sizeof(int32_t)) == cudaSuccess &&
-              cudaMalloc(&xs->sel, S * sizeof(int32_t)) == cudaSuccess &&
               cudaMalloc(&xs->counts, S * c->N * sizeof(int32_t)) == cudaSuccess;
     if (!ok) { micloc_xylo_streams_destroy(xs); return set_error(MICLOC_ERR_CUDA, "cudaMalloc(Xylo stream batch) failed"); }
-    const int rc = micloc_xylo_streams_reset(xs, nullptr, 0, nullptr);
+    rc = micloc_xylo_streams_reset(xs, nullptr, 0, nullptr);
     if (rc) { micloc_xylo_streams_destroy(xs); return rc; }
     *out = xs;
     return MICLOC_OK;
 }
 
-extern "C" int micloc_xylo_streams_latency(micloc_xylo_streams *xs) { return xs ? xs->D : 0; }
+extern "C" int micloc_xylo_streams_latency(micloc_xylo_streams *xs) { return xs ? xs->book.D : 0; }
 
 // shared by push and flush: chain of the new samples (n = 0: flush of the slots in close_sel), then the integer
 // network, DoA and the {0,1} input spikes over each slot's final rows (row stride `rows`)
@@ -1548,37 +1524,39 @@ template <int NBA>
 static void launch_chain_stream(micloc_xylo_streams *xs, const int32_t *close_sel, long long n, long long rows, cudaStream_t st) {
     const micloc_xylo *c = xs->c;
     const ChainParams &p = c->p;
+    const SlotBook &bk = xs->book;
     XyloChainStream sa;
-    sa.state = xs->state; sa.pos_in = xs->pos[xs->pcur]; sa.pos_out = xs->pos[xs->pcur ^ 1]; sa.m_out = xs->m;
+    sa.state = xs->state; sa.pos_in = bk.pos[bk.pcur]; sa.pos_out = bk.pos[bk.pcur ^ 1]; sa.m_out = bk.m;
     sa.close_sel = close_sel; sa.ring = xs->ring; sa.ring_len = xs->ring_len; sa.hist = xs->hist; sa.rows = (int)rows;
-    sa.D = xs->D;
+    sa.D = bk.D;
     const int nw = xs->chain_warps;
     const size_t smem = (size_t)nw * kChainTile * p.M * 2 * sizeof(double);
     cudaFuncSetAttribute(k_xylo_chain_f64<double, NBA, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_xylo_chain_f64<double, NBA, true><<<(unsigned)((xs->S + nw - 1) / nw), 32 * nw, smem, st>>>(
-        xs->xbuf[xs->xcur], xs->q, c->d_ba_b, c->d_ba_a, xs->sgn, xs->flags, p.M, p.half, c->nba, c->F, p.w, p.bipolar, xs->S,
+    k_xylo_chain_f64<double, NBA, true><<<(unsigned)((bk.S + nw - 1) / nw), 32 * nw, smem, st>>>(
+        xs->xbuf[bk.xcur], xs->q, c->d_ba_b, c->d_ba_a, xs->sgn, xs->flags, p.M, p.half, c->nba, c->F, p.w, p.bipolar, bk.S,
         n, sa);
 }
 
+// the chain's positions are flipped by the caller (SlotBook::pushed / flushed)
 static int xylo_streams_advance(micloc_xylo_streams *xs, const int32_t *close_sel, long long n, long long rows,
                                 int8_t *spikes_in_dev, uint8_t *raster_dev, int32_t *counts_dev, int32_t *doa_dev,
                                 int32_t *doa_peak_dev, int32_t peak_win, int32_t *flags_dev, cudaStream_t st) {
     micloc_xylo *c = xs->c;
+    const SlotBook &bk = xs->book;
     if (c->nba <= 3) launch_chain_stream<3>(xs, close_sel, n, rows, st);
     else launch_chain_stream<5>(xs, close_sel, n, rows, st);
     count_launch(1);
     MICLOC_CUDA(cudaGetLastError());
-    xs->pcur ^= 1;
     int32_t *counts = counts_dev ? counts_dev : xs->counts;
-    MICLOC_TRY((launch_lif<true, true>(c, xs->sgn, xs->S, rows, raster_dev, counts, st, xs->m, xs->nstate)));
-    MICLOC_TRY(launch_doa(c, counts, xs->S, doa_dev, doa_peak_dev, peak_win, st, xs->m));
+    MICLOC_TRY((launch_lif<true, true>(c, xs->sgn, bk.S, rows, raster_dev, counts, st, bk.m, xs->nstate)));
+    MICLOC_TRY(launch_doa(c, counts, bk.S, doa_dev, doa_peak_dev, peak_win, st, bk.m));
     if (spikes_in_dev) {
-        const long long r = xs->S * rows;
-        k_xylo_split<<<(unsigned)((r * c->CT + 255) / 256), 256, 0, st>>>(xs->sgn, spikes_in_dev, r, c->CT, c->p.bipolar, xs->m, rows);
+        const long long r = bk.S * rows;
+        k_xylo_split<<<(unsigned)((r * c->CT + 255) / 256), 256, 0, st>>>(xs->sgn, spikes_in_dev, r, c->CT, c->p.bipolar, bk.m, rows);
         count_launch(1);
         MICLOC_CUDA(cudaGetLastError());
     }
-    if (flags_dev) MICLOC_CUDA(cudaMemcpyAsync(flags_dev, xs->flags, (size_t)xs->S * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    if (flags_dev) MICLOC_CUDA(cudaMemcpyAsync(flags_dev, xs->flags, (size_t)bk.S * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
     return MICLOC_OK;
 }
 
@@ -1587,60 +1565,31 @@ extern "C" int micloc_xylo_streams_push(micloc_xylo_streams *xs, const void *fra
                                         int32_t *doa_peak_dev, int32_t peak_win, int32_t *flags_dev, int64_t *n_out_host,
                                         void *stream) {
     if (!xs || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
+    if (!frames_dev) return set_error(MICLOC_ERR_SHAPE, "null frame pointer");
     micloc_xylo *c = xs->c;
     const ChainParams &p = c->p;
-    if (n < 1 || n > xs->max_frame) return set_error(MICLOC_ERR_SHAPE, "frame of %lld samples (stream takes 1..%lld)", (long long)n, xs->max_frame);
-    if (!frames_dev) return set_error(MICLOC_ERR_SHAPE, "null frame pointer");
-    if (in_channels < p.M)
-        return set_error(MICLOC_ERR_SHAPE, "number of channels in the input siganl %d should be the same as the number of microphones %d!", in_channels, p.M);
-    if (dtype != MICLOC_F32 && dtype != MICLOC_I16 && dtype != MICLOC_I32)
-        return set_error(MICLOC_ERR_SHAPE, "dtype must be MICLOC_F32, MICLOC_I16 or MICLOC_I32");
-    for (long long s = 0; s < xs->S; ++s)
-        if (xs->active[(size_t)s] && xs->N[(size_t)s] + n >= (1ll << 31) - 4096)
-            return set_error(MICLOC_ERR_SHAPE, "stream position exceeds 2^31 samples: reset the stream");
+    SlotBook &bk = xs->book;
+    MICLOC_TRY(bk.check_push(dtype, n, in_channels, p.M));
     MICLOC_TRY(check_peak_win(c, doa_peak_dev, peak_win));
     MICLOC_CUDA(cudaSetDevice(xs->device));
     cudaStream_t st = (cudaStream_t)stream;
     // [K-1 history rows | frame] in float64
-    const int nxt = xs->xcur ^ 1;
-    const long long total = xs->S * (xs->hist + n) * p.M;
-    const unsigned ga = (unsigned)((total + 255) / 256);
-    const double *prev = xs->xbuf[xs->xcur];
-    const SlotPos *pos = xs->pos[xs->pcur];
-    if (dtype == MICLOC_F32)
-        k_stream_assemble<float, double><<<ga, 256, 0, st>>>((const float *)frames_dev, prev, xs->xbuf[nxt], pos, xs->S, (int)n, (int)xs->n_prev, in_channels, p.M, xs->hist);
-    else if (dtype == MICLOC_I16)
-        k_stream_assemble<int16_t, double><<<ga, 256, 0, st>>>((const int16_t *)frames_dev, prev, xs->xbuf[nxt], pos, xs->S, (int)n, (int)xs->n_prev, in_channels, p.M, xs->hist);
-    else
-        k_stream_assemble<int32_t, double><<<ga, 256, 0, st>>>((const int32_t *)frames_dev, prev, xs->xbuf[nxt], pos, xs->S, (int)n, (int)xs->n_prev, in_channels, p.M, xs->hist);
-    count_launch(1);
-    MICLOC_CUDA(cudaGetLastError());
-    xs->xcur = nxt;
-    xs->n_prev = n;
+    MICLOC_TRY(bk.assemble(xs->xbuf, frames_dev, dtype, n, in_channels, p.M, xs->hist, st));
     // STHT of the frame rows only (the history rows were the previous push's frame rows)
     {
         const long long rows_in = xs->hist + n;
         const int ntiles = (int)((n + kSTile - 1) / kSTile);
         const size_t smem = xylo_stht_smem(c);
-        dim3 grid((unsigned)(xs->S * ntiles), (unsigned)((p.M + kF64MG - 1) / kF64MG));
+        dim3 grid((unsigned)(bk.S * ntiles), (unsigned)((p.M + kF64MG - 1) / kF64MG));
         MICLOC_CUDA(cudaFuncSetAttribute(k_stht_f64_sparse<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_stht_f64_sparse<double><<<grid, 256, smem, st>>>(xs->xbuf[xs->xcur], c->d_g, xs->q, p.M, p.K, c->n_g, rows_in, ntiles,
+        k_stht_f64_sparse<double><<<grid, 256, smem, st>>>(xs->xbuf[bk.xcur], c->d_g, xs->q, p.M, p.K, c->n_g, rows_in, ntiles,
                                                           (long long)xs->hist);
         count_launch(1);
         MICLOC_CUDA(cudaGetLastError());
     }
-    const long long rows = n + xs->D;
-    MICLOC_TRY(xylo_streams_advance(xs, nullptr, n, rows, spikes_in_dev, raster_dev, counts_dev, doa_dev, doa_peak_dev,
+    MICLOC_TRY(xylo_streams_advance(xs, nullptr, n, n + bk.D, spikes_in_dev, raster_dev, counts_dev, doa_dev, doa_peak_dev,
                                     peak_win, flags_dev, st));
-    for (long long s = 0; s < xs->S; ++s) {
-        const size_t i = (size_t)s;
-        n_out_host[s] = 0;
-        if (!xs->active[i]) continue;
-        xs->N[i] += n;
-        const long long f = xs->N[i] - xs->D > xs->F[i] ? xs->N[i] - xs->D : xs->F[i];
-        n_out_host[s] = f - xs->F[i];
-        xs->F[i] = f;
-    }
+    bk.pushed(n, n_out_host);
     return MICLOC_OK;
 }
 
@@ -1652,20 +1601,13 @@ extern "C" int micloc_xylo_streams_flush(micloc_xylo_streams *xs, const int32_t 
     MICLOC_TRY(check_peak_win(xs->c, doa_peak_dev, peak_win));
     MICLOC_CUDA(cudaSetDevice(xs->device));
     cudaStream_t st = (cudaStream_t)stream;
-    MICLOC_TRY(xylo_upload_slots(xs, slots_host, n_slots, st));
-    const long long rows = xs->max_frame + xs->D;
-    MICLOC_TRY(xylo_streams_advance(xs, xs->sel, 0, rows, spikes_in_dev, raster_dev, counts_dev, doa_dev, doa_peak_dev,
-                                    peak_win, flags_dev, st));
-    for (long long s = 0; s < xs->S; ++s) {
-        const size_t i = (size_t)s;
-        n_out_host[s] = 0;
-        if (!xs->active[i] || !xs->sel_h[i]) continue;
-        n_out_host[s] = xs->N[i] - xs->F[i];
-        xs->F[i] = xs->N[i];
-        xs->active[i] = 0;
-    }
+    SlotBook &bk = xs->book;
+    MICLOC_TRY(bk.upload(slots_host, n_slots, st));
+    MICLOC_TRY(xylo_streams_advance(xs, bk.sel, 0, bk.max_frame + bk.D, spikes_in_dev, raster_dev, counts_dev, doa_dev,
+                                    doa_peak_dev, peak_win, flags_dev, st));
+    bk.flushed(n_out_host);
     if (flags_host) {
-        MICLOC_CUDA(cudaMemcpyAsync(flags_host, xs->flags, (size_t)xs->S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        MICLOC_CUDA(cudaMemcpyAsync(flags_host, xs->flags, (size_t)bk.S * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         MICLOC_CUDA(cudaStreamSynchronize(st));
     }
     return MICLOC_OK;

@@ -23,6 +23,52 @@ def _stream_ptr(device: torch.device):
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+def _check_frames(frames: torch.Tensor, M: int, device: torch.device, num_streams: Optional[int] = None):
+    """The frames of a stream push: [n, channels] (num_streams None) or [num_streams, n, channels], channels >= M, on
+    `device`, float32 / int16 / int32 -> (contiguous frames, dtype code)."""
+    if frames.dim() != (2 if num_streams is None else 3) or frames.shape[-1] < M:
+        raise ValueError(
+            f"number of channels in the input siganl {frames.shape[-1]} should be the same as the number of microphones {M}!")
+    if num_streams is not None and frames.shape[0] != num_streams:
+        raise ValueError(f"frames hold {frames.shape[0]} slots, the batch has {num_streams}")
+    if frames.device != device:
+        raise ValueError(f"frames live on {frames.device}, the stream on {device}")
+    dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frames.dtype)
+    if dt is None:
+        raise ValueError(f"frames must be float32, int16 or int32, got {frames.dtype}")
+    return frames.contiguous(), dt
+
+
+class _SlotBatch:
+    """What the stream batches share: the native batch `_h` of `num_streams` slots on `device`, whose C functions are
+    named `<api>_reset`, `<api>_latency` and `<api>_destroy`, and its slot lists.  A subclass creates the handle and
+    hands it to `_attach`."""
+
+    def _attach(self, lib, h, api: str, num_streams: int, max_frame_len: int, device: torch.device):
+        self._lib, self._h, self._api = lib, h, api
+        self.num_streams, self.max_frame_len, self.device = num_streams, max_frame_len, device
+        self.latency = int(getattr(lib, api + "_latency")(h))
+
+    def close(self):
+        if getattr(self, "_h", None):
+            getattr(self._lib, self._api + "_destroy")(self._h)
+            self._h = None
+
+    __del__ = close
+
+    @staticmethod
+    def _slots(slots):
+        if slots is None:
+            return None, None, 0
+        arr = np.ascontiguousarray(np.atleast_1d(np.asarray(slots)), dtype=np.int32)
+        return arr, arr.ctypes.data_as(C.c_void_p), len(arr)
+
+    def reset(self, slots=None):
+        """Fresh state for the listed slots (None: all); they restart at sample 0."""
+        arr, p, n = self._slots(slots)
+        N.check(getattr(self._lib, self._api + "_reset")(self._h, p, n, _stream_ptr(self.device)))
+
+
 @dataclass
 class ChainSpec:
     """Host constants of one SNN chain (what SNNBeamformer derives, snn_beamformer.py:45-80,342-361)."""
@@ -268,15 +314,7 @@ class SnnStream:
         """One frame in, the samples that became final out: dict(n_out, spikes [n_out, 2M], power [G] and doa [1]
         over those samples, env [n_out, G] + doa_t [n_out] when `want_env`)."""
         e = self.engine
-        if frame.dim() != 2 or frame.shape[1] < e.M:
-            raise ValueError(
-                f"number of channels in the input siganl {frame.shape[-1]} should be the same as the number of microphones {e.M}!")
-        if frame.device != e.device:
-            raise ValueError(f"frame lives on {frame.device}, engine on {e.device}")
-        dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frame.dtype)
-        if dt is None:
-            raise ValueError(f"frame must be float32, int16 or int32, got {frame.dtype}")
-        frame = frame.contiguous()
+        frame, dt = _check_frames(frame, e.M, e.device)
         n = frame.shape[0]
         out = self._outputs(n + self.latency, want_env)
         n_out = C.c_int64()
@@ -297,7 +335,7 @@ class SnnStream:
         return res
 
 
-class SnnStreamBatch:
+class SnnStreamBatch(_SlotBatch):
     """`num_streams` independent recordings ("slots") advanced together (micloc_snn_streams_*): one push hands every
     slot one frame of the same length and runs a fixed number of kernels whatever the number of slots.  Each slot
     behaves as an `SnnStream`; `reset` and `flush` act on a list of slots only, and a flushed slot ignores its rows of
@@ -307,33 +345,10 @@ class SnnStreamBatch:
     def __init__(self, engine: SnnEngine, num_streams: int, max_frame_len: int, fs: float = 48_000.0,
                  rise_time: float = 10e-3, fall_time: float = 100e-3):
         self.engine = engine
-        self._lib = engine._lib
-        self.num_streams = int(num_streams)
-        self.max_frame_len = int(max_frame_len)
         h = C.c_void_p()
-        N.check(self._lib.micloc_snn_streams_create(engine._h, self.num_streams, self.max_frame_len, float(fs),
-                                                    float(rise_time), float(fall_time), C.byref(h)))
-        self._h = h
-        self.latency = int(self._lib.micloc_snn_streams_latency(h))
-
-    def close(self):
-        if getattr(self, "_h", None):
-            self._lib.micloc_snn_streams_destroy(self._h)
-            self._h = None
-
-    __del__ = close
-
-    @staticmethod
-    def _slots(slots):
-        if slots is None:
-            return None, None, 0
-        arr = np.ascontiguousarray(np.atleast_1d(np.asarray(slots)), dtype=np.int32)
-        return arr, arr.ctypes.data_as(C.c_void_p), len(arr)
-
-    def reset(self, slots=None):
-        """Fresh state for the listed slots (None: all); they restart at sample 0."""
-        arr, p, n = self._slots(slots)
-        N.check(self._lib.micloc_snn_streams_reset(self._h, p, n, _stream_ptr(self.engine.device)))
+        N.check(engine._lib.micloc_snn_streams_create(engine._h, int(num_streams), int(max_frame_len), float(fs),
+                                                      float(rise_time), float(fall_time), C.byref(h)))
+        self._attach(engine._lib, h, "micloc_snn_streams", int(num_streams), int(max_frame_len), engine.device)
 
     def _outputs(self, rows, want_env):
         e, S = self.engine, self.num_streams
@@ -348,25 +363,14 @@ class SnnStreamBatch:
         """One frame per slot in, the samples that became final out: dict(n_out numpy int64 [S], spikes [S, n + D, 2M],
         power [S, G], doa [S], + env [S, n + D, G] and doa_t [S, n + D] when `want_env`).  Slot s fills its first
         n_out[s] rows; the other rows, and power / doa of a slot with n_out[s] == 0, are left as allocated."""
-        e = self.engine
-        if frames.dim() != 3 or frames.shape[2] < e.M:
-            raise ValueError(
-                f"number of channels in the input siganl {frames.shape[-1]} should be the same as the number of microphones {e.M}!")
-        if frames.shape[0] != self.num_streams:
-            raise ValueError(f"frames hold {frames.shape[0]} slots, the batch has {self.num_streams}")
-        if frames.device != e.device:
-            raise ValueError(f"frame lives on {frames.device}, engine on {e.device}")
-        dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frames.dtype)
-        if dt is None:
-            raise ValueError(f"frame must be float32, int16 or int32, got {frames.dtype}")
-        frames = frames.contiguous()
+        frames, dt = _check_frames(frames, self.engine.M, self.device, self.num_streams)
         n = frames.shape[1]
         out = self._outputs(n + self.latency, want_env)
         n_out = np.zeros(self.num_streams, dtype=np.int64)
         N.check(self._lib.micloc_snn_streams_push(self._h, _ptr(frames), dt, n, frames.shape[2], _ptr(out["spikes"]),
                                                   _ptr(out["power"]), _ptr(out["doa"]), _ptr(out["env"]),
                                                   _ptr(out["doa_t"]), n_out.ctypes.data_as(C.c_void_p),
-                                                  _stream_ptr(e.device)))
+                                                  _stream_ptr(self.device)))
         out["n_out"] = n_out
         if not want_env:
             del out["env"], out["doa_t"]
@@ -382,7 +386,7 @@ class SnnStreamBatch:
         N.check(self._lib.micloc_snn_streams_flush(self._h, p, ns, _ptr(out["spikes"]), _ptr(out["power"]),
                                                    _ptr(out["doa"]), _ptr(out["env"]), _ptr(out["doa_t"]),
                                                    n_out.ctypes.data_as(C.c_void_p), flags.ctypes.data_as(C.c_void_p),
-                                                   _stream_ptr(self.engine.device)))
+                                                   _stream_ptr(self.device)))
         out["n_out"], out["flags"] = n_out, flags
         if not want_env:
             del out["env"], out["doa_t"]

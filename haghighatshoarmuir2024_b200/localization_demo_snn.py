@@ -21,7 +21,7 @@ import torch
 
 from . import _native as N
 from .array_geometry import ArrayGeometry
-from .engine import SnnEngine, _ptr, _stream_ptr
+from .engine import SnnEngine, _SlotBatch, _check_frames, _ptr, _stream_ptr
 from .filterbank import ButterworthFilterbank
 from .snn_beamformer import SNNBeamformer
 
@@ -133,7 +133,7 @@ class Demo:
             yield self.process_frame(data)
 
 
-class MultibandStreamBatch:
+class MultibandStreamBatch(_SlotBatch):
     """`num_streams` independent recordings ("slots") through the multi-band localiser with its state carried across
     pushes (micloc_snn_mb_streams_*).  N pushed frames give, for every band, what the filterbank of their
     concatenation followed by that band's stream gives (see engine.SnnStreamBatch); every band finalises the same
@@ -146,43 +146,20 @@ class MultibandStreamBatch:
 
     def __init__(self, demo: Demo, num_streams: int, max_frame_len: int):
         self.demo = demo
-        self.num_streams = int(num_streams)
-        self.max_frame_len = int(max_frame_len)
-        self.device = demo.device
         self.time_vec = np.arange(int(round(demo.recording_duration * demo.fs))) / demo.fs
         self.engines = [SnnEngine(beamf.chain_spec(self.time_vec), bf, device=demo.device.index or 0)
                         for beamf, bf in zip(demo.beamfs, demo.bf_mats)]
         self.F, self.M, self.G = len(self.engines), demo.num_mic, len(demo.doa_list)
         self.C2 = 2 * self.M
-        self._lib = N.lib()
+        lib = N.lib()
         sos = np.ascontiguousarray(demo.filterbank.sos_list, dtype=np.float64)           # [F][nsec][6]
         ctxs = (C.c_void_p * self.F)(*[e._h.value for e in self.engines])
         h = C.c_void_p()
-        N.check(self._lib.micloc_snn_mb_streams_create(ctxs, self.F, sos.shape[1], sos.ctypes.data_as(N._dp),
-                                                       demo.doa_list.ctypes.data_as(N._dp), self.num_streams,
-                                                       self.max_frame_len, C.byref(h)))
-        self._h = h
-        self.latency = int(self._lib.micloc_snn_mb_streams_latency(h))
+        N.check(lib.micloc_snn_mb_streams_create(ctxs, self.F, sos.shape[1], sos.ctypes.data_as(N._dp),
+                                                 demo.doa_list.ctypes.data_as(N._dp), int(num_streams),
+                                                 int(max_frame_len), C.byref(h)))
+        self._attach(lib, h, "micloc_snn_mb_streams", int(num_streams), int(max_frame_len), demo.device)
         self._doa_dev = torch.from_numpy(demo.doa_list).to(self.device)
-
-    def close(self):
-        if getattr(self, "_h", None):
-            self._lib.micloc_snn_mb_streams_destroy(self._h)
-            self._h = None
-
-    __del__ = close
-
-    @staticmethod
-    def _slots(slots):
-        if slots is None:
-            return None, None, 0
-        arr = np.ascontiguousarray(np.atleast_1d(np.asarray(slots)), dtype=np.int32)
-        return arr, arr.ctypes.data_as(C.c_void_p), len(arr)
-
-    def reset(self, slots=None):
-        """Fresh state (filterbank included) for the listed slots (None: all); they restart at sample 0."""
-        arr, p, n = self._slots(slots)
-        N.check(self._lib.micloc_snn_mb_streams_reset(self._h, p, n, _stream_ptr(self.device)))
 
     def _outputs(self, rows, want_spikes):
         S, dev = self.num_streams, self.device
@@ -203,17 +180,7 @@ class MultibandStreamBatch:
         -1).  active [S] and doa_deg [S] as in `localize`, the gate on the rms of the frame just pushed (D samples
         ahead of the power window); doa_deg is NaN where inactive or where n_out == 0.  sumsq [S] float64 of the
         frame.  No host synchronisation."""
-        if frames.dim() != 3 or frames.shape[2] < self.M:
-            raise ValueError(
-                f"number of channels in the input siganl {frames.shape[-1]} should be the same as the number of microphones {self.M}!")
-        if frames.shape[0] != self.num_streams:
-            raise ValueError(f"frames hold {frames.shape[0]} slots, the batch has {self.num_streams}")
-        if frames.device != self.device:
-            raise ValueError(f"frames live on {frames.device}, the batch on {self.device}")
-        dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frames.dtype)
-        if dt is None:
-            raise ValueError(f"frames must be float32, int16 or int32, got {frames.dtype}")
-        frames = frames.contiguous()
+        frames, dt = _check_frames(frames, self.M, self.device, self.num_streams)
         S, n, ch = frames.shape
         out = self._outputs(n + self.latency, want_spikes)
         sumsq = torch.empty(S, dtype=torch.float64, device=self.device)

@@ -30,6 +30,7 @@ import torch
 
 from . import _native as N
 from .array_geometry import ArrayGeometry
+from .engine import _SlotBatch, _check_frames, _ptr, _stream_ptr
 from .filterbank import ButterworthFilterbank
 from .snn_beamformer import SNNBeamformer
 
@@ -104,10 +105,6 @@ def quantize_network(bf_mats: Sequence[np.ndarray], tau_vecs: np.ndarray, fs: fl
                        threshold=np.full(n_hidden, thr_q, dtype=np.int16),
                        dash_syn=np.ascontiguousarray(dash_syn.astype(np.int8)),
                        dash_mem=np.ascontiguousarray(dash_mem.astype(np.int8)), scale=float(scale))
-
-
-def _ptr(t: Optional[torch.Tensor]):
-    return None if t is None else C.c_void_p(t.data_ptr())
 
 
 class XyloEngine:
@@ -227,7 +224,7 @@ class XyloEngine:
         return {"counts": counts, "doa": doa, "doa_peak": doa_peak, "raster": raster}
 
 
-class XyloStreamBatch:
+class XyloStreamBatch(_SlotBatch):
     """`num_streams` independent recordings ("slots") through the exact (float64) front end and the integer network
     with their state carried across pushes (micloc_xylo_streams_*).  N pushed frames plus a flush give, for every slot,
     bit for bit what `XyloEngine.run(exact=True)` gives on one clip of their concatenation (in-phase branch: the causal
@@ -242,44 +239,21 @@ class XyloStreamBatch:
     def __init__(self, engine: XyloEngine, num_streams: int, max_frame_len: int, fs: float = 48_000.0,
                  doa_list: Optional[np.ndarray] = None):
         self.engine = engine
-        self.num_streams = int(num_streams)
-        self.max_frame_len = int(max_frame_len)
-        self.device = engine.device
         self.fs = float(fs)
         self.M, self.F, self.G, self.N, self.N_in = engine.M, engine.F, engine.G, engine.N, engine.N_in
-        self._lib = N.lib()
+        lib = N.lib()
         h = C.c_void_p()
-        rc = self._lib.micloc_xylo_streams_create(engine._h, self.num_streams, self.max_frame_len, C.byref(h))
+        rc = lib.micloc_xylo_streams_create(engine._h, int(num_streams), int(max_frame_len), C.byref(h))
         if rc in (N.ERR_CONFIG, N.ERR_UNSUPPORTED):
-            raise N.MiclocError(rc, self._lib.micloc_last_error().decode("utf-8", "replace"))
+            raise N.MiclocError(rc, lib.micloc_last_error().decode("utf-8", "replace"))
         N.check(rc)
-        self._h = h
-        self.latency = int(self._lib.micloc_xylo_streams_latency(h))
+        self._attach(lib, h, "micloc_xylo_streams", int(num_streams), int(max_frame_len), engine.device)
         self._doa_dev = None
         if doa_list is not None:
             doa_list = np.ascontiguousarray(doa_list, dtype=np.float64)
             if doa_list.shape != (self.G,):
                 raise ValueError(f"doa_list should hold {self.G} angles")
             self._doa_dev = torch.from_numpy(doa_list).to(self.device)
-
-    def close(self):
-        if getattr(self, "_h", None):
-            self._lib.micloc_xylo_streams_destroy(self._h)
-            self._h = None
-
-    __del__ = close
-
-    @staticmethod
-    def _slots(slots):
-        if slots is None:
-            return None, None, 0
-        arr = np.ascontiguousarray(np.atleast_1d(np.asarray(slots)), dtype=np.int32)
-        return arr, arr.ctypes.data_as(C.c_void_p), len(arr)
-
-    def reset(self, slots=None):
-        """Fresh state for the listed slots (None: all); they restart at sample 0."""
-        arr, p, n = self._slots(slots)
-        N.check(self._lib.micloc_xylo_streams_reset(self._h, p, n, self.engine._stream()))
 
     def _outputs(self, rows, want_spikes_in, want_raster, peak_win):
         S, dev = self.num_streams, self.device
@@ -304,7 +278,8 @@ class XyloStreamBatch:
             ml = torch.empty(S, dtype=torch.float64, device=self.device)
             trimmed = torch.empty(S, dtype=torch.float64, device=self.device)
             N.check(self._lib.micloc_power_fuse(_ptr(power), F, S, G, _ptr(self._doa_dev), None, None, _ptr(ml),
-                                                _ptr(trimmed), _ptr(fflags), self.device.index or 0, self.engine._stream()))
+                                                _ptr(trimmed), _ptr(fflags), self.device.index or 0,
+                                                _stream_ptr(self.device)))
             nan = torch.full_like(ml, float("nan"))
             out["periodic_ml"] = torch.where(live, ml, nan)
             out["trimmed_periodic_ml"] = torch.where(live, trimmed, nan)
@@ -319,24 +294,14 @@ class XyloStreamBatch:
         clip's bits since its reset; bit 1: the trimmed estimator's IndexError, estimate NaN), spikes_in [S, n + D,
         N_in] / raster [S, n + D, N] on request (slot s fills its first n_out[s] rows).  No host synchronisation
         beyond the row counts."""
-        if frames.dim() != 3 or frames.shape[2] < self.M:
-            raise ValueError(
-                f"number of channels in the input siganl {frames.shape[-1]} should be the same as the number of microphones {self.M}!")
-        if frames.shape[0] != self.num_streams:
-            raise ValueError(f"frames hold {frames.shape[0]} slots, the batch has {self.num_streams}")
-        if frames.device != self.device:
-            raise ValueError(f"frames live on {frames.device}, the batch on {self.device}")
-        dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frames.dtype)
-        if dt is None:
-            raise ValueError(f"frames must be float32, int16 or int32, got {frames.dtype}")
-        frames = frames.contiguous()
+        frames, dt = _check_frames(frames, self.M, self.device, self.num_streams)
         S, n, ch = frames.shape
         out = self._outputs(n + self.latency, want_spikes_in, want_raster, peak_win)
         n_out = np.zeros(S, dtype=np.int64)
         N.check(self._lib.micloc_xylo_streams_push(
             self._h, _ptr(frames), dt, n, ch, _ptr(out["spikes_in"]), _ptr(out["raster"]), _ptr(out["counts"]),
             _ptr(out["doa"]), _ptr(out["doa_peak"]), int(peak_win), _ptr(out["flags"]), n_out.ctypes.data_as(C.c_void_p),
-            self.engine._stream()))
+            _stream_ptr(self.device)))
         out["flags"] = out["flags"] | self._estimators(out, n_out)
         out["n_out"] = n_out
         return out
@@ -353,7 +318,7 @@ class XyloStreamBatch:
         N.check(self._lib.micloc_xylo_streams_flush(
             self._h, p, ns, _ptr(out["spikes_in"]), _ptr(out["raster"]), _ptr(out["counts"]), _ptr(out["doa"]),
             _ptr(out["doa_peak"]), int(peak_win), _ptr(out["flags"]), n_out.ctypes.data_as(C.c_void_p),
-            flags.ctypes.data_as(C.c_void_p), self.engine._stream()))
+            flags.ctypes.data_as(C.c_void_p), _stream_ptr(self.device)))
         fflags = self._estimators(out, n_out).cpu().numpy()
         out.update({"n_out": n_out, "flags": flags | fflags})
         return out

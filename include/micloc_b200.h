@@ -169,7 +169,8 @@ int micloc_snn_stream_flush(micloc_stream *s, int8_t *spikes_dev, float *power_d
  *       n_out = 0, are NOT written.
  *   - flush closes the listed slots like a clip end; outputs as in push with [S][max_frame_len + D] rows;
  *     flags_host [S] (nullable, host): bit 0 = RZCC overflow anywhere in that slot's recording (synchronises).
- *   - reset / flush copy the slot list to the device and synchronise `stream`; a push does not synchronise.
+ *   - reset and flush synchronise `stream` (reset with slots_host NULL too); a push does not synchronise.  This holds
+ *     for every stream batch kind: micloc_snn_streams_*, micloc_snn_mb_streams_* and micloc_xylo_streams_*.
  * Kernel launches per push, whatever S: 5 (frame assembly, STHT, band-pass + RZCC + neuron, Gram, power), of which Gram
  * and power only when power_dev or doa_dev is given; +2 (dense y, envelope) when env_dev or doa_t_dev is given, +1
  * (argmax) when doa_t_dev is given.  The envelope scratch (S (n + D) G floats, twice when env_dev is NULL) is allocated
@@ -213,8 +214,8 @@ int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *slots_host,
  *       at the newest frame, D samples ahead of the samples the power describes.
  *   - flush closes the listed slots (slots_host [n_slots], NULL = every slot) like a clip end; outputs as in push with
  *     [max_frame_len + D] rows; flags_host [S] (nullable, host): bit 0 = RZCC overflow anywhere in that slot's
- *     recording, any band.  reset / flush / flushed slots behave as in micloc_snn_streams_*; reset also restarts the
- *     filterbank of the listed slots from zero state.  reset and flush synchronise `stream`, a push does not.
+ *     recording, any band.  reset / flush / flushed slots and synchronisation behave as in micloc_snn_streams_*;
+ *     reset also restarts the filterbank of the listed slots from zero state.
  * Kernel launches per push, whatever S: 4 F + 2 (filterbank + frame assembly; per band STHT, band-pass + RZCC +
  * neuron, Gram, power; the sum over bands with its estimators), 2 F + 1 when no power, fused output or flags are
  * requested.  1 <= num_streams <= 65535; doa_list [G] (host, nullable: no ML estimators).  The contexts' constants
@@ -378,8 +379,8 @@ int micloc_xylo_process(micloc_xylo *ctx, const int8_t *spikes_in_dev, int64_t B
  *   - Slots, positions, flushed slots, n_out_host and unwritten rows as in micloc_snn_streams_*: slots_host [n_slots]
  *     (NULL = every slot); a slot reset mid-run restarts at 0 while the others go on; a flushed slot ignores later pushes
  *     (n_out = 0, state untouched) until it is reset; n_out_host[s] (host, computed without a synchronisation) is the
- *     number of samples of slot s that became final with this call; reset and flush synchronise `stream`, a push does
- *     not; a push that would take a slot's position to 2^31 - 4096 samples or beyond is refused.
+ *     number of samples of slot s that became final with this call; synchronisation as there; a push that would take
+ *     a slot's position to 2^31 - 4096 samples or beyond is refused.
  *   - push: frames_dev [S][n][in_channels] float32 / int16 / int32, 1 <= n <= max_frame_len (channels >= num_mic are
  *     dropped).  Outputs, all nullable device pointers, over the n_out_host[s] final samples of slot s:
  *       spikes_in_dev [S][n + D][N_in] int8 {0,1} (Demo.spike_encoding's layout);  raster_dev [S][n + D][N] uint8;

@@ -326,6 +326,21 @@ def test_slots_are_independent_under_reset_and_flush():
     assert mb.push(frames[:, :1000])["n_out"].tolist() == [1000 - mb.latency, 0, 0, 0]   # the others were flushed
 
 
+def test_overflow_flag_stays_in_its_slot():
+    """Half a second of digital silence, then signal, overflows the RZCC clusters of slot 1 (as it did when the batch
+    was introduced).  The flush's host flags OR the bands' overflow bits: bit 0 for slot 1 only, as the fused flags of
+    the last push report it."""
+    g = H.load("full_multiband")
+    demo = make_demo(g)
+    lens = [4800] * 10
+    x = recordings(g, 3, sum(lens), seed=8)
+    x[1, 4000:28000] = 0.0
+    mb = demo.stream_batch(3, max_frame_len=4800)
+    calls = run(mb, to_frames(x, torch.int32), lens, want_spikes=False)
+    assert [int(v) & 1 for v in calls[-1]["flags"]] == [0, 1, 0]
+    assert [int(v) & 1 for v in calls[-2]["flags"].cpu()] == [0, 1, 0]
+
+
 def test_activity_gate():
     g = H.load("full_multiband")
     demo = make_demo(g)
