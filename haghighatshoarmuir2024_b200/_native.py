@@ -92,6 +92,8 @@ SYMBOLS = {
                                      C.c_float, _vp, C.c_int, _vp]),
     "micloc_rzcc_encode_f64": (C.c_int, [_vp, _i64, _i64, _i32, _i32, _i32, _vp, C.c_int, _vp]),
     "micloc_hilbert_beamform": (C.c_int, [_vp, _vp, C.c_int, _i64, _i64, _dp, _dp, _i32, _vp, _vp, _vp, _vp]),
+    "micloc_hilbert_set_bf": (C.c_int, [_vp, _dp, _dp, _i32]),
+    "micloc_hilbert_localize": (C.c_int, [_vp, _vp, C.c_int, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp, _vp]),
     "micloc_xylo_create": (C.c_int, [C.POINTER(XyloConfig), C.c_int, C.POINTER(_vp)]),
     "micloc_xylo_destroy": (C.c_int, [_vp]),
     "micloc_xylo_run": (C.c_int, [_vp, _vp, C.c_int, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp]),

@@ -2,6 +2,9 @@
 
 `apply_to_signal` (micloc/beamformer.py:260-292) runs STHT + band-pass + complex
 projection on the GPU (micloc_hilbert_beamform) and returns complex128 `T x G`.
+`localize` and `design_from_template` take batches through micloc_hilbert_localize, which
+gets power, DoA and the design covariance from one Gram matrix of the analytic signal per
+clip and never forms the dense `T x G` output.
 """
 from __future__ import annotations
 
@@ -76,21 +79,24 @@ class Beamformer:
             print("+" * 150)
             print(" designing beamforming matrices for various DoAs ".center(150, "+"))
             print("+" * 150)
-        cov_mat_list = []
         eng = self._engine()
         time_temp = np.asarray(time_temp, dtype=np.float64)
-        for doa in doa_list:
-            delays = self.geometry.delays(theta=doa, normalized=True)
-            td = time_temp.reshape(-1, 1) - delays.reshape(1, -1)
-            td[td < time_temp.min()] = time_temp.min()
-            sig_vec = np.interp(td.ravel(), time_temp, sig_temp).reshape(td.shape)
-            # STHT only: upstream band-passes a copy it never uses (beamformer.py:136-137)
-            x = torch.from_numpy(np.ascontiguousarray(sig_vec, dtype=np.float32)).to(eng.device)
-            q = eng.run_taps(x, want=("q",))["q"][0].cpu().numpy().astype(np.float64)
-            sig_h = np.roll(sig_vec, len(self.kernel) // 2, axis=0) + 1j * q
-            stable_part = min([len(self.kernel), sig_h.shape[0] // 2])
-            stable = sig_h[stable_part:, :]
-            cov_mat_list.append(1 / stable.shape[0] * (stable.conj().T @ stable))
+        T = len(time_temp)
+        # the analytic signal roll(x, K/2) + j STHT(x) without band-pass (upstream band-passes a copy it never uses,
+        # beamformer.py:136-137), covariance over its stable part: one batched device call per chunk of DoAs
+        t_start = min(len(self.kernel), T // 2)
+        chunk = max(1, min(len(doa_list), (256 << 20) // max(1, 4 * T * len(self.geometry))))
+        cov_mat_list = []
+        for d0 in range(0, len(doa_list), chunk):
+            sig = np.empty((min(chunk, len(doa_list) - d0), T, len(self.geometry)), dtype=np.float32)
+            for i, doa in enumerate(doa_list[d0:d0 + chunk]):
+                delays = self.geometry.delays(theta=doa, normalized=True)
+                td = time_temp.reshape(-1, 1) - delays.reshape(1, -1)
+                td[td < time_temp.min()] = time_temp.min()
+                sig[i] = np.interp(td.ravel(), time_temp, sig_temp).reshape(td.shape)
+            x = torch.from_numpy(sig).to(eng.device)
+            cov = eng.hilbert(x, t_start=t_start, bandpass=False, want=("cov",))["cov"].cpu().numpy()
+            cov_mat_list.extend(cov / (T - t_start))
         bf_mat = []
         if not interference_removal:
             for Cm in cov_mat_list:
@@ -106,6 +112,22 @@ class Beamformer:
                 v = vecs[:, -1]
                 bf_mat.append(v / np.linalg.norm(v))
         return np.asarray(bf_mat).T, cov_mat_list
+
+    def localize(self, bf_mat: np.ndarray, audio) -> dict:
+        """Batched hot path: audio [B,T,M] (CUDA tensor, float32/int16) -> dict(doa [B] int32, power [B,G] float32).
+
+        Equals argmax(mean(|apply_to_signal(bf_mat, x)|**2, axis=0)) per clip without the dense T x G array."""
+        bf_mat = np.asarray(bf_mat)
+        num_mic, num_grid = bf_mat.shape
+        num_chan = audio.shape[-1]
+        if num_chan != num_mic:
+            raise ValueError(
+                f"number of channels in the input siganl {num_chan} should be the same as the number of microphones {num_mic}!")
+        eng = self._engine()
+        if getattr(self, "_hbf", None) is None or self._hbf.shape != bf_mat.shape or not np.array_equal(self._hbf, bf_mat):
+            eng.set_hilbert_bf(bf_mat)
+            self._hbf = bf_mat.copy()
+        return eng.hilbert(audio, want=("doa", "power"))
 
     def apply_to_template(self, bf_mat: np.ndarray, template, snr_db: float) -> np.ndarray:
         """beamformer.py:194-258: delayed + noisy array signal, then apply_to_signal."""

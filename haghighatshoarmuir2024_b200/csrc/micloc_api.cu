@@ -69,6 +69,9 @@ struct micloc_snn {
     int last_kernels = 0;
     int sm_count = 148;
     double pole_radius = 1.0;      // largest pole modulus of the band-pass: how fast it forgets (time-segmented kernels)
+    double *d_hW = nullptr;        // [2M][hG] f64: complex steering matrix of micloc_hilbert_localize (Re rows | Im rows)
+    int hG = 0;
+    HilbertScratch hscratch;
 };
 
 // Time segments of the sequential stages (k_chain_blk / k_neuron_seg): the chain's, and neuron segments of
@@ -220,7 +223,8 @@ extern "C" int micloc_snn_create(const micloc_snn_config *cfg, int device, miclo
 extern "C" int micloc_snn_destroy(micloc_snn *c) {
     if (!c) return MICLOC_OK;
     cudaSetDevice(c->device);
-    cudaFree(c->d_taps); cudaFree(c->d_sos); cudaFree(c->d_W); cudaFree(c->d_Wd); cudaFree(c->d_sm_slots);
+    cudaFree(c->d_taps); cudaFree(c->d_sos); cudaFree(c->d_W); cudaFree(c->d_Wd); cudaFree(c->d_sm_slots); cudaFree(c->d_hW);
+    c->hscratch.q.release(); c->hscratch.z.release(); c->hscratch.part.release(); c->hscratch.gram.release();
     c->q.release(); c->spikes.release(); c->vmem.release(); c->gram.release(); c->flags.release(); c->part.release(); c->chunkbuf.release();
     c->rz.release(); c->rzd.release(); c->rspk.release(); c->rflag.release();
     if (c->h_flags_all) cudaFreeHost(c->h_flags_all);
@@ -791,6 +795,39 @@ extern "C" int micloc_hilbert_beamform(micloc_snn *c, const void *audio, int dty
     }
     MICLOC_CUDA(cudaGetLastError());
     return MICLOC_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Beamformer at batch scale: power / DoA / design covariance from the analytic signal's Gram matrix (micloc_hilbert.cu)
+// ---------------------------------------------------------------------------
+extern "C" int micloc_hilbert_set_bf(micloc_snn *c, const double *bf_re, const double *bf_im, int32_t G) {
+    if (!c || !bf_re || !bf_im || G < 1) return set_error(MICLOC_ERR_CONFIG, "bad beamforming matrix (G = %d)", (int)G);
+    MICLOC_CUDA(cudaSetDevice(c->device));
+    MICLOC_CUDA(cudaDeviceSynchronize());       // calls in flight may still read the old matrix
+    const size_t n = (size_t)c->p.M * G;
+    std::vector<double> w(2 * n);
+    std::memcpy(w.data(), bf_re, n * sizeof(double));
+    std::memcpy(w.data() + n, bf_im, n * sizeof(double));
+    if (c->d_hW) cudaFree(c->d_hW);
+    c->d_hW = nullptr; c->hG = 0;
+    MICLOC_CUDA(cudaMalloc(&c->d_hW, w.size() * sizeof(double)));
+    MICLOC_CUDA(cudaMemcpy(c->d_hW, w.data(), w.size() * sizeof(double), cudaMemcpyHostToDevice));
+    c->hG = G;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_hilbert_localize(micloc_snn *c, const void *audio, int dtype, int64_t B, int64_t T,
+                                       int64_t t_start, int bandpass, float *z_dev, double *cov_dev, float *power_dev,
+                                       int32_t *doa_dev, void *stream) {
+    MICLOC_TRY(check_run_args(c, audio, dtype, B, T));
+    if (t_start < 0 || t_start >= T)
+        return set_error(MICLOC_ERR_SHAPE, "t_start = %lld outside [0, T = %lld)", (long long)t_start, (long long)T);
+    if ((power_dev || doa_dev) && !c->d_hW)
+        return set_error(MICLOC_ERR_CONFIG, "power / doa need the steering matrix of micloc_hilbert_set_bf");
+    MICLOC_CUDA(cudaSetDevice(c->device));
+    const HilbertCtx hc{c->p, c->d_taps, c->d_sos, c->pole_radius, c->sm_count, c->d_hW, c->hG};
+    return hilbert_localize(hc, c->hscratch, audio, dtype, B, T, t_start, bandpass, z_dev, cov_dev, power_dev, doa_dev,
+                            (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------

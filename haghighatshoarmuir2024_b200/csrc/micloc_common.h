@@ -114,4 +114,18 @@ int launch_fused(const ChainParams &p, const float *d_taps, const double *d_Wd, 
 bool fused_supported(const ChainParams &p);
 }  // namespace tc
 
+// micloc_hilbert_localize (micloc_hilbert.cu): what it reads from the context, and the scratch it owns there
+struct HilbertCtx {
+    ChainParams p;
+    const float *d_taps, *d_sos;
+    double pole_radius;
+    int sm_count;
+    const double *d_W;      // [2M][G] float64: rows 0..M-1 = Re bf, M..2M-1 = Im bf (null before micloc_hilbert_set_bf)
+    int G;
+};
+struct HilbertScratch { DevBuf q, z, part, gram; };
+int hilbert_localize(const HilbertCtx &hc, HilbertScratch &s, const void *audio, int dtype, long long B, long long T,
+                     long long t_start, int bandpass, float *z_dev, double *cov_dev, float *power_dev, int32_t *doa_dev,
+                     cudaStream_t st);
+
 }  // namespace micloc

@@ -1,0 +1,390 @@
+// micloc_hilbert.cu -- the Hilbert beamformer at batch scale (micloc_hilbert_localize).
+//
+// s_t = zr_t + i zi_t, the band-passed analytic signal, in the real layout z = [zr | zi] ([T][2M]) that k_chain_blk
+// produces.  Everything the Beamformer needs from a clip is its real 2M x 2M Gram matrix G = sum_{t >= t_start} z_t z_t^T:
+//   power[g] = (u_g^T G u_g + v_g^T G v_g) / n_rows,  u = [wr; wi], v = [-wi; wr]   (y_t = sum_m s_tm conj(w_m))
+//   cov      = S^H S = (Grr + Gii) + i (Gri - Gir)                                  (design_from_template)
+// so the dense y [T][G] of micloc_hilbert_beamform is never formed.
+//
+// Kernels per chunk of clips (launch count independent of the chunk's size):
+//   2M <= 16:  k_stht / k_stht_tc -> k_hilbert_gram (roll + band-pass + float64 Gram, z stays on chip) -> k_hilbert_finish
+//   2M >  16:  k_stht / k_stht_tc -> k_hilbert_z (roll + band-pass -> z) -> k_gram_tiled -> k_hilbert_finish
+// k_gram_tc is not used: its fp16 scaling assumes |v| < 15 (membrane values); z of int16 audio is in the thousands.
+#include <cuda_runtime.h>
+
+#include <cmath>
+
+#include "micloc_common.h"
+#include "micloc_staged.cuh"
+
+namespace micloc {
+
+constexpr int kHbLanes = 16;                 // lanes per (clip, segment) unit of k_hilbert_gram: lane c < 2M is channel c
+constexpr int kHbThreads = 128;
+constexpr int kHbUnits = kHbThreads / kHbLanes;
+constexpr int kHbPitch = kHbLanes + 1;       // column 16 stays zero: Gram entries beyond 2M(2M+1)/2 read it
+constexpr int kHbEntries = (kHbLanes * (kHbLanes + 1) / 2 + kHbLanes - 1) / kHbLanes;   // upper-triangle entries per lane
+constexpr int kHbNsecRt = -1;                // NSEC template value: p.nsec sections at run time
+
+// One channel of one (clip, segment): the input of channel c (c < M: np.roll(x, K/2) of microphone c; c >= M: the
+// STHT output q of microphone c - M) through the band-pass sections, kSeg samples at a time, with k_chain_blk's
+// arithmetic (the same fmaf order: z equals run_taps' z tap bit for bit on the sequential plan).
+template <typename IN_T, int NSEC>
+struct HbChannel {
+    float sos[kMaxSections][5];
+    BiquadState bq;
+    const IN_T *xa;
+    const float *xq;
+    bool inphase;
+    int src0, T, M, t_begin;
+
+    __device__ void init(const IN_T *audio, const float *q, const float *band_sos, const ChainParams &p, long long b,
+                         int c, int T_, int t_begin_) {
+        T = T_; M = p.M; t_begin = t_begin_;
+        inphase = c < p.M;
+        xa = audio + b * (long long)T * M + (inphase ? c : 0);
+        xq = q + b * (long long)T * M + (inphase ? 0 : c - M);
+        src0 = (int)(((long long)t_begin - p.half) % T + T) % T;     // (t - K/2) mod T at t = t_begin (np.roll)
+#pragma unroll
+        for (int k = 0; k < kMaxSections; ++k)
+#pragma unroll
+            for (int e = 0; e < 5; ++e) sos[k][e] = band_sos[k * 5 + e];
+        biquad_reset(bq);
+    }
+    // x[i] = input at ts + i for i < t_stop - ts, 0 beyond
+    __device__ __forceinline__ void load(int ts, int t_stop, float (&x)[kSeg]) const {
+        const int left = t_stop - ts;
+        if (inphase) {
+            int s0 = src0 + (ts - t_begin);
+            if (s0 >= T) s0 -= T;
+            const int wrap = T - s0;
+            const IN_T *pp = xa + (long long)s0 * M;
+            if (left >= kSeg && wrap >= kSeg) {
+#pragma unroll
+                for (int i = 0; i < kSeg; ++i) { x[i] = to_f32<IN_T>(*pp); pp += M; }
+            } else {
+#pragma unroll
+                for (int i = 0; i < kSeg; ++i)
+                    x[i] = i < left ? to_f32<IN_T>(pp[(long long)(i < wrap ? i : i - T) * M]) : 0.f;
+            }
+        } else {
+            const float *pp = xq + (long long)ts * M;
+            if (left >= kSeg) {
+#pragma unroll
+                for (int i = 0; i < kSeg; ++i) { x[i] = *pp; pp += M; }
+            } else {
+#pragma unroll
+                for (int i = 0; i < kSeg; ++i) x[i] = i < left ? pp[(long long)i * M] : 0.f;
+            }
+        }
+    }
+    __device__ __forceinline__ float step(float v, int nsec) {
+        constexpr int NS = NSEC >= 0 ? NSEC : kMaxSections;
+#pragma unroll
+        for (int k = 0; k < NS; ++k) {
+            if (NSEC >= 0 || k < nsec) {
+                const float y = fmaf(sos[k][0], v, bq.s1[k]);
+                bq.s1[k] = fmaf(sos[k][1], v, fmaf(-sos[k][3], y, bq.s2[k]));
+                bq.s2[k] = fmaf(sos[k][2], v, -sos[k][4] * y);
+                v = y;
+            }
+        }
+        return v;
+    }
+};
+
+// Time segments (see hilbert_segments): segment s keeps [s seg_len, (s+1) seg_len) and runs the band-pass from `warm` samples
+// before it from zero state (warm = 0 without band-pass: z is then exact in every segment).
+struct HbSegs { int seg_len, warm, nseg; };
+
+// ---------------------------------------------------------------------------
+// 2M <= 16: one unit of 16 lanes per (clip, segment).  Each block of kSeg samples: lane c band-passes channel c into
+// registers and stages it in shared memory as float64; then every lane adds its <= 9 upper-triangle entries of the Gram
+// matrix over the block's rows t >= t_start (float64 FMAs in time order).  part[seg][b][i][j] (i <= j) as k_gram_tiled
+// writes it; z goes to HBM only as the optional debug tap.
+// ---------------------------------------------------------------------------
+template <typename IN_T, int NSEC>
+__global__ void __launch_bounds__(kHbThreads)
+k_hilbert_gram(const IN_T *__restrict__ audio, const float *__restrict__ q, const float *__restrict__ band_sos,
+               float *__restrict__ z_out, double *__restrict__ part, const __grid_constant__ ChainParams p, long long B,
+               long long T64, int t_start, int seg_len, int warm, int nseg) {
+    __shared__ double zs[kHbUnits][kSeg][kHbPitch];
+    const int unit_l = threadIdx.x / kHbLanes, lane = threadIdx.x % kHbLanes;
+    const long long unit = (long long)blockIdx.x * kHbUnits + unit_l;
+    const bool live = unit < B * nseg;
+    const long long b = live ? unit / nseg : 0;
+    const int seg = live ? (int)(unit % nseg) : 0;
+    const int C2 = p.C2, T = (int)T64;
+    const int c = lane < C2 ? lane : C2 - 1;             // idle lanes shadow the last channel and stage zeros
+    const unsigned hmask = 0xffffu << (threadIdx.x & 16);
+    double (*zu)[kHbPitch] = zs[unit_l];
+    for (int i = 0; i < kSeg; ++i) zu[i][kHbLanes] = 0.0;   // (each lane writes the same zero)
+
+    // this lane's Gram entries e = lane + 16 k of the upper triangle, row-major; beyond the triangle: column 16 (zero)
+    const int npair = C2 * (C2 + 1) / 2;
+    int ei[kHbEntries], ej[kHbEntries];
+    double acc[kHbEntries];
+#pragma unroll
+    for (int k = 0; k < kHbEntries; ++k) {
+        int e = lane + kHbLanes * k, i = 0;
+        if (e < npair) {
+            while (e >= C2 - i) { e -= C2 - i; ++i; }
+            ei[k] = i; ej[k] = i + e;
+        } else {
+            ei[k] = ej[k] = kHbLanes;
+        }
+        acc[k] = 0.0;
+    }
+
+    const int start = seg * seg_len, end = min(T, start + seg_len);
+    const int t_begin = max(0, start - warm);
+    const int t_stop = live ? end : t_begin;
+    const int t_lo = max(start, t_start);                // rows of the Gram sum
+    HbChannel<IN_T, NSEC> ch;
+    ch.init(audio, q, band_sos, p, b, c, T, t_begin);
+    const int nsec = p.nsec;
+    float x[kSeg];
+    ch.load(t_begin, t_stop, x);
+    for (int ts = t_begin; ts < t_stop; ts += kSeg) {
+        float v[kSeg];
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i) v[i] = ch.step(x[i], nsec);
+        if (ts + kSeg < t_stop) ch.load(ts + kSeg, t_stop, x);
+        if (ts + kSeg <= start) continue;                // warm-up only (uniform across the unit)
+        if (z_out && lane < C2) {
+            float *zo = z_out + ((long long)b * T + ts) * C2 + lane;
+#pragma unroll
+            for (int i = 0; i < kSeg; ++i)
+                if (ts + i >= start && ts + i < end) zo[(long long)i * C2] = v[i];
+        }
+        const int i0 = max(0, t_lo - ts), i1 = min(kSeg, end - ts);
+        if (i0 >= i1) continue;
+        __syncwarp(hmask);                               // the previous block's reads are done
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i) zu[i][lane] = lane < C2 ? (double)v[i] : 0.0;
+        __syncwarp(hmask);
+        for (int i = i0; i < i1; ++i) {
+#pragma unroll
+            for (int k = 0; k < kHbEntries; ++k) acc[k] = fma(zu[i][ei[k]], zu[i][ej[k]], acc[k]);
+        }
+    }
+    if (!live) return;
+    double *out = part + ((long long)seg * B + b) * C2 * C2;
+#pragma unroll
+    for (int k = 0; k < kHbEntries; ++k)
+        if (ei[k] < kHbLanes) out[ei[k] * C2 + ej[k]] = acc[k];
+}
+
+// ---------------------------------------------------------------------------
+// 2M > 16: z of every (clip, segment, channel) to HBM; k_gram_tiled then sums it.
+// ---------------------------------------------------------------------------
+template <typename IN_T, int NSEC>
+__global__ void __launch_bounds__(kChainBlkThreads)
+k_hilbert_z(const IN_T *__restrict__ audio, const float *__restrict__ q, const float *__restrict__ band_sos,
+            float *__restrict__ z_out, const __grid_constant__ ChainParams p, long long B, long long T64, int seg_len,
+            int warm, int nseg) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int C2 = p.C2, T = (int)T64;
+    if (idx >= B * nseg * C2) return;
+    const int c = (int)(idx % C2);
+    const int seg = (int)((idx / C2) % nseg);
+    const long long b = idx / ((long long)C2 * nseg);
+    const int start = seg * seg_len, end = min(T, start + seg_len);
+    const int t_begin = max(0, start - warm);
+    HbChannel<IN_T, NSEC> ch;
+    ch.init(audio, q, band_sos, p, b, c, T, t_begin);
+    const int nsec = p.nsec;
+    float x[kSeg];
+    ch.load(t_begin, end, x);
+    for (int ts = t_begin; ts < end; ts += kSeg) {
+        float v[kSeg];
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i) v[i] = ch.step(x[i], nsec);
+        if (ts + kSeg < end) ch.load(ts + kSeg, end, x);
+        float *zo = z_out + ((long long)b * T + ts) * C2 + c;
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i)
+            if (ts + i >= start && ts + i < end) zo[(long long)i * C2] = v[i];
+    }
+}
+
+// ---------------------------------------------------------------------------
+// One CTA per clip: G = sum of the nslab partial sums part[slab][b] (upper triangle, slab order: deterministic), then
+//   cov[i][j] = (G[i][j] + G[M+i][M+j], G[i][M+j] - G[M+i][j])
+//   power[g]  = (u^T G u + v^T G v) * inv_n,  u = W[:, g] = [wr; wi], v = [-wi; wr]   (float64, stored as float32)
+//   doa       = first argmax.
+// kSmem: G in shared memory (2M <= 128); otherwise in the global scratch `gram` [B][2M][2M].
+// ---------------------------------------------------------------------------
+template <bool kSmem>
+__global__ void __launch_bounds__(256)
+k_hilbert_finish(const double *__restrict__ part, int nslab, double *__restrict__ gram, const double *__restrict__ W,
+                 int M, int G, long long B, double inv_n, double *__restrict__ cov, float *__restrict__ power,
+                 int32_t *__restrict__ doa) {
+    extern __shared__ __align__(16) double hf_sm[];
+    __shared__ double red_v[256];
+    __shared__ int red_i[256];
+    const long long b = blockIdx.x;
+    const int C2 = 2 * M;
+    double *Gs = kSmem ? hf_sm : gram + b * C2 * C2;
+    for (int e = threadIdx.x; e < C2 * C2; e += blockDim.x) {
+        const int i = e / C2, j = e % C2;
+        const int lo = i < j ? i : j, hi = i < j ? j : i;
+        double s = 0.0;
+        for (int k = 0; k < nslab; ++k) s += part[((long long)k * B + b) * C2 * C2 + lo * C2 + hi];
+        Gs[e] = s;
+    }
+    __syncthreads();
+    if (cov)
+        for (int e = threadIdx.x; e < M * M; e += blockDim.x) {
+            const int i = e / M, j = e % M;
+            cov[(b * M * M + e) * 2] = Gs[i * C2 + j] + Gs[(M + i) * C2 + M + j];
+            cov[(b * M * M + e) * 2 + 1] = Gs[i * C2 + M + j] - Gs[(M + i) * C2 + j];
+        }
+    if (!power && !doa) return;
+    double best = -1.0; int besti = 0x7fffffff;
+    for (int g = threadIdx.x; g < G; g += blockDim.x) {
+        double acc = 0.0;
+        for (int i = 0; i < C2; ++i) {
+            double ru = 0.0, rv = 0.0;
+            for (int j = 0; j < C2; ++j) {
+                const double gij = Gs[i * C2 + j];
+                const double uj = W[(long long)j * G + g];
+                const double vj = j < M ? -W[(long long)(M + j) * G + g] : W[(long long)(j - M) * G + g];
+                ru = fma(gij, uj, ru);
+                rv = fma(gij, vj, rv);
+            }
+            const double ui = W[(long long)i * G + g];
+            const double vi = i < M ? -W[(long long)(M + i) * G + g] : W[(long long)(i - M) * G + g];
+            acc = fma(ui, ru, fma(vi, rv, acc));
+        }
+        acc *= inv_n;
+        if (power) power[b * G + g] = (float)acc;
+        if (acc > best) { best = acc; besti = g; }      // ascending g: first maximum kept
+    }
+    red_v[threadIdx.x] = best; red_i[threadIdx.x] = besti;
+    __syncthreads();
+    for (int s = blockDim.x / 2; s > 0; s >>= 1) {
+        if (threadIdx.x < s) {
+            const double ov = red_v[threadIdx.x + s]; const int oi = red_i[threadIdx.x + s];
+            if (ov > red_v[threadIdx.x] || (ov == red_v[threadIdx.x] && oi < red_i[threadIdx.x])) {
+                red_v[threadIdx.x] = ov; red_i[threadIdx.x] = oi;
+            }
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0 && doa) doa[b] = red_i[0];
+}
+
+// Time segments when the B clips of a chunk are too few chains to fill the GPU: about 3 x 128 chains per SM; a segment
+// is never shorter than its band-pass warm-up (transient below 1e-9 of full scale), and never more than half the clip.
+static HbSegs hilbert_segments(long long B, long long T, int lanes, bool bandpass, double pole_radius, int sm_count) {
+    const HbSegs seq{(int)((T + kSeg - 1) & ~(long long)(kSeg - 1)), 0, 1};
+    const long long chains = B * lanes;
+    if (chains >= 3ll * kChainBlkThreads * sm_count || T < 32768) return seq;
+    int warm = 0;
+    if (bandpass) {
+        if (!(pole_radius > 0.0 && pole_radius < 0.9995)) return seq;
+        warm = (int)std::ceil(std::log(1e-9) / std::log(pole_radius));
+        warm = (warm + kSeg - 1) & ~(kSeg - 1);
+    }
+    long long want = (3ll * kChainBlkThreads * sm_count) / chains;
+    if (want < 1) want = 1;
+    long long seg = (T + want - 1) / want;
+    if (seg < warm) seg = warm;
+    seg = (seg + kSeg - 1) & ~(long long)(kSeg - 1);
+    if (seg * 2 > T) return seq;
+    return {(int)seg, warm, (int)((T + seg - 1) / seg)};
+}
+
+template <typename IN_T, int NSEC>
+static void launch_front(bool narrow, const IN_T *audio, const float *q, const float *sos, float *z, double *part,
+                         const ChainParams &p, long long B, long long T, long long t_start, const HbSegs &sg,
+                         cudaStream_t st) {
+    if (narrow) {
+        const long long units = B * sg.nseg;
+        k_hilbert_gram<IN_T, NSEC><<<(unsigned)((units + kHbUnits - 1) / kHbUnits), kHbThreads, 0, st>>>(
+            audio, q, sos, z, part, p, B, T, (int)t_start, sg.seg_len, sg.warm, sg.nseg);
+    } else {
+        const long long n = B * sg.nseg * p.C2;
+        k_hilbert_z<IN_T, NSEC><<<(unsigned)((n + kChainBlkThreads - 1) / kChainBlkThreads), kChainBlkThreads, 0, st>>>(
+            audio, q, sos, z, p, B, T, sg.seg_len, sg.warm, sg.nseg);
+    }
+}
+
+template <typename IN_T>
+static void launch_front_t(bool narrow, int nsec, const IN_T *audio, const float *q, const float *sos, float *z,
+                           double *part, const ChainParams &p, long long B, long long T, long long t_start,
+                           const HbSegs &sg, cudaStream_t st) {
+    if (nsec == 0) launch_front<IN_T, 0>(narrow, audio, q, sos, z, part, p, B, T, t_start, sg, st);
+    else if (nsec == 2) launch_front<IN_T, 2>(narrow, audio, q, sos, z, part, p, B, T, t_start, sg, st);
+    else launch_front<IN_T, kHbNsecRt>(narrow, audio, q, sos, z, part, p, B, T, t_start, sg, st);
+}
+
+int hilbert_localize(const HilbertCtx &hc, HilbertScratch &s, const void *audio, int dtype, long long B, long long T,
+                     long long t_start, int bandpass, float *z_dev, double *cov_dev, float *power_dev, int32_t *doa_dev,
+                     cudaStream_t st) {
+    const ChainParams &p = hc.p;
+    const int C2 = p.C2;
+    const bool narrow = C2 <= kHbLanes;
+    const bool bp = bandpass != 0;
+    ChainParams pz = p;
+    if (!bp) pz.nsec = 0;
+    const long long nslab_w = (T - t_start + kGtFlush - 1) / kGtFlush;     // k_gram_tiled's slabs (wide arrays)
+    if (!narrow && nslab_w > 65535) return set_error(MICLOC_ERR_UNSUPPORTED, "clip too long for the tiled Gram kernel");
+    // chunks of clips: STHT output, z (wide arrays, unless the caller keeps it) and the slab sums within ~1 GB
+    const size_t esz = dtype == MICLOC_I16 ? 2 : 4;
+    const size_t q_clip = (size_t)T * p.M * sizeof(float);
+    const size_t z_clip = (!narrow && !z_dev) ? (size_t)T * C2 * sizeof(float) : 0;
+    const size_t slab_clip = narrow ? 0 : (size_t)nslab_w * C2 * C2 * sizeof(double);
+    long long chunk = (long long)(((size_t)1 << 30) / (q_clip + z_clip + slab_clip));
+    if (chunk < 1) chunk = 1;
+    if (chunk > 65535) chunk = 65535;
+    if (chunk > B) chunk = B;
+    // the chains of one chunk are what has to fill the GPU: time segments are planned for the chunk
+    const HbSegs sg = hilbert_segments(chunk, T, narrow ? kHbLanes : C2, bp, hc.pole_radius, hc.sm_count);
+    const long long nslab = narrow ? sg.nseg : nslab_w;
+    const size_t part_clip = (size_t)nslab * C2 * C2 * sizeof(double);
+    MICLOC_TRY(s.q.reserve((size_t)chunk * q_clip));
+    if (z_clip) MICLOC_TRY(s.z.reserve((size_t)chunk * z_clip));
+    MICLOC_TRY(s.part.reserve((size_t)chunk * part_clip));
+    const bool smem = (size_t)C2 * C2 * sizeof(double) <= 128 * 1024;
+    if (!smem) MICLOC_TRY(s.gram.reserve((size_t)chunk * C2 * C2 * sizeof(double)));
+    const size_t smem_b = smem ? (size_t)C2 * C2 * sizeof(double) : 0;
+    if (smem) MICLOC_CUDA(cudaFuncSetAttribute(k_hilbert_finish<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               (int)smem_b));
+    const double inv_n = 1.0 / (double)(T - t_start);
+    for (long long b0 = 0; b0 < B; b0 += chunk) {
+        const long long nb = B - b0 < chunk ? B - b0 : chunk;
+        const void *a = (const char *)audio + (size_t)b0 * T * p.M * esz;
+        float *q = (float *)s.q.ptr;
+        float *z = z_dev ? z_dev + (size_t)b0 * T * C2 : (narrow ? nullptr : (float *)s.z.ptr);
+        double *part = (double *)s.part.ptr;
+        MICLOC_TRY(launch_stht_any(p, hc.d_taps, a, dtype, q, nb, T, st));
+        if (dtype == MICLOC_I16)
+            launch_front_t<int16_t>(narrow, pz.nsec, (const int16_t *)a, q, hc.d_sos, z, part, pz, nb, T, t_start, sg, st);
+        else
+            launch_front_t<float>(narrow, pz.nsec, (const float *)a, q, hc.d_sos, z, part, pz, nb, T, t_start, sg, st);
+        count_launch(1);
+        if (!narrow) {
+            const int nblk = (C2 + kGtTile - 1) / kGtTile, nblocks = nblk * (nblk + 1) / 2;
+            k_gram_tiled<<<dim3((unsigned)nb, (unsigned)nblocks, (unsigned)nslab), 256, 0, st>>>(
+                z, part, C2, nb, T, t_start, kGtFlush);
+            count_launch(1);
+        }
+        const size_t o = (size_t)b0;
+        double *cov = cov_dev ? cov_dev + o * p.M * p.M * 2 : nullptr;
+        float *pw = power_dev ? power_dev + o * hc.G : nullptr;
+        int32_t *dd = doa_dev ? doa_dev + o : nullptr;
+        if (smem)
+            k_hilbert_finish<true><<<(unsigned)nb, 256, smem_b, st>>>(part, (int)nslab, nullptr, hc.d_W, p.M, hc.G, nb,
+                                                                      inv_n, cov, pw, dd);
+        else
+            k_hilbert_finish<false><<<(unsigned)nb, 256, 0, st>>>(part, (int)nslab, (double *)s.gram.ptr, hc.d_W, p.M,
+                                                                  hc.G, nb, inv_n, cov, pw, dd);
+        count_launch(1);
+        MICLOC_CUDA(cudaGetLastError());
+    }
+    return MICLOC_OK;
+}
+
+}  // namespace micloc

@@ -238,6 +238,37 @@ class SnnEngine:
         N.check(self._lib.micloc_snn_gram(self._h, _ptr(audio), dt, B, T, int(t_start), _ptr(g), _stream_ptr(self.device)))
         return g
 
+    def set_hilbert_bf(self, bf_complex: np.ndarray):
+        """Steering matrix [M, G] complex of the Hilbert beamformer (`hilbert`); the SNN bf_mat is left as it is."""
+        bf = np.asarray(bf_complex)
+        if bf.ndim != 2 or bf.shape[0] != self.M:
+            raise ValueError(f"bf_mat should have shape (num_mic, num_DoA); got {bf.shape}")
+        re = np.ascontiguousarray(bf.real, dtype=np.float64)
+        im = np.ascontiguousarray(bf.imag, dtype=np.float64) if np.iscomplexobj(bf) else np.zeros_like(re)
+        N.check(self._lib.micloc_hilbert_set_bf(self._h, re.ctypes.data_as(N._dp), im.ctypes.data_as(N._dp),
+                                                bf.shape[1]))
+        self.hilbert_G = bf.shape[1]
+
+    def hilbert(self, audio: torch.Tensor, t_start: int = 0, bandpass: bool = True,
+                want: Sequence[str] = ("doa", "power")) -> Dict[str, torch.Tensor]:
+        """Hilbert beamformer on audio [B,T,M] (micloc_hilbert_localize): the analytic signal s_t (band-passed, or
+        roll + STHT without `bandpass`) over rows t >= t_start gives any of 'doa' [B] int32, 'power' [B,G] float32
+        (mean |s_t . conj(bf_g)|^2), 'cov' [B,M,M] complex128 (sum conj(s_t) s_t^T) and 'z' [B,T,2M] float32 (real |
+        imag of s_t), as device tensors; stream-ordered."""
+        audio, dt = self._check_audio(audio)
+        B, T, _ = audio.shape
+        dev = self.device
+        G = getattr(self, "hilbert_G", 0)
+        mk = lambda name, shape, dtype: torch.empty(shape, dtype=dtype, device=dev) if name in want else None
+        out = {"doa": mk("doa", (B,), torch.int32), "power": mk("power", (B, G), torch.float32),
+               "cov": mk("cov", (B, self.M, self.M, 2), torch.float64), "z": mk("z", (B, T, self.C2), torch.float32)}
+        N.check(self._lib.micloc_hilbert_localize(self._h, _ptr(audio), dt, B, T, int(t_start), int(bool(bandpass)),
+                                                  _ptr(out["z"]), _ptr(out["cov"]), _ptr(out["power"]),
+                                                  _ptr(out["doa"]), _stream_ptr(dev)))
+        if out["cov"] is not None:
+            out["cov"] = torch.view_as_complex(out["cov"])
+        return {k: v for k, v in out.items() if v is not None}
+
     def run_host(self, audio, want_spikes: bool = False, want_power: bool = True, fused: bool = True):
         """End-to-end with HOST buffers (numpy or CPU torch tensors, ideally pinned):
         H2D copy, hot path, D2H copy all inside the C call."""

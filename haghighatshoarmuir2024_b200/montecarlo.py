@@ -30,6 +30,7 @@ class BandSetup:
     band: Sequence[float]
     tau: float
     bf_mat: np.ndarray            # [2M, G]
+    bf_hilbert: Optional[np.ndarray] = None   # [M, G] complex: steering of the Hilbert beamformer arm (run_band_hilbert)
 
 
 def stht_kernel(fs: float, kernel_duration: float) -> np.ndarray:
@@ -115,6 +116,9 @@ class SnrSweep:
         self.bands = bands
         self.specs = [band_chain_spec(self.M, fs, self.kernel, b.band, b.tau, T, bipolar) for b in bands]
         self.engines = [SnnEngine(s, b.bf_mat, device=device) for s, b in zip(self.specs, bands)]
+        for eng, b in zip(self.engines, bands):
+            if b.bf_hilbert is not None:
+                eng.set_hilbert_bf(b.bf_hilbert)
         self.G = bands[0].bf_mat.shape[1]
 
     # ------------------------------------------------------------------
@@ -141,6 +145,17 @@ class SnrSweep:
         RZCC overflow flags); the caller then runs `self.engines[band_idx].refine(audio, out)` once per step."""
         eng = self.engines[band_idx]
         out = eng.run(audio, want_spikes=want_spikes, want_power=want_power, fused=True, refine=refine)
+        if hist is not None:
+            self.histogram(out["doa"], hist)
+        return out
+
+    def run_band_hilbert(self, band_idx: int, audio: torch.Tensor, hist: Optional[torch.Tensor] = None
+                         ) -> Dict[str, torch.Tensor]:
+        """The same batch through the Hilbert beamformer on the band's engine (its STHT and band-pass; steering
+        `bf_hilbert` of the band): dict(doa, power); stream-ordered."""
+        if self.bands[band_idx].bf_hilbert is None:
+            raise ValueError(f"band {band_idx} has no bf_hilbert")
+        out = self.engines[band_idx].hilbert(audio, want=("doa", "power"))
         if hist is not None:
             self.histogram(out["doa"], hist)
         return out

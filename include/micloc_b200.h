@@ -307,6 +307,25 @@ int micloc_hilbert_beamform(micloc_snn *ctx, const void *audio_dev, int dtype, i
                             const double *bf_re_host, const double *bf_im_host, int32_t G,
                             float *y_dev, float *power_dev, int32_t *doa_dev, void *stream);
 
+/* Beamformer at batch scale.  The complex steering matrix of Beamformer.apply_to_signal, bf = bf_re + i bf_im,
+ * [M][G] host float64, kept by the context beside (not instead of) the SNN bf_mat: its own G, its own buffers;
+ * micloc_snn_set_bf is unaffected.  Waits for the device (calls in flight may read the old matrix). */
+int micloc_hilbert_set_bf(micloc_snn *ctx, const double *bf_re_host, const double *bf_im_host, int32_t G);
+/* s_t = analytic signal of clip b: band-passed (bandpass != 0, beamformer.py:281-287) or roll(x, K/2) + j STHT(x)
+ * (bandpass == 0, the form design_from_template uses).  All outputs nullable, device:
+ *   z_dev     [B][T][2M] f32   s_t as (real | imag), debug tap;
+ *   cov_dev   [B][M][M][2] f64 sum_{t >= t_start} conj(s_t[i]) s_t[j]  (re, im);
+ *   power_dev [B][G] f32       mean_{t >= t_start} |sum_m s_t[m] conj(bf[m][g])|^2, as (u^T G u + v^T G v) / (T - t_start)
+ *                              of the real Gram matrix G of (real | imag), u = [Re bf; Im bf], v = [-Im bf; Re bf];
+ *   doa_dev   [B] int32        first argmax of power.
+ * Never forms the dense T x G output.  Stream-ordered (no synchronisation), any B (chunks of <= 65535 clips whose
+ * scratch stays within ~1 GB), f32 / i16 audio, 0 <= t_start < T.  Kernels per chunk: 3 for M <= 8 (STHT, band-pass +
+ * float64 Gram on chip, Gram reduce + cov + power + argmax), 4 for M > 8 (STHT, band-pass -> z, tiled float32 Gram over
+ * 1024-sample slabs, the same last kernel).  power / doa before micloc_hilbert_set_bf -> MICLOC_ERR_CONFIG. */
+int micloc_hilbert_localize(micloc_snn *ctx, const void *audio_dev, int dtype, int64_t B, int64_t T, int64_t t_start,
+                            int bandpass, float *z_dev, double *cov_dev, float *power_dev, int32_t *doa_dev,
+                            void *stream);
+
 /* ---- Xylo integer chain ---------------------------------------------------- */
 /* Network constants are what rockpool's mapper + global_quantize + config_from_specification
  * hand to XyloSim (micloc/xylo_snn_localization.py:268-290); the host package restates that
