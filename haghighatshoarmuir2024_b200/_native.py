@@ -54,6 +54,13 @@ class SynthConfig(C.Structure):
     ]
 
 
+class DesignTemplate(C.Structure):
+    _fields_ = [
+        ("num_mic", _i32), ("r_vec", _dp), ("theta_vec", _dp), ("speed", C.c_double),
+        ("T", _i64), ("time_dev", _vp), ("sig_dev", _vp),
+    ]
+
+
 # every symbol include/micloc_b200.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "micloc_snn_create": (C.c_int, [C.POINTER(SnnConfig), C.c_int, C.POINTER(_vp)]),
@@ -94,6 +101,10 @@ SYMBOLS = {
     "micloc_hilbert_beamform": (C.c_int, [_vp, _vp, C.c_int, _i64, _i64, _dp, _dp, _i32, _vp, _vp, _vp, _vp]),
     "micloc_hilbert_set_bf": (C.c_int, [_vp, _dp, _dp, _i32]),
     "micloc_hilbert_localize": (C.c_int, [_vp, _vp, C.c_int, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp, _vp]),
+    "micloc_design_templates": (C.c_int, [C.POINTER(DesignTemplate), _vp, _i64, _vp, C.c_int, _vp]),
+    "micloc_snn_design": (C.c_int, [_vp, C.POINTER(DesignTemplate), _vp, _i64, _vp, _vp, _vp]),
+    "micloc_hilbert_design": (C.c_int, [_vp, C.POINTER(DesignTemplate), _vp, _i64, C.c_int, _vp, _vp, _vp]),
+    "micloc_design_vectors": (C.c_int, [C.c_int, _vp, _i32, _i64, _vp, _vp, C.c_int, _vp]),
     "micloc_xylo_create": (C.c_int, [C.POINTER(XyloConfig), C.c_int, C.POINTER(_vp)]),
     "micloc_xylo_destroy": (C.c_int, [_vp]),
     "micloc_xylo_run": (C.c_int, [_vp, _vp, C.c_int, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp]),

@@ -113,6 +113,20 @@ class Beamformer:
                 bf_mat.append(v / np.linalg.norm(v))
         return np.asarray(bf_mat).T, cov_mat_list
 
+    def design_on_device(self, template: Tuple[np.ndarray, np.ndarray], doa_list: np.ndarray,
+                         interference_removal: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(bf complex128 `[M, G]`, cov complex128 `[G, M, M]`) designed on the GPU from the template to the steering
+        vectors (micloc_hilbert_design), both device tensors.  cov equals design_from_template's list; every column
+        equals the host's up to a phase (the device makes its entry of largest modulus real and positive)."""
+        try:
+            time_temp, sig_temp = template
+        except Exception:
+            raise ValueError("input template should be a tuple containing (time_in, sig_in) of the template signal!")
+        time_interp = np.arange(np.min(time_temp), np.max(time_temp), step=1 / self.fs)
+        sig_interp = np.interp(time_interp, time_temp, sig_temp)
+        return self._engine().hilbert_design(self.geometry, time_interp, sig_interp, doa_list,
+                                             interference_removal=interference_removal)
+
     def localize(self, bf_mat: np.ndarray, audio) -> dict:
         """Batched hot path: audio [B,T,M] (CUDA tensor, float32/int16) -> dict(doa [B] int32, power [B,G] float32).
 

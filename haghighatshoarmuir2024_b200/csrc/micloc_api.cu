@@ -72,6 +72,7 @@ struct micloc_snn {
     double *d_hW = nullptr;        // [2M][hG] f64: complex steering matrix of micloc_hilbert_localize (Re rows | Im rows)
     int hG = 0;
     HilbertScratch hscratch;
+    DevBuf design_clips, design_cov;        // micloc_snn_design / micloc_hilbert_design: template clips, covariances
 };
 
 // Time segments of the sequential stages (k_chain_blk / k_neuron_seg): the chain's, and neuron segments of
@@ -225,6 +226,7 @@ extern "C" int micloc_snn_destroy(micloc_snn *c) {
     cudaSetDevice(c->device);
     cudaFree(c->d_taps); cudaFree(c->d_sos); cudaFree(c->d_W); cudaFree(c->d_Wd); cudaFree(c->d_sm_slots); cudaFree(c->d_hW);
     c->hscratch.q.release(); c->hscratch.z.release(); c->hscratch.part.release(); c->hscratch.gram.release();
+    c->design_clips.release(); c->design_cov.release();
     c->q.release(); c->spikes.release(); c->vmem.release(); c->gram.release(); c->flags.release(); c->part.release(); c->chunkbuf.release();
     c->rz.release(); c->rzd.release(); c->rspk.release(); c->rflag.release();
     if (c->h_flags_all) cudaFreeHost(c->h_flags_all);
@@ -828,6 +830,120 @@ extern "C" int micloc_hilbert_localize(micloc_snn *c, const void *audio, int dty
     const HilbertCtx hc{c->p, c->d_taps, c->d_sos, c->pole_radius, c->sm_count, c->d_hW, c->hG};
     return hilbert_localize(hc, c->hscratch, audio, dtype, B, T, t_start, bandpass, z_dev, cov_dev, power_dev, doa_dev,
                             (cudaStream_t)stream);
+}
+
+// ---------------------------------------------------------------------------
+// design_from_template on the device (micloc_design.cu): templates -> covariances -> batched eigen-solver
+// ---------------------------------------------------------------------------
+static int design_geom(const micloc_design_template *tp, const double *doa_dev, int64_t G, DesignGeom *geo) {
+    if (!tp) return set_error(MICLOC_ERR_SHAPE, "null template");
+    if (tp->num_mic > kDesignMaxMic)
+        return set_error(MICLOC_ERR_UNSUPPORTED, "design supports num_mic <= %d, got %d", kDesignMaxMic, (int)tp->num_mic);
+    if (tp->num_mic < 1 || !tp->r_vec || !tp->theta_vec || !tp->time_dev || !tp->sig_dev || !doa_dev)
+        return set_error(MICLOC_ERR_SHAPE, "bad template (num_mic %d) or null pointer", (int)tp->num_mic);
+    if (tp->T < 2 || tp->T > (1ll << 30) || G < 1)
+        return set_error(MICLOC_ERR_SHAPE, "bad design shape (T = %lld, G = %lld)", (long long)tp->T, (long long)G);
+    geo->M = tp->num_mic;
+    geo->speed = tp->speed;
+    for (int m = 0; m < tp->num_mic; ++m) { geo->r[m] = tp->r_vec[m]; geo->theta[m] = tp->theta_vec[m]; }
+    return MICLOC_OK;
+}
+
+static int design_ctx_check(micloc_snn *c, const micloc_design_template *tp, const double *doa_dev, int64_t G,
+                            const double *bf_dev, DesignGeom *geo) {
+    if (!c) return set_error(MICLOC_ERR_CONFIG, "null context");
+    MICLOC_TRY(design_geom(tp, doa_dev, G, geo));
+    if (!bf_dev) return set_error(MICLOC_ERR_SHAPE, "null bf output");
+    if (tp->num_mic != c->p.M)
+        return set_error(MICLOC_ERR_SHAPE, "template has %d microphones, the context %d", (int)tp->num_mic, c->p.M);
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_design_templates(const micloc_design_template *tp, const double *doa_dev, int64_t G,
+                                       float *clips_dev, int device, void *stream) {
+    DesignGeom geo;
+    MICLOC_TRY(design_geom(tp, doa_dev, G, &geo));
+    if (!clips_dev) return set_error(MICLOC_ERR_SHAPE, "null clips output");
+    MICLOC_CUDA(cudaSetDevice(device));
+    return launch_design_templates(geo, tp->time_dev, tp->sig_dev, tp->T, doa_dev, G, clips_dev, (cudaStream_t)stream);
+}
+
+extern "C" int micloc_snn_design(micloc_snn *c, const micloc_design_template *tp, const double *doa_dev, int64_t G,
+                                 double *bf_dev, double *cov_dev, void *stream) {
+    DesignGeom geo;
+    MICLOC_TRY(design_ctx_check(c, tp, doa_dev, G, bf_dev, &geo));
+    MICLOC_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const ChainParams &p = c->p;
+    const long long T = tp->T, t_start = T / 4;
+    // clips + STHT output + spikes + membrane of one DoA; chunks within ~1 GB
+    const size_t per = (size_t)T * p.M * (2 * sizeof(float)) + (size_t)T * p.C2 * (1 + sizeof(float));
+    long long chunk = (long long)(((size_t)1 << 30) / per);
+    if (chunk < 1) chunk = 1;
+    if (chunk > 65535) chunk = 65535;
+    if (chunk > G) chunk = G;
+    MICLOC_TRY(c->design_clips.reserve((size_t)chunk * T * p.M * sizeof(float)));
+    MICLOC_TRY(c->q.reserve((size_t)chunk * T * p.M * sizeof(float)));
+    MICLOC_TRY(c->spikes.reserve((size_t)chunk * T * p.C2));
+    MICLOC_TRY(c->vmem.reserve((size_t)chunk * T * p.C2 * sizeof(float)));
+    MICLOC_TRY(c->flags.reserve((size_t)chunk * sizeof(int32_t)));
+    const size_t ncov = (size_t)G * p.C2 * p.C2;
+    double *cov = cov_dev;
+    if (!cov) { MICLOC_TRY(c->design_cov.reserve(ncov * sizeof(double))); cov = (double *)c->design_cov.ptr; }
+    float *clips = (float *)c->design_clips.ptr;
+    for (long long g0 = 0; g0 < G; g0 += chunk) {
+        const long long nb = G - g0 < chunk ? G - g0 : chunk;
+        MICLOC_TRY(launch_design_templates(geo, tp->time_dev, tp->sig_dev, T, doa_dev + g0, nb, clips, st));
+        MICLOC_TRY(run_front(c, sequential_plan(T), clips, MICLOC_F32, nb, T, (float *)c->q.ptr, nullptr,
+                             (int8_t *)c->spikes.ptr, (int32_t *)c->flags.ptr, (float *)c->vmem.ptr, st));
+        k_gram<<<dim3((unsigned)nb, (unsigned)((p.C2 * p.C2 + 255) / 256)), 256, 0, st>>>(
+            (const float *)c->vmem.ptr, cov + (size_t)g0 * p.C2 * p.C2, p.C2, T, t_start);
+        count_launch(1);
+        MICLOC_CUDA(cudaGetLastError());
+    }
+    MICLOC_TRY(launch_design_scale(cov, (long long)ncov, (double)(T - t_start), false, st));
+    MICLOC_TRY(design_vectors(p.bipolar ? 1 : 0, cov, p.M, G, bf_dev, nullptr, st));
+    MICLOC_CUDA(cudaEventRecord(c->ev_last, st));
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_hilbert_design(micloc_snn *c, const micloc_design_template *tp, const double *doa_dev, int64_t G,
+                                     int interference_removal, double *bf_dev, double *cov_dev, void *stream) {
+    DesignGeom geo;
+    MICLOC_TRY(design_ctx_check(c, tp, doa_dev, G, bf_dev, &geo));
+    MICLOC_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const ChainParams &p = c->p;
+    const long long T = tp->T, t_start = p.K < T / 2 ? p.K : T / 2;
+    // the clips of a chunk within ~0.5 GB; micloc_hilbert_localize bounds its own scratch to ~1 GB
+    long long chunk = (long long)(((size_t)512 << 20) / ((size_t)T * p.M * sizeof(float)));
+    if (chunk < 1) chunk = 1;
+    if (chunk > G) chunk = G;
+    MICLOC_TRY(c->design_clips.reserve((size_t)chunk * T * p.M * sizeof(float)));
+    const size_t ncov = (size_t)G * p.M * p.M * 2;
+    double *cov = cov_dev;
+    if (!cov) { MICLOC_TRY(c->design_cov.reserve(ncov * sizeof(double))); cov = (double *)c->design_cov.ptr; }
+    float *clips = (float *)c->design_clips.ptr;
+    const HilbertCtx hc{c->p, c->d_taps, c->d_sos, c->pole_radius, c->sm_count, c->d_hW, c->hG};
+    for (long long g0 = 0; g0 < G; g0 += chunk) {
+        const long long nb = G - g0 < chunk ? G - g0 : chunk;
+        MICLOC_TRY(launch_design_templates(geo, tp->time_dev, tp->sig_dev, T, doa_dev + g0, nb, clips, st));
+        MICLOC_TRY(hilbert_localize(hc, c->hscratch, clips, MICLOC_F32, nb, T, t_start, 0, nullptr,
+                                    cov + (size_t)g0 * p.M * p.M * 2, nullptr, nullptr, st));
+    }
+    // numpy's complex / int multiplies by the reciprocal
+    MICLOC_TRY(launch_design_scale(cov, (long long)ncov, (double)(T - t_start), true, st));
+    return design_vectors(interference_removal ? 3 : 2, cov, p.M, G, bf_dev, nullptr, st);
+}
+
+extern "C" int micloc_design_vectors(int mode, const double *cov_dev, int32_t M, int64_t G, double *bf_dev,
+                                     double *value_dev, int device, void *stream) {
+    if (M > kDesignMaxMic) return set_error(MICLOC_ERR_UNSUPPORTED, "design supports M <= %d, got %d", kDesignMaxMic, (int)M);
+    if (M < 1 || G < 1 || !cov_dev || !bf_dev)
+        return set_error(MICLOC_ERR_SHAPE, "bad solver arguments (M = %d, G = %lld)", (int)M, (long long)G);
+    if (mode < 0 || mode > 3) return set_error(MICLOC_ERR_CONFIG, "design mode %d outside 0..3", mode);
+    MICLOC_CUDA(cudaSetDevice(device));
+    return design_vectors(mode, cov_dev, M, G, bf_dev, value_dev, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------

@@ -128,4 +128,19 @@ int hilbert_localize(const HilbertCtx &hc, HilbertScratch &s, const void *audio,
                      long long t_start, int bandpass, float *z_dev, double *cov_dev, float *power_dev, int32_t *doa_dev,
                      cudaStream_t st);
 
+// design_from_template on the device (micloc_design.cu)
+constexpr int kDesignMaxMic = 64;
+struct DesignGeom {                  // a kernel argument: the array geometry, float64
+    int M;
+    double speed;
+    double r[kDesignMaxMic], theta[kDesignMaxMic];
+};
+// clips [G][T][M] f32 of the template (time, sig [T] f64, device) delayed for every doa [G] (device); G / 65535 launches
+int launch_design_templates(const DesignGeom &geo, const double *time, const double *sig, long long T,
+                            const double *doa, long long G, float *clips, cudaStream_t st);
+// x[0..n) /= d (recip: *= 1 / d); one launch
+int launch_design_scale(double *x, long long n, double d, bool recip, cudaStream_t st);
+// the batched eigen-solver behind micloc_design_vectors (arguments checked by the caller); 1 launch, 3 for mode 3
+int design_vectors(int mode, const double *cov, int M, long long G, double *bf, double *value, cudaStream_t st);
+
 }  // namespace micloc

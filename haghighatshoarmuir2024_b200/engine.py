@@ -39,6 +39,58 @@ def _check_frames(frames: torch.Tensor, M: int, device: torch.device, num_stream
     return frames.contiguous(), dt
 
 
+def _design_template(geometry, time: np.ndarray, sig: np.ndarray, device: torch.device):
+    """micloc_design_template of (geometry, template on the fs grid) -> (struct, the arrays it points at)."""
+    r = np.ascontiguousarray(geometry.r_vec, dtype=np.float64)
+    th = np.ascontiguousarray(geometry.theta_vec, dtype=np.float64)
+    t_d, s_d = _dev64(time, device), _dev64(sig, device)
+    if t_d.dim() != 1 or s_d.shape != t_d.shape:
+        raise ValueError(f"template time and signal must be 1-D of one length; got {tuple(t_d.shape)}, {tuple(s_d.shape)}")
+    tp = N.DesignTemplate()
+    tp.num_mic = len(r)
+    tp.r_vec = r.ctypes.data_as(N._dp)
+    tp.theta_vec = th.ctypes.data_as(N._dp)
+    tp.speed = float(geometry.speed)
+    tp.T = len(t_d)
+    tp.time_dev = _ptr(t_d)
+    tp.sig_dev = _ptr(s_d)
+    return tp, (r, th, t_d, s_d)
+
+
+def _dev64(x, device: torch.device) -> torch.Tensor:
+    """float64 contiguous on `device`; a tensor already there is not copied."""
+    if not isinstance(x, torch.Tensor):
+        x = torch.as_tensor(np.asarray(x, dtype=np.float64))
+    return x.to(device=device, dtype=torch.float64).contiguous()
+
+
+def _doa_tensor(doa, device: torch.device) -> torch.Tensor:
+    return _dev64(doa, device).reshape(-1)
+
+
+def design_vectors(mode: int, cov: torch.Tensor, want_value: bool = False):
+    """The batched float64 design solver alone (micloc_design_vectors) on device covariances: cov [G, 2M, 2M] float64
+    (modes 0 SNN unipolar, 1 SNN bipolar) or [G, M, M] complex128 (modes 2 Hilbert, 3 Hilbert with interference
+    removal) -> bf ([2M, G] float64 for modes 0 / 1, [M, G] complex128 for 2 / 3) and, with want_value, value [G]."""
+    cov = cov.contiguous()
+    G = cov.shape[0]
+    if cov.is_complex():
+        M = cov.shape[1]
+        raw = torch.view_as_real(cov)
+    else:
+        M = cov.shape[1] // 2
+        raw = cov
+    dev = cov.device
+    complex_out = mode in (2, 3)
+    bf = torch.empty((M, G, 2) if complex_out else (2 * M, G), dtype=torch.float64, device=dev)
+    value = torch.empty(G, dtype=torch.float64, device=dev) if want_value else None
+    N.check(N.lib().micloc_design_vectors(int(mode), _ptr(raw), M, G, _ptr(bf), _ptr(value), dev.index,
+                                          _stream_ptr(dev)))
+    if complex_out:
+        bf = torch.view_as_complex(bf)
+    return (bf, value) if want_value else bf
+
+
 class _SlotBatch:
     """What the stream batches share: the native batch `_h` of `num_streams` slots on `device`, whose C functions are
     named `<api>_reset`, `<api>_latency` and `<api>_destroy`, and its slot lists.  A subclass creates the handle and
@@ -268,6 +320,41 @@ class SnnEngine:
         if out["cov"] is not None:
             out["cov"] = torch.view_as_complex(out["cov"])
         return {k: v for k, v in out.items() if v is not None}
+
+    # ------------------------------------------------------------------
+    def design_templates(self, geometry, time: np.ndarray, sig: np.ndarray, doa) -> torch.Tensor:
+        """The template (time, sig) on the fs grid delayed for every DoA: clips [G, T, M] float32 on this GPU
+        (micloc_design_templates)."""
+        tp, keep = _design_template(geometry, time, sig, self.device)
+        doa_d = _doa_tensor(doa, self.device)
+        clips = torch.empty((len(doa_d), tp.T, tp.num_mic), dtype=torch.float32, device=self.device)
+        N.check(self._lib.micloc_design_templates(C.byref(tp), _ptr(doa_d), len(doa_d), _ptr(clips), self.device.index,
+                                                  _stream_ptr(self.device)))
+        return clips
+
+    def snn_design(self, geometry, time: np.ndarray, sig: np.ndarray, doa, want_cov: bool = False):
+        """SNN design on the device (micloc_snn_design; unipolar or bipolar from this chain): (bf [2M, G] float64,
+        cov [G, 2M, 2M] float64 or None), device tensors; this engine's chain must be the one of `time`."""
+        tp, keep = _design_template(geometry, time, sig, self.device)
+        doa_d = _doa_tensor(doa, self.device)
+        G = len(doa_d)
+        bf = torch.empty((self.C2, G), dtype=torch.float64, device=self.device)
+        cov = torch.empty((G, self.C2, self.C2), dtype=torch.float64, device=self.device) if want_cov else None
+        N.check(self._lib.micloc_snn_design(self._h, C.byref(tp), _ptr(doa_d), G, _ptr(bf), _ptr(cov),
+                                            _stream_ptr(self.device)))
+        return bf, cov
+
+    def hilbert_design(self, geometry, time: np.ndarray, sig: np.ndarray, doa, interference_removal: bool = False):
+        """Hilbert design on the device (micloc_hilbert_design): (bf [M, G] complex128, cov [G, M, M] complex128),
+        device tensors."""
+        tp, keep = _design_template(geometry, time, sig, self.device)
+        doa_d = _doa_tensor(doa, self.device)
+        G = len(doa_d)
+        bf = torch.empty((self.M, G, 2), dtype=torch.float64, device=self.device)
+        cov = torch.empty((G, self.M, self.M, 2), dtype=torch.float64, device=self.device)
+        N.check(self._lib.micloc_hilbert_design(self._h, C.byref(tp), _ptr(doa_d), G, int(bool(interference_removal)),
+                                                _ptr(bf), _ptr(cov), _stream_ptr(self.device)))
+        return torch.view_as_complex(bf), torch.view_as_complex(cov)
 
     def run_host(self, audio, want_spikes: bool = False, want_power: bool = True, fused: bool = True):
         """End-to-end with HOST buffers (numpy or CPU torch tensors, ideally pinned):

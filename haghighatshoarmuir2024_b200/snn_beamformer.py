@@ -144,6 +144,23 @@ class SNNBeamformer:
             bf_mat.append(bf_vec)
         return np.asarray(bf_mat).T
 
+    def design_on_device(self, template: Tuple[np.ndarray, np.ndarray], doa_list: np.ndarray) -> torch.Tensor:
+        """Beamforming matrix float64 `[2 num_mic, num_DoA]` on the beamformer's GPU, designed there from the template
+        to the steering vectors (micloc_snn_design): the same covariances as design_from_template and the same
+        unipolar vectors; bipolar columns equal the host's up to a phase of u = Re + i Im (the device makes the entry
+        of largest modulus real and positive).  Only the resampling of the template onto the fs grid runs on the host."""
+        try:
+            time_temp, sig_temp = template
+        except Exception:
+            raise ValueError("input template should be a tuple containing (time_in, sig_in) of the template signal!")
+        time_temp = np.asarray(time_temp, dtype=np.float64)
+        time_interp = np.arange(time_temp.min(), time_temp.max(), step=1 / self.fs)
+        sig_interp = np.interp(time_interp, time_temp, sig_temp)
+        M = len(self.geometry)
+        eng = self.engine(np.zeros((2 * M, 1)), time_interp)
+        bf, _ = eng.snn_design(self.geometry, time_interp, sig_interp, doa_list)
+        return bf
+
     def synthesize_from_template(self, template, snr_db: float, rng=None) -> Tuple[np.ndarray, np.ndarray]:
         """(time, `T x num_mic` noisy array signal) exactly as apply_to_template builds it
         (snn_beamformer.py:230-275); `rng=None` uses numpy's global RNG like the reference."""

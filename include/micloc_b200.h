@@ -326,6 +326,58 @@ int micloc_hilbert_localize(micloc_snn *ctx, const void *audio_dev, int dtype, i
                             int bandpass, float *z_dev, double *cov_dev, float *power_dev, int32_t *doa_dev,
                             void *stream);
 
+/* ---- design_from_template on the device ----------------------------------- */
+/* The template of SNNBeamformer / Beamformer.design_from_template after its resampling onto the fs grid (the host
+ * keeps that O(T) np.interp).  num_mic <= 64 (MICLOC_ERR_UNSUPPORTED beyond), T >= 2. */
+typedef struct {
+    int32_t num_mic;
+    const double *r_vec, *theta_vec;    /* [num_mic] host, float64 (array_geometry.py) */
+    double speed;
+    int64_t T;
+    const double *time_dev, *sig_dev;   /* [T] device, float64: the fs grid and the template on it */
+} micloc_design_template;
+/* clips_dev [G][T][M] f32: the template delayed for every doa_dev [G] (device, f64 rad), exactly as
+ * SNNBeamformer._delayed_template and the Hilbert design loop compute it (float64 delays normalised to start at 0,
+ * td clamped below at time[0], np.interp's formula, one rounding to float32).  1 launch per 65535 DoAs. */
+int micloc_design_templates(const micloc_design_template *tp, const double *doa_dev, int64_t G, float *clips_dev,
+                            int device, void *stream);
+/* SNNBeamformer.design_from_template on the device, mode 0 (unipolar) or 1 (bipolar) from the context's encoder.
+ * C_g = Gram of the membrane signals from t_start = T / 4 on, / (T - t_start), of the context's chain (built for
+ * the template's own time grid).  bf_dev [2M][G] f64 (the micloc_snn_config.bf_mat layout); cov_dev [G][2M][2M] f64,
+ * nullable.  Per chunk of DoAs whose clips and front-end scratch stay within ~1 GB: templates, the staged front end
+ * of micloc_snn_gram (STHT, band-pass + RZCC, neuron filter) and the Gram matrix; per call: 1 scale + 1 solver launch.
+ * The front end reads its overflow flags back once per chunk (as micloc_snn_gram does), which synchronises the
+ * stream; nothing else does. */
+int micloc_snn_design(micloc_snn *ctx, const micloc_design_template *tp, const double *doa_dev, int64_t G,
+                      double *bf_dev, double *cov_dev, void *stream);
+/* Beamformer.design_from_template on the device: cov_g = micloc_hilbert_localize's cov (bandpass = 0,
+ * t_start = min(K, T / 2)) / (T - t_start); mode 2, or mode 3 with interference_removal.  bf_dev [M][G][2] f64
+ * (re, im); cov_dev [G][M][M][2] f64, nullable.  Per chunk of DoAs (clips within ~0.5 GB): templates + the 3 or 4
+ * launches of micloc_hilbert_localize; per call: 1 scale + the solver's launches.  Stream-ordered, no
+ * synchronisation. */
+int micloc_hilbert_design(micloc_snn *ctx, const micloc_design_template *tp, const double *doa_dev, int64_t G,
+                          int interference_removal, double *bf_dev, double *cov_dev, void *stream);
+/* The batched float64 solver alone (cyclic Jacobi, one CTA per matrix, n = 2M <= 128), on device inputs:
+ *   mode 0 (SNN unipolar): cov [G][2M][2M] real PSD -> _find_dc_removed_sing_vec(C, rel_prec = 1e-8): theta = U^T 1,
+ *          bisection between the two largest singular values, U theta / (D - root) normalised; value = root.
+ *          Independent of the eigenvectors' signs, so it needs no phase rule.
+ *   mode 1 (SNN bipolar):  the same cov -> top left singular vector u of (C11 + C22)/2 + i (C12 + C21^T)/2, as the
+ *          column [Re u; Im u]; value = its singular value.
+ *   mode 2 (Hilbert):      cov [G][M][M][2] Hermitian PSD -> top eigenvector; value = its eigenvalue.
+ *   mode 3 (Hilbert, interference removal): the same cov -> C_sum = sum_g C_g + diag(mean(diag(C_sum))) / 10, then
+ *          the top generalised eigenvector of (C_g, C_sum - C_g) (Cholesky of C_sum - C_g), normalised;
+ *          value = the generalised eigenvalue.
+ * bf_dev: [2M][G] for modes 0 and 1, [M][G][2] for modes 2 and 3.  value_dev [G], nullable.
+ * Phase rule (modes 1-3): every complex column is rotated so that its entry of largest modulus (the first such index)
+ * is real and positive.  numpy's SVD leaves an arbitrary LAPACK phase, so device and host columns agree up to a
+ * phase.  The SNN bipolar chain is not exactly invariant under a phase rotation of [Re u; Im u]: device- and
+ * host-designed bipolar matrices can give slightly different SNN power.
+ * Launches: 1 (modes 0-2) or 3 (mode 3: C_sum, Cholesky + whitening, solver).  Stream-ordered, no synchronisation.
+ * M > 64 -> MICLOC_ERR_UNSUPPORTED; G < 1 or a null pointer -> MICLOC_ERR_SHAPE; a mode outside 0..3 ->
+ * MICLOC_ERR_CONFIG. */
+int micloc_design_vectors(int mode, const double *cov_dev, int32_t M, int64_t G, double *bf_dev, double *value_dev,
+                          int device, void *stream);
+
 /* ---- Xylo integer chain ---------------------------------------------------- */
 /* Network constants are what rockpool's mapper + global_quantize + config_from_specification
  * hand to XyloSim (micloc/xylo_snn_localization.py:268-290); the host package restates that
