@@ -365,9 +365,9 @@ int micloc::launch_chain_any(const ChainParams &p, const ChainSegs &segs, const 
                                                   segs.tail, segs.nseg);
     };
     if (dtype == MICLOC_I16)
-        launch(p.nsec == 2 ? k_chain_blk<int16_t, 2> : k_chain_blk<int16_t, 0>, (const int16_t *)audio);
+        launch(p.nsec == 2 ? k_chain_blk<int16_t, 2> : k_chain_blk<int16_t, kNsecRuntime>, (const int16_t *)audio);
     else
-        launch(p.nsec == 2 ? k_chain_blk<float, 2> : k_chain_blk<float, 0>, (const float *)audio);
+        launch(p.nsec == 2 ? k_chain_blk<float, 2> : k_chain_blk<float, kNsecRuntime>, (const float *)audio);
     count_launch(1);
     MICLOC_CUDA(cudaGetLastError());
     return MICLOC_OK;

@@ -124,11 +124,26 @@ __device__ __forceinline__ void biquad_reset(BiquadState &st) {
     for (int k = 0; k < kMaxSections; ++k) { st.s1[k] = 0.f; st.s2[k] = 0.f; }
 }
 
-__device__ __forceinline__ float biquad_step(const float (&sos)[kMaxSections][5], int nsec,
-                                             BiquadState &st, float x) {
+// a band's [kMaxSections][5] coefficients (b0 b1 b2 a1 a2 per section) into registers
+__device__ __forceinline__ void load_sos(float (&sos)[kMaxSections][5], const float *band_sos) {
 #pragma unroll
-    for (int k = 0; k < kMaxSections; ++k) {
-        if (k < nsec) {
+    for (int k = 0; k < kMaxSections; ++k)
+#pragma unroll
+        for (int e = 0; e < 5; ++e) sos[k][e] = band_sos[k * 5 + e];
+}
+
+// NSEC >= 0: that many sections, fixed at compile time (0 passes x through); kNsecRuntime: `nsec` sections.
+// Every float32 band-pass outside the fused kernels runs through this one cascade, so their outputs agree bit for bit
+// (the fmaf nesting and the unfused -a2 * y are part of the result).
+constexpr int kNsecRuntime = -1;
+
+template <int NSEC>
+__device__ __forceinline__ float biquad_cascade(const float (&sos)[kMaxSections][5], int nsec, BiquadState &st,
+                                                float x) {
+    constexpr int NS = NSEC >= 0 ? NSEC : kMaxSections;
+#pragma unroll
+    for (int k = 0; k < NS; ++k) {
+        if (NSEC >= 0 || k < nsec) {
             const float y = fmaf(sos[k][0], x, st.s1[k]);
             st.s1[k] = fmaf(sos[k][1], x, fmaf(-sos[k][3], y, st.s2[k]));
             st.s2[k] = fmaf(sos[k][2], x, -sos[k][4] * y);
@@ -157,10 +172,9 @@ __device__ __forceinline__ float biquad_step(const float (&sos)[kMaxSections][5]
 // flat top of more than kPlateauMax exact zeros, sets `overflow` (the clip is
 // flagged; micloc_rzcc_encode_f64 is the unbounded encoder).
 //
-// Two front ends feed the same cluster logic and give identical spikes:
-//   rzcc_detect         one sample at a time (stream kernel)
-//   rzcc_segment_masks  kSeg samples at once from sign / zero bit masks and the
-//                       per-sample running sums (k_chain_blk, fused kernels)
+// One front end feeds the cluster logic: rzcc_segment_masks, kSeg samples at once
+// from sign / zero bit masks and the per-sample running sums (the fused kernels,
+// and k_chain_blk and k_stream_blk through bandpass_block).
 // ---------------------------------------------------------------------------
 constexpr int kSeg = 32;          // samples between two cluster close checks
 constexpr int kPlateauMax = 16;   // longest run of exact zeros inside a flat top the streaming encoder follows
@@ -288,13 +302,33 @@ __device__ __forceinline__ bool rzcc_flat(float z, float cprev) {
 }
 constexpr float kFlatTrigger = 4.5e-16f;      // a segment whose smallest |z| is below this x |sum| takes the per-sample path
 
-// one sample at a time
-template <typename Emit>
-__device__ __forceinline__ void rzcc_detect(RzccState &s, const RzccStore &st, int bipolar, int w, int t, float z,
-                                            Emit &&emit) {
-    const float cprev = s.csum;
-    s.csum = cprev + z;
-    rzcc_sample(s, st, bipolar, w, t, !rzcc_flat(z, cprev), z > 0.f, cprev, emit);
+// One block of kSeg inputs x through the band-pass (biquad_cascade) and the running sum `csum`, without a branch:
+// what rzcc_segment_masks takes.  Bit (31-i) of `neg` / `zero`: filtered sample i is negative / a flat-top zero
+// (rzcc_flat); cs[i*cs_stride] = running sum after sample i; `any` = OR of the input bits ((any << 1) == 0: every
+// input is +-0, digital silence); out(i, z) sees every filtered sample.  PRED: only samples i < nvalid are filtered, so
+// that the state can carry on into the next block; without it all kSeg are, and the caller discards the state after
+// the last valid sample.
+struct BlockMasks { unsigned neg, zero, any; };
+
+template <int NSEC, bool PRED, typename Out>
+__device__ __forceinline__ BlockMasks bandpass_block(const float (&x)[kSeg], int nvalid,
+                                                     const float (&sos)[kMaxSections][5], int nsec, BiquadState &bq,
+                                                     float &csum, float *cs, int cs_stride, Out &&out) {
+    BlockMasks m{0u, 0u, 0u};
+#pragma unroll
+    for (int i = 0; i < kSeg; ++i) {
+        if (!PRED || i < nvalid) {
+            m.any |= __float_as_uint(x[i]);
+            const float v = biquad_cascade<NSEC>(sos, nsec, bq, x[i]);
+            const float cprev = csum;
+            csum = cprev + v;
+            m.neg |= (__float_as_uint(v) & 0x80000000u) >> i;
+            m.zero |= rzcc_flat(v, cprev) ? (0x80000000u >> i) : 0u;
+            cs[i * cs_stride] = csum;
+            out(i, v);
+        }
+    }
+    return m;
 }
 
 // kSeg samples ts .. ts+nvalid-1 at once.  Bit (31-i) of `neg` / `zero` says that sample ts+i is

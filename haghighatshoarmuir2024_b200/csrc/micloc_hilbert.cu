@@ -6,6 +6,9 @@
 //   cov      = S^H S = (Grr + Gii) + i (Gri - Gir)                                  (design_from_template)
 // so the dense y [T][G] of micloc_hilbert_beamform is never formed.
 //
+// A channel's z is k_chain_blk's: the same input (ClipChannelInput: np.roll of the microphone, or the STHT output) and
+// the same band-pass (biquad_cascade), so z equals run_taps' z tap bit for bit on the sequential plan.
+//
 // Kernels per chunk of clips (launch count independent of the chunk's size):
 //   2M <= 16:  k_stht / k_stht_tc -> k_hilbert_gram (roll + band-pass + float64 Gram, z stays on chip) -> k_hilbert_finish
 //   2M >  16:  k_stht / k_stht_tc -> k_hilbert_z (roll + band-pass -> z) -> k_gram_tiled -> k_hilbert_finish
@@ -24,74 +27,6 @@ constexpr int kHbThreads = 128;
 constexpr int kHbUnits = kHbThreads / kHbLanes;
 constexpr int kHbPitch = kHbLanes + 1;       // column 16 stays zero: Gram entries beyond 2M(2M+1)/2 read it
 constexpr int kHbEntries = (kHbLanes * (kHbLanes + 1) / 2 + kHbLanes - 1) / kHbLanes;   // upper-triangle entries per lane
-constexpr int kHbNsecRt = -1;                // NSEC template value: p.nsec sections at run time
-
-// One channel of one (clip, segment): the input of channel c (c < M: np.roll(x, K/2) of microphone c; c >= M: the
-// STHT output q of microphone c - M) through the band-pass sections, kSeg samples at a time, with k_chain_blk's
-// arithmetic (the same fmaf order: z equals run_taps' z tap bit for bit on the sequential plan).
-template <typename IN_T, int NSEC>
-struct HbChannel {
-    float sos[kMaxSections][5];
-    BiquadState bq;
-    const IN_T *xa;
-    const float *xq;
-    bool inphase;
-    int src0, T, M, t_begin;
-
-    __device__ void init(const IN_T *audio, const float *q, const float *band_sos, const ChainParams &p, long long b,
-                         int c, int T_, int t_begin_) {
-        T = T_; M = p.M; t_begin = t_begin_;
-        inphase = c < p.M;
-        xa = audio + b * (long long)T * M + (inphase ? c : 0);
-        xq = q + b * (long long)T * M + (inphase ? 0 : c - M);
-        src0 = (int)(((long long)t_begin - p.half) % T + T) % T;     // (t - K/2) mod T at t = t_begin (np.roll)
-#pragma unroll
-        for (int k = 0; k < kMaxSections; ++k)
-#pragma unroll
-            for (int e = 0; e < 5; ++e) sos[k][e] = band_sos[k * 5 + e];
-        biquad_reset(bq);
-    }
-    // x[i] = input at ts + i for i < t_stop - ts, 0 beyond
-    __device__ __forceinline__ void load(int ts, int t_stop, float (&x)[kSeg]) const {
-        const int left = t_stop - ts;
-        if (inphase) {
-            int s0 = src0 + (ts - t_begin);
-            if (s0 >= T) s0 -= T;
-            const int wrap = T - s0;
-            const IN_T *pp = xa + (long long)s0 * M;
-            if (left >= kSeg && wrap >= kSeg) {
-#pragma unroll
-                for (int i = 0; i < kSeg; ++i) { x[i] = to_f32<IN_T>(*pp); pp += M; }
-            } else {
-#pragma unroll
-                for (int i = 0; i < kSeg; ++i)
-                    x[i] = i < left ? to_f32<IN_T>(pp[(long long)(i < wrap ? i : i - T) * M]) : 0.f;
-            }
-        } else {
-            const float *pp = xq + (long long)ts * M;
-            if (left >= kSeg) {
-#pragma unroll
-                for (int i = 0; i < kSeg; ++i) { x[i] = *pp; pp += M; }
-            } else {
-#pragma unroll
-                for (int i = 0; i < kSeg; ++i) x[i] = i < left ? pp[(long long)i * M] : 0.f;
-            }
-        }
-    }
-    __device__ __forceinline__ float step(float v, int nsec) {
-        constexpr int NS = NSEC >= 0 ? NSEC : kMaxSections;
-#pragma unroll
-        for (int k = 0; k < NS; ++k) {
-            if (NSEC >= 0 || k < nsec) {
-                const float y = fmaf(sos[k][0], v, bq.s1[k]);
-                bq.s1[k] = fmaf(sos[k][1], v, fmaf(-sos[k][3], y, bq.s2[k]));
-                bq.s2[k] = fmaf(sos[k][2], v, -sos[k][4] * y);
-                v = y;
-            }
-        }
-        return v;
-    }
-};
 
 // Time segments (see hilbert_segments): segment s keeps [s seg_len, (s+1) seg_len) and runs the band-pass from `warm` samples
 // before it from zero state (warm = 0 without band-pass: z is then exact in every segment).
@@ -140,16 +75,18 @@ k_hilbert_gram(const IN_T *__restrict__ audio, const float *__restrict__ q, cons
     const int t_begin = max(0, start - warm);
     const int t_stop = live ? end : t_begin;
     const int t_lo = max(start, t_start);                // rows of the Gram sum
-    HbChannel<IN_T, NSEC> ch;
-    ch.init(audio, q, band_sos, p, b, c, T, t_begin);
+    const ClipChannelInput<IN_T> src(audio, q, p, b, c, T, t_begin);
+    float sos[kMaxSections][5];
+    load_sos(sos, band_sos);
+    BiquadState bq; biquad_reset(bq);
     const int nsec = p.nsec;
     float x[kSeg];
-    ch.load(t_begin, t_stop, x);
+    src.load(t_begin, t_stop, x);
     for (int ts = t_begin; ts < t_stop; ts += kSeg) {
         float v[kSeg];
 #pragma unroll
-        for (int i = 0; i < kSeg; ++i) v[i] = ch.step(x[i], nsec);
-        if (ts + kSeg < t_stop) ch.load(ts + kSeg, t_stop, x);
+        for (int i = 0; i < kSeg; ++i) v[i] = biquad_cascade<NSEC>(sos, nsec, bq, x[i]);
+        if (ts + kSeg < t_stop) src.load(ts + kSeg, t_stop, x);
         if (ts + kSeg <= start) continue;                // warm-up only (uniform across the unit)
         if (z_out && lane < C2) {
             float *zo = z_out + ((long long)b * T + ts) * C2 + lane;
@@ -191,16 +128,18 @@ k_hilbert_z(const IN_T *__restrict__ audio, const float *__restrict__ q, const f
     const long long b = idx / ((long long)C2 * nseg);
     const int start = seg * seg_len, end = min(T, start + seg_len);
     const int t_begin = max(0, start - warm);
-    HbChannel<IN_T, NSEC> ch;
-    ch.init(audio, q, band_sos, p, b, c, T, t_begin);
+    const ClipChannelInput<IN_T> src(audio, q, p, b, c, T, t_begin);
+    float sos[kMaxSections][5];
+    load_sos(sos, band_sos);
+    BiquadState bq; biquad_reset(bq);
     const int nsec = p.nsec;
     float x[kSeg];
-    ch.load(t_begin, end, x);
+    src.load(t_begin, end, x);
     for (int ts = t_begin; ts < end; ts += kSeg) {
         float v[kSeg];
 #pragma unroll
-        for (int i = 0; i < kSeg; ++i) v[i] = ch.step(x[i], nsec);
-        if (ts + kSeg < end) ch.load(ts + kSeg, end, x);
+        for (int i = 0; i < kSeg; ++i) v[i] = biquad_cascade<NSEC>(sos, nsec, bq, x[i]);
+        if (ts + kSeg < end) src.load(ts + kSeg, end, x);
         float *zo = z_out + ((long long)b * T + ts) * C2 + c;
 #pragma unroll
         for (int i = 0; i < kSeg; ++i)
@@ -317,7 +256,7 @@ static void launch_front_t(bool narrow, int nsec, const IN_T *audio, const float
                            const HbSegs &sg, cudaStream_t st) {
     if (nsec == 0) launch_front<IN_T, 0>(narrow, audio, q, sos, z, part, p, B, T, t_start, sg, st);
     else if (nsec == 2) launch_front<IN_T, 2>(narrow, audio, q, sos, z, part, p, B, T, t_start, sg, st);
-    else launch_front<IN_T, kHbNsecRt>(narrow, audio, q, sos, z, part, p, B, T, t_start, sg, st);
+    else launch_front<IN_T, kNsecRuntime>(narrow, audio, q, sos, z, part, p, B, T, t_start, sg, st);
 }
 
 int hilbert_localize(const HilbertCtx &hc, HilbertScratch &s, const void *audio, int dtype, long long B, long long T,

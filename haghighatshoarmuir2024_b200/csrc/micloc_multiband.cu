@@ -42,7 +42,9 @@ k_filterbank(const IN_T *__restrict__ audio, float *__restrict__ out, double *__
         if ((t & 255) == 255) { ss += (double)part; part = 0.f; }
 #pragma unroll
         for (int f = 0; f < 8; ++f)          // (unrolled with a predicate: the states stay in registers)
-            if (f < fp.F) out[((long long)f * B + b) * T * M + t * M + m] = biquad_step(fp.sos[f], fp.nsec, st[f], x);
+            if (f < fp.F)
+                out[((long long)f * B + b) * T * M + t * M + m] =
+                    biquad_cascade<kNsecRuntime>(fp.sos[f], fp.nsec, st[f], x);
     }
     if (sumsq) atomicAdd(sumsq + b, ss + (double)part);
 }

@@ -78,59 +78,36 @@ k_f32_to_f64(const float *__restrict__ x, double *__restrict__ y, long long n) {
 // input -- a block of kSeg exactly-zero input samples anywhere in a segment's span flags the clip as well.  One segment
 // per chain (seg_len >= T, warm = tail = 0) is the sequential recurrence: only an overflowed cluster flags the clip.
 //
-// 32 samples at a time: a per-sample candidate test (rzcc_detect) runs its divergent cluster path on almost every step,
-// because with 32 channels in a warp SOME lane has a zero crossing (ncu: 144 warp instructions per sample).  Here a
-// thread first runs the band-pass and the running sum over a block of kSeg samples without a branch (sign / flat-top
-// bit masks, the running sums of the block in shared memory), then hands the block to rzcc_segment_masks -- the front
-// end of the fused kernels, which visits only the sign changes -- and the next block's 32 inputs travel from HBM to
-// registers meanwhile.  The spike raster must be ZEROED before the launch (launch_chain_any does): only spikes are
-// stored.
+// 32 samples at a time: a per-sample candidate test runs its divergent cluster path on almost every step, because with
+// 32 channels in a warp SOME lane has a zero crossing (ncu: 144 warp instructions per sample).  Here a thread first
+// runs the band-pass and the running sum over a block of kSeg samples without a branch (bandpass_block: sign /
+// flat-top bit masks, the running sums of the block in shared memory), then hands the block to rzcc_segment_masks --
+// the front end of the fused kernels, which visits only the sign changes -- and the next block's 32 inputs travel from
+// HBM to registers meanwhile.  The spike raster must be ZEROED before the launch (launch_chain_any does): only spikes
+// are stored.
 // ---------------------------------------------------------------------------
 constexpr int kChainBlkThreads = 128;
-template <typename IN_T, int NSEC>          // NSEC: biquads of the band-pass (0 = p.nsec at run time)
-__global__ void __launch_bounds__(kChainBlkThreads, 3)
-k_chain_blk(const IN_T *__restrict__ audio, const float *__restrict__ q, const float *__restrict__ band_sos,
-            float *__restrict__ z_out, int8_t *__restrict__ spikes, int32_t *__restrict__ flags,
-            const __grid_constant__ ChainParams p, long long B, long long T64, int nb, int seg_len, int warm, int tail,
-            int nseg) {
-    __shared__ float cs_s[kSeg * kChainBlkThreads];
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const int CT = p.C2 * nb;
-    const bool live = idx < B * nseg * CT;           // (no early return: nothing below is a CTA barrier, but keep the warp whole)
-    const long long idc = live ? idx : 0;
-    const int cc = (int)(idc % CT);
-    const int seg = (int)((idc / CT) % nseg);
-    const long long b = idc / ((long long)CT * nseg);
-    const int band = cc / p.C2, c = cc % p.C2;
-    const int T = (int)T64;
-    constexpr int NS = NSEC ? NSEC : kMaxSections;
 
-    float sos[kMaxSections][5];
-#pragma unroll
-    for (int k = 0; k < kMaxSections; ++k)
-#pragma unroll
-        for (int e = 0; e < 5; ++e) sos[k][e] = band_sos[(band * kMaxSections + k) * 5 + e];
-    const int nsec = NSEC ? NSEC : p.nsec;
+// The input of channel c of clip b from t_begin on: c < M the in-phase x[(t - K/2) mod T] of microphone c (np.roll,
+// snn_beamformer.py:325), c >= M the quadrature q[t] of microphone c - M.  k_chain_blk and the Hilbert front end read
+// their clips through it.
+template <typename IN_T>
+struct ClipChannelInput {
+    const IN_T *xa;
+    const float *xq;
+    bool inphase;
+    int src0, T, M, t_begin;
 
-    const int start = seg * seg_len;
-    const int end = min(T, start + seg_len);
-    const int t_begin = max(0, start - warm);                 // a multiple of kSeg (seg_len and warm are)
-    const int t_stop = live ? min(T, end + tail) : t_begin;
-    BiquadState bq; biquad_reset(bq);
-    RzccState rz; rzcc_reset(rz);
-    int cl_pos[2 * kClusterMax]; float cl_h[2 * kClusterMax];
-    const RzccStore store{cl_pos, cl_h, 1};
-    int8_t *sp = spikes + b * T64 * CT + cc;
-    auto emit = [&](int pos, int sign) { if (pos >= start && pos < end) sp[(long long)pos * CT] = (int8_t)sign; };
-
-    const bool inphase = c < p.M;
-    const IN_T *xa = audio + b * T64 * p.M + (inphase ? c : 0);
-    const float *xq = q + b * T64 * p.M + (inphase ? 0 : c - p.M);
-    const int src0 = (int)(((long long)t_begin - p.half) % T + T) % T;       // (t - K/2) mod T at t = t_begin (np.roll)
-    const int M = p.M;
-    float x[kSeg];
-    auto load_block = [&](int ts) {
-        const int left = t_stop - ts;                      // samples of this block inside the segment (<= 0: none)
+    __device__ __forceinline__ ClipChannelInput(const IN_T *audio, const float *q, const ChainParams &p, long long b,
+                                                int c, int T_, int t_begin_)
+        : inphase(c < p.M), T(T_), M(p.M), t_begin(t_begin_) {
+        xa = audio + b * (long long)T * M + (inphase ? c : 0);
+        xq = q + b * (long long)T * M + (inphase ? 0 : c - M);
+        src0 = (int)(((long long)t_begin - p.half) % T + T) % T;     // (t - K/2) mod T at t = t_begin
+    }
+    // x[i] = input at ts + i for i < t_stop - ts, 0 beyond
+    __device__ __forceinline__ void load(int ts, int t_stop, float (&x)[kSeg]) const {
+        const int left = t_stop - ts;
         if (inphase) {
             int s0 = src0 + (ts - t_begin);
             if (s0 >= T) s0 -= T;
@@ -154,10 +131,46 @@ k_chain_blk(const IN_T *__restrict__ audio, const float *__restrict__ q, const f
                 for (int i = 0; i < kSeg; ++i) x[i] = i < left ? pp[(long long)i * M] : 0.f;
             }
         }
-    };
+    }
+};
+
+template <typename IN_T, int NSEC>          // NSEC: biquads of the band-pass (kNsecRuntime: p.nsec)
+__global__ void __launch_bounds__(kChainBlkThreads, 3)
+k_chain_blk(const IN_T *__restrict__ audio, const float *__restrict__ q, const float *__restrict__ band_sos,
+            float *__restrict__ z_out, int8_t *__restrict__ spikes, int32_t *__restrict__ flags,
+            const __grid_constant__ ChainParams p, long long B, long long T64, int nb, int seg_len, int warm, int tail,
+            int nseg) {
+    __shared__ float cs_s[kSeg * kChainBlkThreads];
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int CT = p.C2 * nb;
+    const bool live = idx < B * nseg * CT;           // (no early return: nothing below is a CTA barrier, but keep the warp whole)
+    const long long idc = live ? idx : 0;
+    const int cc = (int)(idc % CT);
+    const int seg = (int)((idc / CT) % nseg);
+    const long long b = idc / ((long long)CT * nseg);
+    const int band = cc / p.C2, c = cc % p.C2;
+    const int T = (int)T64;
+
+    float sos[kMaxSections][5];
+    load_sos(sos, band_sos + band * kMaxSections * 5);
+    const int nsec = p.nsec;
+
+    const int start = seg * seg_len;
+    const int end = min(T, start + seg_len);
+    const int t_begin = max(0, start - warm);                 // a multiple of kSeg (seg_len and warm are)
+    const int t_stop = live ? min(T, end + tail) : t_begin;
+    BiquadState bq; biquad_reset(bq);
+    RzccState rz; rzcc_reset(rz);
+    int cl_pos[2 * kClusterMax]; float cl_h[2 * kClusterMax];
+    const RzccStore store{cl_pos, cl_h, 1};
+    int8_t *sp = spikes + b * T64 * CT + cc;
+    auto emit = [&](int pos, int sign) { if (pos >= start && pos < end) sp[(long long)pos * CT] = (int8_t)sign; };
+
+    const ClipChannelInput<IN_T> src(audio, q, p, b, c, T, t_begin);
+    float x[kSeg];
     bool unsynced = false;
     float *cs = cs_s + threadIdx.x;
-    load_block(t_begin);
+    src.load(t_begin, t_stop, x);
     for (int ts = t_begin; ts < t_stop; ts += kSeg) {
         const int nvalid = min(kSeg, t_stop - ts);
         if (ts == start && seg > 0) {
@@ -165,37 +178,18 @@ k_chain_blk(const IN_T *__restrict__ audio, const float *__restrict__ q, const f
             const int settled = t_begin + (warm >> 1);
             if ((rz.n1 > 0 && cl_pos[kClusterMax] < settled) || (rz.n0 > 0 && cl_pos[0] < settled)) unsynced = true;
         }
-        // ---- band-pass + running sum of the block, branch-free ----
+        // ---- band-pass + running sum of the block, branch-free (zeros past t_stop too: the loop ends with them) ----
         const float carry = rz.csum;
         float csum = carry;
-        unsigned neg = 0u, zero = 0u, any = 0u;
         const bool keep_z = z_out != nullptr && ts >= start && ts < end;     // (start is a multiple of kSeg)
         float *zo = keep_z ? z_out + (b * T64 + ts) * CT + cc : nullptr;
-#pragma unroll
-        for (int i = 0; i < kSeg; ++i) {
-            float v = x[i];
-            any |= __float_as_uint(v);
-#pragma unroll
-            for (int k = 0; k < NS; ++k) {
-                if (k < nsec) {
-                    const float y = fmaf(sos[k][0], v, bq.s1[k]);
-                    bq.s1[k] = fmaf(sos[k][1], v, fmaf(-sos[k][3], y, bq.s2[k]));
-                    bq.s2[k] = fmaf(sos[k][2], v, -sos[k][4] * y);
-                    v = y;
-                }
-            }
-            const float cprev = csum;
-            csum = cprev + v;
-            neg |= (__float_as_uint(v) & 0x80000000u) >> i;
-            zero |= rzcc_flat(v, cprev) ? (0x80000000u >> i) : 0u;
-            cs[i * kChainBlkThreads] = csum;
-            if (keep_z && ts + i < end) zo[(long long)i * CT] = v;
-        }
+        auto store_z = [&](int i, float v) { if (keep_z && ts + i < end) zo[(long long)i * CT] = v; };
+        const BlockMasks m = bandpass_block<NSEC, false>(x, nvalid, sos, nsec, bq, csum, cs, kChainBlkThreads, store_z);
         // digital silence: a whole block of exactly-zero inputs (either sign)
-        if ((any << 1) == 0u && nvalid == kSeg && nseg > 1) unsynced = true;
+        if ((m.any << 1) == 0u && nvalid == kSeg && nseg > 1) unsynced = true;
         // ---- the next block's inputs on their way while the candidates of this one are handled ----
-        if (ts + kSeg < t_stop) load_block(ts + kSeg);
-        rzcc_segment_masks(rz, store, p.bipolar, p.w, ts, nvalid, neg, zero, cs, kChainBlkThreads, carry, emit);
+        if (ts + kSeg < t_stop) src.load(ts + kSeg, t_stop, x);
+        rzcc_segment_masks(rz, store, p.bipolar, p.w, ts, nvalid, m.neg, m.zero, cs, kChainBlkThreads, carry, emit);
         rz.csum = nvalid == kSeg ? csum : cs[(nvalid - 1) * kChainBlkThreads];
         const bool last = ts + nvalid == T;
         if (last || nvalid == kSeg) rzcc_close(rz, store, p.w, ts + nvalid - 1, last, emit);

@@ -56,7 +56,7 @@ struct ChanState {            // one per (slot, real channel): in-phase | quadra
 // SlotPos and k_stream_assemble (the [K-1 history rows | frame] buffer of every slot): micloc_stream.cuh
 
 // Multi-band frame assembly: one thread per (slot, microphone) steps the F band-pass cascades of the filterbank
-// (biquad_step with the float32 sections of k_filterbank, so band f's rows are micloc_filterbank's bits for the whole
+// (biquad_cascade with the float32 sections of k_filterbank, so band f's rows are micloc_filterbank's bits for the whole
 // recording) from its state in fb_state [F][S][M], and writes band f's [hist_f history rows | frame] buffer cur[f]
 // [S][hist_f + n][M] directly; history from the band's previous buffer prev[f] [S][hist_f + n_prev][M].  A slot at
 // N == 0 (new or reset) starts from zero filter state and zero history.  sumsq [S] (nullable, zeroed by the caller)
@@ -117,7 +117,8 @@ k_mb_stream_assemble(const IN_T *__restrict__ frames, BiquadState *__restrict__ 
                 part = fmaf(x[u], x[u], part);
                 if ((t & 255) == 255) { ss += (double)part; part = 0.f; }
 #pragma unroll
-                for (int f = 0; f < NF; ++f) row[f][(long long)t * M] = biquad_step(ap.fb.sos[f], ap.fb.nsec, st[f], x[u]);
+                for (int f = 0; f < NF; ++f)
+                    row[f][(long long)t * M] = biquad_cascade<kNsecRuntime>(ap.fb.sos[f], ap.fb.nsec, st[f], x[u]);
             }
         }
     }
@@ -139,9 +140,9 @@ static void launch_mb_assemble(int F, unsigned grid, cudaStream_t st, const void
 
 // Band-pass + RZCC of the new samples [N, N + n) of every slot, then the neuron filter of the samples that became
 // final, one thread per (slot, channel) with its state in global memory.  The chain is k_chain_blk's (32-sample blocks:
-// branch-free band-pass and running sum, sign / flat-top masks, rzcc_segment_masks, the next block's inputs loaded
-// meanwhile) with the blocks aligned to ABSOLUTE time: the head and tail of a frame that are no whole aligned block go
-// through the same masks with nvalid < 32, and the clusters are closed exactly where the one-clip chain closes them
+// bandpass_block, rzcc_segment_masks, the next block's inputs loaded meanwhile) with the blocks aligned to ABSOLUTE
+// time: the head and tail of a frame that are no whole aligned block go through the same masks with nvalid < 32 (only
+// the valid samples are filtered), and the clusters are closed exactly where the one-clip chain closes them
 // (after every sample t with t % 32 == 31, and at the end), so the spikes are the one-shot clip's bits.  Spikes go to
 // the thread's ring row (int8 [S][C2][R], R a power of two >= n + D + L + 64) at their absolute position; the neuron
 // then reads the row at t and t - L.  Outputs: spikes / membrane rows [S][rows][C2], row i = sample F + i.
@@ -151,7 +152,7 @@ static void launch_mb_assemble(int F, unsigned grid, cudaStream_t st, const void
 // threads in flight.  152 registers (no spills) leave 13 warps per SM; one-warp CTAs use all 13 (larger CTAs round
 // down), i.e. 61 568 threads on 148 SMs: 4096 slots of 7 microphones (57 344 chains) run in ONE wave.
 constexpr int kStreamBlkThreads = 32;
-template <int NSEC>          // biquads of the band-pass (0 = p.nsec at run time)
+template <int NSEC>          // biquads of the band-pass (kNsecRuntime: p.nsec)
 __global__ void __maxnreg__(152)
 k_stream_blk(const float *__restrict__ xbuf, const float *__restrict__ q, ChanState *__restrict__ state,
              const SlotPos *__restrict__ pos_in, SlotPos *__restrict__ pos_out, int32_t *__restrict__ m_out,
@@ -175,13 +176,8 @@ k_stream_blk(const float *__restrict__ xbuf, const float *__restrict__ q, ChanSt
         pos_out[s] = SlotPos{t_end, F1, (run && flush) ? 0 : ps.active, 0};
         m_out[s] = F1 - F0;
     }
-    constexpr int NS = NSEC ? NSEC : kMaxSections;
-    const int nsec = NSEC ? NSEC : p.nsec;
     float sos[kMaxSections][5];
-#pragma unroll
-    for (int k = 0; k < kMaxSections; ++k)
-#pragma unroll
-        for (int e = 0; e < 5; ++e) sos[k][e] = p.sos[k][e];
+    load_sos(sos, &p.sos[0][0]);
 
     ChanState &st = state[idc];
     BiquadState bq = st.bq;
@@ -223,34 +219,15 @@ k_stream_blk(const float *__restrict__ xbuf, const float *__restrict__ q, ChanSt
         } else {
             for (int i = 0; i < nvalid; ++i) rr[(t + i) & rmask] = 0;
         }
-        // ---- band-pass + running sum of the block, branch-free ----
+        // ---- band-pass + running sum of the block's valid samples (the state carries into the next push) ----
         const float carry = rz.csum;
         float csum = carry;
-        unsigned neg = 0u, zero = 0u;
-#pragma unroll
-        for (int i = 0; i < kSeg; ++i) {
-            if (i < nvalid) {
-                float v = x[i];
-#pragma unroll
-                for (int k = 0; k < NS; ++k) {
-                    if (k < nsec) {
-                        const float y = fmaf(sos[k][0], v, bq.s1[k]);
-                        bq.s1[k] = fmaf(sos[k][1], v, fmaf(-sos[k][3], y, bq.s2[k]));
-                        bq.s2[k] = fmaf(sos[k][2], v, -sos[k][4] * y);
-                        v = y;
-                    }
-                }
-                const float cprev = csum;
-                csum = cprev + v;
-                neg |= (__float_as_uint(v) & 0x80000000u) >> i;
-                zero |= rzcc_flat(v, cprev) ? (0x80000000u >> i) : 0u;
-                cs[i * kStreamBlkThreads] = csum;
-            }
-        }
+        const BlockMasks m = bandpass_block<NSEC, true>(x, nvalid, sos, p.nsec, bq, csum, cs, kStreamBlkThreads,
+                                                        [](int, float) {});
         const int tn = t + nvalid;
         // ---- the next block's inputs on their way while the candidates of this one are handled ----
         if (tn < t_end) load_block(tn, min(kSeg, t_end - tn));
-        rzcc_segment_masks(rz, store, p.bipolar, p.w, t, nvalid, neg, zero, cs, kStreamBlkThreads, carry, emit);
+        rzcc_segment_masks(rz, store, p.bipolar, p.w, t, nvalid, m.neg, m.zero, cs, kStreamBlkThreads, carry, emit);
         rz.csum = csum;
         if ((tn & (kSeg - 1)) == 0) rzcc_close(rz, store, p.w, tn - 1, false, emit);
         t = tn;
@@ -472,7 +449,7 @@ static int band_step(StreamBand &b, const SlotBook &bk, const int32_t *close_sel
     if (!close_sel)
         MICLOC_TRY(launch_stht_any(p, (const float *)b.prm.taps_dev, b.xbuf[bk.xcur], MICLOC_F32, b.q, S, b.hist + n, st));
     const unsigned grid = (unsigned)((S * p.C2 + kStreamBlkThreads - 1) / kStreamBlkThreads);
-    auto kernel = p.nsec == 2 ? k_stream_blk<2> : k_stream_blk<0>;
+    auto kernel = p.nsec == 2 ? k_stream_blk<2> : k_stream_blk<kNsecRuntime>;
     kernel<<<grid, kStreamBlkThreads, 0, st>>>(b.xbuf[bk.xcur], b.q, b.state, bk.pos[bk.pcur], bk.pos[bk.pcur ^ 1], bk.m,
                                               close_sel, b.ring, b.ring_len, b.flags, spikes_dev, b.vmem, p, S, (int)n,
                                               b.hist, (int)rows, bk.D);
