@@ -115,6 +115,12 @@ SYMBOLS = {
     "micloc_xylo_streams_reset": (C.c_int, [_vp, _vp, _i32, _vp]),
     "micloc_xylo_streams_push": (C.c_int, [_vp, _vp, C.c_int, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
     "micloc_xylo_streams_flush": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
+    "micloc_hilbert_streams_create": (C.c_int, [C.POINTER(_vp), _i32, _i32, _dp, _dp, _i32, _i64, C.POINTER(_vp)]),
+    "micloc_hilbert_streams_destroy": (C.c_int, [_vp]),
+    "micloc_hilbert_streams_latency": (C.c_int, [_vp]),
+    "micloc_hilbert_streams_reset": (C.c_int, [_vp, _vp, _i32, _vp]),
+    "micloc_hilbert_streams_push": (C.c_int, [_vp, _vp, C.c_int, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                              _vp, _vp]),
     "micloc_last_error": (C.c_char_p, []),
     "micloc_version": (C.c_int, []),
     "micloc_launch_count": (_i64, []),

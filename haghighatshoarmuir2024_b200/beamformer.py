@@ -4,13 +4,15 @@
 projection on the GPU (micloc_hilbert_beamform) and returns complex128 `T x G`.
 `localize` and `design_from_template` take batches through micloc_hilbert_localize, which
 gets power, DoA and the design covariance from one Gram matrix of the analytic signal per
-clip and never forms the dense `T x G` output.
+clip and never forms the dense `T x G` output.  `HilbertStreamBatch` (and the one-band
+`Beamformer.stream_batch`) runs the same chain over many live recordings, state carried
+from frame to frame (micloc_hilbert_streams_*).
 """
 from __future__ import annotations
 
 import ctypes as C
 from numbers import Number
-from typing import List, Tuple, Union
+from typing import Dict, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -19,7 +21,7 @@ from scipy.signal import butter, hilbert
 
 from . import _native as N
 from .array_geometry import ArrayGeometry
-from .engine import ChainSpec, SnnEngine, _ptr, _stream_ptr
+from .engine import ChainSpec, SnnEngine, _SlotBatch, _check_frames, _ptr, _stream_ptr
 
 Fs = 48_000
 
@@ -143,6 +145,10 @@ class Beamformer:
             self._hbf = bf_mat.copy()
         return eng.hilbert(audio, want=("doa", "power"))
 
+    def stream_batch(self, bf_mat: np.ndarray, num_streams: int, max_frame_len: int) -> "HilbertStreamBatch":
+        """`num_streams` live recordings through this beamformer's own band-pass chain, no filterbank in front."""
+        return HilbertStreamBatch([(self, bf_mat)], num_streams, max_frame_len)
+
     def apply_to_template(self, bf_mat: np.ndarray, template, snr_db: float) -> np.ndarray:
         """beamformer.py:194-258: delayed + noisy array signal, then apply_to_signal."""
         try:
@@ -181,3 +187,85 @@ class Beamformer:
                                                 _stream_ptr(eng.device)))
         yh = y[0].cpu().numpy().astype(np.float64)
         return yh[..., 0] + 1j * yh[..., 1]
+
+
+class HilbertStreamBatch(_SlotBatch):
+    """`num_streams` independent live recordings ("slots") through the Hilbert beamformer with its state carried across
+    pushes (micloc_hilbert_streams_*).  `bands` is a list of (Beamformer, bf_mat [M, G] complex) of one array and one
+    DoA grid; `filterbank` (a ButterworthFilterbank, one band per entry of `bands`) runs in front of them, or, when None,
+    the single band takes the raw frames.  N pushed frames give every band's analytic signal of their concatenation
+    (after the filterbank, if any), with the stream's causal in-phase delay.  Every pushed sample is final at once
+    (latency 0, no flush); `reset(slots)` restarts the listed slots.  The steering matrices are copied at creation."""
+
+    def __init__(self, bands, num_streams: int, max_frame_len: int, filterbank=None, doa_list=None):
+        bands = list(bands)
+        if not bands:
+            raise ValueError("a Hilbert stream batch needs at least one band")
+        if filterbank is not None and len(filterbank.sos_list) != len(bands):
+            raise ValueError(f"the filterbank has {len(filterbank.sos_list)} bands, the batch {len(bands)}")
+        self.bands = bands
+        self.engines = []
+        for beamf, bf_mat in bands:
+            bf_mat = np.asarray(bf_mat)
+            eng = beamf._engine()
+            if getattr(beamf, "_hbf", None) is None or beamf._hbf.shape != bf_mat.shape or not np.array_equal(beamf._hbf, bf_mat):
+                eng.set_hilbert_bf(bf_mat)
+                beamf._hbf = bf_mat.copy()
+            self.engines.append(eng)
+        self.F = len(bands)
+        self.M, self.G = self.engines[0].M, np.asarray(bands[0][1]).shape[1]
+        self.C2 = 2 * self.M
+        self.filterbank = filterbank
+        self.doa_list = None if doa_list is None else np.ascontiguousarray(doa_list, dtype=np.float64)
+        lib = N.lib()
+        sos = None if filterbank is None else np.ascontiguousarray(filterbank.sos_list, dtype=np.float64)
+        ctxs = (C.c_void_p * self.F)(*[e._h.value for e in self.engines])
+        h = C.c_void_p()
+        N.check(lib.micloc_hilbert_streams_create(
+            ctxs, self.F, 0 if sos is None else sos.shape[1], None if sos is None else sos.ctypes.data_as(N._dp),
+            None if self.doa_list is None else self.doa_list.ctypes.data_as(N._dp), int(num_streams),
+            int(max_frame_len), C.byref(h)))
+        self._attach(lib, h, "micloc_hilbert_streams", int(num_streams), int(max_frame_len), self.engines[0].device)
+        self._doa_dev = None if self.doa_list is None else torch.from_numpy(self.doa_list).to(self.device)
+
+    def push(self, frames: torch.Tensor, want: Sequence[str] = ("doa", "power"), rel_threshold: float = 0.0001,
+             full_scale: Optional[float] = None) -> Dict[str, object]:
+        """One frame [num_streams, n, channels] per slot in (int32 / int16 / float32; channels beyond the microphones
+        are dropped), this push's n rows out, as device tensors: any of 'z' [F, S, n, 2M], 'cov' [F, S, M, M]
+        complex128 (sum conj(s_t) s_t^T), 'power' [F, S, G] (mean |s_t . conj(bf_g)|^2), 'power_grid' [S, G] (sum over
+        the bands), 'doa' [S] (its first argmax), 'periodic_ml' / 'trimmed_periodic_ml' [S] (need doa_list) and
+        'flags' [S] (bit 1: the trimmed estimator's IndexError).  With a filterbank, also 'sumsq' [S] of the frame,
+        'active' [S] (its rms against rel_threshold * full_scale, as Demo.localize) and, when 'doa' is wanted and
+        doa_list was given, 'doa_deg' [S] (NaN where inactive).  'n_out' (numpy int64 [S]) is n for every slot.  No
+        host synchronisation."""
+        frames, dt = _check_frames(frames, self.M, self.device, self.num_streams)
+        S, n, ch = frames.shape
+        dev = self.device
+        mk = lambda name, shape, dtype: torch.empty(shape, dtype=dtype, device=dev) if name in want else None
+        out = {"z": mk("z", (self.F, S, n, self.C2), torch.float32),
+               "cov": mk("cov", (self.F, S, self.M, self.M, 2), torch.float64),
+               "power": mk("power", (self.F, S, self.G), torch.float32),
+               "power_grid": mk("power_grid", (S, self.G), torch.float32),
+               "doa": mk("doa", (S,), torch.int32),
+               "periodic_ml": mk("periodic_ml", (S,), torch.float64),
+               "trimmed_periodic_ml": mk("trimmed_periodic_ml", (S,), torch.float64),
+               "flags": mk("flags", (S,), torch.int32)}
+        sumsq = torch.empty(S, dtype=torch.float64, device=dev) if self.filterbank is not None else None
+        n_out = np.zeros(S, dtype=np.int64)
+        N.check(self._lib.micloc_hilbert_streams_push(
+            self._h, _ptr(frames), dt, n, ch, _ptr(out["z"]), _ptr(out["cov"]), _ptr(out["power"]),
+            _ptr(out["power_grid"]), _ptr(out["doa"]), _ptr(out["periodic_ml"]), _ptr(out["trimmed_periodic_ml"]),
+            _ptr(sumsq), _ptr(out["flags"]), n_out.ctypes.data_as(C.c_void_p), _stream_ptr(dev)))
+        if out["cov"] is not None:
+            out["cov"] = torch.view_as_complex(out["cov"])
+        out = {k: v for k, v in out.items() if v is not None}
+        out["n_out"] = n_out
+        if sumsq is not None:
+            if full_scale is None:
+                full_scale = float(torch.iinfo(frames.dtype).max) if not frames.dtype.is_floating_point else 1.0
+            active = torch.sqrt(sumsq / (n * self.M)) >= rel_threshold * full_scale
+            out.update({"sumsq": sumsq, "active": active})
+            if "doa" in out and self._doa_dev is not None:
+                deg = self._doa_dev[out["doa"].long()] * 180 / np.pi
+                out["doa_deg"] = torch.where(active, deg, torch.full_like(deg, float("nan")))
+        return out

@@ -246,6 +246,13 @@ int micloc_snn_get_params(micloc_snn *c, micloc_snn_params *out) {
     return MICLOC_OK;
 }
 
+int micloc::hilbert_ctx(micloc_snn *c, HilbertCtx *out, int *device) {
+    if (!c || !out || !device) return set_error(MICLOC_ERR_CONFIG, "null context");
+    *out = HilbertCtx{c->p, c->d_taps, c->d_sos, c->pole_radius, c->sm_count, c->d_hW, c->hG};
+    *device = c->device;
+    return MICLOC_OK;
+}
+
 extern "C" int micloc_snn_set_bf(micloc_snn *c, const double *bf, int32_t G) {
     if (!c || !bf || G < 1) return set_error(MICLOC_ERR_CONFIG, "bad bf_mat");
     MICLOC_CUDA(cudaSetDevice(c->device));

@@ -124,6 +124,8 @@ struct HilbertCtx {
     int G;
 };
 struct HilbertScratch { DevBuf q, z, part, gram; };
+// what micloc_hilbert_localize reads from context c, and the context's device (the Hilbert stream batches)
+int hilbert_ctx(micloc_snn *c, HilbertCtx *out, int *device);
 int hilbert_localize(const HilbertCtx &hc, HilbertScratch &s, const void *audio, int dtype, long long B, long long T,
                      long long t_start, int bandpass, float *z_dev, double *cov_dev, float *power_dev, int32_t *doa_dev,
                      cudaStream_t st);

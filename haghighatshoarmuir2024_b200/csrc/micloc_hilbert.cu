@@ -13,12 +13,23 @@
 //   2M <= 16:  k_stht / k_stht_tc -> k_hilbert_gram (roll + band-pass + float64 Gram, z stays on chip) -> k_hilbert_finish
 //   2M >  16:  k_stht / k_stht_tc -> k_hilbert_z (roll + band-pass -> z) -> k_gram_tiled -> k_hilbert_finish
 // k_gram_tc is not used: its fp16 scaling assumes |v| < 15 (membrane values); z of int16 audio is in the thousands.
+//
+// HILBERT STREAM BATCHES (micloc_hilbert_streams_*): S live recordings through F band chains, state carried across
+// pushes.  A batch is a SlotBook (micloc_stream.cuh, latency D = 0) plus, per band, the [K-1 history | frame] buffers,
+// the STHT output and one BiquadState per (slot, channel) of the band-pass, all in global memory; with a filterbank,
+// its state [F][S][M] as well.  A slot at N == 0 (new or reset) starts from zero filter state, so reset only rewrites
+// positions.  Per push, whatever S:
+//   k_mb_stream_assemble (filterbank) or k_stream_assemble (none)                                         1
+//   per band: STHT, k_hilbert_gram_stream (2M <= 16) or k_hilbert_z_stream + k_gram_tiled (2M > 16)        2 or 3
+//             k_hilbert_finish when cov, power or a fused output is asked for                              +1
+//   k_power_fuse when power_grid, doa, the estimators or flags are asked for                               +1
 #include <cuda_runtime.h>
 
 #include <cmath>
 
 #include "micloc_common.h"
 #include "micloc_staged.cuh"
+#include "micloc_stream.cuh"
 
 namespace micloc {
 
@@ -31,6 +42,48 @@ constexpr int kHbEntries = (kHbLanes * (kHbLanes + 1) / 2 + kHbLanes - 1) / kHbL
 // Time segments (see hilbert_segments): segment s keeps [s seg_len, (s+1) seg_len) and runs the band-pass from `warm` samples
 // before it from zero state (warm = 0 without band-pass: z is then exact in every segment).
 struct HbSegs { int seg_len, warm, nseg; };
+
+// The float64 Gram matrix of one 16-lane unit (lane c < 2M is channel c): lane `lane` owns the entries
+// e = lane + 16 k of the upper triangle, row-major (beyond the triangle: column 16, which stays zero).  A block of kSeg
+// band-passed samples is staged in the unit's shared rows zu as float64, then every lane adds its <= 9 entries over the
+// block's rows [i0, i1) (float64 FMAs in time order).  The one-shot and the stream kernels accumulate through it.
+struct HbGram {
+    int ei[kHbEntries], ej[kHbEntries];
+    double acc[kHbEntries];
+
+    __device__ __forceinline__ HbGram(double (*zu)[kHbPitch], int lane, int C2) {
+        for (int i = 0; i < kSeg; ++i) zu[i][kHbLanes] = 0.0;   // (each lane writes the same zero)
+        const int npair = C2 * (C2 + 1) / 2;
+#pragma unroll
+        for (int k = 0; k < kHbEntries; ++k) {
+            int e = lane + kHbLanes * k, i = 0;
+            if (e < npair) {
+                while (e >= C2 - i) { e -= C2 - i; ++i; }
+                ei[k] = i; ej[k] = i + e;
+            } else {
+                ei[k] = ej[k] = kHbLanes;
+            }
+            acc[k] = 0.0;
+        }
+    }
+    __device__ __forceinline__ void add_block(double (*zu)[kHbPitch], int lane, int C2, unsigned hmask,
+                                              const float (&v)[kSeg], int i0, int i1) {
+        __syncwarp(hmask);                               // the previous block's reads are done
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i) zu[i][lane] = lane < C2 ? (double)v[i] : 0.0;
+        __syncwarp(hmask);
+        for (int i = i0; i < i1; ++i) {
+#pragma unroll
+            for (int k = 0; k < kHbEntries; ++k) acc[k] = fma(zu[i][ei[k]], zu[i][ej[k]], acc[k]);
+        }
+    }
+    // the upper triangle into out [2M][2M], as k_gram_tiled writes a partial sum
+    __device__ __forceinline__ void store(double *out, int C2) const {
+#pragma unroll
+        for (int k = 0; k < kHbEntries; ++k)
+            if (ei[k] < kHbLanes) out[ei[k] * C2 + ej[k]] = acc[k];
+    }
+};
 
 // ---------------------------------------------------------------------------
 // 2M <= 16: one unit of 16 lanes per (clip, segment).  Each block of kSeg samples: lane c band-passes channel c into
@@ -53,23 +106,7 @@ k_hilbert_gram(const IN_T *__restrict__ audio, const float *__restrict__ q, cons
     const int c = lane < C2 ? lane : C2 - 1;             // idle lanes shadow the last channel and stage zeros
     const unsigned hmask = 0xffffu << (threadIdx.x & 16);
     double (*zu)[kHbPitch] = zs[unit_l];
-    for (int i = 0; i < kSeg; ++i) zu[i][kHbLanes] = 0.0;   // (each lane writes the same zero)
-
-    // this lane's Gram entries e = lane + 16 k of the upper triangle, row-major; beyond the triangle: column 16 (zero)
-    const int npair = C2 * (C2 + 1) / 2;
-    int ei[kHbEntries], ej[kHbEntries];
-    double acc[kHbEntries];
-#pragma unroll
-    for (int k = 0; k < kHbEntries; ++k) {
-        int e = lane + kHbLanes * k, i = 0;
-        if (e < npair) {
-            while (e >= C2 - i) { e -= C2 - i; ++i; }
-            ei[k] = i; ej[k] = i + e;
-        } else {
-            ei[k] = ej[k] = kHbLanes;
-        }
-        acc[k] = 0.0;
-    }
+    HbGram gm(zu, lane, C2);
 
     const int start = seg * seg_len, end = min(T, start + seg_len);
     const int t_begin = max(0, start - warm);
@@ -96,20 +133,10 @@ k_hilbert_gram(const IN_T *__restrict__ audio, const float *__restrict__ q, cons
         }
         const int i0 = max(0, t_lo - ts), i1 = min(kSeg, end - ts);
         if (i0 >= i1) continue;
-        __syncwarp(hmask);                               // the previous block's reads are done
-#pragma unroll
-        for (int i = 0; i < kSeg; ++i) zu[i][lane] = lane < C2 ? (double)v[i] : 0.0;
-        __syncwarp(hmask);
-        for (int i = i0; i < i1; ++i) {
-#pragma unroll
-            for (int k = 0; k < kHbEntries; ++k) acc[k] = fma(zu[i][ei[k]], zu[i][ej[k]], acc[k]);
-        }
+        gm.add_block(zu, lane, C2, hmask, v, i0, i1);
     }
     if (!live) return;
-    double *out = part + ((long long)seg * B + b) * C2 * C2;
-#pragma unroll
-    for (int k = 0; k < kHbEntries; ++k)
-        if (ei[k] < kHbLanes) out[ei[k] * C2 + ej[k]] = acc[k];
+    gm.store(part + ((long long)seg * B + b) * C2 * C2, C2);
 }
 
 // ---------------------------------------------------------------------------
@@ -326,4 +353,345 @@ int hilbert_localize(const HilbertCtx &hc, HilbertScratch &s, const void *audio,
     return MICLOC_OK;
 }
 
+// ---------------------------------------------------------------------------
+// Stream forms.  Channel c of slot s reads the band's [hist | frame] rows: in-phase x[t - K/2] at row hist - K/2 + i,
+// quadrature q at row hist + i (i = t - N, as k_stream_blk), and continues its band-pass from state [S][2M] (zero
+// state at N == 0).  The filter stops after the frame's n samples: the state the next push continues from.
+// ---------------------------------------------------------------------------
+struct StreamChannelInput {
+    const float *src;
+    int M, n;
+    __device__ __forceinline__ StreamChannelInput(const float *xbuf, const float *q, const ChainParams &p, long long s,
+                                                  int c, int hist, int n_)
+        : M(p.M), n(n_) {
+        const long long base = s * ((long long)hist + n) * M;
+        src = c < M ? xbuf + base + (long long)(hist - p.half) * M + c : q + base + (long long)hist * M + (c - M);
+    }
+    // x[i] = input of frame row i0 + i, 0 past the frame
+    __device__ __forceinline__ void load(int i0, float (&x)[kSeg]) const {
+        const float *pp = src + (long long)i0 * M;
+        if (n - i0 >= kSeg) {
+#pragma unroll
+            for (int i = 0; i < kSeg; ++i) { x[i] = *pp; pp += M; }
+        } else {
+#pragma unroll
+            for (int i = 0; i < kSeg; ++i) x[i] = i < n - i0 ? pp[(long long)i * M] : 0.f;
+        }
+    }
+};
+
+// v = band-pass of the block's nv valid inputs (zeros beyond, the state untouched by them)
+template <int NSEC>
+__device__ __forceinline__ void stream_bandpass(const float (&sos)[kMaxSections][5], int nsec, BiquadState &bq,
+                                                const float (&x)[kSeg], int nv, float (&v)[kSeg]) {
+    if (nv == kSeg) {
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i) v[i] = biquad_cascade<NSEC>(sos, nsec, bq, x[i]);
+    } else {
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i) v[i] = i < nv ? biquad_cascade<NSEC>(sos, nsec, bq, x[i]) : 0.f;
+    }
+}
+
+// 2M <= 16: one 16-lane unit per slot (k_hilbert_gram's body through HbGram); part [S][2M][2M] is the single partial
+// sum k_hilbert_finish reads.  Every band's launch writes the same next positions and row counts m = n.
+template <int NSEC>
+__global__ void __launch_bounds__(kHbThreads)
+k_hilbert_gram_stream(const float *__restrict__ xbuf, const float *__restrict__ q, const float *__restrict__ band_sos,
+                      BiquadState *__restrict__ state, const SlotPos *__restrict__ pos_in, SlotPos *__restrict__ pos_out,
+                      int32_t *__restrict__ m_out, float *__restrict__ z_out, double *__restrict__ part,
+                      const __grid_constant__ ChainParams p, long long S, int n, int hist) {
+    __shared__ double zs[kHbUnits][kSeg][kHbPitch];
+    const int unit_l = threadIdx.x / kHbLanes, lane = threadIdx.x % kHbLanes;
+    const long long unit = (long long)blockIdx.x * kHbUnits + unit_l;
+    const bool live = unit < S;
+    const long long s = live ? unit : 0;
+    const int C2 = p.C2;
+    const int c = lane < C2 ? lane : C2 - 1;             // idle lanes shadow the last channel and stage zeros
+    const unsigned hmask = 0xffffu << (threadIdx.x & 16);
+    double (*zu)[kHbPitch] = zs[unit_l];
+    HbGram gm(zu, lane, C2);
+    const SlotPos ps = pos_in[s];
+    BiquadState bq;
+    if (ps.N == 0) biquad_reset(bq);
+    else bq = state[s * C2 + c];
+    float sos[kMaxSections][5];
+    load_sos(sos, band_sos);
+    const int nsec = p.nsec;
+    const StreamChannelInput src(xbuf, q, p, s, c, hist, n);
+    const int t_stop = live ? n : 0;
+    float x[kSeg];
+    if (t_stop > 0) src.load(0, x);
+    for (int ts = 0; ts < t_stop; ts += kSeg) {
+        const int nv = min(kSeg, t_stop - ts);
+        float v[kSeg];
+        stream_bandpass<NSEC>(sos, nsec, bq, x, nv, v);
+        if (ts + kSeg < t_stop) src.load(ts + kSeg, x);
+        if (z_out && lane < C2) {
+            float *zo = z_out + (s * n + ts) * C2 + lane;
+#pragma unroll
+            for (int i = 0; i < kSeg; ++i)
+                if (i < nv) zo[(long long)i * C2] = v[i];
+        }
+        gm.add_block(zu, lane, C2, hmask, v, 0, nv);
+    }
+    if (!live) return;
+    if (lane < C2) state[s * C2 + lane] = bq;
+    if (lane == 0) { pos_out[s] = SlotPos{ps.N + n, ps.N + n, 1, 0}; m_out[s] = n; }
+    gm.store(part + s * C2 * C2, C2);
+}
+
+// 2M > 16: one thread per (slot, channel) writes z [S][n][2M]; k_gram_tiled and k_hilbert_finish follow
+template <int NSEC>
+__global__ void __launch_bounds__(kChainBlkThreads)
+k_hilbert_z_stream(const float *__restrict__ xbuf, const float *__restrict__ q, const float *__restrict__ band_sos,
+                   BiquadState *__restrict__ state, const SlotPos *__restrict__ pos_in, SlotPos *__restrict__ pos_out,
+                   int32_t *__restrict__ m_out, float *__restrict__ z_out, const __grid_constant__ ChainParams p,
+                   long long S, int n, int hist) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int C2 = p.C2;
+    if (idx >= S * C2) return;
+    const int c = (int)(idx % C2);
+    const long long s = idx / C2;
+    const SlotPos ps = pos_in[s];
+    BiquadState bq;
+    if (ps.N == 0) biquad_reset(bq);
+    else bq = state[idx];
+    float sos[kMaxSections][5];
+    load_sos(sos, band_sos);
+    const int nsec = p.nsec;
+    const StreamChannelInput src(xbuf, q, p, s, c, hist, n);
+    float x[kSeg];
+    src.load(0, x);
+    for (int ts = 0; ts < n; ts += kSeg) {
+        const int nv = min(kSeg, n - ts);
+        float v[kSeg];
+        stream_bandpass<NSEC>(sos, nsec, bq, x, nv, v);
+        if (ts + kSeg < n) src.load(ts + kSeg, x);
+        float *zo = z_out + (s * n + ts) * C2 + c;
+#pragma unroll
+        for (int i = 0; i < kSeg; ++i)
+            if (i < nv) zo[(long long)i * C2] = v[i];
+    }
+    state[idx] = bq;
+    if (c == 0) { pos_out[s] = SlotPos{ps.N + n, ps.N + n, 1, 0}; m_out[s] = n; }
+}
+
+// the listed slots (sel == nullptr: all) restart at sample 0
+__global__ void __launch_bounds__(256)
+k_hilbert_stream_reset(SlotPos *__restrict__ pos, const int32_t *__restrict__ sel, long long S) {
+    const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s < S && (!sel || sel[s])) pos[s] = SlotPos{0, 0, 1, 0};
+}
+
 }  // namespace micloc
+
+using namespace micloc;
+
+// one band of a Hilbert stream batch
+struct HilbertStreamBand {
+    HilbertCtx hc;                  // the context's chain constants, taps and band-pass; d_W is the batch's own copy
+    int hist = 0;                   // K - 1
+    float *xbuf[2] = {nullptr, nullptr}, *q = nullptr;
+    BiquadState *state = nullptr;   // [S][2M] band-pass state
+    double *W = nullptr;            // [2M][G] copy of the context's complex steering matrix
+};
+
+struct micloc_hilbert_streams {
+    int F = 0, device = 0, M = 0, G = 0;
+    bool bank = false;              // a filterbank runs in front
+    SlotBook book;
+    HilbertStreamBand band[8];
+    FilterbankParams fb{};
+    BiquadState *fb_state = nullptr;    // [F][S][M]
+    double *doa_list = nullptr;         // [G] on the device, null: no ML estimators
+    float *power = nullptr;             // [F][S][G] per-band power when the caller passes no power_dev
+    float *z = nullptr;                 // [S][max_frame][2M] z scratch of the wide path
+    double *part = nullptr;             // [nslab][S][2M][2M] Gram partial sums (reused band after band)
+    double *gram = nullptr;             // [S][2M][2M] k_hilbert_finish's Gram when it does not fit shared memory
+};
+
+extern "C" int micloc_hilbert_streams_destroy(micloc_hilbert_streams *hs) {
+    if (!hs) return MICLOC_OK;
+    cudaSetDevice(hs->device);
+    hs->book.destroy();
+    for (int f = 0; f < hs->F; ++f) {
+        HilbertStreamBand &b = hs->band[f];
+        cudaFree(b.xbuf[0]); cudaFree(b.xbuf[1]); cudaFree(b.q); cudaFree(b.state); cudaFree(b.W);
+    }
+    cudaFree(hs->fb_state); cudaFree(hs->doa_list); cudaFree(hs->power); cudaFree(hs->z); cudaFree(hs->part);
+    cudaFree(hs->gram);
+    delete hs;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_hilbert_streams_reset(micloc_hilbert_streams *hs, const int32_t *slots_host, int32_t n_slots,
+                                            void *stream) {
+    if (!hs) return set_error(MICLOC_ERR_CONFIG, "null stream");
+    MICLOC_CUDA(cudaSetDevice(hs->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    SlotBook &bk = hs->book;
+    if (slots_host) MICLOC_TRY(bk.upload(slots_host, n_slots, st));
+    k_hilbert_stream_reset<<<(unsigned)((bk.S + 255) / 256), 256, 0, st>>>(bk.pos[bk.pcur], slots_host ? bk.sel : nullptr, bk.S);
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    return bk.reset_done(slots_host != nullptr, st);
+}
+
+static int nslab_of(int C2, long long n) { return C2 <= kHbLanes ? 1 : (int)((n + kGtFlush - 1) / kGtFlush); }
+
+extern "C" int micloc_hilbert_streams_create(micloc_snn *const *ctxs, int32_t F, int32_t n_sections, const double *sos,
+                                             const double *doa_list, int32_t num_streams, int64_t max_frame_len,
+                                             micloc_hilbert_streams **out) {
+    if (!ctxs || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
+    *out = nullptr;
+    if (F < 1 || F > 8) return set_error(MICLOC_ERR_CONFIG, "Hilbert stream batch of %d bands (1..8 supported)", F);
+    if (!sos && F > 1) return set_error(MICLOC_ERR_CONFIG, "%d bands need a filterbank (sos == NULL takes one band)", F);
+    FilterbankParams fb{};
+    if (sos) MICLOC_TRY(filterbank_params(F, n_sections, sos, &fb));
+    HilbertCtx hc[8];
+    int dev[8];
+    for (int f = 0; f < F; ++f) {
+        if (!ctxs[f]) return set_error(MICLOC_ERR_CONFIG, "null context of band %d", f);
+        MICLOC_TRY(hilbert_ctx(ctxs[f], &hc[f], &dev[f]));
+        if (!hc[f].d_W) return set_error(MICLOC_ERR_CONFIG, "band %d has no Hilbert steering matrix (micloc_hilbert_set_bf)", f);
+        if (dev[f] != dev[0])
+            return set_error(MICLOC_ERR_CONFIG, "band %d's context is on device %d, band 0's on device %d", f, dev[f], dev[0]);
+        if (hc[f].p.M != hc[0].p.M || hc[f].G != hc[0].G)
+            return set_error(MICLOC_ERR_SHAPE, "band %d's context has %d microphones and %d DoAs, band 0's %d and %d", f,
+                             hc[f].p.M, hc[f].G, hc[0].p.M, hc[0].G);
+    }
+    MICLOC_CUDA(cudaSetDevice(dev[0]));
+    micloc_hilbert_streams *hs = new micloc_hilbert_streams();
+    hs->F = F; hs->device = dev[0]; hs->M = hc[0].p.M; hs->G = hc[0].G; hs->bank = sos != nullptr; hs->fb = fb;
+    int rc = hs->book.create(num_streams, max_frame_len);
+    const size_t S = (size_t)num_streams, M = (size_t)hs->M, C2 = 2 * M, G = (size_t)hs->G;
+    const bool narrow = (int)C2 <= kHbLanes;
+    for (int f = 0; f < F && !rc; ++f) {
+        HilbertStreamBand &b = hs->band[f];
+        b.hc = hc[f];
+        b.hist = hc[f].p.K - 1;
+        const size_t rows = (size_t)b.hist + (size_t)max_frame_len;
+        if (!(cudaMalloc(&b.xbuf[0], S * rows * M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&b.xbuf[1], S * rows * M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&b.q, S * rows * M * sizeof(float)) == cudaSuccess &&
+              cudaMalloc(&b.state, S * C2 * sizeof(BiquadState)) == cudaSuccess &&
+              cudaMalloc(&b.W, C2 * G * sizeof(double)) == cudaSuccess))
+            rc = set_error(MICLOC_ERR_CUDA, "cudaMalloc(Hilbert stream batch) failed");
+        else if (cudaMemcpy(b.W, hc[f].d_W, C2 * G * sizeof(double), cudaMemcpyDeviceToDevice) != cudaSuccess)
+            rc = set_error(MICLOC_ERR_CUDA, "copy of band %d's steering matrix failed", f);
+        b.hc.d_W = b.W;
+    }
+    const size_t nslab = (size_t)nslab_of((int)C2, max_frame_len);
+    if (!rc && !(cudaMalloc(&hs->power, (size_t)F * S * G * sizeof(float)) == cudaSuccess &&
+                 cudaMalloc(&hs->part, nslab * S * C2 * C2 * sizeof(double)) == cudaSuccess &&
+                 (narrow || cudaMalloc(&hs->z, S * (size_t)max_frame_len * C2 * sizeof(float)) == cudaSuccess) &&
+                 (C2 * C2 * sizeof(double) <= 128 * 1024 || cudaMalloc(&hs->gram, S * C2 * C2 * sizeof(double)) == cudaSuccess) &&
+                 (!hs->bank || cudaMalloc(&hs->fb_state, (size_t)F * S * M * sizeof(BiquadState)) == cudaSuccess) &&
+                 (!doa_list || cudaMalloc(&hs->doa_list, G * sizeof(double)) == cudaSuccess)))
+        rc = set_error(MICLOC_ERR_CUDA, "cudaMalloc(Hilbert stream batch) failed");
+    if (!rc && doa_list && cudaMemcpy(hs->doa_list, doa_list, G * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess)
+        rc = set_error(MICLOC_ERR_CUDA, "Hilbert stream batch set-up failed");
+    if (!rc) rc = micloc_hilbert_streams_reset(hs, nullptr, 0, nullptr);
+    if (rc) { micloc_hilbert_streams_destroy(hs); return rc; }
+    *out = hs;
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_hilbert_streams_latency(micloc_hilbert_streams *hs) { return hs ? hs->book.D : 0; }
+
+// band f's chain over the newest [history | frame] buffers: STHT, band-pass + Gram (z to z_f when given), then cov and
+// power from the Gram; the caller flips the book
+template <int NSEC>
+static int hilbert_stream_band(micloc_hilbert_streams *hs, int f, long long n, float *z_f, double *cov_f, float *power_f,
+                               cudaStream_t st) {
+    HilbertStreamBand &b = hs->band[f];
+    const SlotBook &bk = hs->book;
+    const ChainParams &p = b.hc.p;
+    const long long S = bk.S;
+    const int C2 = p.C2;
+    const float *xb = b.xbuf[bk.xcur];
+    MICLOC_TRY(launch_stht_any(p, b.hc.d_taps, xb, MICLOC_F32, b.q, S, b.hist + n, st));
+    const SlotPos *pin = bk.pos[bk.pcur];
+    SlotPos *pout = bk.pos[bk.pcur ^ 1];
+    const int nslab = nslab_of(C2, n);
+    if (C2 <= kHbLanes) {
+        k_hilbert_gram_stream<NSEC><<<(unsigned)((S + kHbUnits - 1) / kHbUnits), kHbThreads, 0, st>>>(
+            xb, b.q, b.hc.d_sos, b.state, pin, pout, bk.m, z_f, hs->part, p, S, (int)n, b.hist);
+        count_launch(1);
+    } else {
+        float *z = z_f ? z_f : hs->z;
+        k_hilbert_z_stream<NSEC><<<(unsigned)((S * C2 + kChainBlkThreads - 1) / kChainBlkThreads), kChainBlkThreads, 0, st>>>(
+            xb, b.q, b.hc.d_sos, b.state, pin, pout, bk.m, z, p, S, (int)n, b.hist);
+        const int nblk = (C2 + kGtTile - 1) / kGtTile, nblocks = nblk * (nblk + 1) / 2;
+        k_gram_tiled<<<dim3((unsigned)S, (unsigned)nblocks, (unsigned)nslab), 256, 0, st>>>(z, hs->part, C2, S, n, 0, kGtFlush);
+        count_launch(2);
+    }
+    MICLOC_CUDA(cudaGetLastError());
+    if (!cov_f && !power_f) return MICLOC_OK;
+    const double inv_n = 1.0 / (double)n;
+    if (!hs->gram) {
+        const size_t smem_b = (size_t)C2 * C2 * sizeof(double);
+        MICLOC_CUDA(cudaFuncSetAttribute(k_hilbert_finish<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        k_hilbert_finish<true><<<(unsigned)S, 256, smem_b, st>>>(hs->part, nslab, nullptr, b.W, p.M, hs->G, S, inv_n, cov_f,
+                                                                 power_f, nullptr);
+    } else {
+        k_hilbert_finish<false><<<(unsigned)S, 256, 0, st>>>(hs->part, nslab, hs->gram, b.W, p.M, hs->G, S, inv_n, cov_f,
+                                                             power_f, nullptr);
+    }
+    count_launch(1);
+    MICLOC_CUDA(cudaGetLastError());
+    return MICLOC_OK;
+}
+
+extern "C" int micloc_hilbert_streams_push(micloc_hilbert_streams *hs, const void *frames_dev, int dtype, int64_t n,
+                                           int32_t in_channels, float *z_dev, double *cov_dev, float *power_dev,
+                                           float *power_grid_dev, int32_t *doa_dev, double *periodic_ml_dev,
+                                           double *trimmed_ml_dev, double *sumsq_dev, int32_t *flags_dev,
+                                           int64_t *n_out_host, void *stream) {
+    if (!hs || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
+    SlotBook &bk = hs->book;
+    MICLOC_TRY(bk.check_push(dtype, n, in_channels, hs->M));
+    if ((periodic_ml_dev || trimmed_ml_dev) && !hs->doa_list) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
+    if (sumsq_dev && !hs->bank) return set_error(MICLOC_ERR_SHAPE, "sumsq needs the filterbank (sos != NULL at create)");
+    MICLOC_CUDA(cudaSetDevice(hs->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long S = bk.S;
+    if (hs->bank) {
+        MbAssembleParams ap{};
+        ap.fb = hs->fb;
+        for (int f = 0; f < hs->F; ++f) {
+            ap.prev[f] = hs->band[f].xbuf[bk.xcur];
+            ap.cur[f] = hs->band[f].xbuf[bk.xcur ^ 1];
+            ap.hist[f] = hs->band[f].hist;
+        }
+        if (sumsq_dev) MICLOC_CUDA(cudaMemsetAsync(sumsq_dev, 0, (size_t)S * sizeof(double), st));
+        const unsigned grid = (unsigned)((S * hs->M + 127) / 128);
+        auto launch = dtype == MICLOC_F32 ? launch_mb_assemble<float> : dtype == MICLOC_I16 ? launch_mb_assemble<int16_t>
+                                                                                        : launch_mb_assemble<int32_t>;
+        launch(hs->F, grid, st, frames_dev, hs->fb_state, sumsq_dev, bk.pos[bk.pcur], ap, S, (int)n, (int)bk.n_prev,
+               in_channels, hs->M);
+        count_launch(1);
+        MICLOC_CUDA(cudaGetLastError());
+        bk.xcur ^= 1;
+        bk.n_prev = n;
+    } else {
+        MICLOC_TRY(bk.assemble(hs->band[0].xbuf, frames_dev, dtype, n, in_channels, hs->M, hs->band[0].hist, st));
+    }
+    const bool fuse = power_grid_dev || doa_dev || periodic_ml_dev || trimmed_ml_dev || flags_dev;
+    float *power = power_dev ? power_dev : (fuse ? hs->power : nullptr);
+    const int C2 = 2 * hs->M;
+    for (int f = 0; f < hs->F; ++f) {
+        float *z_f = z_dev ? z_dev + (size_t)f * S * n * C2 : nullptr;
+        double *cov_f = cov_dev ? cov_dev + (size_t)f * S * hs->M * hs->M * 2 : nullptr;
+        float *pw_f = power ? power + (size_t)f * S * hs->G : nullptr;
+        const int nsec = hs->band[f].hc.p.nsec;
+        MICLOC_TRY(nsec == 2 ? hilbert_stream_band<2>(hs, f, n, z_f, cov_f, pw_f, st)
+                             : hilbert_stream_band<kNsecRuntime>(hs, f, n, z_f, cov_f, pw_f, st));
+    }
+    bk.pushed(n, n_out_host);
+    if (!fuse) return MICLOC_OK;
+    if (flags_dev) MICLOC_CUDA(cudaMemsetAsync(flags_dev, 0, (size_t)S * sizeof(int32_t), st));
+    return launch_power_fuse(power, hs->F, S, hs->G, hs->doa_list, power_grid_dev, doa_dev, periodic_ml_dev,
+                             trimmed_ml_dev, flags_dev, nullptr, nullptr, st);
+}

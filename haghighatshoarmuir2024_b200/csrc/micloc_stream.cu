@@ -53,90 +53,8 @@ struct ChanState {            // one per (slot, real channel): in-phase | quadra
     NeuronState nr;
 };
 
-// SlotPos and k_stream_assemble (the [K-1 history rows | frame] buffer of every slot): micloc_stream.cuh
-
-// Multi-band frame assembly: one thread per (slot, microphone) steps the F band-pass cascades of the filterbank
-// (biquad_cascade with the float32 sections of k_filterbank, so band f's rows are micloc_filterbank's bits for the whole
-// recording) from its state in fb_state [F][S][M], and writes band f's [hist_f history rows | frame] buffer cur[f]
-// [S][hist_f + n][M] directly; history from the band's previous buffer prev[f] [S][hist_f + n_prev][M].  A slot at
-// N == 0 (new or reset) starts from zero filter state and zero history.  sumsq [S] (nullable, zeroed by the caller)
-// += sum of x^2 over the frame's kept channels, float32 partials of 256 samples added in float64 as in k_filterbank.
-struct MbAssembleParams {
-    FilterbankParams fb;
-    const float *prev[8];
-    float *cur[8];
-    int hist[8];
-};
-
-// NF = F is a template argument: the bands stay in registers, and the unrolled loop body stays small enough for the
-// instruction cache.  A predicated loop over 8 bands inside a 16-sample unroll did not (20 k instructions): 3.5 ms per
-// push at 1024 slots against 2.0 ms at 4096 slots in this form (F = 3, one B200).
-template <typename IN_T, int NF>
-__global__ void __launch_bounds__(128)
-k_mb_stream_assemble(const IN_T *__restrict__ frames, BiquadState *__restrict__ fb_state, double *__restrict__ sumsq,
-                     const SlotPos *__restrict__ pos, const __grid_constant__ MbAssembleParams ap, long long S, int n,
-                     int n_prev, int in_ch, int M) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= S * M) return;
-    const long long s = i / M;
-    const int m = (int)(i % M);
-    const bool fresh = pos[s].N == 0;
-    BiquadState st[NF];
-    float *row[NF];                       // band f's first frame row of this (slot, microphone)
-#pragma unroll
-    for (int f = 0; f < NF; ++f) {
-        if (fresh) biquad_reset(st[f]);
-        else st[f] = fb_state[f * S * M + i];
-        const int hist = ap.hist[f];
-        float *cur = ap.cur[f] + s * ((long long)hist + n) * M + m;
-        const float *prev = ap.prev[f] + (s * ((long long)hist + n_prev) + n_prev) * M + m;
-#pragma unroll 4
-        for (int r = 0; r < hist; ++r) cur[(long long)r * M] = fresh ? 0.f : prev[(long long)r * M];
-        row[f] = cur + (long long)hist * M;
-    }
-    // the frame in blocks of 8 samples, the next block's loads issued before the current one is filtered
-    constexpr int kBlk = 8;
-    const IN_T *src = frames + s * (long long)n * in_ch + m;
-    float nx[kBlk];
-    auto load = [&](int t0) {
-#pragma unroll
-        for (int u = 0; u < kBlk; ++u) nx[u] = t0 + u < n ? (float)src[(long long)(t0 + u) * in_ch] : 0.f;
-    };
-    double ss = 0.0;
-    float part = 0.f;
-    load(0);
-    for (int t0 = 0; t0 < n; t0 += kBlk) {
-        float x[kBlk];
-#pragma unroll
-        for (int u = 0; u < kBlk; ++u) x[u] = nx[u];
-        if (t0 + kBlk < n) load(t0 + kBlk);
-#pragma unroll
-        for (int u = 0; u < kBlk; ++u) {
-            const int t = t0 + u;
-            if (t < n) {
-                part = fmaf(x[u], x[u], part);
-                if ((t & 255) == 255) { ss += (double)part; part = 0.f; }
-#pragma unroll
-                for (int f = 0; f < NF; ++f)
-                    row[f][(long long)t * M] = biquad_cascade<kNsecRuntime>(ap.fb.sos[f], ap.fb.nsec, st[f], x[u]);
-            }
-        }
-    }
-    if (sumsq) atomicAdd(sumsq + s, ss + (double)part);
-#pragma unroll
-    for (int f = 0; f < NF; ++f) fb_state[f * S * M + i] = st[f];
-}
-
-template <typename IN_T>
-static void launch_mb_assemble(int F, unsigned grid, cudaStream_t st, const void *frames, BiquadState *fb_state,
-                               double *sumsq, const SlotPos *pos, const MbAssembleParams &ap, long long S, int n,
-                               int n_prev, int in_ch, int M) {
-    static decltype(&k_mb_stream_assemble<IN_T, 1>) const ks[8] = {
-        k_mb_stream_assemble<IN_T, 1>, k_mb_stream_assemble<IN_T, 2>, k_mb_stream_assemble<IN_T, 3>,
-        k_mb_stream_assemble<IN_T, 4>, k_mb_stream_assemble<IN_T, 5>, k_mb_stream_assemble<IN_T, 6>,
-        k_mb_stream_assemble<IN_T, 7>, k_mb_stream_assemble<IN_T, 8>};
-    ks[F - 1]<<<grid, 128, 0, st>>>((const IN_T *)frames, fb_state, sumsq, pos, ap, S, n, n_prev, in_ch, M);
-}
+// SlotPos, k_stream_assemble (the [K-1 history rows | frame] buffer of every slot) and k_mb_stream_assemble (the same
+// behind a filterbank): micloc_stream.cuh
 
 // Band-pass + RZCC of the new samples [N, N + n) of every slot, then the neuron filter of the samples that became
 // final, one thread per (slot, channel) with its state in global memory.  The chain is k_chain_blk's (32-sample blocks:

@@ -482,6 +482,61 @@ int micloc_xylo_streams_flush(micloc_xylo_streams *xs, const int32_t *slots_host
                               int32_t *doa_peak_dev, int32_t peak_win, int32_t *flags_dev, int64_t *n_out_host,
                               int32_t *flags_host, void *stream);
 
+/* ---- Hilbert stream batches: the Hilbert beamformer over many live recordings ---------------------------------- */
+/* The live Hilbert beamformer (the baseline of every SNN localiser) with its state carried across pushes.  A batch
+ * holds S independent slots (1 <= S <= 65535) over F contexts ctxs[F] (one per band, 1 <= F <= 8, same device, same M),
+ * each with its Hilbert steering matrix set (micloc_hilbert_set_bf) and the same hG; otherwise create returns
+ * MICLOC_ERR_CONFIG (no steering matrix, a device or F out of range, a NULL context) or MICLOC_ERR_SHAPE (M or G differ).
+ *   - sos [F][n_sections][6] (host) != NULL: a Butterworth filterbank (the sections of micloc_filterbank) runs in front
+ *     of the band chains, its state carried: the live multi-band localiser.  sos == NULL: F must be 1 (MICLOC_ERR_CONFIG
+ *     otherwise) and the raw frame goes straight into the band's chain, Beamformer.apply_to_signal's own band-pass
+ *     chain made continuous.
+ *   - Band f's chain is micloc_hilbert_localize's with bandpass = 1: STHT, the context's band-pass, the Gram matrix of
+ *     the analytic signal.  The batch COPIES every band's complex steering matrix at create time (a later
+ *     micloc_hilbert_set_bf leaves the batch as it was); the STHT taps and the band-pass sections are the context's,
+ *     fixed for its lifetime: destroy the batch before its contexts.
+ *   - Concatenation rule: N pushed frames give band f's analytic signal z of the whole recording bit for bit: with a
+ *     filterbank, micloc_filterbank of the concatenation followed by band f's chain; without, the chain on the
+ *     concatenation itself.  As in every stream, the in-phase branch is the causal delay x[t - K/2] (zeros before the
+ *     slot starts; identical to np.roll whenever the recording's last K/2 samples are zero).  On wide arrays (M > 8) the
+ *     STHT runs on the tensor cores, which scale each 256-sample tile by its own largest magnitude: q, and with it z, then
+ *     agrees with the one-shot chain to the tensor-core STHT's tolerance (5e-6 of max |z| measured) rather than bit
+ *     for bit
+ *     (bit for bit again with MICLOC_STHT_FP32 set).
+ *   - Latency 0: every pushed sample is final at once, n_out_host[s] = n for every slot; there is no flush.  reset takes
+ *     a slot list (slots_host [n_slots], NULL = every slot): the listed slots restart at sample 0 with zero filterbank,
+ *     band-pass and STHT history.  reset synchronises `stream`; a push does not.
+ *   - push: frames_dev [S][n][in_channels] float32 / int16 / int32 (int32 wav frames with the recorder's extra channel:
+ *     channels >= M are dropped), 1 <= n <= max_frame_len, in_channels >= M; a push that would take a slot's position to
+ *     2^31 - 4096 samples or beyond is refused.  Outputs, all nullable device pointers, over the n rows of this push:
+ *       z_dev          [F][S][n][2M] f32   s_t as (real | imag), debug tap;
+ *       cov_dev        [F][S][M][M][2] f64 sum_t conj(s_t[i]) s_t[j], not normalised (micloc_hilbert_localize's cov);
+ *       power_dev      [F][S][G] f32       mean_t |s_t . conj(bf_g)|^2;
+ *       power_grid_dev [S][G] f32, doa_dev [S]: the sum over the bands and its first argmax (micloc_power_fuse, for every
+ *                      F);  periodic_ml_dev / trimmed_ml_dev [S] f64: its estimators (need doa_list, MICLOC_ERR_SHAPE
+ *                      otherwise; NaN and flags bit 1 in the reference's IndexError case);
+ *       sumsq_dev      [S] f64: sum of x^2 over the kept channels of the frame, as micloc_snn_mb_streams_push (needs the
+ *                      filterbank: MICLOC_ERR_SHAPE without one);
+ *       flags_dev      [S]: bit 1 as above (there is no RZCC: bit 0 is never set).
+ * Kernel launches per push, whatever S: 1 (frame assembly, with the filterbank when there is one); per band, 2 (STHT,
+ * band-pass + float64 Gram) for M <= 8 or 3 (STHT, band-pass -> z, tiled Gram) for M > 8, +1 (Gram -> cov, power) when
+ * cov, power or a fused output is asked for; +1 (sum over bands, argmax, estimators) when power_grid, doa, the
+ * estimators or flags are asked for.  doa_list [G] (host, nullable).  Device memory: 3 S (K - 1 + max_frame_len) M
+ * floats and S 2M biquad states per band, S G F floats of power scratch, S (2M)^2 doubles of Gram partials per
+ * 1024-sample slab (one slab for M <= 8), S max_frame_len 2M floats of z scratch for M > 8. */
+typedef struct micloc_hilbert_streams micloc_hilbert_streams;
+int micloc_hilbert_streams_create(micloc_snn *const *ctxs, int32_t F, int32_t n_sections, const double *sos,
+                                  const double *doa_list, int32_t num_streams, int64_t max_frame_len,
+                                  micloc_hilbert_streams **out);
+int micloc_hilbert_streams_destroy(micloc_hilbert_streams *hs);
+/* always 0 */
+int micloc_hilbert_streams_latency(micloc_hilbert_streams *hs);
+int micloc_hilbert_streams_reset(micloc_hilbert_streams *hs, const int32_t *slots_host, int32_t n_slots, void *stream);
+int micloc_hilbert_streams_push(micloc_hilbert_streams *hs, const void *frames_dev, int dtype, int64_t n,
+                                int32_t in_channels, float *z_dev, double *cov_dev, float *power_dev,
+                                float *power_grid_dev, int32_t *doa_dev, double *periodic_ml_dev, double *trimmed_ml_dev,
+                                double *sumsq_dev, int32_t *flags_dev, int64_t *n_out_host, void *stream);
+
 /* ---- misc ------------------------------------------------------------------ */
 const char *micloc_last_error(void);
 int micloc_version(void);
