@@ -21,7 +21,7 @@ from scipy.signal import butter, hilbert
 
 from . import _native as N
 from .array_geometry import ArrayGeometry
-from .engine import ChainSpec, SnnEngine, _SlotBatch, _check_frames, _ptr, _stream_ptr
+from .engine import ChainSpec, SnnEngine, _SlotBatch, _activity, _check_frames, _ptr, _stream_ptr
 
 Fs = 48_000
 
@@ -48,6 +48,7 @@ class Beamformer:
         self.device = device
         self.verbose = True
         self._eng = None
+        self._hbf = None            # the engine's Hilbert steering matrix
 
     def _engine(self) -> SnnEngine:
         if self._eng is None:
@@ -57,6 +58,14 @@ class Beamformer:
                              bipolar=False, neuron_decay=0.5, neuron_scale=1.0, neuron_len=1)
             self._eng = SnnEngine(spec, np.zeros((2 * M, 1)), device=self.device)
         return self._eng
+
+    def _hilbert_engine(self, bf_mat: np.ndarray) -> SnnEngine:
+        """The engine with bf_mat [M, G] as its Hilbert steering matrix, uploaded only when it changed."""
+        eng = self._engine()
+        if self._hbf is None or self._hbf.shape != bf_mat.shape or not np.array_equal(self._hbf, bf_mat):
+            eng.set_hilbert_bf(bf_mat)
+            self._hbf = bf_mat.copy()
+        return eng
 
     def hilbert_signal(self, sig_in: np.ndarray) -> np.ndarray:
         """Band-passed analytic signal `T x M` complex128 (beamformer.py:281-287)."""
@@ -139,11 +148,7 @@ class Beamformer:
         if num_chan != num_mic:
             raise ValueError(
                 f"number of channels in the input siganl {num_chan} should be the same as the number of microphones {num_mic}!")
-        eng = self._engine()
-        if getattr(self, "_hbf", None) is None or self._hbf.shape != bf_mat.shape or not np.array_equal(self._hbf, bf_mat):
-            eng.set_hilbert_bf(bf_mat)
-            self._hbf = bf_mat.copy()
-        return eng.hilbert(audio, want=("doa", "power"))
+        return self._hilbert_engine(bf_mat).hilbert(audio, want=("doa", "power"))
 
     def stream_batch(self, bf_mat: np.ndarray, num_streams: int, max_frame_len: int) -> "HilbertStreamBatch":
         """`num_streams` live recordings through this beamformer's own band-pass chain, no filterbank in front."""
@@ -204,14 +209,7 @@ class HilbertStreamBatch(_SlotBatch):
         if filterbank is not None and len(filterbank.sos_list) != len(bands):
             raise ValueError(f"the filterbank has {len(filterbank.sos_list)} bands, the batch {len(bands)}")
         self.bands = bands
-        self.engines = []
-        for beamf, bf_mat in bands:
-            bf_mat = np.asarray(bf_mat)
-            eng = beamf._engine()
-            if getattr(beamf, "_hbf", None) is None or beamf._hbf.shape != bf_mat.shape or not np.array_equal(beamf._hbf, bf_mat):
-                eng.set_hilbert_bf(bf_mat)
-                beamf._hbf = bf_mat.copy()
-            self.engines.append(eng)
+        self.engines = [beamf._hilbert_engine(np.asarray(bf_mat)) for beamf, bf_mat in bands]
         self.F = len(bands)
         self.M, self.G = self.engines[0].M, np.asarray(bands[0][1]).shape[1]
         self.C2 = 2 * self.M
@@ -261,11 +259,9 @@ class HilbertStreamBatch(_SlotBatch):
         out = {k: v for k, v in out.items() if v is not None}
         out["n_out"] = n_out
         if sumsq is not None:
-            if full_scale is None:
-                full_scale = float(torch.iinfo(frames.dtype).max) if not frames.dtype.is_floating_point else 1.0
-            active = torch.sqrt(sumsq / (n * self.M)) >= rel_threshold * full_scale
-            out.update({"sumsq": sumsq, "active": active})
-            if "doa" in out and self._doa_dev is not None:
-                deg = self._doa_dev[out["doa"].long()] * 180 / np.pi
-                out["doa_deg"] = torch.where(active, deg, torch.full_like(deg, float("nan")))
+            out["sumsq"] = sumsq
+            out["active"], doa_deg = _activity(sumsq, n, self.M, frames.dtype, rel_threshold, full_scale,
+                                               out.get("doa"), self._doa_dev)
+            if doa_deg is not None:
+                out["doa_deg"] = doa_deg
         return out

@@ -82,6 +82,10 @@ int filterbank_params(int32_t F, int32_t n_sections, const double *sos, Filterba
 int launch_power_fuse(const float *power, int F, long long B, int G, const double *doa_list, float *power_sum,
                       int32_t *doa, double *ml, double *trimmed, int32_t *flags, const int32_t *rows_b,
                       const int32_t *const *band_flags, cudaStream_t st);
+// the estimator outputs ml / trimmed (nullable) of k_power_fuse need its doa_list
+inline int check_doa_list(const double *doa_list, const void *ml, const void *trimmed) {
+    return (ml || trimmed) && !doa_list ? set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list") : MICLOC_OK;
+}
 // power[b][g] = w_g^T gram_b w_g * inv_T (float64, stored as float32) and doa[b] = first argmax over g, for gram
 // [B][C2][C2] float64.  The one place that picks the power kernel (micloc_snn_run_taps and the stream batches):
 //   k_power_wide               C2 >= 32 and Gram + steering tile in <= 200 KB of shared memory (M <= 72), unless

@@ -15,10 +15,10 @@
 // k_gram_tc is not used: its fp16 scaling assumes |v| < 15 (membrane values); z of int16 audio is in the thousands.
 //
 // HILBERT STREAM BATCHES (micloc_hilbert_streams_*): S live recordings through F band chains, state carried across
-// pushes.  A batch is a SlotBook (micloc_stream.cuh, latency D = 0) plus, per band, the [K-1 history | frame] buffers,
-// the STHT output and one BiquadState per (slot, channel) of the band-pass, all in global memory; with a filterbank,
-// its state [F][S][M] as well.  A slot at N == 0 (new or reset) starts from zero filter state, so reset only rewrites
-// positions.  Per push, whatever S:
+// pushes.  A batch is a SlotBook (latency D = 0) and a BankFront (micloc_stream.cuh, shared with the multi-band SNN
+// batch; it has no filterbank state without a filterbank) plus, per band, the [K-1 history | frame] buffers, the STHT
+// output and one BiquadState per (slot, channel) of the band-pass.  A slot at N == 0 (new or reset) starts from zero
+// filter state, so reset only rewrites positions.  Per push, whatever S:
 //   k_mb_stream_assemble (filterbank) or k_stream_assemble (none)                                         1
 //   per band: STHT, k_hilbert_gram_stream (2M <= 16) or k_hilbert_z_stream + k_gram_tiled (2M > 16)        2 or 3
 //             k_hilbert_finish when cov, power or a fused output is asked for                              +1
@@ -498,14 +498,10 @@ struct HilbertStreamBand {
 };
 
 struct micloc_hilbert_streams {
-    int F = 0, device = 0, M = 0, G = 0;
-    bool bank = false;              // a filterbank runs in front
+    int device = 0;
     SlotBook book;
+    BankFront front;                // fb_state null: no filterbank, the single band takes the raw frames
     HilbertStreamBand band[8];
-    FilterbankParams fb{};
-    BiquadState *fb_state = nullptr;    // [F][S][M]
-    double *doa_list = nullptr;         // [G] on the device, null: no ML estimators
-    float *power = nullptr;             // [F][S][G] per-band power when the caller passes no power_dev
     float *z = nullptr;                 // [S][max_frame][2M] z scratch of the wide path
     double *part = nullptr;             // [nslab][S][2M][2M] Gram partial sums (reused band after band)
     double *gram = nullptr;             // [S][2M][2M] k_hilbert_finish's Gram when it does not fit shared memory
@@ -515,12 +511,12 @@ extern "C" int micloc_hilbert_streams_destroy(micloc_hilbert_streams *hs) {
     if (!hs) return MICLOC_OK;
     cudaSetDevice(hs->device);
     hs->book.destroy();
-    for (int f = 0; f < hs->F; ++f) {
+    for (int f = 0; f < hs->front.F; ++f) {
         HilbertStreamBand &b = hs->band[f];
         cudaFree(b.xbuf[0]); cudaFree(b.xbuf[1]); cudaFree(b.q); cudaFree(b.state); cudaFree(b.W);
     }
-    cudaFree(hs->fb_state); cudaFree(hs->doa_list); cudaFree(hs->power); cudaFree(hs->z); cudaFree(hs->part);
-    cudaFree(hs->gram);
+    hs->front.destroy();
+    cudaFree(hs->z); cudaFree(hs->part); cudaFree(hs->gram);
     delete hs;
     return MICLOC_OK;
 }
@@ -545,27 +541,21 @@ extern "C" int micloc_hilbert_streams_create(micloc_snn *const *ctxs, int32_t F,
                                              micloc_hilbert_streams **out) {
     if (!ctxs || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
     *out = nullptr;
-    if (F < 1 || F > 8) return set_error(MICLOC_ERR_CONFIG, "Hilbert stream batch of %d bands (1..8 supported)", F);
     if (!sos && F > 1) return set_error(MICLOC_ERR_CONFIG, "%d bands need a filterbank (sos == NULL takes one band)", F);
-    FilterbankParams fb{};
-    if (sos) MICLOC_TRY(filterbank_params(F, n_sections, sos, &fb));
     HilbertCtx hc[8];
     int dev[8];
-    for (int f = 0; f < F; ++f) {
-        if (!ctxs[f]) return set_error(MICLOC_ERR_CONFIG, "null context of band %d", f);
+    MICLOC_TRY(check_bands("Hilbert stream batch", ctxs, F, [&](int f, BandShape &b) -> int {
         MICLOC_TRY(hilbert_ctx(ctxs[f], &hc[f], &dev[f]));
         if (!hc[f].d_W) return set_error(MICLOC_ERR_CONFIG, "band %d has no Hilbert steering matrix (micloc_hilbert_set_bf)", f);
-        if (dev[f] != dev[0])
-            return set_error(MICLOC_ERR_CONFIG, "band %d's context is on device %d, band 0's on device %d", f, dev[f], dev[0]);
-        if (hc[f].p.M != hc[0].p.M || hc[f].G != hc[0].G)
-            return set_error(MICLOC_ERR_SHAPE, "band %d's context has %d microphones and %d DoAs, band 0's %d and %d", f,
-                             hc[f].p.M, hc[f].G, hc[0].p.M, hc[0].G);
-    }
+        b = {dev[f], hc[f].p.M, hc[f].G};
+        return MICLOC_OK;
+    }));
     MICLOC_CUDA(cudaSetDevice(dev[0]));
     micloc_hilbert_streams *hs = new micloc_hilbert_streams();
-    hs->F = F; hs->device = dev[0]; hs->M = hc[0].p.M; hs->G = hc[0].G; hs->bank = sos != nullptr; hs->fb = fb;
+    hs->device = dev[0];
     int rc = hs->book.create(num_streams, max_frame_len);
-    const size_t S = (size_t)num_streams, M = (size_t)hs->M, C2 = 2 * M, G = (size_t)hs->G;
+    if (!rc) rc = hs->front.create(F, hc[0].p.M, hc[0].G, num_streams, n_sections, sos, doa_list);
+    const size_t S = (size_t)num_streams, M = (size_t)hc[0].p.M, C2 = 2 * M, G = (size_t)hc[0].G;
     const bool narrow = (int)C2 <= kHbLanes;
     for (int f = 0; f < F && !rc; ++f) {
         HilbertStreamBand &b = hs->band[f];
@@ -583,15 +573,10 @@ extern "C" int micloc_hilbert_streams_create(micloc_snn *const *ctxs, int32_t F,
         b.hc.d_W = b.W;
     }
     const size_t nslab = (size_t)nslab_of((int)C2, max_frame_len);
-    if (!rc && !(cudaMalloc(&hs->power, (size_t)F * S * G * sizeof(float)) == cudaSuccess &&
-                 cudaMalloc(&hs->part, nslab * S * C2 * C2 * sizeof(double)) == cudaSuccess &&
+    if (!rc && !(cudaMalloc(&hs->part, nslab * S * C2 * C2 * sizeof(double)) == cudaSuccess &&
                  (narrow || cudaMalloc(&hs->z, S * (size_t)max_frame_len * C2 * sizeof(float)) == cudaSuccess) &&
-                 (C2 * C2 * sizeof(double) <= 128 * 1024 || cudaMalloc(&hs->gram, S * C2 * C2 * sizeof(double)) == cudaSuccess) &&
-                 (!hs->bank || cudaMalloc(&hs->fb_state, (size_t)F * S * M * sizeof(BiquadState)) == cudaSuccess) &&
-                 (!doa_list || cudaMalloc(&hs->doa_list, G * sizeof(double)) == cudaSuccess)))
+                 (C2 * C2 * sizeof(double) <= 128 * 1024 || cudaMalloc(&hs->gram, S * C2 * C2 * sizeof(double)) == cudaSuccess)))
         rc = set_error(MICLOC_ERR_CUDA, "cudaMalloc(Hilbert stream batch) failed");
-    if (!rc && doa_list && cudaMemcpy(hs->doa_list, doa_list, G * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess)
-        rc = set_error(MICLOC_ERR_CUDA, "Hilbert stream batch set-up failed");
     if (!rc) rc = micloc_hilbert_streams_reset(hs, nullptr, 0, nullptr);
     if (rc) { micloc_hilbert_streams_destroy(hs); return rc; }
     *out = hs;
@@ -633,10 +618,10 @@ static int hilbert_stream_band(micloc_hilbert_streams *hs, int f, long long n, f
     if (!hs->gram) {
         const size_t smem_b = (size_t)C2 * C2 * sizeof(double);
         MICLOC_CUDA(cudaFuncSetAttribute(k_hilbert_finish<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        k_hilbert_finish<true><<<(unsigned)S, 256, smem_b, st>>>(hs->part, nslab, nullptr, b.W, p.M, hs->G, S, inv_n, cov_f,
+        k_hilbert_finish<true><<<(unsigned)S, 256, smem_b, st>>>(hs->part, nslab, nullptr, b.W, p.M, b.hc.G, S, inv_n, cov_f,
                                                                  power_f, nullptr);
     } else {
-        k_hilbert_finish<false><<<(unsigned)S, 256, 0, st>>>(hs->part, nslab, hs->gram, b.W, p.M, hs->G, S, inv_n, cov_f,
+        k_hilbert_finish<false><<<(unsigned)S, 256, 0, st>>>(hs->part, nslab, hs->gram, b.W, p.M, b.hc.G, S, inv_n, cov_f,
                                                              power_f, nullptr);
     }
     count_launch(1);
@@ -651,40 +636,21 @@ extern "C" int micloc_hilbert_streams_push(micloc_hilbert_streams *hs, const voi
                                            int64_t *n_out_host, void *stream) {
     if (!hs || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
     SlotBook &bk = hs->book;
-    MICLOC_TRY(bk.check_push(dtype, n, in_channels, hs->M));
-    if ((periodic_ml_dev || trimmed_ml_dev) && !hs->doa_list) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
-    if (sumsq_dev && !hs->bank) return set_error(MICLOC_ERR_SHAPE, "sumsq needs the filterbank (sos != NULL at create)");
+    BankFront &fr = hs->front;
+    MICLOC_TRY(bk.check_push(dtype, n, in_channels, fr.M));
+    MICLOC_TRY(check_doa_list(fr.doa_list, periodic_ml_dev, trimmed_ml_dev));
+    if (sumsq_dev && !fr.fb_state) return set_error(MICLOC_ERR_SHAPE, "sumsq needs the filterbank (sos != NULL at create)");
     MICLOC_CUDA(cudaSetDevice(hs->device));
     cudaStream_t st = (cudaStream_t)stream;
     const long long S = bk.S;
-    if (hs->bank) {
-        MbAssembleParams ap{};
-        ap.fb = hs->fb;
-        for (int f = 0; f < hs->F; ++f) {
-            ap.prev[f] = hs->band[f].xbuf[bk.xcur];
-            ap.cur[f] = hs->band[f].xbuf[bk.xcur ^ 1];
-            ap.hist[f] = hs->band[f].hist;
-        }
-        if (sumsq_dev) MICLOC_CUDA(cudaMemsetAsync(sumsq_dev, 0, (size_t)S * sizeof(double), st));
-        const unsigned grid = (unsigned)((S * hs->M + 127) / 128);
-        auto launch = dtype == MICLOC_F32 ? launch_mb_assemble<float> : dtype == MICLOC_I16 ? launch_mb_assemble<int16_t>
-                                                                                        : launch_mb_assemble<int32_t>;
-        launch(hs->F, grid, st, frames_dev, hs->fb_state, sumsq_dev, bk.pos[bk.pcur], ap, S, (int)n, (int)bk.n_prev,
-               in_channels, hs->M);
-        count_launch(1);
-        MICLOC_CUDA(cudaGetLastError());
-        bk.xcur ^= 1;
-        bk.n_prev = n;
-    } else {
-        MICLOC_TRY(bk.assemble(hs->band[0].xbuf, frames_dev, dtype, n, in_channels, hs->M, hs->band[0].hist, st));
-    }
+    if (fr.fb_state) MICLOC_TRY(fr.assemble(bk, hs->band, frames_dev, dtype, n, in_channels, sumsq_dev, st));
+    else MICLOC_TRY(bk.assemble(hs->band[0].xbuf, frames_dev, dtype, n, in_channels, fr.M, hs->band[0].hist, st));
     const bool fuse = power_grid_dev || doa_dev || periodic_ml_dev || trimmed_ml_dev || flags_dev;
-    float *power = power_dev ? power_dev : (fuse ? hs->power : nullptr);
-    const int C2 = 2 * hs->M;
-    for (int f = 0; f < hs->F; ++f) {
-        float *z_f = z_dev ? z_dev + (size_t)f * S * n * C2 : nullptr;
-        double *cov_f = cov_dev ? cov_dev + (size_t)f * S * hs->M * hs->M * 2 : nullptr;
-        float *pw_f = power ? power + (size_t)f * S * hs->G : nullptr;
+    float *power = power_dev ? power_dev : (fuse ? fr.power : nullptr);
+    for (int f = 0; f < fr.F; ++f) {
+        float *z_f = z_dev ? z_dev + (size_t)f * S * n * 2 * fr.M : nullptr;
+        double *cov_f = cov_dev ? cov_dev + (size_t)f * S * fr.M * fr.M * 2 : nullptr;
+        float *pw_f = power ? power + (size_t)f * S * fr.G : nullptr;
         const int nsec = hs->band[f].hc.p.nsec;
         MICLOC_TRY(nsec == 2 ? hilbert_stream_band<2>(hs, f, n, z_f, cov_f, pw_f, st)
                              : hilbert_stream_band<kNsecRuntime>(hs, f, n, z_f, cov_f, pw_f, st));
@@ -692,6 +658,5 @@ extern "C" int micloc_hilbert_streams_push(micloc_hilbert_streams *hs, const voi
     bk.pushed(n, n_out_host);
     if (!fuse) return MICLOC_OK;
     if (flags_dev) MICLOC_CUDA(cudaMemsetAsync(flags_dev, 0, (size_t)S * sizeof(int32_t), st));
-    return launch_power_fuse(power, hs->F, S, hs->G, hs->doa_list, power_grid_dev, doa_dev, periodic_ml_dev,
-                             trimmed_ml_dev, flags_dev, nullptr, nullptr, st);
+    return fr.fuse(power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, nullptr, nullptr, st);
 }

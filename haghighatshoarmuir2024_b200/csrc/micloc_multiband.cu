@@ -189,7 +189,7 @@ extern "C" int micloc_power_fuse(const float *power_dev, int32_t F, int64_t B, i
                                  int32_t *flags_dev, int device, void *stream) {
     if (!power_dev) return set_error(MICLOC_ERR_SHAPE, "null argument");
     if (F < 1 || B < 1 || G < 1) return set_error(MICLOC_ERR_SHAPE, "empty input");
-    if ((periodic_ml_dev || trimmed_ml_dev) && !doa_list_dev) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
+    MICLOC_TRY(check_doa_list(doa_list_dev, periodic_ml_dev, trimmed_ml_dev));
     MICLOC_CUDA(cudaSetDevice(device));
     cudaStream_t st = (cudaStream_t)stream;
     if (flags_dev) MICLOC_CUDA(cudaMemsetAsync(flags_dev, 0, (size_t)B * sizeof(int32_t), st));

@@ -27,10 +27,10 @@
 //
 // A MULTI-BAND STREAM BATCH (micloc_snn_mb_streams_*) is the live localiser of micloc/localization_demo_snn.py:125-193
 // made continuous: a Butterworth filterbank on the raw frame, one chain per band, power summed over the bands.  It is
-// one SlotBook plus F StreamBands; the book's latency D = max_f rzcc_lag(w_f) is common, so every band finalises the
-// same samples in a push and every band's k_stream_blk writes the same positions and row counts.  One kernel runs the
-// filterbank with its state carried across pushes and writes every band's [history | frame] rows
-// (k_mb_stream_assemble).  Per push, whatever S:
+// one SlotBook, one BankFront (micloc_stream.cuh, shared with the Hilbert batch) and F StreamBands; the book's latency
+// D = max_f rzcc_lag(w_f) is common, so every band finalises the same samples in a push and every band's k_stream_blk
+// writes the same positions and row counts.  The front's k_mb_stream_assemble runs the filterbank with its state
+// carried across pushes and writes every band's [history | frame] rows.  Per push, whatever S:
 //   k_mb_stream_assemble                                                    1
 //   per band: STHT, k_stream_blk, k_gram, k_power_argmax (into band f's slice of [F][S][G])   4 F
 //   k_power_fuse       sum over bands, argmax, periodic-ML estimators over each slot's final rows   1
@@ -501,21 +501,19 @@ extern "C" int micloc_snn_streams_flush(micloc_stream_batch *sb, const int32_t *
 
 // ---- multi-band stream batches: F bands on one slot book, behind one filterbank ----
 struct micloc_mb_streams {
-    int F = 0, device = 0, M = 0, G = 0;
+    int device = 0;
     SlotBook book;
+    BankFront front;
     StreamBand band[8];
-    FilterbankParams fb{};
-    BiquadState *fb_state = nullptr;    // [F][S][M] filterbank state
-    double *doa_list = nullptr;         // [G] on the device, null: no ML estimators
-    float *power = nullptr;             // [F][S][G] per-band power when the caller passes no power_dev
+    const int32_t *band_flags[8] = {};  // band f's flags, OR-ed into the fused flags
 };
 
 extern "C" int micloc_snn_mb_streams_destroy(micloc_mb_streams *mb) {
     if (!mb) return MICLOC_OK;
     cudaSetDevice(mb->device);
     mb->book.destroy();
-    for (int f = 0; f < mb->F; ++f) band_free(mb->band[f]);
-    cudaFree(mb->fb_state); cudaFree(mb->doa_list); cudaFree(mb->power);
+    for (int f = 0; f < mb->front.F; ++f) band_free(mb->band[f]);
+    mb->front.destroy();
     delete mb;
     return MICLOC_OK;
 }
@@ -525,35 +523,22 @@ extern "C" int micloc_snn_mb_streams_create(micloc_snn *const *ctxs, int32_t F, 
                                             micloc_mb_streams **out) {
     if (!ctxs || !sos || !out) return set_error(MICLOC_ERR_CONFIG, "null argument");
     *out = nullptr;
-    if (F < 1 || F > 8) return set_error(MICLOC_ERR_CONFIG, "multi-band stream batch of %d bands (1..8 supported)", F);
-    FilterbankParams fb;
-    MICLOC_TRY(filterbank_params(F, n_sections, sos, &fb));
     micloc_snn_params prm[8];
-    int D = 0;
-    for (int f = 0; f < F; ++f) {
-        if (!ctxs[f]) return set_error(MICLOC_ERR_CONFIG, "null context of band %d", f);
+    int D = 0;                      // one latency: every band finalises the same samples
+    MICLOC_TRY(check_bands("multi-band stream batch", ctxs, F, [&](int f, BandShape &b) -> int {
         MICLOC_TRY(micloc_snn_get_params(ctxs[f], &prm[f]));
-        if (prm[f].device != prm[0].device)
-            return set_error(MICLOC_ERR_CONFIG, "band %d's context is on device %d, band 0's on device %d", f, prm[f].device, prm[0].device);
-        if (prm[f].chain.M != prm[0].chain.M || prm[f].chain.G != prm[0].chain.G)
-            return set_error(MICLOC_ERR_SHAPE, "band %d's context has %d microphones and %d DoAs, band 0's %d and %d", f,
-                             prm[f].chain.M, prm[f].chain.G, prm[0].chain.M, prm[0].chain.G);
-        D = std::max(D, rzcc_lag(prm[f].chain.w));      // one latency: every band finalises the same samples
-    }
+        b = {prm[f].device, prm[f].chain.M, prm[f].chain.G};
+        D = std::max(D, rzcc_lag(prm[f].chain.w));
+        return MICLOC_OK;
+    }));
     MICLOC_CUDA(cudaSetDevice(prm[0].device));
     micloc_mb_streams *mb = new micloc_mb_streams();
-    mb->F = F; mb->device = prm[0].device; mb->M = prm[0].chain.M; mb->G = prm[0].chain.G; mb->fb = fb;
+    mb->device = prm[0].device;
     mb->book.D = D;
     int rc = mb->book.create(num_streams, max_frame_len);
+    if (!rc) rc = mb->front.create(F, prm[0].chain.M, prm[0].chain.G, num_streams, n_sections, sos, doa_list);
     for (int f = 0; f < F && !rc; ++f) rc = band_alloc(mb->band[f], prm[f], mb->book);
-    const size_t S = (size_t)num_streams;
-    if (!rc && !(cudaMalloc(&mb->fb_state, (size_t)F * S * mb->M * sizeof(BiquadState)) == cudaSuccess &&
-                 cudaMalloc(&mb->power, (size_t)F * S * mb->G * sizeof(float)) == cudaSuccess &&
-                 (!doa_list || cudaMalloc(&mb->doa_list, (size_t)mb->G * sizeof(double)) == cudaSuccess)))
-        rc = set_error(MICLOC_ERR_CUDA, "cudaMalloc(multi-band stream batch) failed");
-    if (!rc && ((doa_list && cudaMemcpy(mb->doa_list, doa_list, (size_t)mb->G * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) ||
-                cudaMemset(mb->fb_state, 0, (size_t)F * S * mb->M * sizeof(BiquadState)) != cudaSuccess))
-        rc = set_error(MICLOC_ERR_CUDA, "multi-band stream batch set-up failed");
+    for (int f = 0; f < F; ++f) mb->band_flags[f] = mb->band[f].flags;
     if (!rc) rc = reset_bands(mb->book, mb->band, F, nullptr, 0, nullptr);
     if (rc) { micloc_snn_mb_streams_destroy(mb); return rc; }
     *out = mb;
@@ -566,16 +551,7 @@ extern "C" int micloc_snn_mb_streams_latency(micloc_mb_streams *mb) { return mb 
 extern "C" int micloc_snn_mb_streams_reset(micloc_mb_streams *mb, const int32_t *slots_host, int32_t n_slots, void *stream) {
     if (!mb) return set_error(MICLOC_ERR_CONFIG, "null stream");
     MICLOC_CUDA(cudaSetDevice(mb->device));
-    return reset_bands(mb->book, mb->band, mb->F, slots_host, n_slots, (cudaStream_t)stream);
-}
-
-// sum over the bands + estimators over each slot's final rows
-static int mb_fuse(micloc_mb_streams *mb, const float *power, float *power_grid_dev, int32_t *doa_dev, double *periodic_ml_dev,
-                   double *trimmed_ml_dev, int32_t *flags_dev, cudaStream_t st) {
-    const int32_t *band_flags[8];
-    for (int f = 0; f < mb->F; ++f) band_flags[f] = mb->band[f].flags;
-    return launch_power_fuse(power, mb->F, mb->book.S, mb->G, mb->doa_list, power_grid_dev, doa_dev, periodic_ml_dev,
-                             trimmed_ml_dev, flags_dev, mb->book.m, band_flags, st);
+    return reset_bands(mb->book, mb->band, mb->front.F, slots_host, n_slots, (cudaStream_t)stream);
 }
 
 extern "C" int micloc_snn_mb_streams_push(micloc_mb_streams *mb, const void *frames_dev, int dtype, int64_t n,
@@ -584,33 +560,18 @@ extern "C" int micloc_snn_mb_streams_push(micloc_mb_streams *mb, const void *fra
                                           double *sumsq_dev, int32_t *flags_dev, int64_t *n_out_host, void *stream) {
     if (!mb || !frames_dev || !n_out_host) return set_error(MICLOC_ERR_SHAPE, "null argument");
     SlotBook &bk = mb->book;
-    MICLOC_TRY(bk.check_push(dtype, n, in_channels, mb->M));
-    if ((periodic_ml_dev || trimmed_ml_dev) && !mb->doa_list) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
+    BankFront &fr = mb->front;
+    MICLOC_TRY(bk.check_push(dtype, n, in_channels, fr.M));
+    MICLOC_TRY(check_doa_list(fr.doa_list, periodic_ml_dev, trimmed_ml_dev));
     MICLOC_CUDA(cudaSetDevice(mb->device));
     cudaStream_t st = (cudaStream_t)stream;
-    MbAssembleParams ap{};
-    ap.fb = mb->fb;
-    for (int f = 0; f < mb->F; ++f) {
-        ap.prev[f] = mb->band[f].xbuf[bk.xcur];
-        ap.cur[f] = mb->band[f].xbuf[bk.xcur ^ 1];
-        ap.hist[f] = mb->band[f].hist;
-    }
-    if (sumsq_dev) MICLOC_CUDA(cudaMemsetAsync(sumsq_dev, 0, (size_t)bk.S * sizeof(double), st));
-    const unsigned grid = (unsigned)((bk.S * mb->M + 127) / 128);
-    auto launch = dtype == MICLOC_F32 ? launch_mb_assemble<float> : dtype == MICLOC_I16 ? launch_mb_assemble<int16_t>
-                                                                                    : launch_mb_assemble<int32_t>;
-    launch(mb->F, grid, st, frames_dev, mb->fb_state, sumsq_dev, bk.pos[bk.pcur], ap, bk.S, (int)n, (int)bk.n_prev,
-           in_channels, mb->M);
-    count_launch(1);
-    MICLOC_CUDA(cudaGetLastError());
-    bk.xcur ^= 1;
-    bk.n_prev = n;
+    MICLOC_TRY(fr.assemble(bk, mb->band, frames_dev, dtype, n, in_channels, sumsq_dev, st));
     const bool fuse = power_dev || power_grid_dev || doa_dev || periodic_ml_dev || trimmed_ml_dev || flags_dev;
-    float *power = power_dev ? power_dev : mb->power;
-    MICLOC_TRY(step_bands(bk, mb->band, mb->F, nullptr, n, n + bk.D, spikes_dev, fuse ? power : nullptr, nullptr, nullptr,
+    float *power = power_dev ? power_dev : fr.power;
+    MICLOC_TRY(step_bands(bk, mb->band, fr.F, nullptr, n, n + bk.D, spikes_dev, fuse ? power : nullptr, nullptr, nullptr,
                           nullptr, n_out_host, st));
     if (!fuse) return MICLOC_OK;
-    return mb_fuse(mb, power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, st);
+    return fr.fuse(power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, bk.m, mb->band_flags, st);
 }
 
 extern "C" int micloc_snn_mb_streams_flush(micloc_mb_streams *mb, const int32_t *slots_host, int32_t n_slots,
@@ -618,15 +579,16 @@ extern "C" int micloc_snn_mb_streams_flush(micloc_mb_streams *mb, const int32_t 
                                            double *periodic_ml_dev, double *trimmed_ml_dev, int32_t *flags_dev,
                                            int64_t *n_out_host, int32_t *flags_host, void *stream) {
     if (!mb || !n_out_host) return set_error(MICLOC_ERR_CONFIG, "null stream");
-    if ((periodic_ml_dev || trimmed_ml_dev) && !mb->doa_list) return set_error(MICLOC_ERR_SHAPE, "the ML estimators need doa_list");
+    BankFront &fr = mb->front;
+    MICLOC_TRY(check_doa_list(fr.doa_list, periodic_ml_dev, trimmed_ml_dev));
     MICLOC_CUDA(cudaSetDevice(mb->device));
     cudaStream_t st = (cudaStream_t)stream;
     const bool fuse = power_dev || power_grid_dev || doa_dev || periodic_ml_dev || trimmed_ml_dev || flags_dev;
-    float *power = power_dev ? power_dev : mb->power;
-    MICLOC_TRY(flush_bands(mb->book, mb->band, mb->F, slots_host, n_slots, spikes_dev, fuse ? power : nullptr, nullptr,
+    float *power = power_dev ? power_dev : fr.power;
+    MICLOC_TRY(flush_bands(mb->book, mb->band, fr.F, slots_host, n_slots, spikes_dev, fuse ? power : nullptr, nullptr,
                            nullptr, nullptr, n_out_host, flags_host, st));
     if (!fuse) return MICLOC_OK;
-    return mb_fuse(mb, power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, st);
+    return fr.fuse(power, power_grid_dev, doa_dev, periodic_ml_dev, trimmed_ml_dev, flags_dev, mb->book.m, mb->band_flags, st);
 }
 
 // ---- the single stream: slot 0 of a one-slot batch ----

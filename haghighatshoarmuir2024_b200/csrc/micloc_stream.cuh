@@ -1,8 +1,8 @@
 // micloc_stream.cuh -- the slot book and frame assembly shared by the stream batches: the float SNN chain's stream and
 // multi-band batches (micloc_stream.cu), the Xylo integer chain's (micloc_xylo.cu) and the Hilbert beamformer's
 // (micloc_hilbert.cu).  The rule of where a slot stands and what a push, flush or reset does to it lives here once; each
-// batch keeps its chain state and flags next to it.  The filterbank assembly serves the multi-band SNN and the Hilbert
-// batches.
+// batch keeps its chain state and flags next to it.  The bank front (BankFront: band context checks, filterbank
+// assembly, DoA list and power fusion) serves the multi-band SNN and the Hilbert batches.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -179,7 +179,7 @@ struct SlotBook {
         return MICLOC_OK;
     }
 
-    // k_stream_assemble of the frames into xbuf[xcur ^ 1], which becomes the newest buffer
+    // k_stream_assemble of the frames into xbuf[xcur ^ 1]
     template <typename OUT_T>
     int assemble(OUT_T *const xbuf[2], const void *frames, int dtype, int64_t n, int32_t in_channels, int M, int hist,
                  cudaStream_t st) {
@@ -194,10 +194,12 @@ struct SlotBook {
             k_stream_assemble<int32_t, OUT_T><<<ga, 256, 0, st>>>((const int32_t *)frames, prev, xbuf[nxt], pos[pcur], S, (int)n, (int)n_prev, in_channels, M, hist);
         count_launch(1);
         MICLOC_CUDA(cudaGetLastError());
-        xcur = nxt;
-        n_prev = n;
+        assembled(n);
         return MICLOC_OK;
     }
+
+    // after the assembly of a frame of n samples into xbuf[xcur ^ 1]: that buffer becomes the newest
+    void assembled(long long n) { xcur ^= 1; n_prev = n; }
 
     // after the owner's reset kernels (listed = a slot list was uploaded): waits for them, the listed slots restart at 0
     int reset_done(bool listed, cudaStream_t st) {
@@ -230,6 +232,78 @@ struct SlotBook {
             F[s] = N[s];
             active[s] = 0;
         }
+    }
+};
+
+struct BandShape { int device, M, G; };
+
+// The band contexts ctxs [F] of a multi-band batch (`kind` in the errors): F in 1..8, none null, all on band 0's device
+// with its M and G.  read(f, shape) reads band f's context for the caller and gives its shape, or an error code.
+template <typename Read>
+int check_bands(const char *kind, micloc_snn *const *ctxs, int32_t F, Read read) {
+    if (F < 1 || F > 8) return set_error(MICLOC_ERR_CONFIG, "%s of %d bands (1..8 supported)", kind, F);
+    BandShape b0{}, b{};
+    for (int f = 0; f < F; ++f) {
+        if (!ctxs[f]) return set_error(MICLOC_ERR_CONFIG, "null context of band %d", f);
+        MICLOC_TRY(read(f, b));
+        if (f == 0) b0 = b;
+        if (b.device != b0.device)
+            return set_error(MICLOC_ERR_CONFIG, "band %d's context is on device %d, band 0's on device %d", f, b.device, b0.device);
+        if (b.M != b0.M || b.G != b0.G)
+            return set_error(MICLOC_ERR_SHAPE, "band %d's context has %d microphones and %d DoAs, band 0's %d and %d", f,
+                             b.M, b.G, b0.M, b0.G);
+    }
+    return MICLOC_OK;
+}
+
+// What sits in front of F band chains on one slot book (multi-band SNN and Hilbert stream batches): the filterbank with
+// its state, the DoA list of the estimators and the per-band power that k_power_fuse adds up.
+struct BankFront {
+    int F = 0, M = 0, G = 0;
+    long long S = 0;
+    FilterbankParams fb{};
+    BiquadState *fb_state = nullptr;    // [F][S][M] filterbank state (never read at N == 0), null: no filterbank
+    double *doa_list = nullptr;         // [G] on the device, null: no ML estimators
+    float *power = nullptr;             // [F][S][G] per-band power when the caller passes no power_dev
+
+    // sos [F][n_sections][6] and doa_list [G] on the host, either may be NULL
+    int create(int F_, int M_, int G_, long long S_, int32_t n_sections, const double *sos, const double *doa_list_host) {
+        if (sos) MICLOC_TRY(filterbank_params(F_, n_sections, sos, &fb));
+        F = F_; M = M_; G = G_; S = S_;
+        if (cudaMalloc(&power, (size_t)F * S * G * sizeof(float)) != cudaSuccess ||
+            (sos && cudaMalloc(&fb_state, (size_t)F * S * M * sizeof(BiquadState)) != cudaSuccess) ||
+            (doa_list_host && (cudaMalloc(&doa_list, (size_t)G * sizeof(double)) != cudaSuccess ||
+                               cudaMemcpy(doa_list, doa_list_host, (size_t)G * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess)))
+            return set_error(MICLOC_ERR_CUDA, "filterbank front set-up failed");
+        return MICLOC_OK;
+    }
+
+    void destroy() { cudaFree(fb_state); cudaFree(doa_list); cudaFree(power); }
+
+    // k_mb_stream_assemble of the frames into every band's xbuf[bk.xcur ^ 1]; sumsq [S] (nullable) is zeroed first
+    template <typename Band>
+    int assemble(SlotBook &bk, const Band *band, const void *frames, int dtype, int64_t n, int32_t in_channels,
+                 double *sumsq, cudaStream_t st) {
+        MbAssembleParams ap{};
+        ap.fb = fb;
+        for (int f = 0; f < F; ++f) {
+            ap.prev[f] = band[f].xbuf[bk.xcur]; ap.cur[f] = band[f].xbuf[bk.xcur ^ 1]; ap.hist[f] = band[f].hist;
+        }
+        if (sumsq) MICLOC_CUDA(cudaMemsetAsync(sumsq, 0, (size_t)S * sizeof(double), st));
+        const unsigned grid = (unsigned)((S * M + 127) / 128);
+        auto launch = dtype == MICLOC_F32 ? launch_mb_assemble<float> : dtype == MICLOC_I16 ? launch_mb_assemble<int16_t>
+                                                                                        : launch_mb_assemble<int32_t>;
+        launch(F, grid, st, frames, fb_state, sumsq, bk.pos[bk.pcur], ap, S, (int)n, (int)bk.n_prev, in_channels, M);
+        count_launch(1);
+        MICLOC_CUDA(cudaGetLastError());
+        bk.assembled(n);
+        return MICLOC_OK;
+    }
+
+    // k_power_fuse over power [F][S][G]: sum over the bands, argmax, estimators (rows_b, band_flags: launch_power_fuse)
+    int fuse(const float *power_fb, float *power_grid, int32_t *doa, double *ml, double *trimmed, int32_t *flags,
+             const int32_t *rows_b, const int32_t *const *band_flags, cudaStream_t st) const {
+        return launch_power_fuse(power_fb, F, S, G, doa_list, power_grid, doa, ml, trimmed, flags, rows_b, band_flags, st);
     }
 };
 

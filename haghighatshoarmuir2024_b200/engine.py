@@ -32,11 +32,26 @@ def _check_frames(frames: torch.Tensor, M: int, device: torch.device, num_stream
     if num_streams is not None and frames.shape[0] != num_streams:
         raise ValueError(f"frames hold {frames.shape[0]} slots, the batch has {num_streams}")
     if frames.device != device:
-        raise ValueError(f"frames live on {frames.device}, the stream on {device}")
+        raise ValueError(f"frames live on {frames.device}, not on {device}")
     dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frames.dtype)
     if dt is None:
         raise ValueError(f"frames must be float32, int16 or int32, got {frames.dtype}")
     return frames.contiguous(), dt
+
+
+def _activity(sumsq: torch.Tensor, rows: int, M: int, dtype: torch.dtype, rel_threshold: float,
+              full_scale: Optional[float], doa=None, doa_list=None, written=None):
+    """The activity gate of micloc/localization_demo_snn.py:136-163 -> (active, doa_deg): active = the frame's rms (sumsq
+    over `rows` samples of M microphones) >= rel_threshold * full_scale (None: an integer `dtype`'s largest value, 1.0
+    for float32); doa_deg = doa_list[doa] in degrees, NaN where inactive or not `written`; None without doa_list."""
+    if full_scale is None:
+        full_scale = float(torch.iinfo(dtype).max) if not dtype.is_floating_point else 1.0
+    active = torch.sqrt(sumsq / (rows * M)) >= rel_threshold * full_scale
+    if doa is None or doa_list is None:
+        return active, None
+    keep, doa = (active, doa) if written is None else (written & active, torch.where(written, doa, 0))
+    deg = doa_list[doa.long()] * 180 / np.pi
+    return active, torch.where(keep, deg, torch.full_like(deg, float("nan")))
 
 
 def _design_template(geometry, time: np.ndarray, sig: np.ndarray, device: torch.device):

@@ -21,7 +21,7 @@ import torch
 
 from . import _native as N
 from .array_geometry import ArrayGeometry
-from .engine import SnnEngine, _SlotBatch, _check_frames, _ptr, _stream_ptr
+from .engine import SnnEngine, _SlotBatch, _activity, _check_frames, _ptr, _stream_ptr
 from .filterbank import ButterworthFilterbank
 from .snn_beamformer import SNNBeamformer
 
@@ -65,15 +65,7 @@ class Demo:
         activity), periodic_ml / trimmed_periodic_ml [B] radians, active [B] bool, power [F, B, G], flags [B])."""
         if frames.dim() == 2:
             frames = frames.unsqueeze(0)
-        if frames.dim() != 3 or frames.shape[2] < self.num_mic:
-            raise ValueError(
-                f"number of channels in the input siganl {frames.shape[-1]} should be the same as the number of microphones {self.num_mic}!")
-        if frames.device != self.device:
-            raise ValueError(f"frames live on {frames.device}, the localiser on {self.device}")
-        dt = {torch.float32: N.F32, torch.int16: N.I16, torch.int32: N.I32}.get(frames.dtype)
-        if dt is None:
-            raise ValueError(f"frames must be float32, int16 or int32, got {frames.dtype}")
-        frames = frames.contiguous()
+        frames, dt = _check_frames(frames, self.num_mic, self.device, frames.shape[0])
         B, T, ch = frames.shape
         F, M, G = len(self.beamfs), self.num_mic, len(self.doa_list)
         lib = N.lib()
@@ -103,13 +95,7 @@ class Demo:
         fflags = torch.empty(B, dtype=torch.int32, device=dev)
         N.check(lib.micloc_power_fuse(_ptr(power), F, B, G, _ptr(self._doa_dev), _ptr(power_grid), _ptr(doa), _ptr(ml),
                                       _ptr(trimmed), _ptr(fflags), dev.index or 0, st))
-        # activity detection (localization_demo_snn.py:136-163): rms over the frame against rel_threshold * full scale
-        if full_scale is None:
-            full_scale = float(torch.iinfo(frames.dtype).max) if not frames.dtype.is_floating_point else 1.0
-        rms = torch.sqrt(sumsq / (T * M))
-        active = rms >= rel_threshold * full_scale
-        doa_deg = torch.where(active, self._doa_dev[doa.long()] * 180 / np.pi,
-                              torch.full_like(rms, float("nan")))
+        active, doa_deg = _activity(sumsq, T, M, frames.dtype, rel_threshold, full_scale, doa, self._doa_dev)
         return {"power_grid": power_grid, "doa": doa, "doa_deg": doa_deg, "periodic_ml": ml, "trimmed_periodic_ml": trimmed,
                 "active": active, "power": power, "flags": flags | fflags, "spikes": spikes if want_spikes else None,
                 "banded": banded}
@@ -189,13 +175,9 @@ class MultibandStreamBatch(_SlotBatch):
             self._h, _ptr(frames), dt, n, ch, _ptr(out["spikes"]), _ptr(out["power"]), _ptr(out["power_grid"]),
             _ptr(out["doa"]), _ptr(out["periodic_ml"]), _ptr(out["trimmed_periodic_ml"]), _ptr(sumsq), _ptr(out["flags"]),
             n_out.ctypes.data_as(C.c_void_p), _stream_ptr(self.device)))
-        if full_scale is None:
-            full_scale = float(torch.iinfo(frames.dtype).max) if not frames.dtype.is_floating_point else 1.0
-        active = torch.sqrt(sumsq / (n * self.M)) >= rel_threshold * full_scale      # as Demo.localize
-        written = out["doa"] >= 0                            # (n_out > 0 without a host-to-device copy)
-        deg = self._doa_dev[torch.where(written, out["doa"], 0).long()] * 180 / np.pi
-        out.update({"n_out": n_out, "active": active, "sumsq": sumsq,
-                    "doa_deg": torch.where(written & active, deg, torch.full_like(deg, float("nan")))})
+        active, doa_deg = _activity(sumsq, n, self.M, frames.dtype, rel_threshold, full_scale, out["doa"], self._doa_dev,
+                                    written=out["doa"] >= 0)         # (n_out > 0 without a host-to-device copy)
+        out.update({"n_out": n_out, "active": active, "sumsq": sumsq, "doa_deg": doa_deg})
         if not want_spikes:
             del out["spikes"]
         return out
